@@ -35,6 +35,14 @@ such as 8 x 32 measure 2-18 % less, depending on the shard size).
             training run and the fused policy + env rollout at 1 M envs (the callers of the hot path) and, at
             --gpus 8, config 5 (PPO loop, 262,144 envs: fused rollout, GAE kernel, all minibatch updates of an
             epoch in one launch with the gradient all-reduce over NVLink peer memory inside the kernel)
+
+    python bench.py ... --dump-outputs DIR
+
+writes, after the timed steps, the output buffers of the last launch of the last timed step (obs, reward, terminated,
+truncated: what VecCarEnv.rollout hands its caller) as DIR/<name>.npy in float32, [steps per launch, DUMP_ENVS(, 18)],
+for the global environment ids np.sort(np.random.default_rng(0).choice(envs, DUMP_ENVS, replace=False)) (and a
+seeded sample of the rows when the launch is too long for DUMP_BYTES).  Actions and resets are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -59,6 +67,8 @@ FLOP_PER_ENV_STEP = 18 * (12 * N_SEG + 4) + 30          # SURVEY §8(d): 5,286
 BYTES_PER_ENV_STEP = 1 + 72 + 4 + 1 + 1
 STATE_BYTES = 48
 METRIC = "CarEnv env-steps/sec"
+DUMP_ENVS = 2048                                         # --dump-outputs: sampled environments (all rows of a 256-step
+DUMP_BYTES = 64 << 20                                    # launch: 44 MB) and the cap on all files together
 
 
 # ----------------------------------------------------------------------------- CPU baseline
@@ -365,6 +375,38 @@ def config5(args):
             "avg_reward_last": hist[-1]["avg_reward"]}
 
 
+def dump_outputs(path, outs, total, lo, world, rank):
+    """Save a seeded sample of this rank's output buffers `outs` (name -> [steps, envs on this rank, ...] CUDA tensor)
+    as path/<name>.npy in float32 on rank 0: the same global environment ids and rows whatever the number of ranks."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+
+    rng = np.random.default_rng(0)
+    ids = np.sort(rng.choice(total, size=min(total, DUMP_ENVS), replace=False))
+    first = next(iter(outs.values()))
+    steps, n, dev = first.shape[0], first.shape[1], first.device
+    row_bytes = len(ids) * 4 * sum(t[0, 0].numel() for t in outs.values())
+    rows = None
+    if steps * row_bytes > DUMP_BYTES:
+        rows = np.sort(rng.choice(steps, size=max(1, DUMP_BYTES // row_bytes), replace=False))
+    cols = torch.from_numpy(ids[(ids >= lo) & (ids < lo + n)] - lo).to(dev)
+    part = {}
+    for name, t in outs.items():
+        s = t.index_select(1, cols)
+        if rows is not None:
+            s = s.index_select(0, torch.from_numpy(rows).to(dev))
+        part[name] = s.float().cpu().numpy()
+    parts = [part]
+    if world > 1:                                       # shards are contiguous env ranges in rank order
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(part, parts, dst=0)
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for name in outs:
+            np.save(os.path.join(path, name + ".npy"), np.concatenate([p[name] for p in parts], axis=1))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -438,6 +480,9 @@ def run_ours(args):
     dev_ms_max = float(t.item())
     value = args.steps * launches * chunk * total / (dev_ms_max * 1e-3)
     slow = env.slow_path_counts()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"obs": obs, "reward": rew, "terminated": term, "truncated": trunc}, total, lo,
+                     world, rank)
 
     # ---- e2e: reference-facing API with HOST buffers (numpy in, numpy out, the reference's dtypes), one env step per call
     e_steps = args.e2e_steps
@@ -623,7 +668,14 @@ def main():
     ap.add_argument("--clock-period", type=float, default=0.01, help="seconds between NVML clock samples")
     ap.add_argument("--no-configs", action="store_true", help="skip BASELINE configs 2 / 3 / 5")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the outputs of the last launch of the last timed step to "
+                         "DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm keeps no output buffers")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

@@ -9,12 +9,23 @@ Everything written here comes out of the reference's own code
 oracle/ref_import.py); nothing is computed by this repository's oracle or
 kernels.  The fixtures pin the oracle (tests/test_oracle_golden.py) and the CUDA
 path (tests/test_gpu_parity.py) on the GPU box, where /root/reference does not
-exist.
+exist.  The one exception is `--from-port`, for the two recordings that were added
+when no reference checkout was at hand: they are then taken from
+oracle/carenv_port.py and from ppo_car_b200.train_ppo.ActorCritic, which were
+unchanged since they last matched the reference in the live tests (the port bit
+for bit on the near-wall track, the network's checkpoint loading strictly into
+lib/model.py:Agent with outputs within 1e-6).  Each file names its source.
 
 Files written:
   carenv_<track>.npz   reset observation + four trajectory groups, each with the
                        action tensor that was played and every per-step output
   gae.npz              Buffer.calculate_advantages on seeded inputs
+  near_wall.npz, near_wall_track.json
+                       the start_destroyed branch (lib/car_env.py:682-686): a
+                       synthetic track whose start pose is 6 px from a wall and
+                       one trajectory group ("destroyed") in the layout above
+  agent_checkpoint.npz a state dict of lib/model.py:Agent (seeded init) and its
+                       log-probability, entropy and value on fixed inputs
   ../../ppo_car_b200/tracks/<track>.json   the two track files (input data in the
                        reference's schema; BASELINE.json names them as workloads)
 """
@@ -30,7 +41,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 
-from oracle.ref_import import RefVecEnv, import_reference, track_path  # noqa: E402
+from oracle.carenv_port import PortVecEnv  # noqa: E402
+from oracle.ref_import import RefVecEnv, import_reference, reference_root, track_path  # noqa: E402
+from tests.synth_tracks import near_wall_track  # noqa: E402
 
 T = 1024
 
@@ -47,8 +60,8 @@ def follower_action(obs: np.ndarray) -> int:
     return {0: 8, 1: 3, -1: 2}[turn]
 
 
-def rollout(track: str, n_envs: int, policy) -> dict:
-    env = RefVecEnv(n_envs, track)
+def rollout(track: str, n_envs: int, policy, vec_env=RefVecEnv) -> dict:
+    env = vec_env(n_envs, track)
     obs = env.reset()
     rec = {k: [] for k in ("actions", "final_obs", "rew", "term", "trunc", "gates_passed", "time_passed", "next_gate_index")}
     for t in range(T):
@@ -124,11 +137,61 @@ def make_gae() -> None:
     np.savez_compressed(os.path.join(HERE, "gae.npz"), **out)
 
 
+def make_near_wall(from_port: bool) -> None:
+    path = near_wall_track(os.path.join(HERE, "near_wall_track.json"))
+    vec_env = PortVecEnv if from_port else RefVecEnv
+    rng = np.random.default_rng(682)
+
+    def policy(t, obs):
+        a = rng.choice(9, size=6, p=[.3, .02, .1, .1, .2, .2, .02, .02, .04])
+        a[0] = 0                                              # one env at full throttle
+        return a
+
+    reset_obs = vec_env(1, path).reset()[0]
+    rec = rollout(path, 6, policy, vec_env)
+    out = {f"destroyed_{k}": v for k, v in rec.items()}
+    source = "oracle/carenv_port.py" if from_port else "lib/car_env.py"
+    np.savez_compressed(os.path.join(HERE, "near_wall.npz"), reset_obs=reset_obs, source=np.array(source), **out)
+
+
+def make_agent(from_port: bool) -> None:
+    import importlib
+
+    import torch
+
+    if from_port:
+        from ppo_car_b200.train_ppo import ActorCritic as Agent
+
+        source = "ppo_car_b200/train_ppo.py:ActorCritic"
+    else:
+        root = reference_root()
+        if root not in sys.path:
+            sys.path.insert(0, root)
+        Agent, source = importlib.import_module("lib.model").Agent, "lib/model.py:Agent"
+    torch.manual_seed(3)
+    net = Agent(18, 9)
+    obs = torch.randn(32, 18)
+    act = torch.randint(0, 9, (32,))
+    with torch.no_grad():
+        if from_port:
+            _, logp, ent, val = net.act(obs, act)
+        else:
+            _, logp, ent, val = net.get_action_and_value(obs, act)
+    out = {"w_" + k: v.numpy() for k, v in net.state_dict().items()}
+    np.savez_compressed(os.path.join(HERE, "agent_checkpoint.npz"), obs=obs.numpy(), act=act.numpy(),
+                        logp=logp.numpy(), entropy=ent.numpy(), value=val.numpy(), source=np.array(source), **out)
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["track", "big_track", "gae"]
+    from_port = "--from-port" in sys.argv
+    which = [w for w in sys.argv[1:] if w != "--from-port"] or ["track", "big_track", "gae", "near_wall", "agent"]
     for w in which:
         if w == "gae":
             make_gae()
+        elif w == "near_wall":
+            make_near_wall(from_port)
+        elif w == "agent":
+            make_agent(from_port)
         else:
             make_track(w)
     print("done")

@@ -24,20 +24,30 @@ def _gpu_traj(out):
                 time_passed=info["time_passed"].cpu().numpy(), next_gate_index=info["next_gate_index"].cpu().numpy())
 
 
+def _golden_group(g, group, T=None, n=None):
+    """One trajectory group of a tests/golden file, its first T steps of the first n envs, as the autoresetting vector
+    env returns it (the reset observation where an episode ended)."""
+    def cut(a):
+        return a[:T, :n]
+
+    done = cut(g[f"{group}_term"] | g[f"{group}_trunc"]).astype(bool)
+    rec = {k: cut(g[f"{group}_{k}"]) for k in ("actions", "rew", "term", "trunc", "gates_passed", "time_passed",
+                                              "next_gate_index")}
+    rec["obs"] = np.where(done[..., None], g["reset_obs"], cut(g[f"{group}_final_obs"]))
+    return rec
+
+
 @pytest.mark.parametrize("name", ["track", "big_track"])
 def test_golden_trajectories_from_the_reference(golden_dir, tracks_dir, name):
     g = np.load(os.path.join(golden_dir, f"carenv_{name}.npz"))
     path = os.path.join(tracks_dir, name + ".json")
     for group in GROUPS:
-        acts = g[f"{group}_actions"]
+        ref = _golden_group(g, group)
+        acts = ref["actions"]
         env = ppo_car_b200.VecCarEnv(acts.shape[1], path)
         obs0, _ = env.reset()
         assert_floats_close(obs0.cpu().numpy(), np.broadcast_to(g["reset_obs"], obs0.shape), "reset obs")
         out = env.rollout(torch.from_numpy(acts).cuda(), store_info=True)
-        done = (g[f"{group}_term"] | g[f"{group}_trunc"]).astype(bool)
-        ref = dict(obs=np.where(done[..., None], g["reset_obs"], g[f"{group}_final_obs"]), rew=g[f"{group}_rew"],
-                   term=g[f"{group}_term"], trunc=g[f"{group}_trunc"], gates_passed=g[f"{group}_gates_passed"],
-                   time_passed=g[f"{group}_time_passed"], next_gate_index=g[f"{group}_next_gate_index"])
         assert_trajectory_matches(_gpu_traj(out), ref, what=f"{name}/{group}")
         if group == "lap":
             assert int(((out["info"]["events"] >> 1) & 1).sum()) == 1
@@ -701,38 +711,51 @@ def test_table_kernel_is_bit_identical_to_the_arithmetic_kernel(tracks_dir, name
         assert a[5] == b[5]
 
 
-def test_cuda_path_against_the_unmodified_reference(tracks_dir, tmp_path):
-    """The CUDA path against the reference's OWN code (lib/car_env.py, unmodified: the /root/reference mount in the
-    build container, the verified oracle/_ref copy on the GPU box) with gymnasium's same-step autoreset emulated:
-    both shipped tracks and the start_destroyed track.  Integers bit-exact, rewards float32(float64 reward),
-    observations 1e-5 relative."""
+def test_cuda_path_against_the_unmodified_reference(golden_dir, tracks_dir, tmp_path):
+    """The CUDA path against the reference's OWN code (lib/car_env.py, unmodified) with gymnasium's same-step autoreset
+    emulated: both shipped tracks and the start_destroyed track.  Always against the stored trajectories
+    (tests/golden: the forward-biased groups of carenv_*.npz, and near_wall.npz, whose `source` names what recorded
+    it); where the reference itself is present ($PPO_CAR_REFERENCE, or the verified oracle/_ref copy), also against
+    fresh trajectories of it.  Integers bit-exact, rewards
+    float32(float64 reward), observations 1e-5 relative."""
     from oracle.ref_import import RefVecEnv, reference_available, track_path
     from tests.synth_tracks import near_wall_track
 
-    if not reference_available():
-        pytest.skip("neither /root/reference nor oracle/_ref (python oracle/make_ref.py) is present")
-    rng = np.random.default_rng(31)
-    cases = [("track", track_path("track.json"), os.path.join(tracks_dir, "track.json"), 240),
-             ("big_track", track_path("big_track.json"), os.path.join(tracks_dir, "big_track.json"), 240)]
-    nw = near_wall_track(str(tmp_path / "near_wall.json"))
-    cases.append(("near_wall", nw, nw, 12))
-    n = 6
-    for name, ref_path, our_path, T in cases:
-        acts = rng.choice(9, size=(T, n), p=[.3, .02, .1, .1, .2, .2, .02, .02, .04]).astype(np.uint8)
-        acts[:, 0] = 0                                          # one env at full throttle: gates, then a crash
-        ref = RefVecEnv(n, ref_path)
-        obs0 = ref.reset()
-        rec = {k: [] for k in ("obs", "rew", "term", "trunc", "gates_passed", "time_passed", "next_gate_index")}
-        for t in range(T):
-            o, r, te, tr, info = ref.step(acts[t])
-            for k, v in (("obs", o), ("rew", r), ("term", te), ("trunc", tr), ("gates_passed", info["gates_passed"]),
-                         ("time_passed", info["time_passed"]), ("next_gate_index", info["next_gate_index"])):
-                rec[k].append(np.array(v))
-        rec = {k: np.stack(v) for k, v in rec.items()}
+    cases = []                                                  # name, track, reset obs, trajectory with its actions
+    for name in ("track", "big_track"):
+        g = np.load(os.path.join(golden_dir, f"carenv_{name}.npz"))
+        cases.append((name, os.path.join(tracks_dir, name + ".json"), g["reset_obs"], _golden_group(g, "fwd", 240, 6)))
+    g = np.load(os.path.join(golden_dir, "near_wall.npz"))
+    cases.append(("near_wall", os.path.join(golden_dir, "near_wall_track.json"), g["reset_obs"],
+                  _golden_group(g, "destroyed")))
+    if reference_available():
+        rng = np.random.default_rng(31)
+        nw = near_wall_track(str(tmp_path / "near_wall.json"))
+        n = 6
+        for name, ref_path, our_path, T in [("track", track_path("track.json"), os.path.join(tracks_dir, "track.json"), 240),
+                                            ("big_track", track_path("big_track.json"),
+                                             os.path.join(tracks_dir, "big_track.json"), 240),
+                                            ("near_wall", nw, nw, 12)]:
+            acts = rng.choice(9, size=(T, n), p=[.3, .02, .1, .1, .2, .2, .02, .02, .04]).astype(np.uint8)
+            acts[:, 0] = 0                                      # one env at full throttle: gates, then a crash
+            ref = RefVecEnv(n, ref_path)
+            obs0 = ref.reset()
+            rec = {k: [] for k in ("obs", "rew", "term", "trunc", "gates_passed", "time_passed", "next_gate_index")}
+            for t in range(T):
+                o, r, te, tr, info = ref.step(acts[t])
+                for k, v in (("obs", o), ("rew", r), ("term", te), ("trunc", tr), ("gates_passed", info["gates_passed"]),
+                             ("time_passed", info["time_passed"]), ("next_gate_index", info["next_gate_index"])):
+                    rec[k].append(np.array(v))
+            rec = {k: np.stack(v) for k, v in rec.items()}
+            rec["actions"] = acts
+            cases.append((name + " (live reference)", our_path, obs0, rec))
+    for name, our_path, obs0, rec in cases:
+        acts = rec["actions"]
+        n, T = acts.shape[1], acts.shape[0]
         env = ppo_car_b200.VecCarEnv(n, our_path)
         g0, _ = env.reset()
-        tol = RTOL_SYNTHETIC if name == "near_wall" else 1e-5
-        assert_floats_close(g0.cpu().numpy(), obs0, f"{name}: reset obs vs reference", rtol=tol)
+        tol = RTOL_SYNTHETIC if name.startswith("near_wall") else 1e-5
+        assert_floats_close(g0.cpu().numpy(), np.broadcast_to(obs0, g0.shape), f"{name}: reset obs vs reference", rtol=tol)
         out = env.rollout(torch.from_numpy(acts).cuda(), store_info=True)
         assert_trajectory_matches(_gpu_traj(out), rec, what=f"{name} vs unmodified reference", rtol=tol)
         assert rec["term"].sum() > 0

@@ -117,14 +117,28 @@ def test_port_against_live_reference_when_available(tracks_dir):
             assert np.array_equal(i1["next_gate_index"], i2["next_gate_index"])
 
 
-def test_port_against_live_reference_start_destroyed(tmp_path):
+def test_port_against_live_reference_start_destroyed(golden_dir, tmp_path):
     """The branch the shipped tracks never take: a start pose inside the collision distance
-    (lib/car_env.py:682-686).  Unmodified reference vs port, bit-exact."""
+    (lib/car_env.py:682-686).  Port vs the stored trajectory (tests/golden/near_wall.npz, its `source` names what
+    recorded it) and, where the unmodified reference is present, vs the reference itself; bit-exact."""
     from oracle.ref_import import RefVecEnv, reference_available
     from tests.synth_tracks import near_wall_track
 
+    g = np.load(os.path.join(golden_dir, "near_wall.npz"))
+    acts = g["destroyed_actions"]
+    port = PortVecEnv(acts.shape[1], os.path.join(golden_dir, "near_wall_track.json"))
+    assert np.array_equal(port.reset(), np.broadcast_to(g["reset_obs"], (acts.shape[1], 18)))
+    for t in range(acts.shape[0]):
+        obs, rew, term, trunc, info = port.step(acts[t])
+        assert term.all() and np.array_equal(term, g["destroyed_term"][t]), t
+        assert np.array_equal(trunc, g["destroyed_trunc"][t]) and np.array_equal(rew, g["destroyed_rew"][t]), t
+        assert np.array_equal(info["final_obs"], g["destroyed_final_obs"][t]), t
+        assert np.array_equal(obs, np.broadcast_to(g["reset_obs"], obs.shape)), t
+        for k in ("gates_passed", "time_passed", "next_gate_index"):
+            assert np.array_equal(info[k], g[f"destroyed_{k}"][t]), (k, t)
+
     if not reference_available():
-        pytest.skip("neither /root/reference nor oracle/_ref is present")
+        return
     path = near_wall_track(str(tmp_path / "near_wall.json"))
     acts = np.random.default_rng(5).integers(0, 9, size=(12, 3))
     ref, port = RefVecEnv(3, path), PortVecEnv(3, path)
@@ -136,15 +150,30 @@ def test_port_against_live_reference_start_destroyed(tmp_path):
         assert np.array_equal(i1["final_obs"], i2["final_obs"]) and np.array_equal(i1["time_passed"], i2["time_passed"])
 
 
-def test_reference_copy_recipe_is_byte_identical(tmp_path):
+def test_reference_copy_recipe_is_byte_identical(tmp_path, monkeypatch):
     """oracle/make_ref.py copies the hot-path files unmodified: when both the mount and the copy exist they are
-    byte-identical, and the MANIFEST hashes verify."""
-    from oracle import ref_import
+    byte-identical, and the MANIFEST hashes verify.  The recipe is also run on a stand-in source tree, so that it is
+    checked without a reference checkout: byte-identical copy, verified MANIFEST, and a changed copy is refused."""
+    from oracle import make_ref, ref_import
 
     copy = ref_import.reference_root(prefer_copy=True)
-    if copy is None or not copy.endswith("_ref"):
-        pytest.skip("oracle/_ref not populated")
-    assert ref_import._copy_is_intact()
-    if os.path.isfile(os.path.join(ref_import._MOUNT, "lib", "car_env.py")):
-        for rel in ("lib/car_env.py", "lib/buffer.py", "tracks/track.json", "tracks/big_track.json"):
-            assert open(os.path.join(copy, rel), "rb").read() == open(os.path.join(ref_import._MOUNT, rel), "rb").read()
+    if copy is not None and copy.endswith("_ref"):
+        assert ref_import._copy_is_intact()
+        if os.path.isfile(os.path.join(ref_import._MOUNT, "lib", "car_env.py")):
+            for rel in ("lib/car_env.py", "lib/buffer.py", "tracks/track.json", "tracks/big_track.json"):
+                assert open(os.path.join(copy, rel), "rb").read() == open(os.path.join(ref_import._MOUNT, rel), "rb").read()
+
+    src, dst = tmp_path / "src", tmp_path / "_ref"
+    for i, rel in enumerate(make_ref.FILES):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(b"stand-in %d\n" % i + bytes(range(256)))
+    monkeypatch.setattr(make_ref, "SRC", str(src))
+    monkeypatch.setattr(make_ref, "DST", str(dst))
+    monkeypatch.setattr(ref_import, "_MOUNT", str(tmp_path / "no_mount"))
+    monkeypatch.setattr(ref_import, "_COPY", str(dst))
+    assert make_ref.make(verbose=False) == str(dst)
+    for rel in make_ref.FILES:
+        assert (dst / rel).read_bytes() == (src / rel).read_bytes()
+    assert ref_import._copy_is_intact() and ref_import.reference_root(prefer_copy=True) == str(dst)
+    (dst / "lib" / "car_env.py").write_bytes(b"changed")
+    assert not ref_import._copy_is_intact() and ref_import.reference_root(prefer_copy=True) is None

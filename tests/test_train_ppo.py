@@ -59,19 +59,31 @@ def test_graph_update_trains():
     assert abs(hist[-1]["lr"] - 3e-4 * 0.99 ** 12) < 1e-9
 
 
-def test_state_dict_loads_into_the_reference_agent():
-    """The checkpoints train_ppo writes (train.py:280-283, 301) carry the reference Agent's keys: a state dict of
-    this harness's network loads strictly into the UNMODIFIED lib/model.py:Agent and both compute the same outputs."""
+def test_state_dict_loads_into_the_reference_agent(golden_dir):
+    """The checkpoints train_ppo writes (train.py:280-283, 301) carry the reference Agent's keys: the stored Agent
+    checkpoint (tests/golden/agent_checkpoint.npz, its `source` names what recorded it) loads strictly into this
+    harness's network, which then computes the stored outputs; where the UNMODIFIED lib/model.py is present, a state
+    dict of this network also loads strictly into its Agent and both compute the same outputs."""
     import importlib
+    import os
     import sys
+
+    import numpy as np
 
     from oracle.ref_import import reference_root
 
+    g = np.load(os.path.join(golden_dir, "agent_checkpoint.npz"))
+    net = ActorCritic(18, 9)
+    net.load_state_dict({k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w_")}, strict=True)
+    with torch.no_grad():
+        _, logp, ent, val = net.act(torch.from_numpy(g["obs"]), torch.from_numpy(g["act"]))
+    assert torch.allclose(logp, torch.from_numpy(g["logp"]), atol=1e-6)
+    assert torch.allclose(ent, torch.from_numpy(g["entropy"]), atol=1e-6)
+    assert val.shape == g["value"].shape and torch.allclose(val, torch.from_numpy(g["value"]), atol=1e-6)
+
     root = reference_root()
     if root is None:
-        pytest.skip("neither /root/reference nor oracle/_ref is present")
-    import os
-
+        return
     if not os.path.isfile(os.path.join(root, "lib", "model.py")):
         pytest.skip("lib/model.py not in the reference copy (re-run oracle/make_ref.py)")
     if root not in sys.path:
