@@ -27,6 +27,10 @@ def gae_reverse_scan(rew, val, term, trunc, last_val, last_term, last_trunc, gam
     if not rew.is_cuda:
         raise _lib.CarEnvError("gae_reverse_scan only runs on CUDA tensors (there is no CPU implementation)")
     T, N = rew.shape
+    for name, out in (("adv_out", adv_out), ("ret_out", ret_out)):      # the kernel writes T * N floats through them
+        if out is not None and (not isinstance(out, torch.Tensor) or out.dtype != torch.float32
+                                or tuple(out.shape) != (T, N) or not out.is_contiguous() or out.device != rew.device):
+            raise ValueError(f"{name} must be a contiguous float32 ({T}, {N}) tensor on {rew.device}")
     f32 = lambda t, shape: t.to(device=rew.device, dtype=torch.float32).reshape(shape).contiguous()
     rew, val, term, trunc = (f32(t, (T, N)) for t in (rew, val, term, trunc))
     last_val, last_term, last_trunc = (f32(t, (N,)) for t in (last_val, last_term, last_trunc))

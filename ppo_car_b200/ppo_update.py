@@ -112,6 +112,8 @@ class FusedPPOUpdate:
             raise ValueError("prof must be an int64 device tensor of n_updates x 4 elements")
         if world > 1 and (self._comm is None or self._comm_world != world):
             raise _lib.CarEnvError("run_epoch(world > 1) needs connect() on every rank first")
+        if idx.shape[0] == 0:            # no updates; an empty idx has no storage (data_ptr 0), which the C ABI refuses
+            return
         if self._epoch_ws is None:
             self._epoch_ws = torch.zeros(self.L.carenv_ppo_epoch_workspace_floats(), device=self.device)
             self._sync = torch.zeros(2, dtype=torch.int32, device=self.device)
