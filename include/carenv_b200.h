@@ -269,6 +269,32 @@ int carenv_policy_rollout_warp(void *handle, const float *w1_actor, const float 
                                float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
                                float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream);
 
+/* Policy evaluation: n_episodes whole episodes of the actor (nn.Linear layout, 18-256-9) on the handle's track in ONE
+ * launch (k_policy_eval, csrc/policy_eval.cuh), one record per episode.  Episode i of the call has the global id
+ * episode0 + i and starts from the start pose; its result depends only on (weights, seed, id, greedy), not on
+ * n_episodes or on how the library schedules the episodes.  The environment state arrays are not touched.
+ *   greedy          1: the argmax of the logits (lowest index on a tie); 0: a sample by inverse CDF on a
+ *                   Philox4x32-10 uniform keyed by `seed`, counter (id low 32 bits, step within the episode,
+ *                   id high 32 bits, 0x4556414C)
+ *   records         [n_episodes], written when the episode ends (terminated or truncated at 1000 steps):
+ *                     ret        float64 sum of the unscaled rewards, in step order
+ *                     length     time_passed of the last step; gates: gates_passed of the last step
+ *                     laps       completed laps; first_lap: time_passed at the first lap, or -1
+ *                     outcome    1 = crash (terminated), 2 = time limit (truncated)
+ *   n_trace         episodes i < n_trace also write their actions to trace_actions [n_trace][1000] and, when
+ *                   trace_u is not NULL and greedy == 0, the uniforms to trace_u [n_trace][1000]; entries past an
+ *                   episode's end are not written.  The environment is deterministic: the actions replay the episode.
+ * Tracks with at most 128 wall segments (CARENV_E_TRACK otherwise).  Float32 CUDA cores; the logits equal those of
+ * carenv_policy_rollout for the same weights and observation. */
+typedef struct {
+    double ret;
+    int32_t length, gates, laps, first_lap, outcome, pad;
+} carenv_eval_record;
+int carenv_policy_eval(void *handle, const float *w1_actor, const float *b1_actor, const float *w2_actor,
+                       const float *b2_actor, long long n_episodes, unsigned long long episode0, int greedy,
+                       unsigned long long seed, carenv_eval_record *records, int n_trace, unsigned char *trace_actions,
+                       float *trace_u, void *stream);
+
 /* All minibatch updates of one PPO epoch in ONE persistent cooperative launch (csrc/ppo_epoch.cuh; replaces the
  * loops of train.py:223-261 — `for _ in range(train_iters): for start in range(0, n_steps, batch_size): ...` — and,
  * with several GPUs, the gradient all-reduce between backward and optimizer.step()).

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(_PKG)
 LIB_PATH = os.environ.get("CARENV_LIB") or os.path.join(_PKG, "libcarenv_b200.so")   # override: kernel experiments
 SOURCES = [os.path.join(_PKG, "csrc", f)
            for f in ("carenv_kernels.cu", "carenv_core.cuh", "carenv_tables.h", "policy_core.cuh", "tc_mlp.cuh",
-                     "ppo_update.cuh", "ppo_epoch.cuh", "policy_rollout.cuh", "policy_abi.cuh")]
+                     "ppo_update.cuh", "ppo_epoch.cuh", "policy_rollout.cuh", "policy_abi.cuh", "policy_eval.cuh")]
 HEADER = os.path.join(ROOT, "include", "carenv_b200.h")
 
 ACT_U8, ACT_I32, ACT_I64 = 0, 1, 2
@@ -112,6 +112,8 @@ def lib():
     L.carenv_policy_rollout_warp.restype = i32
     L.carenv_policy_weights_floats_tc.restype = i32
     L.carenv_policy_rollout_tc.argtypes = L.carenv_policy_rollout.argtypes
+    L.carenv_policy_eval.argtypes = [vp] * 5 + [C.c_longlong, C.c_ulonglong, i32, C.c_ulonglong, vp, i32, vp, vp, vp]
+    L.carenv_policy_eval.restype = i32
     for name in ("carenv_create", "carenv_destroy", "carenv_reset_obs", "carenv_reset", "carenv_step",
                  "carenv_rollout", "carenv_rollout_poses", "carenv_observe", "carenv_step_host", "carenv_step_host_records", "carenv_step_records", "carenv_step_final", "carenv_multi_create", "carenv_multi_destroy", "carenv_multi_reset",
                  "carenv_multi_rollout", "carenv_render", "carenv_host_alloc", "carenv_host_free", "carenv_stats", "gae_reverse_scan", "carenv_bench_ffma", "carenv_set_option", "carenv_policy_rollout", "carenv_policy_rollout_tc"):

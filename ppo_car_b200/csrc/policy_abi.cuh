@@ -365,3 +365,5 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
     if (U == 2) return launch(k_policy_rollout_tc<2, 2>);
     return launch(k_policy_rollout_tc<1, 2>);
 }
+
+#include "policy_eval.cuh"      // carenv_policy_eval: k_policy_eval, whole episodes of one actor per launch

@@ -1,0 +1,185 @@
+"""Policy evaluation on the GPU: whole episodes of one actor in one kernel launch (C ABI ``carenv_policy_eval``).
+
+The reference scores a policy only by watching it (the video logger of train.py:23-50, greedy play every 10
+epochs); ``avg_reward`` of training is a per-step mean over exploring rollouts.  Here every episode of a batch is
+played to its end by ``k_policy_eval`` (csrc/policy_eval.cuh) — greedily or by sampling — and leaves one record:
+its return, length, gates, laps, the step of its first lap and whether it crashed or ran into the 1000-step limit.
+
+    python -m ppo_car_b200.evaluate --checkpoint model.dat --track big_track --episodes 65536 [--greedy]
+    python -m torch.distributed.run --nproc-per-node 8 -m ppo_car_b200.evaluate --checkpoint model.dat ...
+
+Episode ``episode0 + i`` of a call is a fixed function of (weights, seed, id, greedy): a batch can be split over
+calls or ranks at any boundary and gives the same records.
+"""
+from __future__ import annotations
+
+import argparse
+import ctypes as C
+import json
+import math
+import os
+
+import torch
+
+from . import _lib
+from .policy import ACTIONS, HIDDEN, OBS
+
+TIME_LIMIT = 1000                   # steps per episode at most (lib/car_env.py:491)
+RECORD_INT32 = 8                    # carenv_eval_record: double ret; int32 length, gates, laps, first_lap, outcome, pad
+CRASH, TRUNCATED = 1, 2
+SUM_FIELDS = ("count", "ret", "ret_sq", "length", "crashes", "truncations", "lapped", "laps", "first_lap", "gates")
+
+
+def _p(t):
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
+class EvalResult:
+    """Per-episode records of one evaluation call.  ``records`` is the int32 [n, 8] image of the C records;
+    ``ret`` (float64), ``length``, ``gates``, ``laps``, ``first_lap`` (-1 without a lap) and ``outcome``
+    (1 = crash, 2 = time limit) are views of it.  ``trace_actions`` [n_trace, 1000] uint8 (255 past an
+    episode's end) and ``trace_u`` [n_trace, 1000] float32 (sampled calls only) are None without a trace."""
+
+    def __init__(self, records: torch.Tensor, trace_actions: torch.Tensor | None = None,
+                 trace_u: torch.Tensor | None = None):
+        if records.dtype != torch.int32 or records.dim() != 2 or records.shape[1] != RECORD_INT32:
+            raise ValueError("records must be an int32 tensor of shape (n, 8)")
+        self.records = records
+        self.ret = records.view(torch.float64)[:, 0]
+        self.length, self.gates, self.laps = records[:, 2], records[:, 3], records[:, 4]
+        self.first_lap, self.outcome = records[:, 5], records[:, 6]
+        self.trace_actions, self.trace_u = trace_actions, trace_u
+
+    def __len__(self) -> int:
+        return self.records.shape[0]
+
+    def sums(self) -> torch.Tensor:
+        """float64 [10] on the records' device, in the order of SUM_FIELDS: count, sum of returns, sum of squared
+        returns, sum of lengths, crashes, truncations, episodes with a lap, sum of laps, sum of first-lap steps
+        over the lapped episodes, sum of gates.  Sums of shards add up to the sums of their concatenation."""
+        d = torch.float64
+        lapped = self.laps > 0
+        ret = self.ret
+        return torch.stack([
+            torch.tensor(float(len(self)), dtype=d, device=ret.device), ret.sum(), (ret * ret).sum(),
+            self.length.to(d).sum(), (self.outcome == CRASH).to(d).sum(), (self.outcome == TRUNCATED).to(d).sum(),
+            lapped.to(d).sum(), self.laps.to(d).sum(), torch.where(lapped, self.first_lap, 0).to(d).sum(),
+            self.gates.to(d).sum()])
+
+    def summary(self, sums: torch.Tensor | None = None) -> dict:
+        """Means and rates from ``sums`` (e.g. all-reduced over ranks; default: this call's).  ``avg_reward`` is
+        the sum of returns over the sum of lengths: training's metric (times its reward scaling) without the
+        exploration noise and over whole episodes.  Rates are fractions of the episodes; ``std_return`` is the
+        population standard deviation; ``mean_first_lap_steps`` is over the episodes with a lap (None if none)."""
+        s = dict(zip(SUM_FIELDS, (self.sums() if sums is None else sums).tolist()))
+        n = s["count"]
+        if n <= 0:
+            return {"episodes": 0}
+        mean = s["ret"] / n
+        return {"episodes": int(n), "mean_return": mean,
+                "std_return": math.sqrt(max(s["ret_sq"] / n - mean * mean, 0.0)),
+                "avg_reward": s["ret"] / s["length"], "mean_length": s["length"] / n,
+                "crash_rate": s["crashes"] / n, "truncation_rate": s["truncations"] / n,
+                "lap_rate": s["lapped"] / n, "mean_laps": s["laps"] / n,
+                "mean_first_lap_steps": s["first_lap"] / s["lapped"] if s["lapped"] > 0 else None,
+                "mean_gates": s["gates"] / n}
+
+
+def _actor_params(actor, device):
+    params = [actor[0].weight, actor[0].bias, actor[2].weight, actor[2].bias]
+    if [tuple(p.shape) for p in params] != [(HIDDEN, OBS), (HIDDEN,), (ACTIONS, HIDDEN), (ACTIONS,)]:
+        raise ValueError("policy evaluation supports the reference actor only: 18-256-9")
+    if any(p.dtype != torch.float32 or not p.is_contiguous() or p.device != device for p in params):
+        raise ValueError(f"actor parameters must be contiguous float32 tensors on {device}")
+    return [p.detach() for p in params]
+
+
+def evaluate_policy(env, actor, n_episodes: int, greedy: bool = False, seed: int = 0, episode0: int = 0,
+                    trace: int = 0) -> EvalResult:
+    """Play episodes ``episode0 .. episode0 + n_episodes - 1`` of ``actor`` (``nn.Sequential(Linear(18, 256), ReLU,
+    Linear(256, 9))`` on ``env.device``) on ``env``'s track, each from the start pose to its end, in one launch on
+    the current stream.  ``greedy``: argmax actions; else sampled with the Philox stream keyed by ``seed``.  The
+    first ``trace`` episodes also record their actions (and uniforms when sampled).  ``env``'s state is not
+    touched; only its track handle and device are used."""
+    n_episodes, trace = int(n_episodes), int(trace)
+    if n_episodes < 0 or trace < 0:
+        raise ValueError("n_episodes and trace must be >= 0")
+    if not 0 <= int(episode0) < 2 ** 64:
+        raise ValueError("episode0 must fit in 64 bits")
+    dev = env.device
+    params = _actor_params(actor, dev)
+    records = torch.empty((n_episodes, RECORD_INT32), dtype=torch.int32, device=dev)
+    n_trace = min(trace, n_episodes)
+    trace_actions = trace_u = None
+    if trace:
+        trace_actions = torch.full((n_trace, TIME_LIMIT), 255, dtype=torch.uint8, device=dev)
+        if not greedy:
+            trace_u = torch.full((n_trace, TIME_LIMIT), float("nan"), dtype=torch.float32, device=dev)
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        rc = L.carenv_policy_eval(env._handle, *[_p(p) for p in params], n_episodes, int(episode0), int(bool(greedy)),
+                                  int(seed) & (2 ** 64 - 1), _p(records), n_trace, _p(trace_actions), _p(trace_u),
+                                  env._stream())
+    _lib.check(rc, "carenv_policy_eval")
+    return EvalResult(records, trace_actions, trace_u)
+
+
+def load_checkpoint(path: str):
+    """The state dict ``train_ppo`` saves (model.dat / checkpoint_{epoch}.dat, the reference Agent's keys
+    actor.0.weight ... critic.2.bias), loaded strictly into a CPU ActorCritic."""
+    from .train_ppo import ActorCritic
+
+    net = ActorCritic(OBS, ACTIONS, HIDDEN)
+    net.load_state_dict(torch.load(path, map_location="cpu", weights_only=True), strict=True)
+    return net
+
+
+def parse_args(argv=None):
+    p = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
+    p.add_argument("--checkpoint", required=True, help="model.dat / checkpoint_{epoch}.dat written by train_ppo")
+    p.add_argument("--track", default="big_track", help="track name shipped with the package or a JSON path")
+    p.add_argument("--episodes", type=int, default=65536, help="episodes in total over all ranks")
+    p.add_argument("--greedy", action="store_true", help="argmax actions instead of sampled ones")
+    p.add_argument("--seed", type=int, default=0, help="seed of the sampling stream")
+    p.add_argument("--json", default=None, help="write the summary to this file")
+    return p.parse_args(argv)
+
+
+def main(argv=None) -> dict:
+    import torch.distributed as dist
+
+    from . import VecCarEnv, builtin_track
+    from .shard import shard_range
+
+    args = parse_args(argv)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    rank = int(os.environ.get("RANK", "0"))
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local)
+    dev = torch.device("cuda", local)
+    if world > 1 and not dist.is_initialized():
+        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
+        dist.init_process_group("nccl", device_id=dev)
+    track = args.track if os.path.exists(args.track) else builtin_track(args.track)
+    env = VecCarEnv(1, track, device=dev)
+    actor = load_checkpoint(args.checkpoint).actor.to(dev)
+    lo, hi = shard_range(args.episodes, world, rank)            # every rank plays its contiguous share of the ids
+    res = evaluate_policy(env, actor, hi - lo, greedy=args.greedy, seed=args.seed, episode0=lo)
+    sums = res.sums()
+    if world > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+    out = {"checkpoint": args.checkpoint, "track": args.track, "greedy": bool(args.greedy), "seed": args.seed,
+           **res.summary(sums)}
+    if rank == 0:
+        print(json.dumps(out), flush=True)
+        if args.json:
+            with open(args.json, "w") as fh:
+                json.dump(out, fh)
+    env.close()
+    if dist.is_initialized():
+        dist.destroy_process_group()
+    return out
+
+
+if __name__ == "__main__":
+    main()

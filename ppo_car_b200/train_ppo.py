@@ -110,6 +110,12 @@ def parse_args(argv=None):
     p.add_argument("--cuda-graph", action="store_true",
                    help="capture the whole n_steps rollout (policy forward, sampling, env step, buffer rows) in one "
                         "CUDA graph and replay it every epoch: removes the per-step launch overhead at small n_envs")
+    p.add_argument("--eval-every", type=int, default=0,
+                   help="every K epochs play --eval-episodes whole episodes of the current actor on the training track "
+                        "(ppo_car_b200.evaluate, one kernel launch, shared out over the ranks) and add the summary to "
+                        "the epoch's record under \"eval\".  Default 0: no evaluation")
+    p.add_argument("--eval-episodes", type=int, default=1024, help="episodes per evaluation, over all ranks")
+    p.add_argument("--eval-greedy", action="store_true", help="evaluate with argmax actions instead of sampled ones")
     return p.parse_args(argv)
 
 
@@ -199,6 +205,20 @@ def train(args) -> list[dict]:
         pack_policy = pack_policy_weights_tc if not args.fused_cuda_cores else pack_policy_weights
         packed = pack_policy(agent.actor, agent.critic)
         last_val = torch.empty(n, device=dev)
+
+    def evaluate_epoch():
+        """--eval-every: every rank plays its share of the episode ids 0 .. eval_episodes - 1 with the same seed, so
+        every evaluation of a run scores the actor on the same episodes; the sums are all-reduced."""
+        from .evaluate import evaluate_policy
+
+        e_lo, e_hi = shard_range(args.eval_episodes, world, rank)
+        with torch.no_grad():
+            res = evaluate_policy(envs, agent.actor, e_hi - e_lo, greedy=args.eval_greedy, seed=args.seed,
+                                  episode0=e_lo)
+            sums = res.sums()
+        if world > 1:
+            dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+        return res.summary(sums)
 
     graph = None
     if args.cuda_graph and not args.fused_rollout:
@@ -318,10 +338,17 @@ def train(args) -> list[dict]:
                    "episodes": episodes, "policy_loss": s[0], "value_loss": s[1], "entropy": s[2], "total_loss": s[3],
                    "lr": float(fused_upd.lr if fused_upd is not None else opt.param_groups[0]["lr"]), "sps": global_step / (time.time() - t_start),
                    "wall_s": time.time() - t_start}
+            if args.eval_every > 0 and epoch % args.eval_every == 0:
+                rec["eval"] = evaluate_epoch()
             history.append(rec)
             if rank == 0:
                 print(f"Epoch {epoch} done in {rec['wall_s']:.2f}s. Avg reward: {rec['avg_reward']:.4f}. "
                       f"SPS {rec['sps']:.0f}  entropy {rec['entropy']:.3f}", flush=True)
+                if "eval" in rec:
+                    ev = rec["eval"]
+                    print(f"  eval ({ev['episodes']} {'greedy' if args.eval_greedy else 'sampled'} episodes): return "
+                          f"{ev['mean_return']:.3f} +- {ev['std_return']:.3f}, avg reward {ev['avg_reward']:.4f}, "
+                          f"crashes {ev['crash_rate']:.1%}, laps/episode {ev['mean_laps']:.3f}", flush=True)
                 if args.log_json:
                     import json
 
