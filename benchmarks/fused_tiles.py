@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Fused rollout kernels versus shard size: CUDA-core kernel and the tensor-core kernel with 2 or 4
-128-env groups per CTA or 2 groups with a helper thread per environment (option tc_tiles 2 / 4 / 3).  One JSON line per size."""
+"""Fused rollout kernels versus shard size: the CUDA-core kernel (k_policy_rollout, column prefix cuda_core) and the
+tensor-core kernel (k_policy_rollout_tc3, column prefix tc_shared_weight_loads).  One JSON line per size."""
 import json
 import os
 import sys
@@ -26,9 +26,7 @@ for n, T in SIZES:
     obs = env.reset()[0].clone()
     term, trunc, lv = torch.zeros(n, device=dev), torch.zeros(n, device=dev), torch.empty(n, device=dev)
     res = {"n_envs": n, "steps_per_launch": T}
-    for tag, packed, tiles in (("cuda_core", packed_cc, 0), ("tc_tiles2", packed_tc, 2), ("tc_tiles4", packed_tc, 4),
-                              ("tc_2groups_helpers", packed_tc, 3), ("tc_shared_weight_loads", packed_tc, 5)):
-        env.set_option("tc_tiles", tiles)
+    for tag, packed in (("cuda_core", packed_cc), ("tc_shared_weight_loads", packed_tc)):
         for i in range(2):
             ppo_car_b200.fused_rollout(env, packed, buf, obs, term, trunc, seed=1, step0=i * T, last_val=lv)
         torch.cuda.synchronize()

@@ -177,12 +177,12 @@ int carenv_render(void *handle, int n_outer_segments, int n_frames, const int32_
  * batches (at most 2,048 environments, at most 32 wall segments) run by default (identical results);
  * "tab" = 1 / -1 forces / forbids the table kernel (k_rollout_tab: denominators from a shared-memory table) that large
  * launches on tracks with at most 128 segments run by default (identical results);
- * "tc_tiles" picks the kernel behind carenv_policy_rollout_tc (0 = default = 5; 2 / 4 = k_policy_rollout_tc with that
- * many 128-environment groups per CTA, 3 = k_policy_rollout_tc2: environment + policy thread per environment, 5 =
- * k_policy_rollout_tc3: second-layer weight loads shared by the two environments of a tensor-memory lane — variants 3
- * and 5 give the same bits, 2 and 4 differ from them in the last bits of the logits only);
+ * "tc_tiles" = 0 (default) or 5 runs carenv_policy_rollout_tc on k_policy_rollout_tc3, its only kernel; 2, 3 and 4
+ * selected kernels that have been removed, are still accepted here and make carenv_policy_rollout_tc fail with
+ * CARENV_E_INVAL;
  * "tab_slice" = -1 keeps the block-round table kernel where the time-sliced one (k_rollout_tab_sliced) would run;
- * "max_unroll", "block", "smem_pad", "tc_stagger", "host_ranges" select kernel / pipeline variants for measurements. */
+ * "max_unroll", "block", "smem_pad", "host_ranges" select kernel / pipeline variants for measurements;
+ * "tc_stagger" is accepted and has no effect. */
 int carenv_set_option(void *handle, const char *name, int value);
 
 /* Slow-path counters since the last reset of the counters: [0] lines re-evaluated in float64

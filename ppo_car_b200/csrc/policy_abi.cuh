@@ -264,7 +264,7 @@ int carenv_tc_gemm_test(const float *A, const float *B, float *D, void *stream) 
 int carenv_policy_weights_floats_tc(void) { return kTcWeightFloats; }
 
 /* Tensor-core variant of carenv_policy_rollout (same arguments; packed_weights in the layout of
- * ppo_car_b200/policy.py: pack_policy_weights_tc). */
+ * ppo_car_b200/policy.py: pack_policy_weights_tc): k_policy_rollout_tc3. */
 int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
                              unsigned long long seed, unsigned long long step0, double *pos, double *vel,
                              int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
@@ -279,91 +279,35 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
         return fail(CARENV_E_INVAL, "null pointer");
     if (h->host.P.n_seg > kMaxSeg)
         return fail(CARENV_E_TRACK, "the fused rollout kernels support tracks with at most 128 wall segments");
+    if (h->tc_tiles >= 2 && h->tc_tiles <= 4)
+        return fail(CARENV_E_INVAL, "tc_tiles 2, 3 and 4 selected tensor-core rollout kernels that have been removed; "
+                                    "use 0 or 5 (k_policy_rollout_tc3)");
     DeviceGuard guard(h->device);
     if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
     const int table_bytes = (int)h->smem_bytes;
-    // groups per CTA: 2 while 4 would leave SMs without a CTA (one CTA per SM: the weights take 110 KB)
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    // kernel variant (option tc_tiles): 2 / 4 = k_policy_rollout_tc with that many 128-env groups per CTA, 3 =
-    // k_policy_rollout_tc2 (environment + policy thread per environment), 5 = k_policy_rollout_tc3 (second-layer
-    // weight loads shared by the two environments of a TMEM lane, denominators from the table) — the fastest at every
-    // size measured (benchmarks/fused_tiles.py: 12.5 / 87 / 351 us per step at 32,768 / 262,144 / 1,048,576 envs
-    // against 15.8 / 111 / 413 for the best of the others) and the default.
-    int tiles = 5;
-    (void)sms;
-    if (h->tc_tiles >= 2 && h->tc_tiles <= 5) tiles = h->tc_tiles;
-    if (tiles == 5) {                                         // k_policy_rollout_tc3: weight loads shared by two environments
-        int U3 = h->force_generic ? 1 : h->host.P.unroll4;
-        if (h->max_unroll > 0 && U3 > h->max_unroll) U3 = (U3 % h->max_unroll == 0) ? h->max_unroll : 1;
-        const bool tab = U3 >= 2 && h->d_den4 && h->tab >= 0;  // denominators from a (row-skewed) table in shared memory
-        const int n_pairs = h->host.n_pairs;
-        const int row_f4 = ((n_pairs + 7) / 8 * 8) | 1;          // odd number of 16-byte units: rows skewed by one bank group
-        const size_t smem3 = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
-                             (size_t)2 * 2 * tc::kABytes + (size_t)2 * 128 * 12 * sizeof(float) +
-                             (tab ? (size_t)kHeadings * row_f4 * 16 : 0);
-        if (smem3 > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
-        const int grid3 = (n_envs + 255) / 256;
-        auto launch3 = [&](auto kern) -> int {
-            CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
-            kern<<<grid3, 256 + 128 + 32, smem3, static_cast<cudaStream_t>(stream)>>>(
-                h->host.P, h->dev, packed_weights, n_envs, n_steps, env_offset, seed, step0,
-                reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
-                cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-                last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4);
-            CU(cudaGetLastError());
-            return 0;
-        };
-        if (U3 == 4) return tab ? launch3(k_policy_rollout_tc3<4, true>) : launch3(k_policy_rollout_tc3<4, false>);
-        if (U3 == 2) return tab ? launch3(k_policy_rollout_tc3<2, true>) : launch3(k_policy_rollout_tc3<2, false>);
-        return launch3(k_policy_rollout_tc3<1, false>);
-    }
-    if (tiles == 3) {
-        const size_t smem2 = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
-                             (size_t)2 * 2 * tc::kABytes + (size_t)2 * 128 * 12 * sizeof(float);
-        if (smem2 > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
-        const int grid2 = (n_envs + 255) / 256;
-        int U2 = h->force_generic ? 1 : h->host.P.unroll4;
-        if (h->max_unroll > 0 && U2 > h->max_unroll) U2 = (U2 % h->max_unroll == 0) ? h->max_unroll : 1;
-        auto launch2 = [&](auto kern) -> int {
-            CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-            kern<<<grid2, 2 * 256 + 32, smem2, static_cast<cudaStream_t>(stream)>>>(
-                h->host.P, h->dev, packed_weights, n_envs, n_steps, env_offset, seed, step0,
-                reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
-                cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-                last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull,
-                h->tc_stagger >= 0 ? h->tc_stagger : 0);
-            CU(cudaGetLastError());
-            return 0;
-        };
-        if (U2 == 4) return launch2(k_policy_rollout_tc2<4>);
-        if (U2 == 2) return launch2(k_policy_rollout_tc2<2>);
-        return launch2(k_policy_rollout_tc2<1>);
-    }
-    const size_t smem = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
-                        (size_t)tiles * 2 * tc::kABytes;
-    if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
-    const int grid = (n_envs + tiles * 128 - 1) / (tiles * 128);
     int U = h->force_generic ? 1 : h->host.P.unroll4;
     if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
+    const bool tab = U >= 2 && h->d_den4 && h->tab >= 0;    // denominators from a (row-skewed) table in shared memory
+    const int n_pairs = h->host.n_pairs;
+    const int row_f4 = ((n_pairs + 7) / 8 * 8) | 1;         // odd number of 16-byte units: rows skewed by one bank group
+    const size_t smem = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
+                        (size_t)2 * 2 * tc::kABytes + (size_t)2 * 128 * 12 * sizeof(float) +
+                        (tab ? (size_t)kHeadings * row_f4 * 16 : 0);
+    if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
+    const int grid = (n_envs + 255) / 256;
     auto launch = [&](auto kern) -> int {
         CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, tiles * 128 + 32, smem, static_cast<cudaStream_t>(stream)>>>(
+        kern<<<grid, 256 + 128 + 32, smem, static_cast<cudaStream_t>(stream)>>>(
             h->host.P, h->dev, packed_weights, n_envs, n_steps, env_offset, seed, step0,
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
             cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull);
+            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4);
         CU(cudaGetLastError());
         return 0;
     };
-    if (tiles == 4) {
-        if (U == 4) return launch(k_policy_rollout_tc<4, 4>);
-        if (U == 2) return launch(k_policy_rollout_tc<2, 4>);
-        return launch(k_policy_rollout_tc<1, 4>);
-    }
-    if (U == 4) return launch(k_policy_rollout_tc<4, 2>);
-    if (U == 2) return launch(k_policy_rollout_tc<2, 2>);
-    return launch(k_policy_rollout_tc<1, 2>);
+    if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true>) : launch(k_policy_rollout_tc3<4, false>);
+    if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true>) : launch(k_policy_rollout_tc3<2, false>);
+    return launch(k_policy_rollout_tc3<1, false>);
 }
 
 #include "policy_eval.cuh"      // carenv_policy_eval: k_policy_eval, whole episodes of one actor per launch

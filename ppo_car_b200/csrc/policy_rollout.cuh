@@ -136,16 +136,10 @@ k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const fl
     }
 }
 
-// ---- fused rollout, tensor-core version ---------------------------------------------------------------------
-// Same contract as k_policy_rollout, but the two 18->256 layers (23.6 of the 29 kflop per env-step) run on the
-// 5th-gen tensor cores: per step every thread writes its observation row (hi/lo TF32 split, a constant 1 in
-// column 18 carries the bias) into the K-major UMMA operand tile of its 128-env group, one elected thread issues
-// tcgen05.mma kind::tf32 for all kTcTiles groups — D = A_hi*B_hi + A_lo*B_hi + A_hi*B_lo (3xTF32: float32-level
-// accuracy) — into tensor memory, and after the commit barrier every thread reads ITS row of pre-activations
-// back with tcgen05.ld, applies ReLU and the small second layer (FFMA2) and goes on to sampling and the env step.
-// TMEM: 512 columns = kTcTiles x kTcCols; the 256 hidden units of a net are produced in 256 / kTcCols rounds.
-// TILES = 128-env groups per CTA: 4 (512 environment threads, TMEM 4 x 128 columns, two rounds per net) for large
-// shards, 2 (256 threads, 2 x 256 columns, one round per net) for shards that would otherwise leave SMs empty.
+// ---- fused rollout, tensor-core version: packed weights ----------------------------------------------------------
+// k_policy_rollout_tc3 (below) runs the two 18->256 layers (23.6 of the 29 kflop per env-step) on the 5th-gen tensor
+// cores.  Its packed weights hold the first layer of each net as a K-major UMMA B operand (256 units x 24 K, the bias
+// in column 18), split into TF32 hi and lo parts for 3xTF32 products, followed by the second layers for the CUDA cores.
 constexpr int kTcBFloats = tc::kTileN * tc::kK;              // 6,144 floats per B operand
 constexpr int kTcW2Off = 4 * kTcBFloats;                     // [actor hi | actor lo | critic hi | critic lo]
 constexpr int kTcW2cOff = kTcW2Off + kHidden * 10;           // W2 actor as [j][5] pairs, then w2c[j]
@@ -207,252 +201,6 @@ k_pack_policy(const float *__restrict__ w1a, const float *__restrict__ b1a, cons
     out[i] = v;
 }
 
-template <int U, int TILES>
-__global__ void __launch_bounds__(TILES * 128 + 32, 1)
-k_policy_rollout_tc(const __grid_constant__ TrackParams P, const Tables G, const float *__restrict__ weights,
-                    int n_envs, int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
-                    double2 *__restrict__ pos, double2 *__restrict__ vel, int4 *__restrict__ ints,
-                    float *__restrict__ cur_obs, float *__restrict__ cur_term, float *__restrict__ cur_trunc,
-                    double reward_scale, float *__restrict__ obs_buf, float *__restrict__ act_buf,
-                    float *__restrict__ rew_buf, float *__restrict__ val_buf, float *__restrict__ term_buf,
-                    float *__restrict__ trunc_buf, float *__restrict__ logp_buf, float *__restrict__ last_val,
-                    float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode) {
-    constexpr int kTcTiles = TILES;                          // 128-env groups per CTA (+ one MMA-issuing warp)
-    constexpr int kTcCols = 512 / TILES;                     // accumulator columns per group and round
-    constexpr int kTcRounds = kHidden / kTcCols;             // rounds per net
-    static_assert(TILES == 2 || TILES == 4, "TMEM: 512 columns = TILES x (256 or 128)");
-    extern __shared__ __align__(16) unsigned char smem[];
-    // [tables | pad to a 128-byte boundary | weights | A tiles (hi, lo per group)]
-    const int w_off = (int)((tc::smem_u32(smem) + (uint32_t)table_bytes + 127u) / 128u * 128u - tc::smem_u32(smem));
-    float *sw = reinterpret_cast<float *>(smem + w_off);
-    unsigned char *sA = smem + w_off + ((kTcWeightFloats * 4 + 127) / 128 * 128);
-    // per 128-env group: "accumulator ready" (MMA -> group), "accumulator consumed" and "operand rows written"
-    // (group -> MMA issuer).  Groups never wait for each other: no CTA-wide barrier inside the step loop.
-    __shared__ __align__(8) unsigned long long mbar_full[kTcTiles], mbar_cons[kTcTiles], mbar_rows[kTcTiles];
-    __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5;
-    for (int i = tid; i < kTcWeightFloats / 4; i += blockDim.x)
-        reinterpret_cast<float4 *>(sw)[i] = reinterpret_cast<const float4 *>(weights)[i];
-    if (tid == 0)
-        for (int g = 0; g < kTcTiles; ++g) {
-            tc::mbar_init(tc::smem_u32(&mbar_full[g]), 1);
-            tc::mbar_init(tc::smem_u32(&mbar_cons[g]), 128);
-            tc::mbar_init(tc::smem_u32(&mbar_rows[g]), 128);
-        }
-    if (warp == 0) tc::tmem_alloc<512>(&tmem_slot);
-    const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
-    tc::fence_async_smem();
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tbase = tmem_slot;
-    const uint32_t sB = tc::smem_u32(sw);
-    const uint32_t idesc = tc::make_idesc_tf32(128, kTcCols);
-    const int n_forward = n_steps + (last_val ? 1 : 0);      // forward passes per thread
-
-    if (warp == kTcTiles * 4) {
-        // ===== MMA issuer (one elected lane): runs ahead of the groups, throttled only by the barriers =====
-        if ((tid & 31) == 0) {
-            uint32_t p_rows = 0, p_cons = 0;                 // same phase for every group: all advance in lock step here
-            for (int f = 0; f < n_forward; ++f) {
-#pragma unroll 1
-                for (int rnd = 0; rnd < 2 * kTcRounds; ++rnd) {
-                    const int net = rnd / kTcRounds, part = rnd % kTcRounds;
-                    const uint32_t bh = sB + (uint32_t)((2 * net) * kTcBFloats * 4 + part * (kTcCols / 8) * tc::kSBO);
-                    const uint32_t bl = bh + (uint32_t)(kTcBFloats * 4);
-#pragma unroll 1
-                    for (int g = 0; g < kTcTiles; ++g) {
-                        if (rnd == 0) tc::mbar_wait(tc::smem_u32(&mbar_rows[g]), p_rows);      // this step's rows
-                        if (f > 0 || rnd > 0) tc::mbar_wait(tc::smem_u32(&mbar_cons[g]), p_cons);  // D_g read out
-                        tc::tc_fence_after();
-                        const uint32_t ah = tc::smem_u32(sA + g * 2 * tc::kABytes), al = ah + tc::kABytes;
-                        const uint32_t d = tbase + (uint32_t)(g * kTcCols);
-#pragma unroll
-                        for (int pr = 0; pr < 3; ++pr) {
-                            const uint32_t a0 = (pr == 1) ? al : ah, b0 = (pr == 2) ? bl : bh;
-#pragma unroll
-                            for (int ks = 0; ks < tc::kK / 8; ++ks)
-                                tc::mma_tf32(d, tc::make_smem_desc(a0 + ks * 2 * tc::kLBO),
-                                             tc::make_smem_desc(b0 + ks * 2 * tc::kLBO), idesc, (pr | ks) != 0);
-                        }
-                        tc::mma_commit(tc::smem_u32(&mbar_full[g]));
-                    }
-                    if (rnd == 0) p_rows ^= 1u;
-                    if (f > 0 || rnd > 0) p_cons ^= 1u;
-                }
-            }
-        }
-    } else {
-        // ===== environment threads: one thread = one environment = one TMEM lane of its group =====
-        const int group = tid >> 7, row = tid & 127;
-        const uint32_t my_tmem = tbase + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(group * kTcCols);
-        unsigned char *myA = sA + group * 2 * tc::kABytes;   // hi tile, then lo tile
-        const uint32_t full_bar = tc::smem_u32(&mbar_full[group]), cons_bar = tc::smem_u32(&mbar_cons[group]);
-        const uint32_t rows_bar = tc::smem_u32(&mbar_rows[group]);
-        uint32_t parity = 0;
-
-        const int e_raw = blockIdx.x * (kTcTiles * 128) + tid;
-        const bool active = e_raw < n_envs;
-        const int e = active ? e_raw : n_envs - 1;           // idle threads shadow the last env (no stores)
-
-        EnvState s;
-        {
-            const double2 p = pos[e], v = vel[e];
-            const int4 q = ints[e];
-            s.px = p.x; s.py = p.y; s.vx = v.x; s.vy = v.y;
-            s.k = q.x; s.t = q.y; s.next_gate = q.z; s.passed = q.w;
-        }
-        float obs[kObsDim];
-        {
-            const float2 *src = reinterpret_cast<const float2 *>(cur_obs + (size_t)e * kObsDim);
-#pragma unroll
-            for (int i = 0; i < kObsDim / 2; ++i) { const float2 v = src[i]; obs[2 * i] = v.x; obs[2 * i + 1] = v.y; }
-        }
-        float tc_ = cur_term[e], uc = cur_trunc[e];
-        const uint32_t gid = (uint32_t)(env_offset + e);
-
-        // one forward pass of both nets for the observation in `obs`
-        auto forward = [&](PolicyOut &po) {
-            // this thread's operand row: obs | 1 | 0...  split into TF32 hi and lo.  The previous pass's MMAs have
-            // completed (their last "accumulator ready" was awaited), so the tile may be overwritten.
-#pragma unroll
-            for (int c = 0; c < tc::kKChunks; ++c) {
-                float hi[4], lo[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int k = 4 * c + j;
-                    const float x = k < kObsDim ? obs[k < kObsDim ? k : 0] : (k == kObsDim ? 1.0f : 0.0f);
-                    hi[j] = tc::to_tf32(x);
-                    lo[j] = tc::to_tf32(x - hi[j]);
-                }
-                const int off = tc::operand_offset(row, 4 * c);
-                *reinterpret_cast<float4 *>(myA + off) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-                *reinterpret_cast<float4 *>(myA + tc::kABytes + off) = make_float4(lo[0], lo[1], lo[2], lo[3]);
-            }
-            tc::fence_async_smem();
-            tc::mbar_arrive(rows_bar);
-            float2 L[5];
-#pragma unroll
-            for (int q = 0; q < 5; ++q) L[q] = make_float2(0.0f, 0.0f);
-            float2 V = make_float2(0.0f, 0.0f);
-#pragma unroll 1
-            for (int rnd = 0; rnd < 2 * kTcRounds; ++rnd) {
-                const int net = rnd / kTcRounds, part = rnd % kTcRounds;   // net 0 = actor, 1 = critic
-                tc::mbar_wait(full_bar, parity);
-                parity ^= 1u;
-                tc::tc_fence_after();
-                if (net == 0) {
-                    const float2 *w2 = reinterpret_cast<const float2 *>(sw + kTcW2Off) + (size_t)(part * kTcCols) * 5;
-#pragma unroll 1
-                    for (int c = 0; c < kTcCols; c += 16) {
-                        float v[16];
-                        tc::tmem_ld16(my_tmem + c, v);
-                        if (c + 16 == kTcCols) { tc::tc_fence_before(); tc::mbar_arrive(cons_bar); }   // D_g is free again
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) {
-                            const float h = fmaxf(v[i], 0.0f);
-#pragma unroll
-                            for (int q = 0; q < 5; ++q) L[q] = __ffma2_rn(make_float2(h, h), w2[(c + i) * 5 + q], L[q]);
-                        }
-                    }
-                } else {
-                    const float4 *wc = reinterpret_cast<const float4 *>(sw + kTcW2cOff + part * kTcCols);
-#pragma unroll 1
-                    for (int c = 0; c < kTcCols; c += 16) {
-                        float v[16];
-                        tc::tmem_ld16(my_tmem + c, v);
-                        if (c + 16 == kTcCols) { tc::tc_fence_before(); tc::mbar_arrive(cons_bar); }
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float4 w4 = wc[c / 4 + i];
-                            V = __ffma2_rn(make_float2(fmaxf(v[4 * i], 0.0f), fmaxf(v[4 * i + 1], 0.0f)),
-                                           make_float2(w4.x, w4.y), V);
-                            V = __ffma2_rn(make_float2(fmaxf(v[4 * i + 2], 0.0f), fmaxf(v[4 * i + 3], 0.0f)),
-                                           make_float2(w4.z, w4.w), V);
-                        }
-                    }
-                }
-            }
-            const float *tail = sw + kTcTailOff;
-#pragma unroll
-            for (int q = 0; q < 5; ++q) {
-                po.logit[2 * q] = L[q].x + tail[2 * q];
-                po.logit[2 * q + 1] = L[q].y + tail[2 * q + 1];
-            }
-            po.value = (V.x + V.y) + tail[10];
-        };
-
-        PolicyOut po;
-        for (int t = 0; t < n_steps; ++t) {
-            const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
-            forward(po);
-            const unsigned long long gs = step0 + (unsigned long long)t;
-            const uint32_t bits = philox_uniform_bits((uint32_t)seed, (uint32_t)(seed >> 32), gid, (uint32_t)gs,
-                                                      (uint32_t)(gs >> 32), 0x43415245u);
-            const float u = (float)(bits >> 8) * (1.0f / 16777216.0f);
-            float logp, us;
-            const int a = sample_action(po, u, logp, us);
-            if (active) {
-                if (obs_mode == kObsPose) {
-                    store_pose(reinterpret_cast<PoseRec *>(obs_buf) + idx, s, obs[2], obs[3]);
-                } else {
-                    float2 *dst = reinterpret_cast<float2 *>(obs_buf + idx * kObsDim);
-#pragma unroll
-                    for (int i = 0; i < kObsDim / 2; ++i) dst[i] = make_float2(obs[2 * i], obs[2 * i + 1]);
-                }
-                act_buf[idx] = (float)a;
-                val_buf[idx] = po.value;
-                logp_buf[idx] = logp;
-                term_buf[idx] = tc_;
-                trunc_buf[idx] = uc;
-                if (u_dbg) u_dbg[idx] = u;
-            }
-            StepResult o;
-            env_step<U>(s, a, reward_scale, P, T, o, active ? stats : nullptr);
-            if (active) rew_buf[idx] = o.reward;
-#pragma unroll
-            for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];
-            tc_ = o.terminated ? 1.0f : 0.0f;
-            uc = o.truncated ? 1.0f : 0.0f;
-        }
-        if (last_val) forward(po);                           // bootstrap value of the final observation
-        if (active) {
-            pos[e] = make_double2(s.px, s.py);
-            vel[e] = make_double2(s.vx, s.vy);
-            ints[e] = make_int4(s.k, s.t, s.next_gate, s.passed);
-            float2 *dst = reinterpret_cast<float2 *>(cur_obs + (size_t)e * kObsDim);
-#pragma unroll
-            for (int i = 0; i < kObsDim / 2; ++i) dst[i] = make_float2(obs[2 * i], obs[2 * i + 1]);
-            cur_term[e] = tc_;
-            cur_trunc[e] = uc;
-            if (last_val) last_val[e] = po.value;
-        }
-    }
-    tc::tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tc::tmem_dealloc<512>(tbase);
-}
-
-// ---- fused rollout, tensor cores, TWO threads per environment ---------------------------------------------------
-// k_policy_rollout_tc walks one dependent chain of ~6,900 instructions per environment and step (operand row ->
-// MMA -> 256 + 256 hidden units through the CUDA-core second layer -> sampling -> env step); with one 256-env CTA
-// per SM (shards of 32,768 envs, BASELINE config 5) that chain IS the step time.  Measured per step (cycle stamps,
-// benchmarks/tc2_phase_profile.py): env step 9.4k cycles, second layer 13k — of which 11k are the shared-memory
-// pipe delivering the broadcast weights (16 bytes x 32 lanes per LDS.128 = two return cycles; both 128-env groups
-// run their second layer at the same time because their MMAs complete together).  Here
-//   * every environment has an ENVIRONMENT thread (operand row, Buffer rows, Philox, hidden units 0..127 of the
-//     actor, sampling, env step) and a POLICY thread on the same TMEM lane (hidden units 128..255 of the actor —
-//     partial logits to the environment thread through shared memory — then the whole critic and the value row,
-//     off the critical path: it runs while the environment thread samples and steps);
-//   * the second-layer weight loads are software-pipelined by hand (second_layer_chunk16);
-//   * the issuer lane is a polling state machine per 128-env group (actor MMAs as two N = 128 halves with their
-//     own commit barriers, the critic's N = 256 MMAs as soon as the actor columns are read out), so the groups are
-//     independent (option tc_stagger delays group 1's start so that one group's second layer would run beside the
-//     other group's env step; measured: no effect on the step time, default 0).
-// The critic sums its 256 products in the order of the other kernels (same value bits); the logits are the sum of two
-// 128-unit partial chains, so they differ from the other kernels' in the last bits.
-// (Second-layer weights from the constant bank as uniform LDCU operands were measured too: 65 cycles per hidden
-// unit instead of 27 — the uniform load path delivers one 8-byte operand per ~12 cycles per scheduler.)
 // Two hidden units (h0, h1) of the actor through the 256 -> 9 layer: w = their ten weight pairs as five float4
 // ([unit][5] float2 layout), L[q] = logits (2q, 2q + 1).
 __device__ __forceinline__ void second_layer_pair(float h0, float h1, const float4 (&w)[5], float2 (&L)[5]) {
@@ -468,349 +216,25 @@ __device__ __forceinline__ void second_layer_pair(float h0, float h1, const floa
     L[4] = __ffma2_rn(make_float2(h1, h1), make_float2(w[4].z, w[4].w), L[4]);
 }
 
-// Sixteen hidden units (TMEM columns already in v, weights at shared address a = [unit][5] float2).  Two hidden units
-// = five 16-byte weight loads + ten FFMA2.  Left to itself the compiler issues each load right before its first use
-// (one load in flight: 30 cycles of shared-memory latency per two FFMA2, 71 cycles per hidden unit measured); here
-// the loads of the NEXT pair are issued — as ordered volatile loads — before the current pair is consumed.
-__device__ __forceinline__ void second_layer_chunk16(uint32_t a, const float (&v)[16], float2 (&L)[5]) {
-    float4 wa[5], wb[5];
-#pragma unroll
-    for (int r = 0; r < 5; ++r) wa[r] = tc::lds128(a + 16u * r);
-#pragma unroll
-    for (int i = 0; i < 8; i += 2) {
-#pragma unroll
-        for (int r = 0; r < 5; ++r) wb[r] = tc::lds128(a + 80u * (i + 1) + 16u * r);
-        second_layer_pair(fmaxf(v[2 * i], 0.0f), fmaxf(v[2 * i + 1], 0.0f), wa, L);
-        if (i + 2 < 8) {
-#pragma unroll
-            for (int r = 0; r < 5; ++r) wa[r] = tc::lds128(a + 80u * (i + 2) + 16u * r);
-        }
-        second_layer_pair(fmaxf(v[2 * i + 2], 0.0f), fmaxf(v[2 * i + 3], 0.0f), wb, L);
-    }
-}
-
-#ifdef CARENV_TC2_PROF          // per-phase cycle counts of one environment / policy thread (kernel tuning builds only)
-#define TC2_T(i) do { const long long now_ = clock64(); prof_[i] += now_ - last_; last_ = now_; } while (0)
-#else
-#define TC2_T(i) do { } while (0)
-#endif
-template <int U>
-__global__ void __launch_bounds__(2 * 256 + 32, 1)
-k_policy_rollout_tc2(const __grid_constant__ TrackParams P, const Tables G, const float *__restrict__ weights,
-                     int n_envs, int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
-                     double2 *__restrict__ pos, double2 *__restrict__ vel, int4 *__restrict__ ints,
-                     float *__restrict__ cur_obs, float *__restrict__ cur_term, float *__restrict__ cur_trunc,
-                     double reward_scale, float *__restrict__ obs_buf, float *__restrict__ act_buf,
-                     float *__restrict__ rew_buf, float *__restrict__ val_buf, float *__restrict__ term_buf,
-                     float *__restrict__ trunc_buf, float *__restrict__ logp_buf, float *__restrict__ last_val,
-                     float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode,
-                     int stagger_cycles) {
-    constexpr int kGroups = 2, kCols = 256, kHalf = 128, kEnvThreads = kGroups * 128;
-    extern __shared__ __align__(16) unsigned char smem[];
-    // [tables | pad to a 128-byte boundary | weights | A tiles (hi, lo per group) | logits [group][128][12]]
-    const int w_off = (int)((tc::smem_u32(smem) + (uint32_t)table_bytes + 127u) / 128u * 128u - tc::smem_u32(smem));
-    float *sw = reinterpret_cast<float *>(smem + w_off);
-    unsigned char *sA = smem + w_off + ((kTcWeightFloats * 4 + 127) / 128 * 128);
-    float *s_logit = reinterpret_cast<float *>(sA + kGroups * 2 * tc::kABytes);
-    __shared__ __align__(8) unsigned long long mb_rows[kGroups], mb_full_lo[kGroups], mb_full_hi[kGroups],
-        mb_cons_a[kGroups], mb_full_c[kGroups], mb_cons_c[kGroups], mb_logit[kGroups];
-    __shared__ uint32_t tmem_slot;
-    // the warp index through a shuffle: the compiler then knows that it — and every role branch below — is warp-uniform
-    const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-    for (int i = tid; i < kTcWeightFloats / 4; i += blockDim.x)
-        reinterpret_cast<float4 *>(sw)[i] = reinterpret_cast<const float4 *>(weights)[i];
-    if (tid == 0)
-        for (int g = 0; g < kGroups; ++g) {
-            tc::mbar_init(tc::smem_u32(&mb_rows[g]), 128);
-            tc::mbar_init(tc::smem_u32(&mb_full_lo[g]), 1);
-            tc::mbar_init(tc::smem_u32(&mb_full_hi[g]), 1);
-            tc::mbar_init(tc::smem_u32(&mb_cons_a[g]), 256);
-            tc::mbar_init(tc::smem_u32(&mb_full_c[g]), 1);
-            tc::mbar_init(tc::smem_u32(&mb_cons_c[g]), 128);
-            tc::mbar_init(tc::smem_u32(&mb_logit[g]), 128);
-        }
-    if (warp == 0) tc::tmem_alloc<512>(&tmem_slot);
-    const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
-    tc::fence_async_smem();
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tbase = tmem_slot;
-    const int n_forward = n_steps + (last_val ? 1 : 0);
-
-    if (warp == 2 * kEnvThreads / 32) {
-        // ===== MMA issuer (one lane): a polling state machine per group, so the groups never wait for each other =====
-        if ((tid & 31) == 0) {
-            const uint32_t sB = tc::smem_u32(sw);
-            const uint32_t idesc_half = tc::make_idesc_tf32(128, kHalf), idesc_full = tc::make_idesc_tf32(128, kCols);
-            int f[kGroups] = {0, 0}, stage[kGroups] = {0, 0};
-            int open = n_forward > 0 ? kGroups : 0;
-            auto issue = [&](uint32_t d, uint32_t ah, uint32_t bh, uint32_t idesc) {     // D = Ah*Bh + Al*Bh + Ah*Bl
-                const uint32_t al = ah + tc::kABytes, bl = bh + (uint32_t)(kTcBFloats * 4);
-#pragma unroll
-                for (int pr = 0; pr < 3; ++pr) {
-                    const uint32_t a0 = (pr == 1) ? al : ah, b0 = (pr == 2) ? bl : bh;
-#pragma unroll
-                    for (int ks = 0; ks < tc::kK / 8; ++ks)
-                        tc::mma_tf32(d, tc::make_smem_desc(a0 + ks * 2 * tc::kLBO), tc::make_smem_desc(b0 + ks * 2 * tc::kLBO),
-                                     idesc, (pr | ks) != 0);
-                }
-            };
-            for (long long spin = 0; open > 0; ++spin) {
-                if (spin > (1ll << 28)) __trap();                    // a protocol error must not hang the GPU box
-#pragma unroll
-                for (int g = 0; g < kGroups; ++g) {
-                    if (f[g] == n_forward) continue;
-                    const uint32_t par = (uint32_t)(f[g] & 1);
-                    const uint32_t ah = tc::smem_u32(sA + g * 2 * tc::kABytes);
-                    const uint32_t d = tbase + (uint32_t)(g * kCols);
-                    if (stage[g] == 0) {
-                        // this pass's operand rows are written and the previous pass's critic columns are read out
-                        if (!tc::mbar_test(tc::smem_u32(&mb_rows[g]), par)) continue;
-                        if (f[g] > 0 && !tc::mbar_test(tc::smem_u32(&mb_cons_c[g]), par ^ 1u)) continue;
-                        tc::tc_fence_after();
-                        issue(d, ah, sB, idesc_half);                                        // actor units 0..127
-                        tc::mma_commit(tc::smem_u32(&mb_full_lo[g]));
-                        issue(d + kHalf, ah, sB + (uint32_t)((kHalf / 8) * tc::kSBO), idesc_half);   // actor units 128..255
-                        tc::mma_commit(tc::smem_u32(&mb_full_hi[g]));
-                        stage[g] = 1;
-                    } else {
-                        if (!tc::mbar_test(tc::smem_u32(&mb_cons_a[g]), par)) continue;      // the actor columns are read out
-                        tc::tc_fence_after();
-                        issue(d, ah, sB + (uint32_t)(2 * kTcBFloats * 4), idesc_full);       // critic, 256 units
-                        tc::mma_commit(tc::smem_u32(&mb_full_c[g]));
-                        stage[g] = 0;
-                        if (++f[g] == n_forward) --open;
-                    }
-                }
-            }
-        }
-    } else {
-        const bool policy = warp >= kEnvThreads / 32;
-        const int lt = policy ? tid - kEnvThreads : tid;
-        const int group = lt >> 7, row = lt & 127;
-        const int e_raw = blockIdx.x * kEnvThreads + lt;
-        const bool active = e_raw < n_envs;
-        const int e = active ? e_raw : n_envs - 1;           // idle threads shadow the last env (no stores)
-        float *my_logit = s_logit + (size_t)(group * 128 + row) * 12;
-        const uint32_t my_tmem = tbase + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(group * kCols);
-        const uint32_t w2s = tc::smem_u32(sw + kTcW2Off);            // [unit][5] float2 pairs
-        const uint32_t b_cons_a = tc::smem_u32(&mb_cons_a[group]);
-        const uint32_t b_logit = tc::smem_u32(&mb_logit[group]), b_full_c = tc::smem_u32(&mb_full_c[group]);
-
-        if (policy) {
-            // ===== policy threads: the second layers of both nets for the environment on this TMEM lane =====
-            // The per-thread allocation of a 17-warp CTA is 96 registers (five warps on one scheduler's file); the
-            // policy threads take 80 (two pairs of hidden units' weights in flight), the environment threads get 112.
-            asm volatile("setmaxnreg.dec.sync.aligned.u32 80;\n");
-            const uint32_t b_full_hi = tc::smem_u32(&mb_full_hi[group]), b_cons_c = tc::smem_u32(&mb_cons_c[group]);
-            const float *tail = sw + kTcTailOff;
-            const float4 *wc = reinterpret_cast<const float4 *>(sw + kTcW2cOff);
-#ifdef CARENV_TC2_PROF
-            long long prof_[8] = {0, 0, 0, 0, 0, 0, 0, 0}, last_ = clock64();
-#endif
-            for (int f = 0; f < n_forward; ++f) {
-                const uint32_t par = (uint32_t)(f & 1);
-                float2 L[5];
-#pragma unroll
-                for (int q = 0; q < 5; ++q) L[q] = make_float2(0.0f, 0.0f);
-                tc::mbar_wait(b_full_hi, par);
-                tc::tc_fence_after();
-                TC2_T(0);
-#pragma unroll 1
-                for (int c = kHalf; c < kCols; c += 16) {               // hidden units 128..255
-                    float v[16];
-                    tc::tmem_ld16(my_tmem + c, v);
-                    if (c + 16 == kCols) { tc::tc_fence_before(); tc::mbar_arrive(b_cons_a); }   // this half is read out
-                    second_layer_chunk16(w2s + (uint32_t)c * 40u, v, L);
-                }
-                reinterpret_cast<float4 *>(my_logit)[0] = make_float4(L[0].x, L[0].y, L[1].x, L[1].y);
-                reinterpret_cast<float4 *>(my_logit)[1] = make_float4(L[2].x, L[2].y, L[3].x, L[3].y);
-                reinterpret_cast<float2 *>(my_logit)[4] = L[4];
-                tc::mbar_arrive(b_logit);                            // release: the partial logits are visible
-                TC2_T(1);
-                tc::mbar_wait(b_full_c, par);
-                tc::tc_fence_after();
-                TC2_T(2);
-                float2 V = make_float2(0.0f, 0.0f);
-#pragma unroll 1
-                for (int c = 0; c < kCols; c += 16) {
-                    float v[16];
-                    tc::tmem_ld16(my_tmem + c, v);
-                    if (c + 16 == kCols) { tc::tc_fence_before(); tc::mbar_arrive(b_cons_c); }
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float4 w = wc[c / 4 + i];
-                        V = __ffma2_rn(make_float2(fmaxf(v[4 * i], 0.0f), fmaxf(v[4 * i + 1], 0.0f)), make_float2(w.x, w.y), V);
-                        V = __ffma2_rn(make_float2(fmaxf(v[4 * i + 2], 0.0f), fmaxf(v[4 * i + 3], 0.0f)), make_float2(w.z, w.w), V);
-                    }
-                }
-                const float value = (V.x + V.y) + tail[10];
-                if (active) {
-                    if (f < n_steps) val_buf[(size_t)f * (size_t)n_envs + (size_t)e] = value;
-                    else last_val[e] = value;                        // bootstrap value of the final observation
-                }
-                TC2_T(3);
-            }
-#ifdef CARENV_TC2_PROF
-            if (blockIdx.x == 0 && lt == 0)
-                printf("tc2 policy thread cycles/step: wait_actor %lld actor %lld wait_critic %lld critic %lld\n",
-                       prof_[0] / n_forward, prof_[1] / n_forward, prof_[2] / n_forward, prof_[3] / n_forward);
-#endif
-        } else {
-            // ===== environment threads =====
-            asm volatile("setmaxnreg.inc.sync.aligned.u32 112;\n");
-            unsigned char *myA = sA + group * 2 * tc::kABytes;   // hi tile, then lo tile
-            const uint32_t b_rows = tc::smem_u32(&mb_rows[group]), b_full_lo = tc::smem_u32(&mb_full_lo[group]);
-            const float *tail = sw + kTcTailOff;
-            EnvState s;
-            {
-                const double2 p = pos[e], v = vel[e];
-                const int4 q = ints[e];
-                s.px = p.x; s.py = p.y; s.vx = v.x; s.vy = v.y;
-                s.k = q.x; s.t = q.y; s.next_gate = q.z; s.passed = q.w;
-            }
-            float obs[kObsDim];
-            {
-                const float2 *src = reinterpret_cast<const float2 *>(cur_obs + (size_t)e * kObsDim);
-#pragma unroll
-                for (int i = 0; i < kObsDim / 2; ++i) { const float2 v = src[i]; obs[2 * i] = v.x; obs[2 * i + 1] = v.y; }
-            }
-            float tc_ = cur_term[e], uc = cur_trunc[e];
-            const uint32_t gid = (uint32_t)(env_offset + e);
-
-            // operand row of pass f: obs | 1 | 0...  split into TF32 hi and lo
-            auto write_row = [&](int f) {
-                if (f > 0) tc::mbar_wait(b_full_c, (uint32_t)((f - 1) & 1));   // the previous pass's MMAs have read the tile
-#pragma unroll
-                for (int c = 0; c < tc::kKChunks; ++c) {
-                    float hi[4], lo[4];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const int k = 4 * c + j;
-                        const float x = k < kObsDim ? obs[k < kObsDim ? k : 0] : (k == kObsDim ? 1.0f : 0.0f);
-                        hi[j] = tc::to_tf32(x);
-                        lo[j] = tc::to_tf32(x - hi[j]);
-                    }
-                    const int off = tc::operand_offset(row, 4 * c);
-                    *reinterpret_cast<float4 *>(myA + off) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<float4 *>(myA + tc::kABytes + off) = make_float4(lo[0], lo[1], lo[2], lo[3]);
-                }
-                tc::fence_async_smem();
-                tc::mbar_arrive(b_rows);
-            };
-
-            if (group == 1 && stagger_cycles > 0) {                  // tuning hook (see the header)
-                const long long t0 = clock64();
-                while (clock64() - t0 < (long long)stagger_cycles) { }
-            }
-#ifdef CARENV_TC2_PROF
-            long long prof_[8] = {0, 0, 0, 0, 0, 0, 0, 0}, last_ = clock64();
-#endif
-            for (int t = 0; t < n_steps; ++t) {
-                const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
-                write_row(t);
-                TC2_T(0);
-                // Philox and the Buffer rows that do not depend on the action, while the tensor core and the policy thread work
-                const unsigned long long gs = step0 + (unsigned long long)t;
-                const uint32_t bits = philox_uniform_bits((uint32_t)seed, (uint32_t)(seed >> 32), gid, (uint32_t)gs,
-                                                          (uint32_t)(gs >> 32), 0x43415245u);
-                const float u = (float)(bits >> 8) * (1.0f / 16777216.0f);
-                if (active) {
-                    if (obs_mode == kObsPose) {
-                        store_pose(reinterpret_cast<PoseRec *>(obs_buf) + idx, s, obs[2], obs[3]);
-                    } else {
-                        float2 *dst = reinterpret_cast<float2 *>(obs_buf + idx * kObsDim);
-#pragma unroll
-                        for (int i = 0; i < kObsDim / 2; ++i) dst[i] = make_float2(obs[2 * i], obs[2 * i + 1]);
-                    }
-                    term_buf[idx] = tc_;
-                    trunc_buf[idx] = uc;
-                    if (u_dbg) u_dbg[idx] = u;
-                }
-                TC2_T(1);
-                float2 L[5];
-#pragma unroll
-                for (int q = 0; q < 5; ++q) L[q] = make_float2(0.0f, 0.0f);
-                tc::mbar_wait(b_full_lo, (uint32_t)(t & 1));
-                tc::tc_fence_after();
-#pragma unroll 1
-                for (int c = 0; c < kHalf; c += 16) {                   // hidden units 0..127
-                    float v[16];
-                    tc::tmem_ld16(my_tmem + c, v);
-                    if (c + 16 == kHalf) { tc::tc_fence_before(); tc::mbar_arrive(b_cons_a); }   // this half is read out
-                    second_layer_chunk16(w2s + (uint32_t)c * 40u, v, L);
-                }
-                TC2_T(5);
-                tc::mbar_wait(b_logit, (uint32_t)(t & 1));           // acquire: the policy thread's partial logits
-                TC2_T(2);
-                PolicyOut po;
-                {
-                    const float4 p0 = reinterpret_cast<const float4 *>(my_logit)[0], p1 = reinterpret_cast<const float4 *>(my_logit)[1];
-                    const float2 p2 = reinterpret_cast<const float2 *>(my_logit)[4];
-                    po.logit[0] = (L[0].x + p0.x) + tail[0]; po.logit[1] = (L[0].y + p0.y) + tail[1];
-                    po.logit[2] = (L[1].x + p0.z) + tail[2]; po.logit[3] = (L[1].y + p0.w) + tail[3];
-                    po.logit[4] = (L[2].x + p1.x) + tail[4]; po.logit[5] = (L[2].y + p1.y) + tail[5];
-                    po.logit[6] = (L[3].x + p1.z) + tail[6]; po.logit[7] = (L[3].y + p1.w) + tail[7];
-                    po.logit[8] = (L[4].x + p2.x) + tail[8]; po.logit[9] = (L[4].y + p2.y) + tail[9];
-                    po.value = 0.0f;
-                }
-                float logp, us;
-                const int a = sample_action(po, u, logp, us);
-                if (active) {
-                    act_buf[idx] = (float)a;
-                    logp_buf[idx] = logp;
-                }
-                TC2_T(3);
-                StepResult o;
-                env_step<U>(s, a, reward_scale, P, T, o, active ? stats : nullptr);
-                if (active) rew_buf[idx] = o.reward;
-#pragma unroll
-                for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];
-                tc_ = o.terminated ? 1.0f : 0.0f;
-                uc = o.truncated ? 1.0f : 0.0f;
-                TC2_T(4);
-            }
-#ifdef CARENV_TC2_PROF
-            if (blockIdx.x == 0 && lt == 0)
-                printf("tc2 env thread cycles/step: row %lld philox+stores %lld wait+actor_lo %lld wait_partial %lld sample %lld env_step %lld\n",
-                       prof_[0] / n_steps, prof_[1] / n_steps, prof_[5] / n_steps, prof_[2] / n_steps, prof_[3] / n_steps, prof_[4] / n_steps);
-#endif
-            if (last_val) {                                          // one more pass: the policy thread writes the bootstrap value
-                write_row(n_steps);
-                tc::mbar_wait(b_full_lo, (uint32_t)(n_steps & 1));
-                tc::tc_fence_before();
-                tc::mbar_arrive(b_cons_a);
-            }
-            if (active) {
-                pos[e] = make_double2(s.px, s.py);
-                vel[e] = make_double2(s.vx, s.vy);
-                ints[e] = make_int4(s.k, s.t, s.next_gate, s.passed);
-                float2 *dst = reinterpret_cast<float2 *>(cur_obs + (size_t)e * kObsDim);
-#pragma unroll
-                for (int i = 0; i < kObsDim / 2; ++i) dst[i] = make_float2(obs[2 * i], obs[2 * i + 1]);
-                cur_term[e] = tc_;
-                cur_trunc[e] = uc;
-            }
-        }
-    }
-    tc::tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tc::tmem_dealloc<512>(tbase);
-}
-
 // ---- fused rollout, tensor cores, every second-layer weight load shared by TWO environments --------------------
-// ncu of k_policy_rollout_tc2 (profiles/r2_policy_tc2_ncu.txt): the 256 -> 9 layer is bound by the shared-memory
-// RETURN path — a broadcast LDS.128 delivers 16 bytes to 32 lanes in two wavefronts, i.e. the weights of ONE packed
-// FFMA2 per cycle and SM, half of what the FMA pipes take — and all warps run that phase together because their
-// MMAs complete together (the pipe is ~100 % busy for 11k of a step's 29k cycles, 41 % on average).  Here every
-// weight load feeds two environments: the environment thread of lane r in group 0 runs hidden units 0..127 for
-// BOTH environments on TMEM lane r (group 0's and group 1's columns), its twin in group 1 runs units 128..255 for
-// both, and the two exchange the partial logits of each other's environment through shared memory.  The critic is
-// done by 128 critic threads, lane r for both environments of the lane as well, off the critical path.  One CTA =
-// 256 environment threads + 128 critic threads + the issuer warp (13 warps, 128 registers each at launch; the critic
-// warps hand 64 of theirs to the environment warps).  Logits = (units 0..127) + (units 128..255) + bias, the order
-// of k_policy_rollout_tc2: bit-identical to it; values bit-identical to every other kernel.
+// Same contract as k_policy_rollout.  Per step every environment thread writes its observation row (hi/lo TF32 split,
+// a constant 1 in column 18 carries the bias) into the K-major UMMA operand tile of its 128-env group, one elected
+// thread issues tcgen05.mma kind::tf32 — D = A_hi*B_hi + A_lo*B_hi + A_hi*B_lo (3xTF32: float32-level accuracy) — into
+// tensor memory, and the threads read their rows of pre-activations back with tcgen05.ld and run ReLU and the second
+// layers on the CUDA cores (FFMA2).
+// The 256 -> 9 layer is bound by the shared-memory RETURN path (ncu, DESIGN.md §7 "Round 2"): a broadcast
+// LDS.128 delivers 16 bytes to 32 lanes in two wavefronts, i.e. the weights of ONE packed FFMA2 per cycle and SM, half
+// of what the FMA pipes take — and all warps run that phase together because their MMAs complete together (with one
+// environment per weight load the pipe is ~100 % busy for 11k of a step's 29k cycles).  So here every weight load
+// feeds two environments: the environment thread of lane r in group 0 runs hidden units 0..127 for BOTH environments
+// on TMEM lane r (group 0's and group 1's columns), its twin in group 1 runs units 128..255 for both, and the two
+// exchange the partial logits of each other's environment through shared memory.  The loads are software-pipelined
+// by hand (the next pair of hidden units' weights in flight as ordered volatile loads; left to itself the compiler
+// issues each load right before its first use).  The critic is done by 128 critic threads, lane r for both
+// environments of the lane as well, off the critical path.  One CTA = 256 environment threads + 128 critic threads +
+// the issuer warp (13 warps, 128 registers each at launch; the critic warps hand 64 of theirs to the environment
+// warps).  Logits = (units 0..127) + (units 128..255) + bias, the same operands in the same order on both threads of
+// a lane; value = (even units + odd units) + bias.
 __device__ __forceinline__ void second_layer_chunk16_x2(uint32_t a, const float (&va)[16], const float (&vb)[16],
                                                         float2 (&La)[5], float2 (&Lb)[5]) {
     float4 wa[5], wb[5];

@@ -81,17 +81,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t mbar_smem, uint32_t parity) {
     __trap();
 }
 
-// One non-blocking probe of a phase (for an issuer that serves several independent groups).
-__device__ __forceinline__ bool mbar_test(uint32_t mbar_smem, uint32_t parity) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"     // test_wait never suspends the thread
-        "selp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(done) : "r"(mbar_smem), "r"(parity) : "memory");
-    return done != 0;
-}
-
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }

@@ -200,8 +200,8 @@ def train(args) -> list[dict]:
         # small shards (the reference's 24 environments): one warp per environment, parameters read in place
         warp_rollout = (not args.fused_cuda_cores and n <= WARP_ROLLOUT_MAX_ENVS and len(envs.track.walls) <= 32)
 
-        # tensor-core kernel (256- or 512-environment CTAs, chosen by the library from the shard size); it is also
-        # the faster one for tiny shards (24 envs: 12.7 vs 14.4 us per step, benchmarks/fused_rollout.py)
+        # otherwise the tensor-core kernel (k_policy_rollout_tc3, 256-environment CTAs), or the CUDA-core kernel with
+        # --fused-cuda-cores
         pack_policy = pack_policy_weights_tc if not args.fused_cuda_cores else pack_policy_weights
         packed = pack_policy(agent.actor, agent.critic)
         last_val = torch.empty(n, device=dev)

@@ -26,6 +26,12 @@ Files written:
                        one trajectory group ("destroyed") in the layout above
   agent_checkpoint.npz a state dict of lib/model.py:Agent (seeded init) and its
                        log-probability, entropy and value on fixed inputs
+  fused_tc3.npz        NOT from the reference: `python tests/golden/make_golden.py
+                       fused_tc3` on a GPU records a fused rollout of this
+                       repository's tensor-core kernel (k_policy_rollout_tc3)
+                       with the agent_checkpoint.npz weights, so that
+                       tests/test_fused_rollout.py can require the same bits
+                       from every later build
   ../../ppo_car_b200/tracks/<track>.json   the two track files (input data in the
                        reference's schema; BASELINE.json names them as workloads)
 """
@@ -182,6 +188,43 @@ def make_agent(from_port: bool) -> None:
                         logp=logp.numpy(), entropy=ent.numpy(), value=val.numpy(), source=np.array(source), **out)
 
 
+FUSED_TC3 = dict(n_envs=300, n_steps=64, seed=21, step0=7)   # one full 256-env CTA and a ragged one
+
+
+def fused_tc3_rollout(tc_tiles: int = 0) -> dict:
+    """The rollout pinned by fused_tc3.npz: the agent_checkpoint.npz network on big_track through
+    ppo_car_b200.fused_rollout (tensor-core packing), with the handle option tc_tiles set to `tc_tiles`."""
+    import torch
+
+    import ppo_car_b200
+    from ppo_car_b200.train_ppo import ActorCritic
+
+    dev = torch.device("cuda")
+    ck = np.load(os.path.join(HERE, "agent_checkpoint.npz"))
+    net = ActorCritic(18, 9).to(dev)
+    net.load_state_dict({k[2:]: torch.from_numpy(ck[k]) for k in ck.files if k.startswith("w_")})
+    n, T = FUSED_TC3["n_envs"], FUSED_TC3["n_steps"]
+    env = ppo_car_b200.VecCarEnv(n, ppo_car_b200.builtin_track("big_track"), reward_scaling=0.1, float_flags=True)
+    env.set_option("tc_tiles", tc_tiles)
+    buf = ppo_car_b200.Buffer((18,), T, n, dev)
+    cur_obs = env.reset()[0].clone()
+    cur_term, cur_trunc, last_val = (torch.zeros(n, device=dev), torch.zeros(n, device=dev),
+                                     torch.empty(n, device=dev))
+    packed = ppo_car_b200.pack_policy_weights_tc(net.actor, net.critic)
+    ppo_car_b200.fused_rollout(env, packed, buf, cur_obs, cur_term, cur_trunc, seed=FUSED_TC3["seed"],
+                               step0=FUSED_TC3["step0"], last_val=last_val)
+    torch.cuda.synchronize()
+    return dict(act_buf=buf.act_buf.to(torch.uint8).cpu().numpy(), logprob_buf=buf.logprob_buf.cpu().numpy(),
+                val_buf=buf.val_buf.cpu().numpy(), rew_buf=buf.rew_buf.cpu().numpy(),
+                last_val=last_val.cpu().numpy(), cur_obs=cur_obs.cpu().numpy())
+
+
+def make_fused_tc3() -> None:
+    out = fused_tc3_rollout()
+    np.savez_compressed(os.path.join(HERE, "fused_tc3.npz"),
+                        source=np.array("ppo_car_b200.fused_rollout: k_policy_rollout_tc3"), **out)
+
+
 if __name__ == "__main__":
     from_port = "--from-port" in sys.argv
     which = [w for w in sys.argv[1:] if w != "--from-port"] or ["track", "big_track", "gae", "near_wall", "agent"]
@@ -192,6 +235,8 @@ if __name__ == "__main__":
             make_near_wall(from_port)
         elif w == "agent":
             make_agent(from_port)
+        elif w == "fused_tc3":
+            make_fused_tc3()
         else:
             make_track(w)
     print("done")

@@ -28,12 +28,10 @@ def test_pack_layout_matches_header_constants():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n,tensor_cores", [(24, False), (1000, False), (24, 2), (1000, 2), (1000, 4), (2049, 4),
-                                            (1300, 2), (24, 3), (1000, 3), (1300, 3), (24, 5), (1000, 5), (1300, 5)])
+@pytest.mark.parametrize("n,tensor_cores", [(24, False), (1000, False), (24, 5), (1000, 5), (1300, 5), (2049, 5)])
 def test_fused_rollout_matches_torch_policy_and_env_kernel(tracks_dir, n, tensor_cores):
-    """tensor_cores: False = CUDA-core kernel, 2 / 4 = tensor-core kernel with that many 128-env groups per CTA,
-    3 = two groups with a policy thread per environment (k_policy_rollout_tc2), 5 = weight loads shared by the two
-    environments of a TMEM lane (k_policy_rollout_tc3)."""
+    """tensor_cores: False = CUDA-core kernel (k_policy_rollout), 5 = tensor-core kernel (k_policy_rollout_tc3, option
+    tc_tiles 5).  2049 envs leave one environment in the last 256-env CTA."""
     dev = torch.device("cuda")
     path = os.path.join(tracks_dir, "big_track.json")
     T = 300
@@ -155,30 +153,20 @@ def test_warp_per_environment_fused_rollout(tracks_dir, n, track_name):
 
 
 @pytest.mark.gpu
-def test_two_thread_kernels_agree_bit_for_bit(tracks_dir):
-    """k_policy_rollout_tc2 and k_policy_rollout_tc3 sum the logits in the same order ((units 0..127) + (units
-    128..255) + bias) and the values in the order of every other kernel: identical rollouts, bit for bit; the
-    values also equal the 4-group kernel's."""
-    dev = torch.device("cuda")
-    path = os.path.join(tracks_dir, "big_track.json")
-    n, T = 1500, 200
-    torch.manual_seed(9)
-    net = ActorCritic(18, 9).to(dev)
-    packed = ppo_car_b200.pack_policy_weights_tc(net.actor, net.critic)
-    res = {}
-    for tiles in (3, 5, 4):
-        env = ppo_car_b200.VecCarEnv(n, path, reward_scaling=0.1, float_flags=True)
-        env.set_option("tc_tiles", tiles)
-        buf = ppo_car_b200.Buffer((18,), T, n, dev)
-        o = env.reset()[0].clone()
-        z1, z2, lv = torch.zeros(n, device=dev), torch.zeros(n, device=dev), torch.empty(n, device=dev)
-        ppo_car_b200.fused_rollout(env, packed, buf, o, z1, z2, seed=4, step0=0, last_val=lv)
-        res[tiles] = (buf.obs_buf.clone(), buf.act_buf.clone(), buf.logprob_buf.clone(), buf.val_buf.clone(),
-                      buf.rew_buf.clone(), lv.clone(), o.clone())
-    for a, b in zip(res[3], res[5]):
-        assert torch.equal(a, b)
-    # the 4-group kernel: same values wherever the trajectories have not diverged yet (step 0 at least)
-    assert torch.equal(res[3][3][0], res[4][3][0])
+def test_tensor_core_rollout_reproduces_pinned_bits(golden_dir):
+    """k_policy_rollout_tc3 against tests/golden/fused_tc3.npz (one full 256-env CTA and a ragged one, 64 steps,
+    bootstrap values): actions, log-probabilities, values, rewards, last values and final observations bit for bit.
+    Option tc_tiles 0 and 5 select this kernel; 2, 3 and 4 named kernels that have been removed and are refused."""
+    from tests.golden.make_golden import fused_tc3_rollout
+
+    ref = np.load(os.path.join(golden_dir, "fused_tc3.npz"))
+    for tiles in (0, 5):
+        got = fused_tc3_rollout(tiles)
+        for k, v in got.items():
+            assert v.dtype == ref[k].dtype and np.array_equal(v, ref[k]), (tiles, k)
+    for tiles in (2, 3, 4):
+        with pytest.raises(ppo_car_b200.CarEnvError, match="removed"):
+            fused_tc3_rollout(tiles)
 
 
 @pytest.mark.gpu
