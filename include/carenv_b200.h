@@ -225,7 +225,9 @@ int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs,
 /* Tensor-core variant of the fused rollout: the two 18->256 layers run as tcgen05.mma kind::tf32 (3xTF32
  * split, float32-level accuracy) with accumulators in tensor memory; same arguments and results (to float32
  * rounding of the network outputs) as carenv_policy_rollout.  packed_weights: device
- * float[carenv_policy_weights_floats_tc()] from ppo_car_b200.policy.pack_policy_weights_tc. */
+ * float[carenv_policy_weights_floats_tc()] from ppo_car_b200.policy.pack_policy_weights_tc.  On tracks whose
+ * denominator table does not fit next to the weights in 227 KB of shared memory (above about 80 wall segments) it
+ * computes the denominators instead, so every track of up to 128 segments with few enough gates runs. */
 int carenv_policy_weights_floats_tc(void);
 int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
                              unsigned long long seed, unsigned long long step0, double *pos, double *vel,

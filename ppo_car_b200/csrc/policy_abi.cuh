@@ -200,6 +200,7 @@ int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs,
     if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
     const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
     const size_t smem = (size_t)table_bytes + sizeof(float) * kPolicyFloats;
+    if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the CUDA-core rollout kernel");
     const int grid = (n_envs + kPolicyBlock - 1) / kPolicyBlock;
     int U = h->force_generic ? 1 : h->host.P.unroll4;   // the fused kernels are instantiated for 4, 2, 1
     if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
@@ -287,12 +288,15 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
     const int table_bytes = (int)h->smem_bytes;
     int U = h->force_generic ? 1 : h->host.P.unroll4;
     if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
-    const bool tab = U >= 2 && h->d_den4 && h->tab >= 0;    // denominators from a (row-skewed) table in shared memory
     const int n_pairs = h->host.n_pairs;
     const int row_f4 = ((n_pairs + 7) / 8 * 8) | 1;         // odd number of 16-byte units: rows skewed by one bank group
-    const size_t smem = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
-                        (size_t)2 * 2 * tc::kABytes + (size_t)2 * 128 * 12 * sizeof(float) +
-                        (tab ? (size_t)kHeadings * row_f4 * 16 : 0);
+    const size_t smem_base = (size_t)table_bytes + 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) +
+                             (size_t)2 * 2 * tc::kABytes + (size_t)2 * 128 * 12 * sizeof(float);
+    const size_t tab_bytes = (size_t)kHeadings * row_f4 * 16;
+    // denominators from a (row-skewed) table in shared memory where it fits (tracks of up to about 80 segments);
+    // otherwise the arithmetic instantiation of the same U, which gives the same results
+    const bool tab = U >= 2 && h->d_den4 && h->tab >= 0 && smem_base + tab_bytes <= 227 * 1024;
+    const size_t smem = smem_base + (tab ? tab_bytes : 0);
     if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
     const int grid = (n_envs + 255) / 256;
     auto launch = [&](auto kern) -> int {
