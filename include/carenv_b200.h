@@ -297,6 +297,29 @@ int carenv_policy_eval(void *handle, const float *w1_actor, const float *b1_acto
                        unsigned long long seed, carenv_eval_record *records, int n_trace, unsigned char *trace_actions,
                        float *trace_u, void *stream);
 
+/* Several tracks in the fused rollout and in policy evaluation, one launch each.  `multi` is a multi-track handle
+ * (carenv_multi_create); every track of it must have at most 128 wall segments (CARENV_E_TRACK otherwise).  Track ids
+ * outside 0..n_tracks - 1 are clamped as in carenv_multi_rollout.  Each call reads the tracks' segment counts from the
+ * handle with one small copy that synchronises with `stream`.
+ *   carenv_policy_rollout_tc_multi   carenv_policy_rollout_tc with environment e on track track_ids[e] (device int32
+ *       [n_envs]); the random stream is keyed by the global env id as before, so every environment's rows are
+ *       bit-identical to carenv_policy_rollout_tc on its track alone.  obs_buf always holds [n_steps][n_envs][18]
+ *       observations: pose records do not carry a track.
+ *   carenv_policy_eval_multi   carenv_policy_eval with episode i of the call on track episode_tracks[i] (device int32
+ *       [n_episodes]); each episode starts from its track's start pose, and its record equals the one
+ *       carenv_policy_eval gives for the same id on that track alone. */
+int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const float *packed_weights, int n_envs,
+                                   int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                                   double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                   float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                   float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf, float *logp_buf,
+                                   float *last_val, float *u_dbg, void *stream);
+int carenv_policy_eval_multi(void *multi, const int32_t *episode_tracks, const float *w1_actor, const float *b1_actor,
+                             const float *w2_actor, const float *b2_actor, long long n_episodes,
+                             unsigned long long episode0, int greedy, unsigned long long seed,
+                             carenv_eval_record *records, int n_trace, unsigned char *trace_actions, float *trace_u,
+                             void *stream);
+
 /* All minibatch updates of one PPO epoch in ONE persistent cooperative launch (csrc/ppo_epoch.cuh; replaces the
  * loops of train.py:223-261 — `for _ in range(train_iters): for start in range(0, n_steps, batch_size): ...` — and,
  * with several GPUs, the gradient all-reduce between backward and optimizer.step()).

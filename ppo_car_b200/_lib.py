@@ -114,6 +114,10 @@ def lib():
     L.carenv_policy_rollout_tc.argtypes = L.carenv_policy_rollout.argtypes
     L.carenv_policy_eval.argtypes = [vp] * 5 + [C.c_longlong, C.c_ulonglong, i32, C.c_ulonglong, vp, i32, vp, vp, vp]
     L.carenv_policy_eval.restype = i32
+    L.carenv_policy_rollout_tc_multi.argtypes = [vp, vp] + L.carenv_policy_rollout_tc.argtypes[1:]
+    L.carenv_policy_rollout_tc_multi.restype = i32
+    L.carenv_policy_eval_multi.argtypes = [vp, vp] + L.carenv_policy_eval.argtypes[1:]
+    L.carenv_policy_eval_multi.restype = i32
     for name in ("carenv_create", "carenv_destroy", "carenv_reset_obs", "carenv_reset", "carenv_step",
                  "carenv_rollout", "carenv_rollout_poses", "carenv_observe", "carenv_step_host", "carenv_step_host_records", "carenv_step_records", "carenv_step_final", "carenv_multi_create", "carenv_multi_destroy", "carenv_multi_reset",
                  "carenv_multi_rollout", "carenv_render", "carenv_host_alloc", "carenv_host_free", "carenv_stats", "gae_reverse_scan", "carenv_bench_ffma", "carenv_set_option", "carenv_policy_rollout", "carenv_policy_rollout_tc"):

@@ -305,13 +305,63 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
             h->host.P, h->dev, packed_weights, n_envs, n_steps, env_offset, seed, step0,
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
             cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4);
+            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4,
+            nullptr, nullptr, 0, nullptr);
         CU(cudaGetLastError());
         return 0;
     };
     if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true>) : launch(k_policy_rollout_tc3<4, false>);
     if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true>) : launch(k_policy_rollout_tc3<2, false>);
     return launch(k_policy_rollout_tc3<1, false>);
+}
+
+/* Largest wall-segment count over the tracks of a multi-track handle: the handle keeps its TrackParams on the device
+ * only, so this is one small strided copy, synchronous with `stream`. */
+static int multi_max_seg(const MultiTrack *m, cudaStream_t stream, int *max_seg) {
+    std::vector<int> n_seg((size_t)m->n_tracks);
+    CU(cudaMemcpy2DAsync(n_seg.data(), sizeof(int), &m->d_params[0].n_seg, sizeof(TrackParams), sizeof(int),
+                         (size_t)m->n_tracks, cudaMemcpyDeviceToHost, stream));
+    CU(cudaStreamSynchronize(stream));
+    *max_seg = 0;
+    for (int v : n_seg) *max_seg = v > *max_seg ? v : *max_seg;
+    return 0;
+}
+
+/* carenv_policy_rollout_tc on several tracks (k_policy_rollout_tc3<0, false>): environment e runs on track
+ * track_ids[e] of the multi-track handle (clamped to 0..n_tracks - 1 as carenv_multi_rollout does). */
+int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const float *packed_weights, int n_envs,
+                                   int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                                   double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                   float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                   float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                   float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    MultiTrack *m = static_cast<MultiTrack *>(multi);
+    if (!m) return fail(CARENV_E_INVAL, "null handle");
+    if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
+    if (n_envs == 0) return 0;
+    if (!track_ids || !packed_weights || !pos || !vel || !ints || !cur_obs || !cur_term || !cur_trunc || !obs_buf ||
+        !act_buf || !rew_buf || !val_buf || !term_buf || !trunc_buf || !logp_buf)
+        return fail(CARENV_E_INVAL, "null pointer");
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int max_seg = 0;
+    if (const int rc = multi_max_seg(m, st, &max_seg)) return rc;
+    if (max_seg > kMaxSeg)
+        return fail(CARENV_E_TRACK, "the fused rollout kernels support tracks with at most 128 wall segments");
+    // no staged tables: weights after a 128-byte alignment pad, A tiles, exchanged partial logits
+    const size_t smem = 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) + (size_t)2 * 2 * tc::kABytes +
+                        (size_t)2 * 128 * 12 * sizeof(float);
+    static const TrackParams kNoTrack{};                     // P and G of the single-track instantiations: unused
+    auto kern = k_policy_rollout_tc3<0, false>;
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(n_envs + 255) / 256, 256 + 128 + 32, smem, st>>>(
+        kNoTrack, Tables{}, packed_weights, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
+        reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale,
+        obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, m->d_stats, 0, kObsFull,
+        nullptr, 0, 0, m->d_params, m->d_tables, m->n_tracks, track_ids);
+    CU(cudaGetLastError());
+    return 0;
 }
 
 #include "policy_eval.cuh"      // carenv_policy_eval: k_policy_eval, whole episodes of one actor per launch

@@ -17,6 +17,10 @@
 //               chains, in the same order, as the actor part of policy_forward — the CUDA-core rollout's logits.
 //               The step loop's trip count is warp-uniform (lanes without an episode step along and discard their
 //               results) so that the wall tests keep their uniform constant-bank operands (DESIGN §3).
+//   k_policy_eval<0>   several tracks (carenv_policy_eval_multi): a slot that claims episode i moves to the start pose
+//               and reset observation of track episode_tracks[i] (as k_reset_multi) and steps with env_step<0> on that
+//               track's TrackParams / Tables in global memory (as k_rollout_multi); nothing else changes, so episode i
+//               on track k gives the record k_policy_eval gives on track k alone.
 #pragma once
 
 extern "C++" {
@@ -62,12 +66,16 @@ __device__ __forceinline__ void actor_forward(const float (&obs)[kPolicyObs], co
     out.value = 0.0f;
 }
 
+// U == 0 keeps its 16 table pointers and the track pointer in registers (the single-track tables are shared-memory
+// offsets): 3 CTAs per SM, 168 registers, where 4 CTAs (128 registers) spill.
 template <int U>
-__global__ void __launch_bounds__(kEvalBlock, 4)
+__global__ void __launch_bounds__(kEvalBlock, U == 0 ? 3 : 4)
 k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::Params W, long long n_episodes,
               unsigned long long episode0, int greedy, unsigned long long seed,
               carenv_eval_record *__restrict__ records, int n_trace, unsigned char *__restrict__ trace_actions,
-              float *__restrict__ trace_u, unsigned long long *counter, unsigned long long *stats, int table_bytes) {
+              float *__restrict__ trace_u, unsigned long long *counter, unsigned long long *stats, int table_bytes,
+              const TrackParams *__restrict__ mt_params, const Tables *__restrict__ mt_tables, int n_tracks,
+              const int *__restrict__ episode_tracks) {
     extern __shared__ __align__(16) unsigned char smem[];
     float *sw = reinterpret_cast<float *>(smem + table_bytes);
     for (int i = threadIdx.x; i < (kHidden / 2) * kActorPairFloats; i += blockDim.x) {
@@ -83,7 +91,9 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
     }
     if (threadIdx.x < kEvalTail)
         sw[(kHidden / 2) * kActorPairFloats + threadIdx.x] = threadIdx.x < kActions ? W.b2a[threadIdx.x] : 0.0f;
-    const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
+    // U == 0 (several tracks): nothing is staged, every lane reads its episode's track tables
+    const Tables T = U == 0 ? Tables{} : stage_tables(G, P.n_gates, P.n_seg, smem);   // ends with __syncthreads()
+    if constexpr (U == 0) __syncthreads();
 
     const int lane = threadIdx.x & 31;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -94,6 +104,17 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
 #pragma unroll
     for (int i = 0; i < kObsDim; ++i) obs[i] = P.reset_obs[i];
 
+    int tr = 0;                            // U == 0: the track of the lane's episode
+    // U == 0: the start pose and reset observation of track `tr` (k_reset_multi); env_step's autoreset would go back
+    // to the previous episode's track
+    auto start_on_track = [&]() {
+        const TrackParams &Q = mt_params[tr];
+        s.px = Q.start_x; s.py = Q.start_y; s.vx = 0.0; s.vy = 0.0;
+        s.k = 0; s.t = 0; s.next_gate = 0; s.passed = 0;
+#pragma unroll
+        for (int i = 0; i < kObsDim; ++i) obs[i] = Q.reset_obs[i];
+    };
+    if constexpr (U == 0) start_on_track();
     long long ep = -1;                     // episode index i of this call held by the lane (-1: none)
     bool drained = false;                  // the counter has run past n_episodes: the lane claims nothing more
     double ret = 0.0;
@@ -110,6 +131,10 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
             const unsigned long long i = base + (unsigned long long)__popc(m & lt_mask);
             if (i < (unsigned long long)n_episodes) {
                 ep = (long long)i; ret = 0.0; laps = 0; first_lap = -1;
+                if constexpr (U == 0) {
+                    tr = min(max(episode_tracks[i], 0), n_tracks - 1);
+                    start_on_track();
+                }
             } else {
                 drained = true;
             }
@@ -139,7 +164,8 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
             a = sample_action(po, u, logp, us);
         }
         StepResult o;
-        env_step<U>(s, a, 1.0, P, T, o, stats);
+        if constexpr (U == 0) env_step<0>(s, a, 1.0, mt_params[tr], mt_tables[tr], o, stats);
+        else env_step<U>(s, a, 1.0, P, T, o, stats);
         if (live) {
             if (ep < n_trace) {
                 const size_t ti = (size_t)ep * kTimeLimit + (size_t)step;
@@ -170,6 +196,47 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
 }  // extern "C++"
 
 /* ---- C ABI (include/carenv_b200.h) ---- */
+// One launch of an evaluation kernel: a persistent grid of at most one wave (CARENV_EVAL_CTAS > 0 caps it further,
+// a test hook so that a few slots play many episodes each) and a claim counter that lives for the call.  `m` and
+// `episode_tracks` only for the multi-track instantiation (else null).
+static int launch_eval(void (*kern)(const TrackParams, const Tables, const ppo::Params, long long, unsigned long long,
+                                    int, unsigned long long, carenv_eval_record *, int, unsigned char *, float *,
+                                    unsigned long long *, unsigned long long *, int, const TrackParams *,
+                                    const Tables *, int, const int *),
+                       int device, const TrackParams &P, const Tables &G, int table_bytes, const MultiTrack *m,
+                       const int32_t *episode_tracks, const ppo::Params &W, long long n_episodes,
+                       unsigned long long episode0, int greedy, unsigned long long seed, carenv_eval_record *records,
+                       int n_trace, unsigned char *trace_actions, float *trace_u, unsigned long long *stats,
+                       cudaStream_t st) {
+    const size_t smem = (size_t)table_bytes + sizeof(float) * kEvalFloats;
+    const char *cap_env = getenv("CARENV_EVAL_CTAS");
+    const long long cap = cap_env ? atoll(cap_env) : 0;
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int sms = 0, per_sm = 0;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kEvalBlock, smem));
+    long long grid = (n_episodes + kEvalBlock - 1) / kEvalBlock;
+    const long long resident = (long long)sms * (per_sm > 0 ? per_sm : 1);
+    if (grid > resident) grid = resident;
+    if (cap > 0 && grid > cap) grid = cap;
+    // The claim counter lives for one call, allocated and freed in stream order: calls on one handle may run
+    // concurrently on different streams.
+    unsigned long long *counter = nullptr;
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&counter), sizeof(unsigned long long), st));
+    cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st);
+    if (e == cudaSuccess) {
+        kern<<<(unsigned)grid, kEvalBlock, smem, st>>>(P, G, W, n_episodes, episode0, greedy ? 1 : 0, seed, records,
+                                                      n_trace, trace_actions, trace_u, counter, stats, table_bytes,
+                                                      m ? m->d_params : nullptr, m ? m->d_tables : nullptr,
+                                                      m ? m->n_tracks : 0, episode_tracks);
+        e = cudaGetLastError();
+    }
+    const cudaError_t ef = cudaFreeAsync(counter, st);
+    if (e != cudaSuccess) return cuda_fail(e, "k_policy_eval launch");
+    CU(ef);
+    return 0;
+}
+
 int carenv_policy_eval(void *handle, const float *w1a, const float *b1a, const float *w2a, const float *b2a,
                        long long n_episodes, unsigned long long episode0, int greedy, unsigned long long seed,
                        carenv_eval_record *records, int n_trace, unsigned char *trace_actions, float *trace_u,
@@ -186,40 +253,36 @@ int carenv_policy_eval(void *handle, const float *w1a, const float *b1a, const f
     DeviceGuard guard(h->device);
     if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
     const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
-    const size_t smem = (size_t)table_bytes + sizeof(float) * kEvalFloats;
     int U = h->force_generic ? 1 : h->host.P.unroll4;   // as carenv_policy_rollout: instantiated for 4, 2, 1
     if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
-    // Test hook: CARENV_EVAL_CTAS > 0 caps the grid, so that a few slots play many episodes each.
-    const char *cap_env = getenv("CARENV_EVAL_CTAS");
-    const long long cap = cap_env ? atoll(cap_env) : 0;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     const ppo::Params W{w1a, b1a, w2a, b2a, nullptr, nullptr, nullptr, nullptr};
-    auto launch = [&](auto kern) -> int {
-        CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int sms = 0, per_sm = 0;
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kEvalBlock, smem));
-        long long grid = (n_episodes + kEvalBlock - 1) / kEvalBlock;
-        const long long resident = (long long)sms * (per_sm > 0 ? per_sm : 1);
-        if (grid > resident) grid = resident;
-        if (cap > 0 && grid > cap) grid = cap;
-        // The claim counter lives for one call, allocated and freed in stream order: calls on one handle may run
-        // concurrently on different streams.
-        unsigned long long *counter = nullptr;
-        CU(cudaMallocAsync(reinterpret_cast<void **>(&counter), sizeof(unsigned long long), st));
-        cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st);
-        if (e == cudaSuccess) {
-            kern<<<(unsigned)grid, kEvalBlock, smem, st>>>(h->host.P, h->dev, W, n_episodes, episode0, greedy ? 1 : 0,
-                                                          seed, records, n_trace, trace_actions, trace_u, counter,
-                                                          h->d_stats, table_bytes);
-            e = cudaGetLastError();
-        }
-        const cudaError_t ef = cudaFreeAsync(counter, st);
-        if (e != cudaSuccess) return cuda_fail(e, "k_policy_eval launch");
-        CU(ef);
-        return 0;
-    };
-    if (U == 4) return launch(k_policy_eval<4>);
-    if (U == 2) return launch(k_policy_eval<2>);
-    return launch(k_policy_eval<1>);
+    auto kern = U == 4 ? k_policy_eval<4> : (U == 2 ? k_policy_eval<2> : k_policy_eval<1>);
+    return launch_eval(kern, h->device, h->host.P, h->dev, table_bytes, nullptr, nullptr, W, n_episodes, episode0,
+                       greedy, seed, records, n_trace, trace_actions, trace_u, h->d_stats,
+                       static_cast<cudaStream_t>(stream));
+}
+
+/* carenv_policy_eval on several tracks (k_policy_eval<0>): episode i of the call plays on track episode_tracks[i] of
+ * the multi-track handle (clamped to 0..n_tracks - 1) and gives the record carenv_policy_eval gives on that track. */
+int carenv_policy_eval_multi(void *multi, const int32_t *episode_tracks, const float *w1a, const float *b1a,
+                             const float *w2a, const float *b2a, long long n_episodes, unsigned long long episode0,
+                             int greedy, unsigned long long seed, carenv_eval_record *records, int n_trace,
+                             unsigned char *trace_actions, float *trace_u, void *stream) {
+    MultiTrack *m = static_cast<MultiTrack *>(multi);
+    if (!m) return fail(CARENV_E_INVAL, "null handle");
+    if (n_episodes < 0) return fail(CARENV_E_INVAL, "negative n_episodes");
+    if (!episode_tracks || !w1a || !b1a || !w2a || !b2a || !records) return fail(CARENV_E_INVAL, "null pointer");
+    if (n_trace < 0) return fail(CARENV_E_INVAL, "negative n_trace");
+    if (n_trace > 0 && !trace_actions) return fail(CARENV_E_INVAL, "n_trace > 0 needs trace_actions");
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int max_seg = 0;
+    if (const int rc = multi_max_seg(m, st, &max_seg)) return rc;
+    if (max_seg > kMaxSeg) return fail(CARENV_E_TRACK, "policy evaluation supports tracks with at most 128 wall segments");
+    if (n_episodes == 0) return 0;
+    static const TrackParams kNoTrack{};                     // P and G of the single-track instantiations: unused
+    const ppo::Params W{w1a, b1a, w2a, b2a, nullptr, nullptr, nullptr, nullptr};
+    return launch_eval(k_policy_eval<0>, m->device, kNoTrack, Tables{}, 0, m, episode_tracks, W, n_episodes, episode0,
+                       greedy, seed, records, n_trace, trace_actions, trace_u, m->d_stats, st);
 }

@@ -235,6 +235,10 @@ __device__ __forceinline__ void second_layer_pair(float h0, float h1, const floa
 // the issuer warp (13 warps, 128 registers each at launch; the critic warps hand 64 of theirs to the environment
 // warps).  Logits = (units 0..127) + (units 128..255) + bias, the same operands in the same order on both threads of
 // a lane; value = (even units + odd units) + bias.
+// U == 0 is the multi-track instantiation (carenv_policy_rollout_tc_multi): each environment thread reads
+// track_ids[e] once and steps with env_step<0> on that track's TrackParams / Tables in global memory (the arrays of
+// the multi-track handle), as k_rollout_multi does; no track tables are staged and P / G are unused.  Tracks may
+// differ within a warp: the barrier protocol does not care, every environment thread still arrives once per phase.
 __device__ __forceinline__ void second_layer_chunk16_x2(uint32_t a, const float (&va)[16], const float (&vb)[16],
                                                         float2 (&La)[5], float2 (&Lb)[5]) {
     float4 wa[5], wb[5];
@@ -265,7 +269,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
                      float *__restrict__ rew_buf, float *__restrict__ val_buf, float *__restrict__ term_buf,
                      float *__restrict__ trunc_buf, float *__restrict__ logp_buf, float *__restrict__ last_val,
                      float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode,
-                     const float4 *__restrict__ den4, int n_pairs, int row_f4) {
+                     const float4 *__restrict__ den4, int n_pairs, int row_f4, const TrackParams *__restrict__ mt_params,
+                     const Tables *__restrict__ mt_tables, int n_tracks, const int *__restrict__ track_ids) {
     constexpr int kGroups = 2, kCols = 256, kHalf = 128, kEnvThreads = kGroups * 128, kCriticThreads = 128;
     extern __shared__ __align__(16) unsigned char smem[];
     // [tables | pad to a 128-byte boundary | weights | A tiles (hi, lo per group) | exchanged partial logits [group][128][12]
@@ -299,7 +304,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
         tc::mbar_init(tc::smem_u32(&mb_xchg), kEnvThreads);
     }
     if (warp == 0) tc::tmem_alloc<512>(&tmem_slot);
-    const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
+    // U == 0 (several tracks): nothing is staged, every environment thread reads its own track's tables
+    const Tables T = U == 0 ? Tables{} : stage_tables(G, P.n_gates, P.n_seg, smem);   // ends with __syncthreads()
     tc::fence_async_smem();
     tc::tc_fence_before();
     __syncthreads();
@@ -389,6 +395,10 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
         const int e_raw = blockIdx.x * kEnvThreads + tid;
         const bool active = e_raw < n_envs;
         const int e = active ? e_raw : n_envs - 1;           // idle threads shadow the last env (no stores)
+        // U == 0: this environment's track, its constants and tables read through pointers as in k_rollout_multi
+        const int tr = U == 0 ? min(max(track_ids[e], 0), n_tracks - 1) : 0;
+        const TrackParams &PE = U == 0 ? mt_params[tr] : P;
+        const Tables TE = U == 0 ? mt_tables[tr] : T;
         const uint32_t lane_tmem = tbase + ((uint32_t)((warp & 3) * 32) << 16);
         const uint32_t w2s = tc::smem_u32(sw + kTcW2Off) + (uint32_t)(group * kHalf) * 40u;   // this thread's 128 hidden units
         const uint32_t b_full_mine = group == 0 ? b_full_lo : b_full_hi;
@@ -497,7 +507,7 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
                 logp_buf[idx] = logp;
             }
             StepResult o;
-            env_step<U, TAB>(s, a, reward_scale, P, T, o, active ? stats : nullptr, nullptr, TAB ? &tv : nullptr);
+            env_step<U, TAB>(s, a, reward_scale, PE, TE, o, active ? stats : nullptr, nullptr, TAB ? &tv : nullptr);
             if (active) rew_buf[idx] = o.reward;
 #pragma unroll
             for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];

@@ -10,6 +10,9 @@ its return, length, gates, laps, the step of its first lap and whether it crashe
 
 Episode ``episode0 + i`` of a call is a fixed function of (weights, seed, id, greedy): a batch can be split over
 calls or ranks at any boundary and gives the same records.
+
+Several tracks (``--track big_track,track``, or a ``MultiTrackVecEnv``): episode ``g`` plays on track ``g % n_tracks``
+by default (``carenv_policy_eval_multi``, still one launch), and the summary gains ``"by_track"``.
 """
 from __future__ import annotations
 
@@ -41,9 +44,16 @@ class EvalResult:
     episode's end) and ``trace_u`` [n_trace, 1000] float32 (sampled calls only) are None without a trace."""
 
     def __init__(self, records: torch.Tensor, trace_actions: torch.Tensor | None = None,
-                 trace_u: torch.Tensor | None = None):
+                 trace_u: torch.Tensor | None = None, track: torch.Tensor | None = None, n_tracks: int | None = None):
+        """``track`` [n] (int, on the records' device) and ``n_tracks``: the track of every episode of a
+        multi-track call (None for single-track calls)."""
         if records.dtype != torch.int32 or records.dim() != 2 or records.shape[1] != RECORD_INT32:
             raise ValueError("records must be an int32 tensor of shape (n, 8)")
+        if (track is None) != (n_tracks is None):
+            raise ValueError("pass both track and n_tracks, or neither")
+        if track is not None and (tuple(track.shape) != (records.shape[0],) or track.device != records.device):
+            raise ValueError("track must hold one id per record, on the records' device")
+        self.track, self.n_tracks = track, (None if n_tracks is None else int(n_tracks))
         self.records = records
         self.ret = records.view(torch.float64)[:, 0]
         self.length, self.gates, self.laps = records[:, 2], records[:, 3], records[:, 4]
@@ -65,6 +75,26 @@ class EvalResult:
             self.length.to(d).sum(), (self.outcome == CRASH).to(d).sum(), (self.outcome == TRUNCATED).to(d).sum(),
             lapped.to(d).sum(), self.laps.to(d).sum(), torch.where(lapped, self.first_lap, 0).to(d).sum(),
             self.gates.to(d).sum()])
+
+    def sums_by_track(self) -> torch.Tensor:
+        """float64 [n_tracks, 10]: :meth:`sums` of the episodes of each track (multi-track calls only).  Rows of
+        shards add up like :meth:`sums`."""
+        if self.track is None:
+            raise ValueError("sums_by_track needs the track column of a multi-track evaluation")
+        d = torch.float64
+        lapped = self.laps > 0
+        ret = self.ret
+        cols = torch.stack([
+            torch.ones_like(ret), ret, ret * ret, self.length.to(d), (self.outcome == CRASH).to(d),
+            (self.outcome == TRUNCATED).to(d), lapped.to(d), self.laps.to(d),
+            torch.where(lapped, self.first_lap, 0).to(d), self.gates.to(d)], dim=1)
+        out = torch.zeros((self.n_tracks, len(SUM_FIELDS)), dtype=d, device=ret.device)
+        return out.index_add_(0, self.track.to(device=ret.device, dtype=torch.int64), cols)
+
+    def summary_by_track(self, sums_by_track: torch.Tensor | None = None) -> list[dict]:
+        """One :meth:`summary` per track from ``sums_by_track`` (e.g. all-reduced; default: this call's)."""
+        rows = self.sums_by_track() if sums_by_track is None else sums_by_track
+        return [self.summary(r) for r in rows]
 
     def summary(self, sums: torch.Tensor | None = None) -> dict:
         """Means and rates from ``sums`` (e.g. all-reduced over ranks; default: this call's).  ``avg_reward`` is
@@ -94,19 +124,48 @@ def _actor_params(actor, device):
     return [p.detach() for p in params]
 
 
+def default_episode_tracks(n_episodes: int, n_tracks: int, episode0: int = 0, device=None) -> torch.Tensor:
+    """Track of global episode id ``g``: ``g % n_tracks`` (int32 [n_episodes]); a batch split over calls or ranks
+    gets the same assignment."""
+    return ((int(episode0) % n_tracks + torch.arange(n_episodes, dtype=torch.int64, device=device)) % n_tracks
+            ).to(torch.int32)
+
+
 def evaluate_policy(env, actor, n_episodes: int, greedy: bool = False, seed: int = 0, episode0: int = 0,
-                    trace: int = 0) -> EvalResult:
+                    trace: int = 0, episode_tracks=None) -> EvalResult:
     """Play episodes ``episode0 .. episode0 + n_episodes - 1`` of ``actor`` (``nn.Sequential(Linear(18, 256), ReLU,
     Linear(256, 9))`` on ``env.device``) on ``env``'s track, each from the start pose to its end, in one launch on
     the current stream.  ``greedy``: argmax actions; else sampled with the Philox stream keyed by ``seed``.  The
     first ``trace`` episodes also record their actions (and uniforms when sampled).  ``env``'s state is not
-    touched; only its track handle and device are used."""
+    touched; only its track handle and device are used.
+
+    With a :class:`MultiTrackVecEnv`, episode ``i`` of the call plays on track ``episode_tracks[i]`` (default: the
+    global id modulo the number of tracks, :func:`default_episode_tracks`) and its record equals the single-track
+    record of the same id on that track; the result has a ``track`` column and per-track sums."""
+    from .vec_env import MultiTrackVecEnv
+
     n_episodes, trace = int(n_episodes), int(trace)
     if n_episodes < 0 or trace < 0:
         raise ValueError("n_episodes and trace must be >= 0")
     if not 0 <= int(episode0) < 2 ** 64:
         raise ValueError("episode0 must fit in 64 bits")
     dev = env.device
+    multi = isinstance(env, MultiTrackVecEnv)
+    if episode_tracks is not None and not multi:
+        raise ValueError("episode_tracks needs a MultiTrackVecEnv")
+    if multi:
+        n_tracks = len(env.track_paths)
+        if episode_tracks is None:
+            tracks = default_episode_tracks(n_episodes, n_tracks, episode0, dev)
+        else:
+            tracks = torch.as_tensor(episode_tracks).reshape(-1)
+            if tracks.numel() != n_episodes:
+                raise ValueError(f"expected {n_episodes} episode tracks, got {tracks.numel()}")
+            if tracks.dtype.is_floating_point or tracks.dtype == torch.bool:
+                raise ValueError("episode_tracks must be integers")
+            if n_episodes and (int(tracks.min()) < 0 or int(tracks.max()) >= n_tracks):
+                raise ValueError(f"episode tracks must be in 0..{n_tracks - 1}")
+            tracks = tracks.to(device=dev, dtype=torch.int32).contiguous()
     params = _actor_params(actor, dev)
     records = torch.empty((n_episodes, RECORD_INT32), dtype=torch.int32, device=dev)
     n_trace = min(trace, n_episodes)
@@ -116,6 +175,13 @@ def evaluate_policy(env, actor, n_episodes: int, greedy: bool = False, seed: int
         if not greedy:
             trace_u = torch.full((n_trace, TIME_LIMIT), float("nan"), dtype=torch.float32, device=dev)
     L = _lib.lib()
+    if multi:
+        with torch.cuda.device(dev):
+            rc = L.carenv_policy_eval_multi(env._multi, _p(tracks), *[_p(p) for p in params], n_episodes, int(episode0),
+                                            int(bool(greedy)), int(seed) & (2 ** 64 - 1), _p(records), n_trace,
+                                            _p(trace_actions), _p(trace_u), env._stream())
+        _lib.check(rc, "carenv_policy_eval_multi")
+        return EvalResult(records, trace_actions, trace_u, track=tracks, n_tracks=n_tracks)
     with torch.cuda.device(dev):
         rc = L.carenv_policy_eval(env._handle, *[_p(p) for p in params], n_episodes, int(episode0), int(bool(greedy)),
                                   int(seed) & (2 ** 64 - 1), _p(records), n_trace, _p(trace_actions), _p(trace_u),
@@ -137,7 +203,9 @@ def load_checkpoint(path: str):
 def parse_args(argv=None):
     p = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     p.add_argument("--checkpoint", required=True, help="model.dat / checkpoint_{epoch}.dat written by train_ppo")
-    p.add_argument("--track", default="big_track", help="track name shipped with the package or a JSON path")
+    p.add_argument("--track", default="big_track",
+                   help="track name shipped with the package or a JSON path; a comma-separated list plays episode g on "
+                        "track g %% n_tracks and adds per-track summaries under \"by_track\"")
     p.add_argument("--episodes", type=int, default=65536, help="episodes in total over all ranks")
     p.add_argument("--greedy", action="store_true", help="argmax actions instead of sampled ones")
     p.add_argument("--seed", type=int, default=0, help="seed of the sampling stream")
@@ -148,7 +216,7 @@ def parse_args(argv=None):
 def main(argv=None) -> dict:
     import torch.distributed as dist
 
-    from . import VecCarEnv, builtin_track
+    from . import MultiTrackVecEnv, VecCarEnv, builtin_track
     from .shard import shard_range
 
     args = parse_args(argv)
@@ -160,16 +228,25 @@ def main(argv=None) -> dict:
     if world > 1 and not dist.is_initialized():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
-    track = args.track if os.path.exists(args.track) else builtin_track(args.track)
-    env = VecCarEnv(1, track, device=dev)
+    names = args.track.split(",")
+    paths = [t if os.path.exists(t) else builtin_track(t) for t in names]
+    if len(paths) == 1:
+        env = VecCarEnv(1, paths[0], device=dev)
+    else:
+        env = MultiTrackVecEnv(track_paths=paths, track_ids=[0], device=dev)
     actor = load_checkpoint(args.checkpoint).actor.to(dev)
     lo, hi = shard_range(args.episodes, world, rank)            # every rank plays its contiguous share of the ids
     res = evaluate_policy(env, actor, hi - lo, greedy=args.greedy, seed=args.seed, episode0=lo)
     sums = res.sums()
+    by_track = res.sums_by_track() if len(paths) > 1 else None
     if world > 1:
         dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+        if by_track is not None:
+            dist.all_reduce(by_track, op=dist.ReduceOp.SUM)
     out = {"checkpoint": args.checkpoint, "track": args.track, "greedy": bool(args.greedy), "seed": args.seed,
            **res.summary(sums)}
+    if by_track is not None:
+        out["by_track"] = [{"track": name, **summ} for name, summ in zip(names, res.summary_by_track(by_track))]
     if rank == 0:
         print(json.dumps(out), flush=True)
         if args.json:

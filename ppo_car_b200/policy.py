@@ -118,7 +118,14 @@ def fused_rollout(env, packed: torch.Tensor, buf, cur_obs: torch.Tensor, cur_ter
                   tensor_cores: bool | None = None) -> None:
     """Fill every row of ``buf`` (ppo_car_b200.Buffer) with one launch and leave the rollout state in
     ``cur_obs / cur_term / cur_trunc`` (in place).  ``step0`` is the global step index of row 0 (it
-    selects the random stream together with ``seed`` and ``env_offset + env``)."""
+    selects the random stream together with ``seed`` and ``env_offset + env``).
+
+    ``env`` may be a :class:`MultiTrackVecEnv` (C ABI carenv_policy_rollout_tc_multi): every environment runs on its
+    track (``env.track_ids``) and its rows are bit-identical to a single-track run on that track.  That needs the
+    tensor-core packing and full observation rows (no ``Buffer(compact_obs=True)``)."""
+    from .vec_env import MultiTrackVecEnv
+
+    multi = isinstance(env, MultiTrackVecEnv)
     n, T = env.num_envs, buf.capacity
     for name, t, shape in (("cur_obs", cur_obs, (n, OBS)), ("cur_term", cur_term, (n,)), ("cur_trunc", cur_trunc, (n,)),
                            ("last_val", last_val, (n,)), ("u_dbg", u_dbg, (T, n))):
@@ -129,10 +136,26 @@ def fused_rollout(env, packed: torch.Tensor, buf, cur_obs: torch.Tensor, cur_ter
     rows = buf.pose_buf if compact else buf.obs_buf
     if tuple(rows.shape) != ((T, n, 4) if compact else (T, n, OBS)):
         raise ValueError("buffer shape does not match the environment")
-    env.set_option("pose_rows", int(compact))               # obs_buf argument = 32-byte pose records
     L = _lib.lib()
     if tensor_cores is None:                                # the two packings have different sizes
         tensor_cores = packed.numel() == L.carenv_policy_weights_floats_tc()
+    if multi:
+        if compact:
+            raise ValueError("several tracks need full observation rows: pose records do not carry a track "
+                             "(use Buffer(compact_obs=False))")
+        if not tensor_cores:
+            raise ValueError("several tracks run on the tensor-core kernel only: pack the weights with "
+                             "pack_policy_weights_tc")
+        with torch.cuda.device(env.device):
+            rc = L.carenv_policy_rollout_tc_multi(
+                env._multi, _p(env.track_ids), _p(packed), n, T, int(env_offset), int(seed) & (2 ** 64 - 1),
+                int(step0), _p(env.pos), _p(env.vel), _p(env.ints), _p(cur_obs), _p(cur_term), _p(cur_trunc),
+                float(env.reward_scaling), _p(rows), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf),
+                _p(buf.term_buf), _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream())
+        _lib.check(rc, "carenv_policy_rollout_tc_multi")
+        buf.ptr = T
+        return
+    env.set_option("pose_rows", int(compact))               # obs_buf argument = 32-byte pose records
     fn = L.carenv_policy_rollout_tc if tensor_cores else L.carenv_policy_rollout
     with torch.cuda.device(env.device):
         rc = fn(env._handle, _p(packed), n, T, int(env_offset), int(seed) & (2 ** 64 - 1), int(step0), _p(env.pos),

@@ -7,6 +7,7 @@ statistics (train.py:272-274, avg_reward) cross the shards: one small all-reduce
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -18,6 +19,17 @@ def shard_range(n_total: int, world_size: int, rank: int) -> tuple[int, int]:
     base, extra = divmod(n_total, world_size)
     lo = rank * base + min(rank, extra)
     return lo, lo + base + (1 if rank < extra else 0)
+
+
+def track_blocks(n_total: int, n_tracks: int, lo: int, hi: int) -> np.ndarray:
+    """Track of each global env lo .. hi - 1 when n_total envs share n_tracks tracks: env g runs on track
+    g * n_tracks // n_total, i.e. contiguous, balanced blocks (warps of the fused rollout kernel are then nearly all
+    single-track), independent of how the envs are sharded.  int32 [hi - lo]."""
+    if not (1 <= n_tracks <= n_total):
+        raise ValueError("need 1 <= n_tracks <= n_total")
+    if not (0 <= lo <= hi <= n_total):
+        raise ValueError("env range out of bounds")
+    return (np.arange(lo, hi, dtype=np.int64) * n_tracks // n_total).astype(np.int32)
 
 
 def allreduce_rollout_stats(reward_sum: torch.Tensor, n_steps: torch.Tensor, episodes: torch.Tensor | None = None):

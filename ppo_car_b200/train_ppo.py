@@ -21,6 +21,10 @@ kernel launch, and with more than one process (torchrun) every rank owns an env 
 are averaged with one NCCL all-reduce per minibatch step (12,298 floats).
 
     python -m ppo_car_b200.train_ppo --track big_track --n-envs 24 --n-epochs 200
+
+Several tracks: ``--track big_track,track,my_track.json`` trains ONE policy on all of them.  Global env g of N runs on
+track g * K // N (contiguous blocks), every rank steps its shard as a MultiTrackVecEnv, and every epoch record gains
+``"by_track"`` (avg_reward and episodes per track, over all ranks).
 """
 from __future__ import annotations
 
@@ -33,8 +37,8 @@ import torch
 import torch.distributed as dist
 import torch.nn as nn
 
-from . import Buffer, VecCarEnv, builtin_track
-from .shard import allreduce_rollout_stats, shard_range
+from . import Buffer, MultiTrackVecEnv, VecCarEnv, builtin_track
+from .shard import allreduce_rollout_stats, shard_range, track_blocks
 
 
 def _ortho(layer: nn.Linear, gain: float) -> nn.Linear:
@@ -73,7 +77,9 @@ def parse_args(argv=None):
                    help="directory for checkpoint_{epoch}.dat (every 10 epochs) and model.dat (at exit), the "
                         "reference's files (train.py:280-283, 301); a sub-directory named after --run-name is created. "
                         "Default: no checkpoints")
-    p.add_argument("--track", default="big_track", help="track name shipped with the package or a JSON path")
+    p.add_argument("--track", default="big_track",
+                   help="track name shipped with the package or a JSON path, or a comma-separated list of them: one "
+                        "policy trained on every track, env g of N on track g * K // N")
     p.add_argument("--n-envs", type=int, default=16, help="total environments over all ranks")
     p.add_argument("--n-epochs", type=int, default=200)
     p.add_argument("--n-steps", type=int, default=1024)
@@ -119,7 +125,28 @@ def parse_args(argv=None):
     return p.parse_args(argv)
 
 
+def track_list(args) -> tuple[list[str], list[str]]:
+    """(names, paths) of ``--track``: one entry, or several from a comma-separated list.  With several tracks the
+    options that have no multi-track path are refused here, before any device work."""
+    names = [args.track] if os.path.exists(args.track) else args.track.split(",")
+    paths = [t if os.path.exists(t) else builtin_track(t) for t in names]
+    if len(paths) > 1:
+        for flag, on, why in (("--compact-obs", args.compact_obs, "pose records do not carry a track"),
+                              ("--fused-cuda-cores", args.fused_cuda_cores,
+                               "the multi-track fused rollout runs on the tensor cores"),
+                              ("--cuda-graph", args.cuda_graph,
+                               "the eager rollout is not captured; --fused-rollout is one launch per epoch")):
+            if on:
+                raise SystemExit(f"{flag} does not work with several tracks: {why}")
+        if args.n_envs < len(paths):
+            raise SystemExit(f"--n-envs {args.n_envs} is smaller than the number of tracks ({len(paths)}): "
+                             "every track needs at least one environment")
+    return names, paths
+
+
 def train(args) -> list[dict]:
+    names, paths = track_list(args)
+    multi = len(paths) > 1
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -129,12 +156,16 @@ def train(args) -> list[dict]:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(args.seed)                       # same initial weights on every rank
-    track = args.track if os.path.exists(args.track) else builtin_track(args.track)
     lo, hi = shard_range(args.n_envs, world, rank)
     n = hi - lo
     T = args.n_steps
 
-    envs = VecCarEnv(n, track, device=dev, reward_scaling=args.reward_scaling, float_flags=True, with_info=False)
+    if multi:
+        envs = MultiTrackVecEnv(track_paths=paths, track_ids=track_blocks(args.n_envs, len(paths), lo, hi), device=dev,
+                                reward_scaling=args.reward_scaling, float_flags=True)
+    else:
+        envs = VecCarEnv(n, paths[0], device=dev, reward_scaling=args.reward_scaling, float_flags=True,
+                         with_info=False)
     obs_dim = envs.single_observation_space.shape
     agent = ActorCritic(obs_dim[0], envs.single_action_space.n).to(dev)
     graph_update = bool(args.graph_update)                 # with world > 1 the NCCL all-reduce is captured too
@@ -198,7 +229,8 @@ def train(args) -> list[dict]:
                              pack_policy_weights_tc)
 
         # small shards (the reference's 24 environments): one warp per environment, parameters read in place
-        warp_rollout = (not args.fused_cuda_cores and n <= WARP_ROLLOUT_MAX_ENVS and len(envs.track.walls) <= 32)
+        warp_rollout = (not multi and not args.fused_cuda_cores and n <= WARP_ROLLOUT_MAX_ENVS
+                        and len(envs.track.walls) <= 32)
 
         # otherwise the tensor-core kernel (k_policy_rollout_tc3, 256-environment CTAs), or the CUDA-core kernel with
         # --fused-cuda-cores
@@ -216,9 +248,28 @@ def train(args) -> list[dict]:
             res = evaluate_policy(envs, agent.actor, e_hi - e_lo, greedy=args.eval_greedy, seed=args.seed,
                                   episode0=e_lo)
             sums = res.sums()
+            by_track = res.sums_by_track() if multi else None
         if world > 1:
             dist.all_reduce(sums, op=dist.ReduceOp.SUM)
-        return res.summary(sums)
+            if by_track is not None:
+                dist.all_reduce(by_track, op=dist.ReduceOp.SUM)
+        out = res.summary(sums)
+        if by_track is not None:
+            out["by_track"] = [{"track": name, **summ} for name, summ in zip(names, res.summary_by_track(by_track))]
+        return out
+
+    def rollout_by_track():
+        """avg_reward and episodes of this epoch's rollout per track, summed over the ranks."""
+        tid = envs.track_ids.to(torch.int64)
+        z = torch.zeros((3, len(paths)), dtype=torch.float64, device=dev)
+        z[0].index_add_(0, tid, buf.rew_buf.sum(0).double())
+        z[1].index_add_(0, tid, torch.full((n,), float(T), dtype=torch.float64, device=dev))
+        z[2].index_add_(0, tid, (buf.term_buf.sum(0) + buf.trunc_buf.sum(0)).double())
+        if world > 1:
+            dist.all_reduce(z, op=dist.ReduceOp.SUM)
+        r, st, ep = z.tolist()
+        return [{"track": name, "avg_reward": r[k] / st[k] / args.reward_scaling, "episodes": ep[k]}
+                for k, name in enumerate(names)]
 
     graph = None
     if args.cuda_graph and not args.fused_rollout:
@@ -260,6 +311,7 @@ def train(args) -> list[dict]:
                 adv, ret = buf.calculate_advantages(boot, next_term.reshape(1, -1), next_trunc.reshape(1, -1))
             rew_sum, steps, episodes = allreduce_rollout_stats(buf.rew_buf.sum(), torch.tensor(float(T * n), device=dev),
                                                                buf.term_buf.sum() + buf.trunc_buf.sum())
+            by_track = rollout_by_track() if multi else None
             obs_b, act_b, val_b, logp_b = buf.get()
             obs_f = obs_b if args.compact_obs else obs_b.view(-1, *obs_dim)      # pose records / observations
             act_f, logp_f = act_b.view(-1), logp_b.view(-1)
@@ -338,12 +390,16 @@ def train(args) -> list[dict]:
                    "episodes": episodes, "policy_loss": s[0], "value_loss": s[1], "entropy": s[2], "total_loss": s[3],
                    "lr": float(fused_upd.lr if fused_upd is not None else opt.param_groups[0]["lr"]), "sps": global_step / (time.time() - t_start),
                    "wall_s": time.time() - t_start}
+            if by_track is not None:
+                rec["by_track"] = by_track
             if args.eval_every > 0 and epoch % args.eval_every == 0:
                 rec["eval"] = evaluate_epoch()
             history.append(rec)
             if rank == 0:
                 print(f"Epoch {epoch} done in {rec['wall_s']:.2f}s. Avg reward: {rec['avg_reward']:.4f}. "
                       f"SPS {rec['sps']:.0f}  entropy {rec['entropy']:.3f}", flush=True)
+                if by_track is not None:
+                    print("  by track: " + ", ".join(f"{b['track']} {b['avg_reward']:.4f}" for b in by_track), flush=True)
                 if "eval" in rec:
                     ev = rec["eval"]
                     print(f"  eval ({ev['episodes']} {'greedy' if args.eval_greedy else 'sampled'} episodes): return "
