@@ -346,6 +346,58 @@ int carenv_ppo_epoch(float *w1_actor, float *b1_actor, float *w2_actor, float *b
                      double max_grad_norm, float *sums4, float *workspace, int *sync_words, void *comm, int n_ctas,
                      long long *prof, void *stream);
 
+/* Populations: P independent policies ("members") trained side by side in one process, one launch per stage for all
+ * of them (csrc/population.cuh).  Member p owns its parameters, Adam state, hyperparameters, seed and n environments,
+ * which are columns p*n .. p*n + n - 1 of every [N] / [T][N] array (N = P*n); members never exchange data.
+ * Parameters are stacked nn.Linear tensors: w1 [P][256][18], b1 [P][256], w2_actor [P][9][256], b2_actor [P][9],
+ * w2_critic [P][1][256], b2_critic [P][1].  Every call refuses n_members or n_envs_per_member <= 0, a negative n_steps
+ * and null pointers (CARENV_E_INVAL).
+ *   carenv_pack_policy_pop   carenv_pack_policy for every member in one launch: packed_out [P][floats], block p
+ *       bit-identical to carenv_pack_policy of member p.
+ *   carenv_policy_rollout_warp_pop / carenv_policy_rollout_tc_pop   one launch plays all members' rollouts (replaces,
+ *       per member, the loop of train.py:173-195 as carenv_policy_rollout_warp / _tc do).  Member p keys its random
+ *       stream with seeds[p] (device uint64 [P]) and its member-local env index, so its rows are bit-identical to
+ *       carenv_policy_rollout_warp / _tc run alone on member p with env_offset 0 and n environments.  The warp kernel
+ *       takes tracks of at most 32 wall segments, the tensor-core kernel tracks of at most 128 (CARENV_E_TRACK
+ *       otherwise).  obs_buf holds full [T][N][18] rows: the handle's pose_rows option must be 0.
+ *   carenv_ppo_epoch_pop   all n_updates minibatch updates of an epoch for every member in ONE cluster launch
+ *       (replaces, per member, train.py:223-261 as carenv_ppo_epoch does): one thread-block cluster of
+ *       carenv_ppo_epoch_pop_cluster_size() CTAs per member, gradients reduced through distributed shared memory.
+ *         idx                  device int64 [P][n_updates][batch]: global rows of obs / act / ... (member p's own)
+ *         lr, clip_ratio, vf_coef, ent_coef, max_grad_norm   device float [P]
+ *         exp_avg, exp_avg_sq  device float [P][12,298] (flat parameter layout); step device int [P];
+ *         sums4                device float [P][4]: policy loss, value loss, entropy, total loss, accumulated
+ *       Deterministic, and member p's results do not depend on the other members; not bit-identical to
+ *       carenv_ppo_epoch (another reduction order).  Needs no workspace.
+ *   carenv_ppo_epoch_pop_resident_clusters   how many clusters of the update kernel the current device keeps resident
+ *       at once (cudaOccupancyMaxActiveClusters). */
+int carenv_pack_policy_pop(int tensor_cores, int n_members, const float *w1_actor, const float *b1_actor,
+                           const float *w2_actor, const float *b2_actor, const float *w1_critic, const float *b1_critic,
+                           const float *w2_critic, const float *b2_critic, float *packed_out, void *stream);
+int carenv_policy_rollout_warp_pop(void *handle, int n_members, const float *w1_actor, const float *b1_actor,
+                                   const float *w2_actor, const float *b2_actor, const float *w1_critic,
+                                   const float *b1_critic, const float *w2_critic, const float *b2_critic,
+                                   int n_envs_per_member, int n_steps, const unsigned long long *seeds,
+                                   unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                   float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                   float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                   float *logp_buf, float *last_val, float *u_dbg, void *stream);
+int carenv_policy_rollout_tc_pop(void *handle, int n_members, const float *packed_weights, int n_envs_per_member,
+                                 int n_steps, const unsigned long long *seeds, unsigned long long step0, double *pos,
+                                 double *vel, int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc,
+                                 double reward_scale, float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                 float *term_buf, float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg,
+                                 void *stream);
+int carenv_ppo_epoch_pop_cluster_size(void);
+int carenv_ppo_epoch_pop_resident_clusters(int *n_clusters);
+int carenv_ppo_epoch_pop(int n_members, float *w1_actor, float *b1_actor, float *w2_actor, float *b2_actor,
+                         float *w1_critic, float *b1_critic, float *w2_critic, float *b2_critic, const float *obs,
+                         const long long *idx, const float *act, const float *old_logp, const float *adv,
+                         const float *ret, int batch, int n_updates, const float *lr, const float *clip_ratio,
+                         const float *vf_coef, const float *ent_coef, const float *max_grad_norm, double beta1,
+                         double beta2, double eps, float *exp_avg, float *exp_avg_sq, int *step, float *sums4,
+                         void *stream);
+
 /* Test hook for the tensor-core building blocks (csrc/tc_mlp.cuh): D[128][256] = A[128][24] * B[256][24]^T,
  * tcgen05.mma kind::tf32 with the accumulator in tensor memory; device pointers, row-major float32. */
 int carenv_tc_gemm_test(const float *A, const float *B, float *D, void *stream);

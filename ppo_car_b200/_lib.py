@@ -15,7 +15,8 @@ ROOT = os.path.dirname(_PKG)
 LIB_PATH = os.environ.get("CARENV_LIB") or os.path.join(_PKG, "libcarenv_b200.so")   # override: kernel experiments
 SOURCES = [os.path.join(_PKG, "csrc", f)
            for f in ("carenv_kernels.cu", "carenv_core.cuh", "carenv_tables.h", "policy_core.cuh", "tc_mlp.cuh",
-                     "ppo_update.cuh", "ppo_epoch.cuh", "policy_rollout.cuh", "policy_abi.cuh", "policy_eval.cuh")]
+                     "ppo_update.cuh", "ppo_epoch.cuh", "policy_rollout.cuh", "policy_abi.cuh", "policy_eval.cuh",
+                     "population.cuh")]
 HEADER = os.path.join(ROOT, "include", "carenv_b200.h")
 
 ACT_U8, ACT_I32, ACT_I64 = 0, 1, 2
@@ -118,6 +119,15 @@ def lib():
     L.carenv_policy_rollout_tc_multi.restype = i32
     L.carenv_policy_eval_multi.argtypes = [vp, vp] + L.carenv_policy_eval.argtypes[1:]
     L.carenv_policy_eval_multi.restype = i32
+    L.carenv_pack_policy_pop.argtypes = [i32, i32] + [vp] * 10
+    L.carenv_policy_rollout_warp_pop.argtypes = [vp, i32] + [vp] * 8 + [i32, i32, vp, C.c_ulonglong] + [vp] * 6 + \
+        [f64] + [vp] * 10
+    L.carenv_policy_rollout_tc_pop.argtypes = [vp, i32, vp, i32, i32, vp, C.c_ulonglong] + [vp] * 6 + [f64] + [vp] * 10
+    L.carenv_ppo_epoch_pop.argtypes = [i32] + [vp] * 8 + [vp] * 6 + [i32, i32] + [vp] * 5 + [f64, f64, f64] + [vp] * 5
+    L.carenv_ppo_epoch_pop_resident_clusters.argtypes = [vp]
+    for name in ("carenv_pack_policy_pop", "carenv_policy_rollout_warp_pop", "carenv_policy_rollout_tc_pop",
+                 "carenv_ppo_epoch_pop", "carenv_ppo_epoch_pop_cluster_size", "carenv_ppo_epoch_pop_resident_clusters"):
+        getattr(L, name).restype = i32
     for name in ("carenv_create", "carenv_destroy", "carenv_reset_obs", "carenv_reset", "carenv_step",
                  "carenv_rollout", "carenv_rollout_poses", "carenv_observe", "carenv_step_host", "carenv_step_host_records", "carenv_step_records", "carenv_step_final", "carenv_multi_create", "carenv_multi_destroy", "carenv_multi_reset",
                  "carenv_multi_rollout", "carenv_render", "carenv_host_alloc", "carenv_host_free", "carenv_stats", "gae_reverse_scan", "carenv_bench_ffma", "carenv_set_option", "carenv_policy_rollout", "carenv_policy_rollout_tc"):

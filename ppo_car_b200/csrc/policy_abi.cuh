@@ -220,6 +220,33 @@ int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs,
 }
 
 /* Small batches: one warp per environment, network parameters in nn.Linear layout (k_policy_rollout_warp). */
+// n_members == 0: one policy (k_policy_rollout_warp<false>); otherwise n_members stacked policies with n_envs
+// environments each and seeds[p] (k_policy_rollout_warp<true>, carenv_policy_rollout_warp_pop).
+static int policy_rollout_warp_launch(Handle *h, const ppo::Params &W, int n_members, int n_envs, int n_steps,
+                                      int env_offset, unsigned long long seed, const unsigned long long *seeds,
+                                      unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                      float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                      float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                      float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    if (h->host.P.n_seg > 32)
+        return fail(CARENV_E_TRACK, "the warp-per-environment rollout kernel supports tracks with at most 32 wall segments");
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
+    const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
+    const size_t smem = (size_t)table_bytes + sizeof(float) * kWpFloats;
+    if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the warp-per-environment rollout kernel");
+    auto kern = n_members > 0 ? k_policy_rollout_warp<true> : k_policy_rollout_warp<false>;
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const dim3 grid((n_envs + 3) / 4, n_members > 0 ? n_members : 1);
+    kern<<<grid, 128, smem, static_cast<cudaStream_t>(stream)>>>(
+        h->host.P, h->dev, W, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
+        reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale, obs_buf,
+        act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, h->d_stats, table_bytes,
+        h->pose_rows ? kObsPose : kObsFull, seeds, n_members * n_envs);
+    CU(cudaGetLastError());
+    return 0;
+}
+
 int carenv_policy_rollout_warp(void *handle, const float *w1a, const float *b1a, const float *w2a, const float *b2a,
                                const float *w1c, const float *b1c, const float *w2c, const float *b2c, int n_envs,
                                int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
@@ -234,22 +261,10 @@ int carenv_policy_rollout_warp(void *handle, const float *w1a, const float *b1a,
     if (!w1a || !b1a || !w2a || !b2a || !w1c || !b1c || !w2c || !b2c || !pos || !vel || !ints || !cur_obs || !cur_term ||
         !cur_trunc || !obs_buf || !act_buf || !rew_buf || !val_buf || !term_buf || !trunc_buf || !logp_buf)
         return fail(CARENV_E_INVAL, "null pointer");
-    if (h->host.P.n_seg > 32)
-        return fail(CARENV_E_TRACK, "the warp-per-environment rollout kernel supports tracks with at most 32 wall segments");
-    DeviceGuard guard(h->device);
-    if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
-    const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
-    const size_t smem = (size_t)table_bytes + sizeof(float) * kWpFloats;
-    if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the warp-per-environment rollout kernel");
-    CU(cudaFuncSetAttribute(k_policy_rollout_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const ppo::Params W{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c};
-    k_policy_rollout_warp<<<(n_envs + 3) / 4, 128, smem, static_cast<cudaStream_t>(stream)>>>(
-        h->host.P, h->dev, W, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
-        reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale, obs_buf,
-        act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, h->d_stats, table_bytes,
-        h->pose_rows ? kObsPose : kObsFull);
-    CU(cudaGetLastError());
-    return 0;
+    return policy_rollout_warp_launch(h, ppo::Params{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c}, 0, n_envs, n_steps,
+                                      env_offset, seed, nullptr, step0, pos, vel, ints, cur_obs, cur_term, cur_trunc,
+                                      reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
+                                      last_val, u_dbg, stream);
 }
 
 /* Test hook: D[128,256] = A[128,24] * B[256,24]^T on the tensor cores (tcgen05, kind::tf32). */
@@ -264,20 +279,14 @@ int carenv_tc_gemm_test(const float *A, const float *B, float *D, void *stream) 
 
 int carenv_policy_weights_floats_tc(void) { return kTcWeightFloats; }
 
-/* Tensor-core variant of carenv_policy_rollout (same arguments; packed_weights in the layout of
- * ppo_car_b200/policy.py: pack_policy_weights_tc): k_policy_rollout_tc3. */
-int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
-                             unsigned long long seed, unsigned long long step0, double *pos, double *vel,
-                             int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
-                             float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
-                             float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
-    Handle *h = static_cast<Handle *>(handle);
-    if (!h) return fail(CARENV_E_INVAL, "null handle");
-    if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
-    if (n_envs == 0) return 0;
-    if (!packed_weights || !pos || !vel || !ints || !cur_obs || !cur_term || !cur_trunc || !obs_buf || !act_buf ||
-        !rew_buf || !val_buf || !term_buf || !trunc_buf || !logp_buf)
-        return fail(CARENV_E_INVAL, "null pointer");
+// k_policy_rollout_tc3 on a single-track handle.  n_members == 0: one policy; otherwise n_members packed policies
+// [n_members][kTcWeightFloats] with n_envs environments each and seeds[p] (carenv_policy_rollout_tc_pop).
+static int policy_rollout_tc_launch(Handle *h, const float *packed_weights, int n_members, int n_envs, int n_steps,
+                                    int env_offset, unsigned long long seed, const unsigned long long *seeds,
+                                    unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                    float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                    float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                    float *logp_buf, float *last_val, float *u_dbg, void *stream) {
     if (h->host.P.n_seg > kMaxSeg)
         return fail(CARENV_E_TRACK, "the fused rollout kernels support tracks with at most 128 wall segments");
     if (h->tc_tiles >= 2 && h->tc_tiles <= 4)
@@ -298,7 +307,7 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
     const bool tab = U >= 2 && h->d_den4 && h->tab >= 0 && smem_base + tab_bytes <= 227 * 1024;
     const size_t smem = smem_base + (tab ? tab_bytes : 0);
     if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the tensor-core rollout kernel");
-    const int grid = (n_envs + 255) / 256;
+    const dim3 grid((n_envs + 255) / 256, n_members > 0 ? n_members : 1);
     auto launch = [&](auto kern) -> int {
         CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<grid, 256 + 128 + 32, smem, static_cast<cudaStream_t>(stream)>>>(
@@ -306,13 +315,37 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
             cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
             last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4,
-            nullptr, nullptr, 0, nullptr);
+            nullptr, nullptr, 0, nullptr, seeds, n_members * n_envs);
         CU(cudaGetLastError());
         return 0;
     };
+    if (n_members > 0) {
+        if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true, true>) : launch(k_policy_rollout_tc3<4, false, true>);
+        if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true, true>) : launch(k_policy_rollout_tc3<2, false, true>);
+        return launch(k_policy_rollout_tc3<1, false, true>);
+    }
     if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true>) : launch(k_policy_rollout_tc3<4, false>);
     if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true>) : launch(k_policy_rollout_tc3<2, false>);
     return launch(k_policy_rollout_tc3<1, false>);
+}
+
+/* Tensor-core variant of carenv_policy_rollout (same arguments; packed_weights in the layout of
+ * ppo_car_b200/policy.py: pack_policy_weights_tc): k_policy_rollout_tc3. */
+int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                             unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                             int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                             float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                             float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    Handle *h = static_cast<Handle *>(handle);
+    if (!h) return fail(CARENV_E_INVAL, "null handle");
+    if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
+    if (n_envs == 0) return 0;
+    if (!packed_weights || !pos || !vel || !ints || !cur_obs || !cur_term || !cur_trunc || !obs_buf || !act_buf ||
+        !rew_buf || !val_buf || !term_buf || !trunc_buf || !logp_buf)
+        return fail(CARENV_E_INVAL, "null pointer");
+    return policy_rollout_tc_launch(h, packed_weights, 0, n_envs, n_steps, env_offset, seed, nullptr, step0, pos, vel,
+                                    ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
+                                    term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream);
 }
 
 /* Largest wall-segment count over the tracks of a multi-track handle: the handle keeps its TrackParams on the device
@@ -359,9 +392,10 @@ int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const 
         kNoTrack, Tables{}, packed_weights, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
         reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale,
         obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, m->d_stats, 0, kObsFull,
-        nullptr, 0, 0, m->d_params, m->d_tables, m->n_tracks, track_ids);
+        nullptr, 0, 0, m->d_params, m->d_tables, m->n_tracks, track_ids, nullptr, 0);
     CU(cudaGetLastError());
     return 0;
 }
 
 #include "policy_eval.cuh"      // carenv_policy_eval: k_policy_eval, whole episodes of one actor per launch
+#include "population.cuh"       // carenv_*_pop: independent policies trained side by side (member-batched kernels)

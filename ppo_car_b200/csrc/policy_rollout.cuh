@@ -146,14 +146,48 @@ constexpr int kTcW2cOff = kTcW2Off + kHidden * 10;           // W2 actor as [j][
 constexpr int kTcTailOff = kTcW2cOff + kHidden;              // b2[0..9], b2c, pad
 constexpr int kTcWeightFloats = kTcTailOff + 12;             // 27,404 floats
 
+// ---- populations of independent members (POP instantiations, carenv_policy_rollout_*_pop) ----------------------
+// Member p's parameters in stacked nn.Linear-layout tensors [P][256][18], [P][256], [P][9][256], [P][9], ...
+__device__ __forceinline__ ppo::Params member_params(const ppo::Params &W, int p) {
+    const size_t q = (size_t)p;
+    return ppo::Params{W.w1a + q * kHidden * kObsDim, W.b1a + q * kHidden, W.w2a + q * kActions * kHidden,
+                       W.b2a + q * kActions,          W.w1c + q * kHidden * kObsDim, W.b1c + q * kHidden,
+                       W.w2c + q * kHidden,           W.b2c + q};
+}
+
+// Moves every per-environment pointer to column col0 (the member's first environment): afterwards the kernel indexes
+// them with the member-local env e and, for the [T, N] rows, with the population's row stride N.
+__device__ __forceinline__ void pop_shift_columns(int col0, double2 *__restrict__ &pos, double2 *__restrict__ &vel,
+                                                  int4 *__restrict__ &ints, float *__restrict__ &cur_obs,
+                                                  float *__restrict__ &cur_term, float *__restrict__ &cur_trunc,
+                                                  float *__restrict__ &last_val, float *__restrict__ &obs_buf,
+                                                  float *__restrict__ &act_buf, float *__restrict__ &rew_buf,
+                                                  float *__restrict__ &val_buf, float *__restrict__ &term_buf,
+                                                  float *__restrict__ &trunc_buf, float *__restrict__ &logp_buf,
+                                                  float *__restrict__ &u_dbg) {
+    const size_t c = (size_t)col0;
+    pos += c; vel += c; ints += c;
+    cur_obs += c * kObsDim; cur_term += c; cur_trunc += c;
+    if (last_val) last_val += c;
+    obs_buf += c * kObsDim;                                  // full observation rows only (the launchers refuse poses)
+    act_buf += c; rew_buf += c; val_buf += c; term_buf += c; trunc_buf += c; logp_buf += c;
+    if (u_dbg) u_dbg += c;
+}
+
 // Packing of the reference network's parameters (nn.Linear layout: weight [out][in], lib/model.py:10-26) into the
 // two layouts above, one thread per packed float: runs after every optimiser epoch, so it is one launch and not
 // forty small tensor operations (13 ms per epoch in PyTorch, as much as the rollout of 32,768 envs x 1,024 steps).
-template <bool TC>
+// POP (carenv_pack_policy_pop): blockIdx.y = member p of stacked parameters [P][...], output block p of [P][floats].
+template <bool TC, bool POP = false>
 __global__ void __launch_bounds__(256)
 k_pack_policy(const float *__restrict__ w1a, const float *__restrict__ b1a, const float *__restrict__ w2a,
               const float *__restrict__ b2a, const float *__restrict__ w1c, const float *__restrict__ b1c,
               const float *__restrict__ w2c, const float *__restrict__ b2c, float *__restrict__ out) {
+    if constexpr (POP) {
+        const ppo::Params m = member_params(ppo::Params{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c}, blockIdx.y);
+        w1a = m.w1a; b1a = m.b1a; w2a = m.w2a; b2a = m.b2a; w1c = m.w1c; b1c = m.b1c; w2c = m.w2c; b2c = m.b2c;
+        out += (size_t)blockIdx.y * (TC ? kTcWeightFloats : kPolicyFloats);
+    }
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     float v = 0.0f;
     if (TC) {
@@ -259,7 +293,10 @@ __device__ __forceinline__ void second_layer_chunk16_x2(uint32_t a, const float 
     }
 }
 
-template <int U, bool TAB>
+// POP (carenv_policy_rollout_tc_pop, single-track U only): blockIdx.y = member p, as in k_policy_rollout_warp<true>:
+// packed weights [P][kTcWeightFloats], seeds[p], n_envs environments per member at columns p * n_envs + e of arrays
+// with row_stride columns.
+template <int U, bool TAB, bool POP = false>
 __global__ void __launch_bounds__(256 + 128 + 32, 1)
 k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, const float *__restrict__ weights,
                      int n_envs, int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
@@ -270,9 +307,20 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
                      float *__restrict__ trunc_buf, float *__restrict__ logp_buf, float *__restrict__ last_val,
                      float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode,
                      const float4 *__restrict__ den4, int n_pairs, int row_f4, const TrackParams *__restrict__ mt_params,
-                     const Tables *__restrict__ mt_tables, int n_tracks, const int *__restrict__ track_ids) {
+                     const Tables *__restrict__ mt_tables, int n_tracks, const int *__restrict__ track_ids,
+                     const unsigned long long *__restrict__ seeds, int row_stride) {
+    static_assert(!POP || U != 0, "populations run on one track");
     constexpr int kGroups = 2, kCols = 256, kHalf = 128, kEnvThreads = kGroups * 128, kCriticThreads = 128;
     extern __shared__ __align__(16) unsigned char smem[];
+    int stride = n_envs;
+    if constexpr (POP) {
+        const int p = blockIdx.y;
+        weights += (size_t)p * kTcWeightFloats;
+        seed = seeds[p];
+        stride = row_stride;
+        pop_shift_columns(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
+                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg);
+    }
     // [tables | pad to a 128-byte boundary | weights | A tiles (hi, lo per group) | exchanged partial logits [group][128][12]
     //  | TAB: the denominator table of k_rollout_tab, ONE copy whose rows are skewed by 16 bytes (row_f4 is odd in
     //    16-byte units): threads of a quarter warp with different headings mostly hit different bank groups (about
@@ -381,8 +429,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
             }
             const float value_a = (Va.x + Va.y) + bias, value_b = (Vb.x + Vb.y) + bias;
             if (f < n_steps) {
-                if (ea_raw < n_envs) val_buf[(size_t)f * (size_t)n_envs + (size_t)ea_raw] = value_a;
-                if (eb_raw < n_envs) val_buf[(size_t)f * (size_t)n_envs + (size_t)eb_raw] = value_b;
+                if (ea_raw < n_envs) val_buf[(size_t)f * (size_t)stride + (size_t)ea_raw] = value_a;
+                if (eb_raw < n_envs) val_buf[(size_t)f * (size_t)stride + (size_t)eb_raw] = value_b;
             } else {                                                 // bootstrap values of the final observations
                 if (ea_raw < n_envs) last_val[ea_raw] = value_a;
                 if (eb_raw < n_envs) last_val[eb_raw] = value_b;
@@ -443,7 +491,7 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
         };
 
         for (int t = 0; t < n_steps; ++t) {
-            const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
+            const size_t idx = (size_t)t * (size_t)stride + (size_t)e;
             const uint32_t par = (uint32_t)(t & 1);
             write_row(t);
             const unsigned long long gs = step0 + (unsigned long long)t;
@@ -550,6 +598,12 @@ constexpr int kWpRow = 20;                                   // first-layer row:
 constexpr int kWpW2 = 12;                                    // actor second-layer row: W2[0..8][j], pad
 constexpr int kWpFloats = 2 * kHidden * kWpRow + kHidden * kWpW2 + kHidden + 12;   // 13,580 floats = 54,320 B
 
+// POP (carenv_policy_rollout_warp_pop): a population of independent members, blockIdx.y = member p.  W points at the
+// stacked parameters [P][...] of all members, seeds[p] keys member p's random stream, n_envs is the member's
+// environment count and env e of member p is global column p * n_envs + e of every [N] and [T, N] array
+// (row_stride = N).  The CTA stages member p's parameters and otherwise runs the single-policy code unchanged, so
+// member p's rows are those of k_policy_rollout_warp<false> on that member alone with env_offset = 0.
+template <bool POP>
 __global__ void __launch_bounds__(128)
 k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, const ppo::Params W, int n_envs, int n_steps,
                       int env_offset, unsigned long long seed, unsigned long long step0, double2 *__restrict__ pos,
@@ -558,23 +612,34 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
                       float *__restrict__ obs_buf, float *__restrict__ act_buf, float *__restrict__ rew_buf,
                       float *__restrict__ val_buf, float *__restrict__ term_buf, float *__restrict__ trunc_buf,
                       float *__restrict__ logp_buf, float *__restrict__ last_val, float *__restrict__ u_dbg,
-                      unsigned long long *stats, int table_bytes, int obs_mode) {
+                      unsigned long long *stats, int table_bytes, int obs_mode, const unsigned long long *__restrict__ seeds,
+                      int row_stride) {
     extern __shared__ __align__(16) unsigned char smem[];
+    ppo::Params Wm = W;
+    int stride = n_envs;
+    if constexpr (POP) {
+        const int p = blockIdx.y;
+        Wm = member_params(W, p);
+        seed = seeds[p];
+        stride = row_stride;
+        pop_shift_columns(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
+                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg);
+    }
     float *sw1 = reinterpret_cast<float *>(smem + table_bytes);   // [512][20]: rows 0..255 actor, 256..511 critic
     float *sw2 = sw1 + 2 * kHidden * kWpRow;                      // [256][12]
     float *swc = sw2 + kHidden * kWpW2;                           // [256]
     float *stail = swc + kHidden;                                 // b2a[0..8], 0, b2c, 0
     for (int i = threadIdx.x; i < 2 * kHidden * kWpRow; i += blockDim.x) {
         const int r = i / kWpRow, c = i - r * kWpRow, j = r & (kHidden - 1);
-        const float *w1 = r < kHidden ? W.w1a : W.w1c, *b1 = r < kHidden ? W.b1a : W.b1c;
+        const float *w1 = r < kHidden ? Wm.w1a : Wm.w1c, *b1 = r < kHidden ? Wm.b1a : Wm.b1c;
         sw1[i] = c < kObsDim ? w1[j * kObsDim + c] : (c == kObsDim ? b1[j] : 0.0f);
     }
     for (int i = threadIdx.x; i < kHidden * kWpW2; i += blockDim.x) {
         const int j = i / kWpW2, q = i - j * kWpW2;
-        sw2[i] = q < kActions ? W.w2a[q * kHidden + j] : 0.0f;
+        sw2[i] = q < kActions ? Wm.w2a[q * kHidden + j] : 0.0f;
     }
-    for (int i = threadIdx.x; i < kHidden; i += blockDim.x) swc[i] = W.w2c[i];
-    if (threadIdx.x < 12) stail[threadIdx.x] = threadIdx.x < kActions ? W.b2a[threadIdx.x] : (threadIdx.x == 10 ? W.b2c[0] : 0.0f);
+    for (int i = threadIdx.x; i < kHidden; i += blockDim.x) swc[i] = Wm.w2c[i];
+    if (threadIdx.x < 12) stail[threadIdx.x] = threadIdx.x < kActions ? Wm.b2a[threadIdx.x] : (threadIdx.x == 10 ? Wm.b2c[0] : 0.0f);
     const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
     const int e = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
@@ -645,7 +710,7 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
 
     PolicyOut po;
     for (int t = 0; t < n_steps; ++t) {
-        const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
+        const size_t idx = (size_t)t * (size_t)stride + (size_t)e;
         forward(po, true);
         const unsigned long long gs = step0 + (unsigned long long)t;
         const uint32_t bits = philox_uniform_bits((uint32_t)seed, (uint32_t)(seed >> 32), gid, (uint32_t)gs,
