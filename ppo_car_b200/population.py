@@ -36,6 +36,10 @@ DEFAULTS = {"learning_rate": 3e-4, "learning_rate_decay": 0.99, "clip_ratio": 0.
             "max_grad_norm": 1.0}
 STATE_KEYS = ("actor.0.weight", "actor.0.bias", "actor.2.weight", "actor.2.bias",
               "critic.0.weight", "critic.0.bias", "critic.2.weight", "critic.2.bias")
+# the largest seed s whose minibatch generator seed s * 1000 + 1 (PopulationPPOUpdate, as train_ppo seeds rank 0) fits
+# in the 64 bits a torch.Generator takes
+MAX_SEED = (2 ** 64 - 2) // 1000                    # 18446744073709551
+SEED_RANGE = f"seeds must be in 0 .. {MAX_SEED} (the minibatch generator of seed s is seeded s * 1000 + 1 < 2^64)"
 
 
 def _p(t):
@@ -56,8 +60,8 @@ def parse_seeds(spec: str) -> list[int]:
             seeds.extend(range(int(a), int(b) + 1))
         else:
             seeds.append(int(part))
-    if any(s < 0 or s >= 2 ** 63 for s in seeds):
-        raise ValueError("seeds must be in 0 .. 2^63 - 1")
+    if any(s < 0 or s > MAX_SEED for s in seeds):
+        raise ValueError(SEED_RANGE)
     if len(set(seeds)) != len(seeds):
         raise ValueError(f"--seeds {spec!r} repeats a seed")
     return seeds
@@ -96,8 +100,8 @@ class Population:
             raise ValueError("a population needs at least one member")
         if int(n_envs_per_member) < 1:
             raise ValueError("n_envs_per_member must be at least 1")
-        if any(s < 0 or s >= 2 ** 63 for s in seeds):
-            raise ValueError("seeds must be in 0 .. 2^63 - 1")
+        if any(s < 0 or s > MAX_SEED for s in seeds):
+            raise ValueError(SEED_RANGE)
         hp = hparams if isinstance(hparams, (list, tuple)) else [hparams or {}] * len(seeds)
         if len(hp) != len(seeds):
             raise ValueError("hparams must be one dict or one dict per member")

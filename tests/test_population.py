@@ -37,7 +37,8 @@ def test_parse_seeds():
     assert popmod.parse_seeds("0,5,9") == [0, 5, 9]
     assert popmod.parse_seeds("0-2,7") == [0, 1, 2, 7]
     assert popmod.parse_seeds("4") == [4]
-    for bad in ("", "3-1", "1,1", "a", "0,,1", "-1"):
+    assert popmod.parse_seeds("18446744073709551") == [popmod.MAX_SEED]       # the largest s with s * 1000 + 1 < 2^64
+    for bad in ("", "3-1", "1,1", "a", "0,,1", "-1", "18446744073709552"):
         with pytest.raises(ValueError):
             popmod.parse_seeds(bad)
 
@@ -76,6 +77,7 @@ def test_members_are_sharded_over_ranks():
     (["--seeds", "3-1"], "seed range"),
     (["--learning-rate", ","], "empty"),
     (["--batch-size", "2000"], "--batch-size"),
+    (["--seeds", "18446744073709552"], "0 .. 18446744073709551"),     # s * 1000 + 1 overflows 64 bits
 ])
 def test_refusals_come_before_any_device_work(argv, words, monkeypatch):
     monkeypatch.setattr(torch.cuda, "set_device", lambda *a: pytest.fail("device work before the refusal"))
@@ -92,6 +94,8 @@ def test_population_refuses_bad_arguments():
         Population([0, 1], 4, [{}])
     with pytest.raises(ValueError):
         Population([0], 4, {"gamma": 0.9})
+    with pytest.raises(ValueError, match="18446744073709551"):
+        Population([popmod.MAX_SEED + 1], 4)
     with pytest.raises(ValueError):
         PopulationPPOUpdate(SimpleNamespace(), 1)
 
