@@ -370,7 +370,14 @@ int carenv_ppo_epoch(float *w1_actor, float *b1_actor, float *w2_actor, float *b
  *       Deterministic, and member p's results do not depend on the other members; not bit-identical to
  *       carenv_ppo_epoch (another reduction order).  Needs no workspace.
  *   carenv_ppo_epoch_pop_resident_clusters   how many clusters of the update kernel the current device keeps resident
- *       at once (cudaOccupancyMaxActiveClusters). */
+ *       at once (cudaOccupancyMaxActiveClusters).
+ *   carenv_policy_eval_pop   carenv_policy_eval of every member in ONE launch: n_episodes_per_member episodes (global
+ *       ids episode0 .. episode0 + n - 1) of each member's actor (w1_actor .. b2_actor as above) on the handle's track.
+ *       Member p samples with seeds[p] (device uint64 [P]) and writes records [P][n] (block p) and, for its first
+ *       n_trace episodes, trace_actions / trace_u [P][n_trace][1000] (block p), so member p's records and traces
+ *       equal carenv_policy_eval of member p with seed seeds[p].  Refuses n_members outside 1..65535, a negative
+ *       n_episodes_per_member or n_trace, n_trace > 0 without trace_actions and null pointers (CARENV_E_INVAL) and
+ *       tracks over 128 wall segments (CARENV_E_TRACK); 0 episodes launch nothing. */
 int carenv_pack_policy_pop(int tensor_cores, int n_members, const float *w1_actor, const float *b1_actor,
                            const float *w2_actor, const float *b2_actor, const float *w1_critic, const float *b1_critic,
                            const float *w2_critic, const float *b2_critic, float *packed_out, void *stream);
@@ -397,6 +404,11 @@ int carenv_ppo_epoch_pop(int n_members, float *w1_actor, float *b1_actor, float 
                          const float *vf_coef, const float *ent_coef, const float *max_grad_norm, double beta1,
                          double beta2, double eps, float *exp_avg, float *exp_avg_sq, int *step, float *sums4,
                          void *stream);
+int carenv_policy_eval_pop(void *handle, int n_members, const float *w1_actor, const float *b1_actor,
+                           const float *w2_actor, const float *b2_actor, long long n_episodes_per_member,
+                           unsigned long long episode0, int greedy, const unsigned long long *seeds,
+                           carenv_eval_record *records, int n_trace, unsigned char *trace_actions, float *trace_u,
+                           void *stream);
 
 /* Test hook for the tensor-core building blocks (csrc/tc_mlp.cuh): D[128][256] = A[128][24] * B[256][24]^T,
  * tcgen05.mma kind::tf32 with the accumulator in tensor memory; device pointers, row-major float32. */

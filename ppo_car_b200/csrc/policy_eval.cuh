@@ -21,6 +21,10 @@
 //               and reset observation of track episode_tracks[i] (as k_reset_multi) and steps with env_step<0> on that
 //               track's TrackParams / Tables in global memory (as k_rollout_multi); nothing else changes, so episode i
 //               on track k gives the record k_policy_eval gives on track k alone.
+//   k_policy_eval<U, true>   a population (carenv_policy_eval_pop): blockIdx.y = member p.  The CTA stages member p's
+//               actor from the stacked [P][...] tensors and keys its random stream with seeds[p]; member p claims from
+//               counter[p] and writes its own blocks of the records and traces.  The rest is the single-member code,
+//               so member p's records are those of k_policy_eval<U> on member p alone.
 #pragma once
 
 extern "C++" {
@@ -68,29 +72,43 @@ __device__ __forceinline__ void actor_forward(const float (&obs)[kPolicyObs], co
 
 // U == 0 keeps its 16 table pointers and the track pointer in registers (the single-track tables are shared-memory
 // offsets): 3 CTAs per SM, 168 registers, where 4 CTAs (128 registers) spill.
-template <int U>
+template <int U, bool POP = false>
 __global__ void __launch_bounds__(kEvalBlock, U == 0 ? 3 : 4)
 k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::Params W, long long n_episodes,
               unsigned long long episode0, int greedy, unsigned long long seed,
               carenv_eval_record *__restrict__ records, int n_trace, unsigned char *__restrict__ trace_actions,
               float *__restrict__ trace_u, unsigned long long *counter, unsigned long long *stats, int table_bytes,
               const TrackParams *__restrict__ mt_params, const Tables *__restrict__ mt_tables, int n_tracks,
-              const int *__restrict__ episode_tracks) {
+              const int *__restrict__ episode_tracks, const unsigned long long *__restrict__ seeds) {
+    static_assert(!POP || U != 0, "populations play on one track");
     extern __shared__ __align__(16) unsigned char smem[];
+    const float *w1a = W.w1a, *b1a = W.b1a, *w2a = W.w2a, *b2a = W.b2a;
+    // POP: member p's block of a [P][per] array starts at p * per.  The record, trace and counter offsets are formed
+    // where they are used, not added to the base pointers up front: held across the step loop, those pointers made
+    // k_policy_eval<4, true> spill at the 128 registers of 4 CTAs per SM.
+    auto member_block = [&](size_t per) -> size_t {
+        if constexpr (POP) return (size_t)blockIdx.y * per;
+        else return 0;
+    };
+    if constexpr (POP) {
+        const size_t p = blockIdx.y;           // the actor only: the critic pointers are null
+        w1a += p * kHidden * kObsDim; b1a += p * kHidden; w2a += p * kActions * kHidden; b2a += p * kActions;
+        seed = seeds[p];
+    }
     float *sw = reinterpret_cast<float *>(smem + table_bytes);
     for (int i = threadIdx.x; i < (kHidden / 2) * kActorPairFloats; i += blockDim.x) {
         const int p = i / kActorPairFloats, c = i - p * kActorPairFloats;   // as k_pack_policy<false>, actor half
         float v = 0.0f;
-        if (c < 36) v = W.w1a[(2 * p + (c & 1)) * kObsDim + (c >> 1)];
-        else if (c < 38) v = W.b1a[2 * p + (c - 36)];
+        if (c < 36) v = w1a[(2 * p + (c & 1)) * kObsDim + (c >> 1)];
+        else if (c < 38) v = b1a[2 * p + (c - 36)];
         else if (c >= 40) {
             const int d = c - 40, q = d >> 2, sft = (d >> 1) & 1, row = 2 * q + (d & 1);
-            v = row < kActions ? W.w2a[row * kHidden + 2 * p + sft] : 0.0f;
+            v = row < kActions ? w2a[row * kHidden + 2 * p + sft] : 0.0f;
         }
         sw[i] = v;
     }
     if (threadIdx.x < kEvalTail)
-        sw[(kHidden / 2) * kActorPairFloats + threadIdx.x] = threadIdx.x < kActions ? W.b2a[threadIdx.x] : 0.0f;
+        sw[(kHidden / 2) * kActorPairFloats + threadIdx.x] = threadIdx.x < kActions ? b2a[threadIdx.x] : 0.0f;
     // U == 0 (several tracks): nothing is staged, every lane reads its episode's track tables
     const Tables T = U == 0 ? Tables{} : stage_tables(G, P.n_gates, P.n_seg, smem);   // ends with __syncthreads()
     if constexpr (U == 0) __syncthreads();
@@ -125,7 +143,7 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
         if (!m) return;
         const int leader = __ffs(m) - 1;
         unsigned long long base = 0;
-        if (lane == leader) base = atomicAdd(counter, (unsigned long long)__popc(m));
+        if (lane == leader) base = atomicAdd(counter + member_block(1), (unsigned long long)__popc(m));
         base = __shfl_sync(0xffffffffu, base, leader);
         if (want) {
             const unsigned long long i = base + (unsigned long long)__popc(m & lt_mask);
@@ -168,7 +186,7 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
         else env_step<U>(s, a, 1.0, P, T, o, stats);
         if (live) {
             if (ep < n_trace) {
-                const size_t ti = (size_t)ep * kTimeLimit + (size_t)step;
+                const size_t ti = member_block((size_t)n_trace * kTimeLimit) + (size_t)ep * kTimeLimit + (size_t)step;
                 trace_actions[ti] = (unsigned char)a;
                 if (trace_u && !greedy) trace_u[ti] = u;
             }
@@ -182,7 +200,7 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
                 r.ret = ret;
                 r.length = o.time_passed; r.gates = o.gates_passed; r.laps = laps; r.first_lap = first_lap;
                 r.outcome = o.terminated ? 1 : 2; r.pad = 0;
-                records[ep] = r;
+                records[member_block((size_t)n_episodes) + ep] = r;
                 ep = -1;
             }
         }
@@ -196,18 +214,20 @@ k_policy_eval(const __grid_constant__ TrackParams P, const Tables G, const ppo::
 }  // extern "C++"
 
 /* ---- C ABI (include/carenv_b200.h) ---- */
-// One launch of an evaluation kernel: a persistent grid of at most one wave (CARENV_EVAL_CTAS > 0 caps it further,
-// a test hook so that a few slots play many episodes each) and a claim counter that lives for the call.  `m` and
-// `episode_tracks` only for the multi-track instantiation (else null).
+// One launch of an evaluation kernel: a persistent grid (ctas_per_member, n_members) of at most one wave in all
+// (CARENV_EVAL_CTAS > 0 caps ctas_per_member further, a test hook so that a few slots play many episodes each) and one
+// claim counter per member that lives for the call.  With more members than one wave holds, each member gets one CTA
+// and the later CTAs wait to become resident: CTAs never wait for each other.  `m` and `episode_tracks` only for the
+// multi-track instantiation, `seeds` only for the population instantiations (else null).
 static int launch_eval(void (*kern)(const TrackParams, const Tables, const ppo::Params, long long, unsigned long long,
                                     int, unsigned long long, carenv_eval_record *, int, unsigned char *, float *,
                                     unsigned long long *, unsigned long long *, int, const TrackParams *,
-                                    const Tables *, int, const int *),
+                                    const Tables *, int, const int *, const unsigned long long *),
                        int device, const TrackParams &P, const Tables &G, int table_bytes, const MultiTrack *m,
-                       const int32_t *episode_tracks, const ppo::Params &W, long long n_episodes,
-                       unsigned long long episode0, int greedy, unsigned long long seed, carenv_eval_record *records,
-                       int n_trace, unsigned char *trace_actions, float *trace_u, unsigned long long *stats,
-                       cudaStream_t st) {
+                       const int32_t *episode_tracks, const ppo::Params &W, int n_members, long long n_episodes,
+                       unsigned long long episode0, int greedy, unsigned long long seed,
+                       const unsigned long long *seeds, carenv_eval_record *records, int n_trace,
+                       unsigned char *trace_actions, float *trace_u, unsigned long long *stats, cudaStream_t st) {
     const size_t smem = (size_t)table_bytes + sizeof(float) * kEvalFloats;
     const char *cap_env = getenv("CARENV_EVAL_CTAS");
     const long long cap = cap_env ? atoll(cap_env) : 0;
@@ -217,24 +237,33 @@ static int launch_eval(void (*kern)(const TrackParams, const Tables, const ppo::
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kEvalBlock, smem));
     long long grid = (n_episodes + kEvalBlock - 1) / kEvalBlock;
     const long long resident = (long long)sms * (per_sm > 0 ? per_sm : 1);
-    if (grid > resident) grid = resident;
+    const long long wave = resident / n_members > 1 ? resident / n_members : 1;
+    if (grid > wave) grid = wave;
     if (cap > 0 && grid > cap) grid = cap;
-    // The claim counter lives for one call, allocated and freed in stream order: calls on one handle may run
+    // The claim counters live for one call, allocated and freed in stream order: calls on one handle may run
     // concurrently on different streams.
+    const size_t counter_bytes = sizeof(unsigned long long) * (size_t)n_members;
     unsigned long long *counter = nullptr;
-    CU(cudaMallocAsync(reinterpret_cast<void **>(&counter), sizeof(unsigned long long), st));
-    cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st);
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&counter), counter_bytes, st));
+    cudaError_t e = cudaMemsetAsync(counter, 0, counter_bytes, st);
     if (e == cudaSuccess) {
-        kern<<<(unsigned)grid, kEvalBlock, smem, st>>>(P, G, W, n_episodes, episode0, greedy ? 1 : 0, seed, records,
-                                                      n_trace, trace_actions, trace_u, counter, stats, table_bytes,
-                                                      m ? m->d_params : nullptr, m ? m->d_tables : nullptr,
-                                                      m ? m->n_tracks : 0, episode_tracks);
+        kern<<<dim3((unsigned)grid, (unsigned)n_members), kEvalBlock, smem, st>>>(
+            P, G, W, n_episodes, episode0, greedy ? 1 : 0, seed, records, n_trace, trace_actions, trace_u, counter,
+            stats, table_bytes, m ? m->d_params : nullptr, m ? m->d_tables : nullptr, m ? m->n_tracks : 0,
+            episode_tracks, seeds);
         e = cudaGetLastError();
     }
     const cudaError_t ef = cudaFreeAsync(counter, st);
     if (e != cudaSuccess) return cuda_fail(e, "k_policy_eval launch");
     CU(ef);
     return 0;
+}
+
+// The instantiation for the handle's track, as carenv_policy_rollout chooses it: U = 4, 2 or 1.
+static int eval_unroll(const Handle *h) {
+    int U = h->force_generic ? 1 : h->host.P.unroll4;
+    if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
+    return U;
 }
 
 int carenv_policy_eval(void *handle, const float *w1a, const float *b1a, const float *w2a, const float *b2a,
@@ -253,12 +282,39 @@ int carenv_policy_eval(void *handle, const float *w1a, const float *b1a, const f
     DeviceGuard guard(h->device);
     if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
     const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
-    int U = h->force_generic ? 1 : h->host.P.unroll4;   // as carenv_policy_rollout: instantiated for 4, 2, 1
-    if (h->max_unroll > 0 && U > h->max_unroll) U = (U % h->max_unroll == 0) ? h->max_unroll : 1;
+    const int U = eval_unroll(h);
     const ppo::Params W{w1a, b1a, w2a, b2a, nullptr, nullptr, nullptr, nullptr};
     auto kern = U == 4 ? k_policy_eval<4> : (U == 2 ? k_policy_eval<2> : k_policy_eval<1>);
-    return launch_eval(kern, h->device, h->host.P, h->dev, table_bytes, nullptr, nullptr, W, n_episodes, episode0,
-                       greedy, seed, records, n_trace, trace_actions, trace_u, h->d_stats,
+    return launch_eval(kern, h->device, h->host.P, h->dev, table_bytes, nullptr, nullptr, W, 1, n_episodes, episode0,
+                       greedy, seed, nullptr, records, n_trace, trace_actions, trace_u, h->d_stats,
+                       static_cast<cudaStream_t>(stream));
+}
+
+/* carenv_policy_eval for a population (k_policy_eval<U, true>): n_episodes episodes of each of n_members actors
+ * stacked [P][...] in one launch; member p plays with seeds[p] and writes records [p][n_episodes] and traces
+ * [p][n_trace][1000], the records and traces carenv_policy_eval gives for member p alone with seeds[p]. */
+int carenv_policy_eval_pop(void *handle, int n_members, const float *w1a, const float *b1a, const float *w2a,
+                           const float *b2a, long long n_episodes, unsigned long long episode0, int greedy,
+                           const unsigned long long *seeds, carenv_eval_record *records, int n_trace,
+                           unsigned char *trace_actions, float *trace_u, void *stream) {
+    Handle *h = static_cast<Handle *>(handle);
+    if (!h) return fail(CARENV_E_INVAL, "null handle");
+    if (n_members <= 0 || n_members > 65535) return fail(CARENV_E_INVAL, "n_members must be in 1..65535");
+    if (n_episodes < 0) return fail(CARENV_E_INVAL, "negative n_episodes");
+    if (!w1a || !b1a || !w2a || !b2a || !seeds || !records) return fail(CARENV_E_INVAL, "null pointer");
+    if (n_trace < 0) return fail(CARENV_E_INVAL, "negative n_trace");
+    if (n_trace > 0 && !trace_actions) return fail(CARENV_E_INVAL, "n_trace > 0 needs trace_actions");
+    if (h->host.P.n_seg > kMaxSeg)
+        return fail(CARENV_E_TRACK, "policy evaluation supports tracks with at most 128 wall segments");
+    if (n_episodes == 0) return 0;
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return fail(CARENV_E_NOGPU, "cannot select the handle's CUDA device");
+    const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
+    const int U = eval_unroll(h);
+    const ppo::Params W{w1a, b1a, w2a, b2a, nullptr, nullptr, nullptr, nullptr};
+    auto kern = U == 4 ? k_policy_eval<4, true> : (U == 2 ? k_policy_eval<2, true> : k_policy_eval<1, true>);
+    return launch_eval(kern, h->device, h->host.P, h->dev, table_bytes, nullptr, nullptr, W, n_members, n_episodes,
+                       episode0, greedy, 0, seeds, records, n_trace, trace_actions, trace_u, h->d_stats,
                        static_cast<cudaStream_t>(stream));
 }
 
@@ -283,6 +339,6 @@ int carenv_policy_eval_multi(void *multi, const int32_t *episode_tracks, const f
     if (n_episodes == 0) return 0;
     static const TrackParams kNoTrack{};                     // P and G of the single-track instantiations: unused
     const ppo::Params W{w1a, b1a, w2a, b2a, nullptr, nullptr, nullptr, nullptr};
-    return launch_eval(k_policy_eval<0>, m->device, kNoTrack, Tables{}, 0, m, episode_tracks, W, n_episodes, episode0,
-                       greedy, seed, records, n_trace, trace_actions, trace_u, m->d_stats, st);
+    return launch_eval(k_policy_eval<0>, m->device, kNoTrack, Tables{}, 0, m, episode_tracks, W, 1, n_episodes,
+                       episode0, greedy, seed, nullptr, records, n_trace, trace_actions, trace_u, m->d_stats, st);
 }

@@ -13,6 +13,9 @@ calls or ranks at any boundary and gives the same records.
 
 Several tracks (``--track big_track,track``, or a ``MultiTrackVecEnv``): episode ``g`` plays on track ``g % n_tracks``
 by default (``carenv_policy_eval_multi``, still one launch), and the summary gains ``"by_track"``.
+
+Several actors (:func:`evaluate_population`, ``--checkpoint a.dat,b.dat,...``): the same episode ids of every actor in
+one launch (``carenv_policy_eval_pop``); each actor's records are those ``evaluate_policy`` gives it alone.
 """
 from __future__ import annotations
 
@@ -190,6 +193,59 @@ def evaluate_policy(env, actor, n_episodes: int, greedy: bool = False, seed: int
     return EvalResult(records, trace_actions, trace_u)
 
 
+def evaluate_population(env, actor_params, n_episodes: int, greedy: bool = False, seeds=0, episode0: int = 0,
+                        trace: int = 0) -> list[EvalResult]:
+    """:func:`evaluate_policy` of P actors in one launch (``carenv_policy_eval_pop``): episodes ``episode0 ..
+    episode0 + n_episodes - 1`` of every member on ``env``'s track.  ``actor_params`` are the four stacked actor
+    tensors ``w1 [P, 256, 18], b1 [P, 256], w2 [P, 9, 256], b2 [P, 9]`` (``Population.params[:4]``), contiguous float32
+    on ``env.device``; ``seeds`` is one seed for every member or a list of P.  Returns one :class:`EvalResult` per
+    member whose records (views of one ``[P, n, 8]`` tensor) and traces equal ``evaluate_policy`` of that member's
+    actor with its seed.  Populations play on one track: a :class:`MultiTrackVecEnv` is refused."""
+    from .vec_env import MultiTrackVecEnv
+
+    if isinstance(env, MultiTrackVecEnv):
+        raise ValueError("evaluate_population plays on one track; a MultiTrackVecEnv is not supported")
+    n_episodes, trace = int(n_episodes), int(trace)
+    if n_episodes < 0 or trace < 0:
+        raise ValueError("n_episodes and trace must be >= 0")
+    if not 0 <= int(episode0) < 2 ** 64:
+        raise ValueError("episode0 must fit in 64 bits")
+    dev = env.device
+    params = list(actor_params)
+    P = params[0].shape[0] if len(params) == 4 and params[0].dim() == 3 else 0
+    if [tuple(p.shape) for p in params] != [(P, HIDDEN, OBS), (P, HIDDEN), (P, ACTIONS, HIDDEN), (P, ACTIONS)]:
+        raise ValueError("actor_params must be the stacked reference actor tensors [P, 256, 18], [P, 256], "
+                         "[P, 9, 256], [P, 9]")
+    if not 1 <= P <= 65535:
+        raise ValueError("a population has 1 .. 65535 members")
+    if any(p.dtype != torch.float32 or not p.is_contiguous() or p.device != dev for p in params):
+        raise ValueError(f"actor parameters must be contiguous float32 tensors on {dev}")
+    seeds = [int(seeds)] * P if isinstance(seeds, int) else [int(s) for s in seeds]
+    if len(seeds) != P:
+        raise ValueError(f"expected one seed or {P} seeds, got {len(seeds)}")
+    seeds = [s & (2 ** 64 - 1) for s in seeds]                 # as evaluate_policy
+    records = torch.empty((P, n_episodes, RECORD_INT32), dtype=torch.int32, device=dev)
+    n_trace = min(trace, n_episodes)
+    trace_actions = trace_u = None
+    if trace:
+        trace_actions = torch.full((P, n_trace, TIME_LIMIT), 255, dtype=torch.uint8, device=dev)
+        if not greedy:
+            trace_u = torch.full((P, n_trace, TIME_LIMIT), float("nan"), dtype=torch.float32, device=dev)
+    results = [EvalResult(records[p], None if trace_actions is None else trace_actions[p],
+                          None if trace_u is None else trace_u[p]) for p in range(P)]
+    if n_episodes == 0:
+        return results
+    # a pinned, stream-ordered copy: a pageable one would wait for the work already queued on the device
+    seeds_dev = torch.tensor([s - 2 ** 64 if s >= 2 ** 63 else s for s in seeds], dtype=torch.int64).pin_memory()
+    with torch.cuda.device(dev):
+        seeds_dev = seeds_dev.to(dev, non_blocking=True)
+        rc = _lib.lib().carenv_policy_eval_pop(env._handle, P, *[_p(p.detach()) for p in params], n_episodes,
+                                               int(episode0), int(bool(greedy)), _p(seeds_dev), _p(records), n_trace,
+                                               _p(trace_actions), _p(trace_u), env._stream())
+    _lib.check(rc, "carenv_policy_eval_pop")
+    return results
+
+
 def load_checkpoint(path: str):
     """The state dict ``train_ppo`` saves (model.dat / checkpoint_{epoch}.dat, the reference Agent's keys
     actor.0.weight ... critic.2.bias), loaded strictly into a CPU ActorCritic."""
@@ -200,9 +256,22 @@ def load_checkpoint(path: str):
     return net
 
 
+def checkpoint_list(spec: str) -> list[str]:
+    """``--checkpoint``: one path (kept whole when it names a file, commas included) or a comma-separated list."""
+    if os.path.exists(spec):
+        return [spec]
+    paths = [c.strip() for c in spec.split(",")]
+    if not all(paths):
+        raise SystemExit(f"empty entry in --checkpoint {spec!r}")
+    return paths
+
+
 def parse_args(argv=None):
     p = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
-    p.add_argument("--checkpoint", required=True, help="model.dat / checkpoint_{epoch}.dat written by train_ppo")
+    p.add_argument("--checkpoint", required=True,
+                   help="model.dat / checkpoint_{epoch}.dat written by train_ppo; a comma-separated list (e.g. every "
+                        "member_*/model.dat of a population) scores all of them in one launch with the same --seed and "
+                        "prints one summary per checkpoint under \"checkpoints\"")
     p.add_argument("--track", default="big_track",
                    help="track name shipped with the package or a JSON path; a comma-separated list plays episode g on "
                         "track g %% n_tracks and adds per-track summaries under \"by_track\"")
@@ -220,6 +289,11 @@ def main(argv=None) -> dict:
     from .shard import shard_range
 
     args = parse_args(argv)
+    names = args.track.split(",")
+    ckpts = checkpoint_list(args.checkpoint)
+    if len(ckpts) > 1 and len(names) > 1:
+        raise SystemExit("several checkpoints are scored on one track; pass several checkpoints or several tracks, "
+                         "not both")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -228,25 +302,35 @@ def main(argv=None) -> dict:
     if world > 1 and not dist.is_initialized():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
-    names = args.track.split(",")
     paths = [t if os.path.exists(t) else builtin_track(t) for t in names]
     if len(paths) == 1:
         env = VecCarEnv(1, paths[0], device=dev)
     else:
         env = MultiTrackVecEnv(track_paths=paths, track_ids=[0], device=dev)
-    actor = load_checkpoint(args.checkpoint).actor.to(dev)
     lo, hi = shard_range(args.episodes, world, rank)            # every rank plays its contiguous share of the ids
-    res = evaluate_policy(env, actor, hi - lo, greedy=args.greedy, seed=args.seed, episode0=lo)
-    sums = res.sums()
-    by_track = res.sums_by_track() if len(paths) > 1 else None
-    if world > 1:
-        dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+    if len(ckpts) > 1:
+        actors = [load_checkpoint(c).actor for c in ckpts]
+        stacked = [torch.stack([getattr(a[i], k).detach() for a in actors]).to(dev).contiguous()
+                   for i, k in ((0, "weight"), (0, "bias"), (2, "weight"), (2, "bias"))]
+        results = evaluate_population(env, stacked, hi - lo, greedy=args.greedy, seeds=args.seed, episode0=lo)
+        sums = torch.stack([r.sums() for r in results])         # [P, 10]
+        if world > 1:
+            dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+        out = {"checkpoints": [{"checkpoint": c, "track": args.track, "greedy": bool(args.greedy), "seed": args.seed,
+                                **r.summary(s)} for c, r, s in zip(ckpts, results, sums)]}
+    else:
+        actor = load_checkpoint(args.checkpoint).actor.to(dev)
+        res = evaluate_policy(env, actor, hi - lo, greedy=args.greedy, seed=args.seed, episode0=lo)
+        sums = res.sums()
+        by_track = res.sums_by_track() if len(paths) > 1 else None
+        if world > 1:
+            dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+            if by_track is not None:
+                dist.all_reduce(by_track, op=dist.ReduceOp.SUM)
+        out = {"checkpoint": args.checkpoint, "track": args.track, "greedy": bool(args.greedy), "seed": args.seed,
+               **res.summary(sums)}
         if by_track is not None:
-            dist.all_reduce(by_track, op=dist.ReduceOp.SUM)
-    out = {"checkpoint": args.checkpoint, "track": args.track, "greedy": bool(args.greedy), "seed": args.seed,
-           **res.summary(sums)}
-    if by_track is not None:
-        out["by_track"] = [{"track": name, **summ} for name, summ in zip(names, res.summary_by_track(by_track))]
+            out["by_track"] = [{"track": name, **summ} for name, summ in zip(names, res.summary_by_track(by_track))]
     if rank == 0:
         print(json.dumps(out), flush=True)
         if args.json:

@@ -404,6 +404,15 @@ def train_population(args) -> dict:
                 pop.decay_lr()
                 lr_now = pop.lr.tolist()                         # train_ppo records the decayed rate
                 sums = (pop.sums / args.train_iters).tolist()
+                evals = None
+                if args.eval_every > 0 and epoch % args.eval_every == 0:
+                    from .evaluate import evaluate_population
+
+                    with torch.no_grad():                    # every member in one launch, with its own seed
+                        res = evaluate_population(env, pop.params[:4], args.eval_episodes, greedy=args.eval_greedy,
+                                                  seeds=pop.seeds)
+                        eval_sums = torch.stack([r.sums() for r in res]).cpu()
+                    evals = [r.summary(s) for r, s in zip(res, eval_sums)]
                 wall = time.time() - t_start
                 for p in range(pop.P):
                     seed, h = mine[p]
@@ -411,13 +420,8 @@ def train_population(args) -> dict:
                            "avg_reward": stats[p][0] / float(T * n) / args.reward_scaling, "episodes": stats[p][1],
                            "policy_loss": sums[p][0], "value_loss": sums[p][1], "entropy": sums[p][2],
                            "total_loss": sums[p][3], "lr": lr_now[p], "wall_s": wall}
-                    if args.eval_every > 0 and epoch % args.eval_every == 0:
-                        from .evaluate import evaluate_policy
-
-                        with torch.no_grad():
-                            res = evaluate_policy(env, pop.member_actor(p), args.eval_episodes, greedy=args.eval_greedy,
-                                                  seed=seed)
-                        rec["eval"] = res.summary()
+                    if evals is not None:
+                        rec["eval"] = evals[p]
                         eval_ret[p] = rec["eval"]["mean_return"]
                     history.append(rec)
                     print(json.dumps(rec), flush=True)
