@@ -12,6 +12,9 @@ Member ``p`` is initialised, rolled out and given minibatches exactly as ``train
 its first epoch's rollout is bit-identical to that run's; its updates differ from ``k_ppo_epoch``'s only in the
 summation order of the gradient.
 
+``--pbt-every K`` turns on population-based training (:mod:`ppo_car_b200.pbt`): every K epochs the weakest members
+take perturbed copies of the best members' training state.
+
     python -m ppo_car_b200.population --track big_track --n-envs 24 --n-epochs 200 --seeds 0-31 \\
         --learning-rate 3e-4,1e-3
 """
@@ -34,6 +37,10 @@ from .policy import ACTIONS, OBS, WARP_ROLLOUT_MAX_ENVS
 HPARAMS = ("learning_rate", "learning_rate_decay", "clip_ratio", "ent_coef", "vf_coef", "max_grad_norm")
 DEFAULTS = {"learning_rate": 3e-4, "learning_rate_decay": 0.99, "clip_ratio": 0.2, "ent_coef": 0.001, "vf_coef": 0.5,
             "max_grad_norm": 1.0}
+# the [P] float32 device tensor of Population that holds each hyperparameter (lr: the current, decayed rate)
+HPARAM_ATTRS = {"learning_rate": "lr", "learning_rate_decay": "lr_decay", "clip_ratio": "clip_ratio",
+                "ent_coef": "ent_coef", "vf_coef": "vf_coef", "max_grad_norm": "max_grad_norm"}
+CAPPED_AT_ONE = ("learning_rate_decay", "clip_ratio")         # a perturbed value is clamped to at most 1.0
 STATE_KEYS = ("actor.0.weight", "actor.0.bias", "actor.2.weight", "actor.2.bias",
               "critic.0.weight", "critic.0.bias", "critic.2.weight", "critic.2.bias")
 # the largest seed s whose minibatch generator seed s * 1000 + 1 (PopulationPPOUpdate, as train_ppo seeds rank 0) fits
@@ -171,6 +178,68 @@ class Population:
         """StepLR(gamma = learning_rate_decay) of every member, as ``train_ppo`` applies after each epoch."""
         self.lr.mul_(self.lr_decay)
 
+    def current_hparams(self) -> list[dict]:
+        """Every member's hyperparameters as the kernels use them now (``learning_rate``: the current, decayed rate),
+        one dict per member with the keys of :data:`HPARAMS`, as Python floats of the float32 values."""
+        cols = torch.stack([getattr(self, HPARAM_ATTRS[k]) for k in HPARAMS], 1).tolist()
+        return [dict(zip(HPARAMS, row)) for row in cols]
+
+    def _state_tensors(self):
+        return list(self.params) + [self.exp_avg, self.exp_avg_sq]
+
+    def state_rows(self, idx) -> tuple[torch.Tensor, torch.Tensor]:
+        """The full training state of members ``idx`` as new tensors: float32 ``[k, S]`` (the eight parameter tensors,
+        ``exp_avg``, ``exp_avg_sq``, then the hyperparameters in HPARAMS order) and their int32 step counts ``[k]``."""
+        i = torch.as_tensor(list(idx), dtype=torch.int64).to(self.device)
+        parts = [t[i].reshape(len(i), -1) for t in self._state_tensors()]
+        parts.append(torch.stack([getattr(self, HPARAM_ATTRS[k])[i] for k in HPARAMS], 1))
+        return torch.cat(parts, 1), self.step_count[i]
+
+    def set_rows(self, dst, rows: torch.Tensor, steps: torch.Tensor, factors=None) -> None:
+        """Write :meth:`state_rows` images into members ``dst``, then scale hyperparameter ``name`` of ``dst[j]`` by
+        ``factors[j][name]`` (a float32 product on the device; a scaled ``clip_ratio`` or ``learning_rate_decay`` is
+        clamped to at most 1.0).  Names missing from a member's dict keep the copied value bit for bit."""
+        dst = list(dst)
+        if not dst:
+            return
+        factors = list(factors) if factors is not None else [{}] * len(dst)
+        if len(factors) != len(dst) or rows.shape[0] != len(dst) or steps.shape[0] != len(dst):
+            raise ValueError("one state row, step count and factor dict per destination")
+        if len(set(dst)) != len(dst) or not all(0 <= d < self.P for d in dst):
+            raise ValueError(f"destinations must be distinct members of 0 .. {self.P - 1}")
+        unknown = {k for f in factors for k in f} - set(HPARAMS)
+        if unknown:
+            raise ValueError(f"unknown hyperparameters {sorted(unknown)}")
+        d = torch.as_tensor(dst, dtype=torch.int64).to(self.device)
+        with torch.no_grad():
+            off = 0
+            for t in self._state_tensors():
+                w = t[0].numel()
+                t[d] = rows[:, off:off + w].reshape(len(dst), *t.shape[1:])
+                off += w
+            self.step_count[d] = steps.to(torch.int32)
+            for k, name in enumerate(HPARAMS):
+                v = rows[:, off + k]
+                if any(name in f for f in factors):
+                    v = v * torch.tensor([f.get(name, 1.0) for f in factors], dtype=torch.float32, device=self.device)
+                    if name in CAPPED_AT_ONE:
+                        cap = [1.0 if name in f else float("inf") for f in factors]
+                        v = torch.minimum(v, torch.tensor(cap, dtype=torch.float32, device=self.device))
+                getattr(self, HPARAM_ATTRS[name])[d] = v
+
+    def copy_members(self, dst, src, factors=None) -> None:
+        """PBT's exploit and explore: member ``src[j]``'s weights, Adam moments, step count and hyperparameters (the
+        current learning rate included) into member ``dst[j]``, then :meth:`set_rows`'s scaling by ``factors[j]``.
+        Every source is read before any destination is written.  Seeds, environments and minibatch generators stay
+        with their slots."""
+        dst, src = list(dst), list(src)
+        if not all(0 <= s < self.P for s in src):
+            raise ValueError(f"sources must be members of 0 .. {self.P - 1}")
+        if len(src) != len(dst):
+            raise ValueError("one source per destination")
+        if src:
+            self.set_rows(dst, *self.state_rows(src), factors)
+
 
 def _stream(dev):
     return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
@@ -283,6 +352,17 @@ def parse_args(argv=None):
     p = argparse.ArgumentParser(description="train a population of independent PPO policies in one process",
                                 add_help=False)
     p.add_argument("--seeds", default="0", help="seeds of the members: a range 0-31, a list 0,5,9, or a mix")
+    p.add_argument("--pbt-every", type=int, default=0,
+                   help="population-based training: every K epochs score every member (--eval-episodes, "
+                        "--eval-greedy) and replace the bottom --pbt-fraction with perturbed copies of the top.  "
+                        "Default 0: off (the other --pbt-* flags then do nothing)")
+    p.add_argument("--pbt-fraction", type=float, default=0.25,
+                   help="fraction f in (0, 0.5] of the members replaced per round, and of those they copy from")
+    p.add_argument("--pbt-explore", default="learning_rate,ent_coef",
+                   help="comma-separated hyperparameters scaled by 0.8 or 1.2 after a copy (names of --learning-rate "
+                        "etc. with underscores; empty: copy only)")
+    p.add_argument("--pbt-seed", type=int, default=0,
+                   help="seed of the PBT decisions and of the sampled fitness evaluation (the same on every rank)")
     mine, rest = p.parse_known_args(argv)
     # lists are kept here (check_args parses them); train_ppo's parser sees one value of each
     first = lambda k, v: v.split(",")[0].strip() or str(DEFAULTS[k])
@@ -297,6 +377,8 @@ def parse_args(argv=None):
                 rest[i] = flag + "=" + first(k, a.split("=", 1)[1])
     args = train_args(rest)
     args.seeds = mine.seeds
+    args.pbt_every, args.pbt_fraction = mine.pbt_every, mine.pbt_fraction
+    args.pbt_explore, args.pbt_seed = mine.pbt_explore, mine.pbt_seed
     for k in HPARAMS:
         setattr(args, k + "_list", getattr(mine, k, None) or str(getattr(args, k)))
     return args
@@ -323,7 +405,26 @@ def check_args(args) -> tuple[list[dict], list[tuple[int, dict]]]:
         raise SystemExit("the population is empty")
     if not 2 <= args.batch_size <= 1024:
         raise SystemExit("--batch-size must be in 2..1024")
-    return expand_grid(seeds, lists)
+    settings, members = expand_grid(seeds, lists)
+    if args.pbt_every < 0:
+        raise SystemExit("--pbt-every must be >= 0 (0: no population-based training)")
+    if args.pbt_every > 0:
+        from .pbt import parse_explore
+
+        if not 0.0 < args.pbt_fraction <= 0.5:
+            raise SystemExit("--pbt-fraction must be in (0, 0.5]")
+        if int(len(members) * args.pbt_fraction) == 0:
+            raise SystemExit(f"--pbt-fraction {args.pbt_fraction:g} of {len(members)} members replaces none: "
+                             "floor(P * f) must be at least 1")
+        try:
+            parse_explore(args.pbt_explore)
+        except ValueError as e:
+            raise SystemExit(str(e))
+        if not 0 <= args.pbt_seed < 2 ** 64:
+            raise SystemExit("--pbt-seed must be in 0 .. 2^64 - 1")
+        if args.eval_episodes < 1:
+            raise SystemExit("--eval-episodes must be at least 1 with --pbt-every: it scores the members")
+    return settings, members
 
 
 def summarize(results: list[dict], settings: list[dict]) -> list[dict]:
@@ -345,14 +446,23 @@ def summarize(results: list[dict], settings: list[dict]) -> list[dict]:
 
 def train_population(args) -> dict:
     """Train every member of the grid for ``args.n_epochs`` epochs; returns {"history": [per-epoch member records of
-    this rank], "final": [one record per member, all ranks], "summary": rows of :func:`summarize`}."""
+    this rank], "final": [one record per member, all ranks], "summary": rows of :func:`summarize`}.
+
+    With ``args.pbt_every = K > 0`` a population-based-training round (:func:`pbt.pbt_round`) follows every K-th epoch
+    but the last; epoch records then gain ``"current_hparams"``, final records ``"current_hparams"`` and
+    ``"ancestry"`` (``[epoch, parent]`` per copy), and the result ``"lineage"`` (this rank's lineage records) and
+    ``"pbt_best"`` (the best member by the last round's fitness, when there was a round)."""
     from . import Buffer, VecCarEnv, builtin_track
+    from . import pbt
     from .shard import shard_range
 
     settings, members = check_args(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    pbt_on = args.pbt_every > 0
+    if pbt_on and world > len(members):
+        raise SystemExit(f"--pbt-every needs at least one member per rank ({len(members)} members, {world} ranks)")
     track = args.track if os.path.exists(args.track) else builtin_track(args.track)
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -363,6 +473,7 @@ def train_population(args) -> dict:
     mine = members[lo:hi]
     n, T = args.n_envs, args.n_steps
     history, final = [], []
+    lineage, fitness = [], None
     if mine:
         pop = Population([s for s, _ in mine], n, [h for _, h in mine], dev)
         N = pop.num_envs
@@ -383,6 +494,17 @@ def train_population(args) -> dict:
                 os.makedirs(d, exist_ok=True)
                 torch.save(pop.member_state_dict(p_local), os.path.join(d, name))
 
+        def emit(rec):
+            print(json.dumps(rec), flush=True)
+            if args.log_json:
+                with open(args.log_json + (f".rank{rank}" if world > 1 else ""), "a") as fh:
+                    fh.write(json.dumps(rec) + "\n")
+
+        if pbt_on:
+            counts = [b - a for a, b in (shard_range(len(members), world, r) for r in range(world))]
+            explore = pbt.parse_explore(args.pbt_explore)
+            gen = torch.Generator().manual_seed(args.pbt_seed)
+            ancestry = [[] for _ in range(pop.P)]
         eval_ret = [None] * pop.P
         t_start = time.time()
         try:
@@ -413,6 +535,7 @@ def train_population(args) -> dict:
                                                   seeds=pop.seeds)
                         eval_sums = torch.stack([r.sums() for r in res]).cpu()
                     evals = [r.summary(s) for r, s in zip(res, eval_sums)]
+                current = pop.current_hparams() if pbt_on else None
                 wall = time.time() - t_start
                 for p in range(pop.P):
                     seed, h = mine[p]
@@ -423,11 +546,18 @@ def train_population(args) -> dict:
                     if evals is not None:
                         rec["eval"] = evals[p]
                         eval_ret[p] = rec["eval"]["mean_return"]
+                    if pbt_on:
+                        rec["current_hparams"] = current[p]
                     history.append(rec)
-                    print(json.dumps(rec), flush=True)
-                    if args.log_json:
-                        with open(args.log_json + (f".rank{rank}" if world > 1 else ""), "a") as fh:
-                            fh.write(json.dumps(rec) + "\n")
+                    emit(rec)
+                # a round after the last epoch would only overwrite final weights that nothing trains further
+                if pbt_on and epoch % args.pbt_every == 0 and epoch < args.n_epochs:
+                    fitness, lines = pbt.pbt_round(pop, env, args, epoch // args.pbt_every - 1, epoch, lo, counts,
+                                                   gen, explore)
+                    for line in lines:
+                        ancestry[line["member"] - lo].append([epoch, line["parent"]])
+                        lineage.append(line)
+                        emit(line)
                 if epoch % 10 == 0:
                     for p in range(pop.P):
                         save(p, f"checkpoint_{epoch}.dat")
@@ -438,6 +568,10 @@ def train_population(args) -> dict:
         last = history[-pop.P:] if history else []
         final = [{"member": r["member"], "seed": r["seed"], "hparams": r["hparams"], "avg_reward": r["avg_reward"],
                   "eval_return": eval_ret[i]} for i, r in enumerate(last)]
+        if pbt_on:
+            current = pop.current_hparams()
+            for i, r in enumerate(final):
+                r["current_hparams"], r["ancestry"] = current[i], ancestry[i]
     if world > 1:
         gathered = [None] * world
         dist.all_gather_object(gathered, final)
@@ -451,7 +585,18 @@ def train_population(args) -> dict:
             if "eval_return_mean" in row:
                 line += f", eval return {row['eval_return_mean']:.3f} +- {row['eval_return_std']:.3f}"
             print(line, flush=True)
-    return {"history": history, "final": final, "summary": summary}
+    out = {"history": history, "final": final, "summary": summary}
+    if pbt_on:
+        out["lineage"] = lineage
+        if fitness is not None:                      # every rank holds every member's fitness of the last round
+            best = min(range(len(fitness)), key=lambda g: (-fitness[g], g))
+            out["pbt_best"] = {"member": best, "fitness": fitness[best],
+                               "current_hparams": next(r for r in final if r["member"] == best)["current_hparams"]}
+            if rank == 0:
+                h = ", ".join(f"{k}={v:g}" for k, v in out["pbt_best"]["current_hparams"].items())
+                print(f"best member by last PBT fitness: {best} (mean return {fitness[best]:.3f}) now [{h}]",
+                      flush=True)
+    return out
 
 
 def main(argv=None):
