@@ -73,7 +73,7 @@ int carenv_reset(void *handle, int n_envs, double *pos, double *vel, int32_t *in
 
 /* One CarEnv.step for every environment, with the same-step autoreset of
  * gymnasium.vector.AsyncVectorEnv (lib/car_env.py:693-760; train.py:138,185).
- *   actions     [n_envs] of action_dtype, values 0..8
+ *   actions     [n_envs] of action_dtype, values 0..8; any other value (in any dtype) does nothing, like 8
  *   reward_scale            TransformReward factor (train.py:65,68); reward_out = float32(r * scale)
  *   obs_out     [n_envs][18] float32; the RESET observation where the episode ended
  *   reward_out  [n_envs] float32

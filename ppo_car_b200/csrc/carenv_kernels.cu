@@ -159,6 +159,14 @@ struct DeviceGuard {
 constexpr int kBlock = CARENV_BLOCK;
 constexpr int kWarpPerEnvMax = 2048;   // n_envs up to which k_rollout_warp is launched (tracks with <= 32 segments)
 
+// The action index of one element of the caller's action array.  An action outside 0..8 does nothing (decode_action);
+// a 64-bit action must not be truncated into that range first (2^32 + 1 is not action 1).  The same rule as
+// narrow_actions_i64 on the host path.
+template <typename ActT> __device__ __forceinline__ int action_index(ActT a) { return (int)a; }
+template <> __device__ __forceinline__ int action_index<int64_t>(int64_t a) {
+    return (unsigned long long)a < 8ull ? (int)a : 8;
+}
+
 template <typename FlagT> __device__ __forceinline__ FlagT make_flag(int v);
 template <> __device__ __forceinline__ uint8_t make_flag<uint8_t>(int v) { return (uint8_t)v; }
 template <> __device__ __forceinline__ float make_flag<float>(int v) { return v ? 1.0f : 0.0f; }
@@ -281,11 +289,11 @@ k_rollout(const __grid_constant__ TrackParams P, const Tables G, int n_envs, int
         s.px = p.x; s.py = p.y; s.vx = v.x; s.vy = v.y;
         s.k = q.x; s.t = q.y; s.next_gate = q.z; s.passed = q.w;
     }
-    int a_next = (int)actions[e];
+    int a_next = action_index(actions[e]);
     for (int t = 0; t < n_steps; ++t) {
         const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
         const int a = a_next;
-        if (t + 1 < n_steps) a_next = (int)actions[idx + (size_t)n_envs];   // next step's action is in flight during this step
+        if (t + 1 < n_steps) a_next = action_index(actions[idx + (size_t)n_envs]);   // next step's action is in flight during this step
         StepResult o;
         env_step<U>(s, a, reward_scale, P, T, o, stats, nullptr, nullptr, fobs_out ? fobs_out + idx * kObsDim : nullptr);
         if (obs_mode == kObsFull) {
@@ -351,11 +359,11 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
             s.px = p.x; s.py = p.y; s.vx = v.x; s.vy = v.y;
             s.k = q.x; s.t = q.y; s.next_gate = q.z; s.passed = q.w;
         }
-        int a_next = (int)actions[e];
+        int a_next = action_index(actions[e]);
         for (int t = 0; t < n_steps; ++t) {
             const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
             const int a = a_next;
-            if (t + 1 < n_steps) a_next = (int)actions[idx + (size_t)n_envs];
+            if (t + 1 < n_steps) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
             env_step<U, true>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
@@ -443,11 +451,11 @@ k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, cons
             s.px = pp.x; s.py = pp.y; s.vx = v.x; s.vy = v.y;
             s.k = qq.x; s.t = qq.y; s.next_gate = qq.z; s.passed = qq.w;
         }
-        int a_next = (int)actions[(size_t)t0 * (size_t)n_envs + (size_t)e];
+        int a_next = action_index(actions[(size_t)t0 * (size_t)n_envs + (size_t)e]);
         for (int t = t0; t < t1; ++t) {
             const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
             const int a = a_next;
-            if (t + 1 < t1) a_next = (int)actions[idx + (size_t)n_envs];
+            if (t + 1 < t1) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
             env_step<U, true>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
@@ -500,11 +508,11 @@ k_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, int n_envs
         s.k = q.x; s.t = q.y; s.next_gate = q.z; s.passed = q.w;
     }
     unsigned long long *my_stats = lane == 0 ? stats : nullptr;
-    int a_next = (int)actions[e];
+    int a_next = action_index(actions[e]);
     for (int t = 0; t < n_steps; ++t) {
         const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
         const int a = a_next;
-        if (t + 1 < n_steps) a_next = (int)actions[idx + (size_t)n_envs];
+        if (t + 1 < n_steps) a_next = action_index(actions[idx + (size_t)n_envs]);
         StepResult o;
         env_step<kWarpPerEnv>(s, a, reward_scale, P, T, o, my_stats, &ws, nullptr,
                               (fobs_out && lane == 0) ? fobs_out + idx * kObsDim : nullptr);
@@ -643,7 +651,7 @@ k_rollout_multi(const TrackParams *__restrict__ params, const Tables *__restrict
     for (int t = 0; t < n_steps; ++t) {
         const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
         StepResult o;
-        env_step<0>(s, (int)actions[idx], reward_scale, P, T, o, stats);
+        env_step<0>(s, action_index(actions[idx]), reward_scale, P, T, o, stats);
         if (obs_out) {
             float2 *dst = reinterpret_cast<float2 *>(obs_out + idx * kObsDim);
 #pragma unroll
