@@ -513,10 +513,12 @@ __device__ __forceinline__ void cast_walls_warp(const EnvState &s, const Tables 
 // dist[i] (pixels, float32) for ray i = heading + 30*i degrees; returns destroyed.
 // U = segments per loop iteration.  U > 1 requires (checked on the host, TrackParams::unroll) that
 // n_seg and every polyline start are multiples of U; the body is then U segments of straight-line
-// code (about 1.5 KB each) — small enough to stay in the instruction cache, which a full unroll of
-// 24 segments is not (measured: 1.5 "no instruction" stalls per issue and a slower kernel).
+// code (about 1.5 KB each).
+// NS > 0 (U > 1 only): the track has exactly NS segments (and its unroll is U); the loop is unrolled over all of them.
+// Round 1 measured a full unroll of 24 segments as instruction-cache bound (1.5 "no instruction" stalls per issue);
+// with the pair arithmetic the 24-segment wall block is about 900 instructions and 4.4 % faster (DESIGN.md §3).
 // TAB (U > 1 only): denominators from the per-track table `tv` (k_rollout_tab) instead of being recomputed.
-template <int U, bool TAB = false>
+template <int U, bool TAB = false, int NS = 0>
 CE_HD bool cast_walls(const EnvState &s, const TrackParams &P, const Tables &T, float dist[kNumRays],
                       unsigned long long *stats, const WarpSeg *ws = nullptr, const TabView *tv = nullptr) {
     const float R0 = kNoHitR;
@@ -545,13 +547,20 @@ CE_HD bool cast_walls(const EnvState &s, const TrackParams &P, const Tables &T, 
 #pragma unroll
         for (int l = 0; l < 6; ++l) { w.Rp[l] = R0; w.Rm[l] = -R0; w.gq[l] = 1.0e30f; }
         w.gu = 1.0e30f;
-#pragma unroll 1
-        for (int j0 = 0; j0 < P.n_seg; j0 += U) {
+        auto segments = [&](int j0) {                       // segments j0 .. j0 + U - 1
             if (P.segf[j0].chain_start) wall_chain_start2(w, P.segf[j0]);
 #pragma unroll
             for (int u = 0; u < U; u += 2)
                 wall_pair<TAB>(w, P.segf[j0 + u], P.segd[j0 + u], P.segf[j0 + u + 1], P.segd[j0 + u + 1], s.px, s.py,
                                tb, (j0 + u) >> 1);
+        };
+        if (NS > 0) {
+            // every segment index is a constant: the records are constant-bank operands, no indexed loads, no loop
+#pragma unroll
+            for (int j0 = 0; j0 < NS; j0 += U) segments(j0);
+        } else {
+#pragma unroll 1
+            for (int j0 = 0; j0 < P.n_seg; j0 += U) segments(j0);
         }
 #pragma unroll
         for (int l = 0; l < 6; ++l) { Rp[l] = w.Rp[l]; Rm[l] = w.Rm[l]; gq[l] = w.gq[l]; }
@@ -651,7 +660,7 @@ CE_HD void pose_observation(const EnvState &s, float vx10, float vy10, const flo
 // ---- one CarEnv.step with same-step autoreset --------------------------------------------------
 // `final_obs` (optional, 18 floats): receives the observation of the state the step ended in BEFORE the autoreset —
 // gymnasium's info["final_observation"]; it equals o.obs wherever the episode did not end.
-template <int U, bool TAB = false>
+template <int U, bool TAB = false, int NS = 0>
 CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackParams &P, const Tables &T,
                     StepResult &o, unsigned long long *stats, const WarpSeg *ws = nullptr, const TabView *tv = nullptr,
                     float *final_obs = nullptr) {
@@ -673,7 +682,7 @@ CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackPar
     integrate(s, thrust, k_pre, T);
 
     float dist[kNumRays];
-    bool destroyed = cast_walls<U, TAB>(s, P, T, dist, stats, ws, tv);
+    bool destroyed = cast_walls<U, TAB, NS>(s, P, T, dist, stats, ws, tv);
     destroyed = destroyed || (P.start_destroyed != 0);
     s.t += 1;
     o.terminated = 0; o.truncated = 0;

@@ -16,6 +16,8 @@
 //   k_rollout_tab_sliced   the same for launches of >= 75,776 environments and >= 4 steps, with an SM's env-steps cut
 //               into 16 equal per-warp intervals (jobs that straddle two warps are split in time): four warps per
 //               scheduler until the launch ends.
+//               Both table kernels also come as <U, NS> instantiations for the segment counts of the shipped tracks
+//               (24 and 16): the segment loop fully unrolled, every segment record a constant-bank operand.
 //   k_rollout_multi / k_reset_multi / k_render   a track id per environment in one launch; headless rgb_array frames.
 //   csrc/policy_rollout.cuh (included below)   k_policy_rollout / k_policy_rollout_tc / _tc2 / _tc3: policy forward +
 //               sampling + env step + Buffer rows in one launch (CUDA cores / tcgen05 tensor cores, policy_core.cuh,
@@ -320,7 +322,7 @@ k_rollout(const __grid_constant__ TrackParams P, const Tables G, int n_envs, int
 #define CARENV_TAB_THREADS 512
 #endif
 constexpr int kTabThreads = CARENV_TAB_THREADS;
-template <typename ActT, typename FlagT, int U>
+template <typename ActT, typename FlagT, int U, int NS = 0>
 __global__ void __launch_bounds__(kTabThreads, 1)
 k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4, int n_pairs,
               int row_f4, int copies, int table_bytes, int n_envs, int n_steps, int epb_main, int n_main, int epb_last,
@@ -365,7 +367,7 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
             const int a = a_next;
             if (t + 1 < n_steps) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
-            env_step<U, true>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
+            env_step<U, true, NS>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
                 float2 *dst = reinterpret_cast<float2 *>(obs_out + idx * kObsDim);
 #pragma unroll
@@ -393,7 +395,7 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
 // is at least n_steps long, so the first part has finished by then; the flag makes it safe).  Every warp is busy for
 // the same number of steps and every scheduler keeps four warps until the very end.  Per-environment arithmetic is
 // untouched: results are bit-identical to k_rollout_tab / k_rollout.
-template <typename ActT, typename FlagT, int U>
+template <typename ActT, typename FlagT, int U, int NS = 0>
 __global__ void __launch_bounds__(kTabThreads, 1)
 k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4, int n_pairs,
                      int row_f4, int copies, int table_bytes, int n_envs, int n_steps, int *__restrict__ flags,
@@ -457,7 +459,7 @@ k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, cons
             const int a = a_next;
             if (t + 1 < t1) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
-            env_step<U, true>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
+            env_step<U, true, NS>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
                 float2 *dst = reinterpret_cast<float2 *>(obs_out + idx * kObsDim);
 #pragma unroll
@@ -783,6 +785,9 @@ template <typename ActT, typename FlagT>
 int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, double *vel, int32_t *ints,
                        const void *actions, double reward_scale, float *obs_out, float *reward_out, void *term_out,
                        void *trunc_out, int32_t *info_out, cudaStream_t stream, int obs_mode) {
+    // The segment loop fully unrolled (NS = n_seg) for the segment counts of the shipped tracks, big_track (24) and
+    // track.json (16): no indexed constant loads and no loop overhead (DESIGN.md §3).  Other tracks run the U loop.
+    const int n_seg = h->host.P.n_seg;
     const int n_pairs = h->host.n_pairs;
     const int row_f4 = (n_pairs + 7) / 8 * 8;                // rows are multiples of 128 bytes
     const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
@@ -830,6 +835,8 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
                     CU(cudaGetLastError());
                     return 0;
                 };
+                if (U == 6 && n_seg == 24) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 6, 24>);
+                if (U == 4 && n_seg == 16) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 4, 16>);
                 if (U == 6) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 6>);
                 if (U == 4) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 4>);
                 return launch_s(k_rollout_tab_sliced<ActT, FlagT, 2>);
@@ -859,6 +866,8 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
         CU(cudaGetLastError());
         return 0;
     };
+    if (U == 6 && n_seg == 24) return launch(k_rollout_tab<ActT, FlagT, 6, 24>);
+    if (U == 4 && n_seg == 16) return launch(k_rollout_tab<ActT, FlagT, 4, 16>);
     if (U == 6) return launch(k_rollout_tab<ActT, FlagT, 6>);
     if (U == 4) return launch(k_rollout_tab<ActT, FlagT, 4>);
     return launch(k_rollout_tab<ActT, FlagT, 2>);
