@@ -332,7 +332,18 @@ int carenv_policy_eval_multi(void *multi, const int32_t *episode_tracks, const f
  *                order, so every rank applies bit-identical updates; every rank must make the same sequence of calls.
  *   n_ctas       0 = default (64, or ceil(batch / 8) if larger); must be the same on every rank
  *   prof         NULL, or device int64 [n_updates][4]: nanosecond stamps of update start and of the three grid barriers
- * Other arguments as carenv_ppo_grad / carenv_ppo_adam. */
+ * Other arguments as carenv_ppo_grad / carenv_ppo_adam.
+ *
+ * carenv_ppo_epoch_kl: carenv_ppo_epoch with PPO's divergence statistics and an early stop.  Update u's statistics are
+ * taken over its minibatch (all ranks' samples) at the parameters before its step, log ratio = new_logp - old_logp:
+ *   kl_out      device float [n_updates][2]: approx KL mean((ratio - 1) - log ratio) and clip fraction
+ *               mean(|ratio - 1| > clip_ratio); rows after the stopping update are NaN
+ *   n_done      device int: the updates that applied a step; step advances by n_done
+ *   target_kl   update u applies no step, and the launch ends, when its approx KL > target_kl (compared in double; no
+ *               1.5 factor); +inf gives the statistics with every step applied, bit-identical to carenv_ppo_epoch
+ * CARENV_E_INVAL for a null kl_out or n_done and for a target_kl that is NaN or <= 0.  Every rank reaches the same
+ * decision from the same bits.  With a communicator the exchange count is kept on the device across these calls; a
+ * carenv_ppo_epoch call after one reads it back (one synchronising copy). */
 #define CARENV_IPC_HANDLE_BYTES 64
 int carenv_ppo_comm_create(int world, int rank, void **comm, unsigned char *ipc_handle_out /* [64] */);
 int carenv_ppo_comm_connect(void *comm, const unsigned char *all_handles /* [world][64], rank order */);
@@ -345,6 +356,13 @@ int carenv_ppo_epoch(float *w1_actor, float *b1_actor, float *w2_actor, float *b
                      float *exp_avg_sq, const float *lr, int *step, double beta1, double beta2, double eps,
                      double max_grad_norm, float *sums4, float *workspace, int *sync_words, void *comm, int n_ctas,
                      long long *prof, void *stream);
+int carenv_ppo_epoch_kl(float *w1_actor, float *b1_actor, float *w2_actor, float *b2_actor, float *w1_critic,
+                        float *b1_critic, float *w2_critic, float *b2_critic, const float *obs, const long long *idx,
+                        const float *act, const float *old_logp, const float *adv, const float *ret, int batch,
+                        int n_updates, double clip_ratio, double vf_coef, double ent_coef, float *exp_avg,
+                        float *exp_avg_sq, const float *lr, int *step, double beta1, double beta2, double eps,
+                        double max_grad_norm, float *sums4, float *workspace, int *sync_words, void *comm, int n_ctas,
+                        long long *prof, void *stream, double target_kl, float *kl_out, int *n_done);
 
 /* Populations: P independent policies ("members") trained side by side in one process, one launch per stage for all
  * of them (csrc/population.cuh).  Member p owns its parameters, Adam state, hyperparameters, seed and n environments,
@@ -369,6 +387,9 @@ int carenv_ppo_epoch(float *w1_actor, float *b1_actor, float *w2_actor, float *b
  *         sums4                device float [P][4]: policy loss, value loss, entropy, total loss, accumulated
  *       Deterministic, and member p's results do not depend on the other members; not bit-identical to
  *       carenv_ppo_epoch (another reduction order).  Needs no workspace.
+ *   carenv_ppo_epoch_pop_kl   carenv_ppo_epoch_pop with carenv_ppo_epoch_kl's statistics and stop rule, per member:
+ *       kl_out device float [P][n_updates][2], n_done device int [P]; one target_kl for every member, each member stops
+ *       on its own and its bits do not depend on the other members.  Same refusals as carenv_ppo_epoch_kl.
  *   carenv_ppo_epoch_pop_resident_clusters   how many clusters of the update kernel the current device keeps resident
  *       at once (cudaOccupancyMaxActiveClusters).
  *   carenv_policy_eval_pop   carenv_policy_eval of every member in ONE launch: n_episodes_per_member episodes (global
@@ -404,6 +425,13 @@ int carenv_ppo_epoch_pop(int n_members, float *w1_actor, float *b1_actor, float 
                          const float *vf_coef, const float *ent_coef, const float *max_grad_norm, double beta1,
                          double beta2, double eps, float *exp_avg, float *exp_avg_sq, int *step, float *sums4,
                          void *stream);
+int carenv_ppo_epoch_pop_kl(int n_members, float *w1_actor, float *b1_actor, float *w2_actor, float *b2_actor,
+                            float *w1_critic, float *b1_critic, float *w2_critic, float *b2_critic, const float *obs,
+                            const long long *idx, const float *act, const float *old_logp, const float *adv,
+                            const float *ret, int batch, int n_updates, const float *lr, const float *clip_ratio,
+                            const float *vf_coef, const float *ent_coef, const float *max_grad_norm, double beta1,
+                            double beta2, double eps, float *exp_avg, float *exp_avg_sq, int *step, float *sums4,
+                            void *stream, double target_kl, float *kl_out, int *n_done);
 int carenv_policy_eval_pop(void *handle, int n_members, const float *w1_actor, const float *b1_actor,
                            const float *w2_actor, const float *b2_actor, long long n_episodes_per_member,
                            unsigned long long episode0, int greedy, const unsigned long long *seeds,

@@ -103,6 +103,8 @@ def lib():
     L.carenv_ppo_epoch.argtypes = [vp] * 8 + [vp] * 6 + [i32, i32, f64, f64, f64, vp, vp, vp, vp, f64, f64, f64, f64,
                                                          vp, vp, vp, vp, i32, vp, vp]
     L.carenv_ppo_epoch.restype = i32
+    L.carenv_ppo_epoch_kl.argtypes = L.carenv_ppo_epoch.argtypes + [f64, vp, vp]
+    L.carenv_ppo_epoch_kl.restype = i32
     L.carenv_pack_policy.argtypes = [i32] + [vp] * 10
     L.carenv_pack_policy.restype = i32
     L.carenv_policy_weights_floats.restype = i32
@@ -124,11 +126,12 @@ def lib():
         [f64] + [vp] * 10
     L.carenv_policy_rollout_tc_pop.argtypes = [vp, i32, vp, i32, i32, vp, C.c_ulonglong] + [vp] * 6 + [f64] + [vp] * 10
     L.carenv_ppo_epoch_pop.argtypes = [i32] + [vp] * 8 + [vp] * 6 + [i32, i32] + [vp] * 5 + [f64, f64, f64] + [vp] * 5
+    L.carenv_ppo_epoch_pop_kl.argtypes = L.carenv_ppo_epoch_pop.argtypes + [f64, vp, vp]
     L.carenv_ppo_epoch_pop_resident_clusters.argtypes = [vp]
     L.carenv_policy_eval_pop.argtypes = [vp, i32] + [vp] * 4 + [C.c_longlong, C.c_ulonglong, i32, vp, vp, i32, vp, vp,
                                                                vp]
     for name in ("carenv_pack_policy_pop", "carenv_policy_rollout_warp_pop", "carenv_policy_rollout_tc_pop",
-                 "carenv_ppo_epoch_pop", "carenv_ppo_epoch_pop_cluster_size", "carenv_ppo_epoch_pop_resident_clusters",
+                 "carenv_ppo_epoch_pop", "carenv_ppo_epoch_pop_kl", "carenv_ppo_epoch_pop_cluster_size", "carenv_ppo_epoch_pop_resident_clusters",
                  "carenv_policy_eval_pop"):
         getattr(L, name).restype = i32
     for name in ("carenv_create", "carenv_destroy", "carenv_reset_obs", "carenv_reset", "carenv_step",

@@ -68,6 +68,8 @@ struct PpoComm {
     ppo::Exchange *local = nullptr;
     ppo::Exchange *peer[ppo::kMaxWorld] = {};
     unsigned long long seq = 0;           // updates completed so far (advances identically on every rank)
+    unsigned long long *d_seq = nullptr;  // the same count on the device, kept there by carenv_ppo_epoch_kl launches
+    bool seq_on_device = false;           // d_seq, not seq, is current (a KL launch came last)
 };
 
 int carenv_ppo_comm_create(int world, int rank, void **comm, unsigned char *ipc_handle_out) {
@@ -119,24 +121,31 @@ int carenv_ppo_comm_destroy(void *comm) {
     for (int r = 0; r < c->world; ++r)
         if (r != c->rank && c->peer[r]) cudaIpcCloseMemHandle(c->peer[r]);
     if (c->local) cudaFree(c->local);
+    if (c->d_seq) cudaFree(c->d_seq);
     delete c;
     return 0;
 }
 
 int carenv_ppo_epoch_workspace_floats(void) { return ppo::kMaxCtas * ppo::kLocalPad + 2 * ppo::kMaxCtas + 8 * ppo::kMaxCtas + ppo::kLocalPad; }
 
-int carenv_ppo_epoch(float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c, float *w2c, float *b2c,
-                     const float *obs, const long long *idx, const float *act, const float *old_logp,
-                     const float *adv, const float *ret, int batch, int n_updates, double clip_ratio, double vf_coef,
-                     double ent_coef, float *exp_avg, float *exp_avg_sq, const float *lr, int *step, double beta1,
-                     double beta2, double eps, double max_grad_norm, float *sums4, float *workspace, int *sync_words,
-                     void *comm, int n_ctas, long long *prof, void *stream) {
+// carenv_ppo_epoch and carenv_ppo_epoch_kl: kl_out == nullptr launches k_ppo_epoch<8>, otherwise k_ppo_epoch<8, true>
+static int ppo_epoch_launch(float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c, float *w2c,
+                            float *b2c, const float *obs, const long long *idx, const float *act, const float *old_logp,
+                            const float *adv, const float *ret, int batch, int n_updates, double clip_ratio,
+                            double vf_coef, double ent_coef, float *exp_avg, float *exp_avg_sq, const float *lr,
+                            int *step, double beta1, double beta2, double eps, double max_grad_norm, float *sums4,
+                            float *workspace, int *sync_words, void *comm, int n_ctas, long long *prof, void *stream,
+                            double target_kl, float *kl_out, int *n_done) {
     if (batch < 2 || batch > ppo::kMaxBatch) return fail(CARENV_E_INVAL, "batch must be in 2..1024");
     if (n_updates < 0) return fail(CARENV_E_INVAL, "negative n_updates");
     if (!w1a || !b1a || !w2a || !b2a || !w1c || !b1c || !w2c || !b2c || !obs || !idx || !act || !old_logp || !adv ||
         !ret || !exp_avg || !exp_avg_sq || !lr || !step || !sums4 || !workspace || !sync_words)
         return fail(CARENV_E_INVAL, "null pointer");
-    if (n_updates == 0) return 0;
+    const bool kl = kl_out != nullptr;
+    if (n_updates == 0) {
+        if (kl) CU(cudaMemsetAsync(n_done, 0, sizeof(int), static_cast<cudaStream_t>(stream)));
+        return 0;
+    }
     PpoComm *c = static_cast<PpoComm *>(comm);
     int G = n_ctas > 0 ? n_ctas : 64;
     const int need = (batch + ppo::kEpochSamples - 1) / ppo::kEpochSamples;
@@ -162,22 +171,63 @@ int carenv_ppo_epoch(float *w1a, float *b1a, float *w2a, float *b2a, float *w1c,
     A.err = sync_words + 1;
     A.world = 1; A.rank = 0;
     A.prof = prof;
+    A.target_kl = target_kl; A.kl_out = kl_out; A.n_done = n_done;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (c && c->world > 1) {
         if (c->device != dev) return fail(CARENV_E_INVAL, "the communicator belongs to another device");
         for (int r = 0; r < c->world; ++r)
             if (!c->peer[r]) return fail(CARENV_E_INVAL, "communicator not connected (carenv_ppo_comm_connect)");
+        if (kl) {
+            // an early stop exchanges fewer updates than the launch holds: the kernel keeps the count on the device
+            if (!c->d_seq) CU(cudaMalloc(reinterpret_cast<void **>(&c->d_seq), sizeof(unsigned long long)));
+            if (!c->seq_on_device) {
+                CU(cudaMemcpyAsync(c->d_seq, &c->seq, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
+                c->seq_on_device = true;
+            }
+            A.seq_dev = c->d_seq;
+        } else if (c->seq_on_device) {       // after carenv_ppo_epoch_kl: fetch the count the device advanced
+            CU(cudaMemcpyAsync(&c->seq, c->d_seq, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            c->seq_on_device = false;
+        }
         A.world = c->world; A.rank = c->rank; A.seq_base = c->seq;
         for (int r = 0; r < c->world; ++r) A.peer[r] = c->peer[r];
     }
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     CU(cudaMemsetAsync(sync_words, 0, sizeof(int), st));
     void *args[] = {&A};
-    CU(cudaFuncSetAttribute(ppo::k_ppo_epoch<ppo::kEpochSamples>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            ppo::kEpochSmemBytes));
-    CU(cudaLaunchCooperativeKernel(reinterpret_cast<void *>(ppo::k_ppo_epoch<ppo::kEpochSamples>), dim3(G),
-                                   dim3(ppo::kEpochThreads), args, ppo::kEpochSmemBytes, st));
-    if (c) c->seq += (unsigned long long)n_updates;
+    auto kern = kl ? ppo::k_ppo_epoch<ppo::kEpochSamples, true> : ppo::k_ppo_epoch<ppo::kEpochSamples>;
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ppo::kEpochSmemBytes));
+    CU(cudaLaunchCooperativeKernel(reinterpret_cast<void *>(kern), dim3(G), dim3(ppo::kEpochThreads), args,
+                                   ppo::kEpochSmemBytes, st));
+    if (c && !kl) c->seq += (unsigned long long)n_updates;
     return 0;
+}
+
+int carenv_ppo_epoch(float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c, float *w2c, float *b2c,
+                     const float *obs, const long long *idx, const float *act, const float *old_logp,
+                     const float *adv, const float *ret, int batch, int n_updates, double clip_ratio, double vf_coef,
+                     double ent_coef, float *exp_avg, float *exp_avg_sq, const float *lr, int *step, double beta1,
+                     double beta2, double eps, double max_grad_norm, float *sums4, float *workspace, int *sync_words,
+                     void *comm, int n_ctas, long long *prof, void *stream) {
+    return ppo_epoch_launch(w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, obs, idx, act, old_logp, adv, ret, batch, n_updates,
+                            clip_ratio, vf_coef, ent_coef, exp_avg, exp_avg_sq, lr, step, beta1, beta2, eps,
+                            max_grad_norm, sums4, workspace, sync_words, comm, n_ctas, prof, stream, 0.0, nullptr,
+                            nullptr);
+}
+
+int carenv_ppo_epoch_kl(float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c, float *w2c,
+                        float *b2c, const float *obs, const long long *idx, const float *act, const float *old_logp,
+                        const float *adv, const float *ret, int batch, int n_updates, double clip_ratio,
+                        double vf_coef, double ent_coef, float *exp_avg, float *exp_avg_sq, const float *lr, int *step,
+                        double beta1, double beta2, double eps, double max_grad_norm, float *sums4, float *workspace,
+                        int *sync_words, void *comm, int n_ctas, long long *prof, void *stream, double target_kl,
+                        float *kl_out, int *n_done) {
+    if (!kl_out || !n_done) return fail(CARENV_E_INVAL, "null pointer");
+    if (!(target_kl > 0.0)) return fail(CARENV_E_INVAL, "target_kl must be positive (+inf: statistics only)");
+    return ppo_epoch_launch(w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, obs, idx, act, old_logp, adv, ret, batch, n_updates,
+                            clip_ratio, vf_coef, ent_coef, exp_avg, exp_avg_sq, lr, step, beta1, beta2, eps,
+                            max_grad_norm, sums4, workspace, sync_words, comm, n_ctas, prof, stream, target_kl, kl_out,
+                            n_done);
 }
 
 int carenv_policy_weights_floats(void) { return kPolicyFloats; }

@@ -61,6 +61,10 @@ struct PopEpochArgs {
     float *m, *v;                     // [P][12,298] Adam moments, flat parameter layout
     int *step;                        // [P]
     float *sums4;                     // [P][4]
+    // k_ppo_epoch_pop<true> only: statistics and early stop, per member
+    double target_kl;                 // a member stops at its first update whose approx KL exceeds it (+inf: never)
+    float *kl_out;                    // [P][n_updates][2] approx KL, clip fraction; NaN after the stopping update
+    int *n_done;                      // [P] updates that applied a step
 };
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -89,11 +93,16 @@ __device__ __forceinline__ float4 dsmem_ld4(uint32_t addr) {
     return v;
 }
 
+// KL = true: k_ppo_epoch<8, true>'s statistics and stop rule per member (carenv_ppo_epoch_pop_kl).  Each CTA's KL and
+// clip sums form a second float4 of its stats line, read over DSMEM and folded in the same fixed order as the first,
+// so every CTA of the cluster sees the same totals, takes the same exit and still reaches the final cluster barrier.
+template <bool KL = false>
 __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const PopEpochArgs A) {
     using namespace ppo;
     constexpr int SMAX = kEpochSamples;
     constexpr int kZ = 10;                               // 9 logits + the value per sample
     constexpr int kFold = kZ * SMAX;
+    constexpr int kParts = KL ? 5 : 3;                   // policy loss, entropy, value loss (, KL term, clipped)
     static_assert(SMAX * kIn <= kEpochThreads, "one thread per staged observation element");
     extern __shared__ __align__(16) float s_dyn[];
     float *const s_m = s_dyn, *const s_v = s_dyn + kLocalK * kH;
@@ -102,10 +111,12 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     __shared__ __align__(16) float s_x[SMAX][20];
     __shared__ float s_red[8][kFold];
     __shared__ __align__(16) float s_z[SMAX][12];
-    __shared__ float s_part[SMAX][3];
+    __shared__ float s_part[SMAX][kParts];
     __shared__ float s_red8[8];
     __shared__ __align__(16) float4 s_line;              // slice sum of squares, loss partial sums of the CTA's samples
     __shared__ float4 s_tot;
+    __shared__ __align__(16) float4 s_line_kl;           // KL: KL and clip sums of the CTA's samples
+    __shared__ float2 s_tot_kl;
     __shared__ float s_bias[2];
     __shared__ float s_b2[kZ], s_b2m[kZ], s_b2v[kZ];
 
@@ -126,6 +137,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     const int step0 = A.step[p];
     const float lr = A.lr[p], clip_ratio = A.clip_ratio[p], vf_coef = A.vf_coef[p], ent_coef = A.ent_coef[p];
     const float max_grad_norm = A.max_grad_norm[p];
+    int n_run = A.n_updates, n_eval = A.n_updates;      // KL: updates that applied a step / formed statistics
     const uint32_t a_g = tc::smem_u32(s_g), a_slice = tc::smem_u32(s_slice), a_line = tc::smem_u32(&s_line);
 
     float w[kLocalK];
@@ -184,6 +196,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
             a_inv = 1.0f / fmaxf(sqrtf(var), 1.0e-5f);
         }
         float lp0 = 0.0f, lp1 = 0.0f, lp2 = 0.0f;       // loss partial sums of the CTA's samples (thread 0)
+        float lp3 = 0.0f, lp4 = 0.0f;                   // KL: KL and clip sums of the CTA's samples (thread 0)
 
         // ---- phase A: the CTA's samples, chunk by chunk
         for (int ch = 0; ch < n_chunks; ++ch) {
@@ -266,9 +279,15 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
                         s_z[j][q] = g_lp * ((a == q ? 1.0f : 0.0f) - pr[q]) + ent_coef * invB * pr[q] * (lp[q] + H);
                     s_z[j][kQ] = vf_coef * d * invB;
                     p0 = fmaxf(t1, t2); p1 = H; p2 = 0.5f * d * d;
+                    if constexpr (KL) {
+                        const float log_r = new_lp - c_olp;
+                        s_part[j][3] = (ratio - 1.0f) - log_r;
+                        s_part[j][4] = fabsf(ratio - 1.0f) > clip_ratio ? 1.0f : 0.0f;
+                    }
                 } else {
 #pragma unroll
                     for (int q = 0; q < kZ; ++q) s_z[j][q] = 0.0f;
+                    if constexpr (KL) { s_part[j][3] = 0.0f; s_part[j][4] = 0.0f; }
                 }
                 s_part[j][0] = p0; s_part[j][1] = p1; s_part[j][2] = p2;
             }
@@ -276,6 +295,10 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
             if (j == 0) {
 #pragma unroll
                 for (int s = 0; s < SMAX; ++s) { lp0 += s_part[s][0]; lp1 += s_part[s][1]; lp2 += s_part[s][2]; }
+                if constexpr (KL) {
+#pragma unroll
+                    for (int s = 0; s < SMAX; ++s) { lp3 += s_part[s][3]; lp4 += s_part[s][4]; }
+                }
             }
 
             // ---- backward: the 48 parameters of unit j, one fma chain over all of the CTA's samples
@@ -340,6 +363,9 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
         {
             const float ssum = block_sum_256(ss, s_red8);
             if (j == 0) s_line = make_float4(ssum, lp0, lp1, lp2);
+            if constexpr (KL) {
+                if (j == 0) s_line_kl = make_float4(lp3, lp4, 0.0f, 0.0f);
+            }
         }
         if (j == 64) {                                                // bias corrections of this step
             const int t_step = step0 + u + 1;
@@ -371,9 +397,27 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
                     tot.z += __shfl_xor_sync(0xffffffffu, tot.z, o); tot.w += __shfl_xor_sync(0xffffffffu, tot.w, o);
                 }
                 if (lane == 0) s_tot = tot;
+                if constexpr (KL) {
+                    const float4 l2 = lane < kPopCluster ? dsmem_ld4(dsmem_map(tc::smem_u32(&s_line_kl), (uint32_t)lane))
+                                                         : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                    float2 t2 = make_float2(l2.x, l2.y);
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) {
+                        t2.x += __shfl_xor_sync(0xffffffffu, t2.x, o); t2.y += __shfl_xor_sync(0xffffffffu, t2.y, o);
+                    }
+                    if (lane == 0) s_tot_kl = t2;
+                }
             }
             __syncthreads();
             const float4 tot = s_tot;
+            if constexpr (KL) {                                       // the same bits in every CTA of the cluster
+                const float kl = s_tot_kl.x * invB, clip_frac = s_tot_kl.y * invB;
+                if (r == 0 && j == 0) {
+                    float *row = A.kl_out + 2 * (pq * (size_t)A.n_updates + (size_t)u);
+                    row[0] = kl; row[1] = clip_frac;
+                }
+                if ((double)kl > A.target_kl) { n_run = u; n_eval = u + 1; break; }
+            }
             const float coef = fminf(max_grad_norm / (sqrtf(tot.x) + 1.0e-6f), 1.0f);    // clip_grad_norm_
             if (r == 0 && j == 0) {
                 float *sums = A.sums4 + 4 * pq;
@@ -418,7 +462,13 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
             const int f = local_to_flat(kLocalK * kH + j);
             *param_ptr(P, f) = s_b2[j]; gm[f] = s_b2m[j]; gv[f] = s_b2v[j];
         }
-        if (j == 0) A.step[p] = step0 + A.n_updates;
+        if constexpr (KL) {
+            float *rows = A.kl_out + 2 * pq * (size_t)A.n_updates;
+            for (int i = 2 * n_eval + j; i < 2 * A.n_updates; i += kEpochThreads) rows[i] = __int_as_float(0x7fc00000);
+            if (j == 0) { A.step[p] = step0 + n_run; A.n_done[p] = n_run; }
+        } else {
+            if (j == 0) A.step[p] = step0 + A.n_updates;
+        }
     }
 }
 
@@ -511,19 +561,60 @@ static void ppo_epoch_pop_config(cudaLaunchConfig_t *cfg, cudaLaunchAttribute *a
     cfg->numAttrs = 1;
 }
 
-static int ppo_epoch_pop_attributes() {
-    CU(cudaFuncSetAttribute(k_ppo_epoch_pop, cudaFuncAttributeMaxDynamicSharedMemorySize, kPopSmemBytes));
-    if (kPopCluster > 8) CU(cudaFuncSetAttribute(k_ppo_epoch_pop, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+static int ppo_epoch_pop_attributes(bool kl) {
+    const void *kern = kl ? reinterpret_cast<const void *>(k_ppo_epoch_pop<true>)
+                          : reinterpret_cast<const void *>(k_ppo_epoch_pop<false>);
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kPopSmemBytes));
+    if (kPopCluster > 8) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     return 0;
 }
 
 int carenv_ppo_epoch_pop_resident_clusters(int *n_clusters) {
     if (!n_clusters) return fail(CARENV_E_INVAL, "null pointer");
-    if (const int rc = ppo_epoch_pop_attributes()) return rc;
+    if (const int rc = ppo_epoch_pop_attributes(false)) return rc;
     cudaLaunchConfig_t cfg;
     cudaLaunchAttribute attr;
     ppo_epoch_pop_config(&cfg, &attr, 1, nullptr);
-    CU(cudaOccupancyMaxActiveClusters(n_clusters, k_ppo_epoch_pop, &cfg));
+    CU(cudaOccupancyMaxActiveClusters(n_clusters, k_ppo_epoch_pop<false>, &cfg));
+    return 0;
+}
+
+// carenv_ppo_epoch_pop and carenv_ppo_epoch_pop_kl: kl_out == nullptr launches k_ppo_epoch_pop<false>
+static int ppo_epoch_pop_launch(int n_members, float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c,
+                                float *w2c, float *b2c, const float *obs, const long long *idx, const float *act,
+                                const float *old_logp, const float *adv, const float *ret, int batch, int n_updates,
+                                const float *lr, const float *clip_ratio, const float *vf_coef, const float *ent_coef,
+                                const float *max_grad_norm, double beta1, double beta2, double eps, float *exp_avg,
+                                float *exp_avg_sq, int *step, float *sums4, void *stream, double target_kl,
+                                float *kl_out, int *n_done) {
+    if (n_members <= 0 || n_members > 0x7fffffff / kPopCluster)
+        return fail(CARENV_E_INVAL, "n_members must be positive (and n_members * cluster size below 2^31)");
+    if (batch < 2 || batch > ppo::kMaxBatch) return fail(CARENV_E_INVAL, "batch must be in 2..1024");
+    if (n_updates < 0) return fail(CARENV_E_INVAL, "negative n_updates");
+    if (!w1a || !b1a || !w2a || !b2a || !w1c || !b1c || !w2c || !b2c || !obs || !idx || !act || !old_logp || !adv ||
+        !ret || !lr || !clip_ratio || !vf_coef || !ent_coef || !max_grad_norm || !exp_avg || !exp_avg_sq || !step ||
+        !sums4)
+        return fail(CARENV_E_INVAL, "null pointer");
+    const bool kl = kl_out != nullptr;
+    if (n_updates == 0) {
+        if (kl) CU(cudaMemsetAsync(n_done, 0, sizeof(int) * (size_t)n_members, static_cast<cudaStream_t>(stream)));
+        return 0;
+    }
+    PopEpochArgs A;
+    memset(&A, 0, sizeof(A));
+    A.P = ppo::MutableParams{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c};
+    A.obs = obs; A.idx = idx; A.act = act; A.old_logp = old_logp; A.adv = adv; A.ret = ret;
+    A.B = batch; A.n_updates = n_updates;
+    A.lr = lr; A.clip_ratio = clip_ratio; A.vf_coef = vf_coef; A.ent_coef = ent_coef; A.max_grad_norm = max_grad_norm;
+    A.beta1 = (float)beta1; A.beta2 = (float)beta2; A.eps = (float)eps;
+    A.m = exp_avg; A.v = exp_avg_sq; A.step = step; A.sums4 = sums4;
+    A.target_kl = target_kl; A.kl_out = kl_out; A.n_done = n_done;
+    if (const int rc = ppo_epoch_pop_attributes(kl)) return rc;
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute attr;
+    ppo_epoch_pop_config(&cfg, &attr, n_members, static_cast<cudaStream_t>(stream));
+    if (kl) CU(cudaLaunchKernelEx(&cfg, k_ppo_epoch_pop<true>, A));
+    else CU(cudaLaunchKernelEx(&cfg, k_ppo_epoch_pop<false>, A));
     return 0;
 }
 
@@ -533,27 +624,21 @@ int carenv_ppo_epoch_pop(int n_members, float *w1a, float *b1a, float *w2a, floa
                          const float *lr, const float *clip_ratio, const float *vf_coef, const float *ent_coef,
                          const float *max_grad_norm, double beta1, double beta2, double eps, float *exp_avg,
                          float *exp_avg_sq, int *step, float *sums4, void *stream) {
-    if (n_members <= 0 || n_members > 0x7fffffff / kPopCluster)
-        return fail(CARENV_E_INVAL, "n_members must be positive (and n_members * cluster size below 2^31)");
-    if (batch < 2 || batch > ppo::kMaxBatch) return fail(CARENV_E_INVAL, "batch must be in 2..1024");
-    if (n_updates < 0) return fail(CARENV_E_INVAL, "negative n_updates");
-    if (!w1a || !b1a || !w2a || !b2a || !w1c || !b1c || !w2c || !b2c || !obs || !idx || !act || !old_logp || !adv ||
-        !ret || !lr || !clip_ratio || !vf_coef || !ent_coef || !max_grad_norm || !exp_avg || !exp_avg_sq || !step ||
-        !sums4)
-        return fail(CARENV_E_INVAL, "null pointer");
-    if (n_updates == 0) return 0;
-    PopEpochArgs A;
-    memset(&A, 0, sizeof(A));
-    A.P = ppo::MutableParams{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c};
-    A.obs = obs; A.idx = idx; A.act = act; A.old_logp = old_logp; A.adv = adv; A.ret = ret;
-    A.B = batch; A.n_updates = n_updates;
-    A.lr = lr; A.clip_ratio = clip_ratio; A.vf_coef = vf_coef; A.ent_coef = ent_coef; A.max_grad_norm = max_grad_norm;
-    A.beta1 = (float)beta1; A.beta2 = (float)beta2; A.eps = (float)eps;
-    A.m = exp_avg; A.v = exp_avg_sq; A.step = step; A.sums4 = sums4;
-    if (const int rc = ppo_epoch_pop_attributes()) return rc;
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute attr;
-    ppo_epoch_pop_config(&cfg, &attr, n_members, static_cast<cudaStream_t>(stream));
-    CU(cudaLaunchKernelEx(&cfg, k_ppo_epoch_pop, A));
-    return 0;
+    return ppo_epoch_pop_launch(n_members, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, obs, idx, act, old_logp, adv, ret,
+                                batch, n_updates, lr, clip_ratio, vf_coef, ent_coef, max_grad_norm, beta1, beta2, eps,
+                                exp_avg, exp_avg_sq, step, sums4, stream, 0.0, nullptr, nullptr);
+}
+
+int carenv_ppo_epoch_pop_kl(int n_members, float *w1a, float *b1a, float *w2a, float *b2a, float *w1c, float *b1c,
+                            float *w2c, float *b2c, const float *obs, const long long *idx, const float *act,
+                            const float *old_logp, const float *adv, const float *ret, int batch, int n_updates,
+                            const float *lr, const float *clip_ratio, const float *vf_coef, const float *ent_coef,
+                            const float *max_grad_norm, double beta1, double beta2, double eps, float *exp_avg,
+                            float *exp_avg_sq, int *step, float *sums4, void *stream, double target_kl,
+                            float *kl_out, int *n_done) {
+    if (!kl_out || !n_done) return fail(CARENV_E_INVAL, "null pointer");
+    if (!(target_kl > 0.0)) return fail(CARENV_E_INVAL, "target_kl must be positive (+inf: statistics only)");
+    return ppo_epoch_pop_launch(n_members, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, obs, idx, act, old_logp, adv, ret,
+                                batch, n_updates, lr, clip_ratio, vf_coef, ent_coef, max_grad_norm, beta1, beta2, eps,
+                                exp_avg, exp_avg_sq, step, sums4, stream, target_kl, kl_out, n_done);
 }

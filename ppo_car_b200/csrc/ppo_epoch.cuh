@@ -77,6 +77,11 @@ struct EpochArgs {
     Exchange *peer[kMaxWorld];        // peer[rank] is the local buffer
     unsigned long long seq_base;      // updates completed by earlier launches (same on every rank)
     long long *prof;                  // optional [n_updates][4] globaltimer stamps of CTA 0: start, barrier 1, 2, 3
+    // k_ppo_epoch<SMAX, true> only: statistics and early stop
+    double target_kl;                 // stop at the first update whose approx KL exceeds it (+inf: never)
+    float *kl_out;                    // [n_updates][2] approx KL, clip fraction; NaN after the stopping update
+    int *n_done;                      // updates that applied a step
+    unsigned long long *seq_dev;      // world > 1: the exchanged-update count, read at launch and advanced at exit
 };
 
 // local element e -> index in the flat layout W1a b1a W2a b2a W1c b1c W2c b2c
@@ -205,17 +210,25 @@ __device__ __forceinline__ float adam_quotient(float num, float v, float inv_sqr
 constexpr int kEpochSamples = 8;                     // samples per CTA: G = max(64, ceil(B / 8)) CTAs cover B <= 1,024
 constexpr int kEpochSmemBytes = 2 * kLocalK * kH * (int)sizeof(float);   // Adam moments of the 48 x 256 unit parameters
 
-template <int SMAX>
+// KL = true adds the PPO diagnostics and the early stop (carenv_ppo_epoch_kl): phase A also sums each sample's
+// (ratio - 1) - log ratio and |ratio - 1| > clip_ratio; the two CTA sums ride in the partial-gradient row at columns
+// kLocal, kLocal + 1 and are reduced (over the CTAs, then the ranks) by two extra threads of CTA 0 in phase B, outside
+// the slice sum of squares, so the parameter arithmetic keeps its bits.  Phase C divides them by the sample count,
+// CTA 0 records them, and when the KL exceeds target_kl every CTA of every rank (the totals are the same bits
+// everywhere) skips that update's step and leaves the loop.  With several GPUs the exchange sequence base lives in
+// device memory (seq_dev), because only the device knows how many updates a launch exchanged.
+template <int SMAX, bool KL = false>
 __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs A) {
     static_assert(SMAX * kIn <= kEpochThreads, "one thread per staged observation element");
     constexpr int kZ = 10;                               // 9 logits + the value per sample
     constexpr int kFold = kZ * SMAX;
+    constexpr int kParts = KL ? 5 : 3;                   // policy loss, entropy, value loss (, KL term, clipped)
     extern __shared__ __align__(16) float s_dyn[];       // m [48][256] | v [48][256]: this CTA's copy of the Adam moments
     float *const s_m = s_dyn, *const s_v = s_dyn + kLocalK * kH;
     __shared__ __align__(16) float s_x[SMAX][20];        // observation rows of the CTA's samples
     __shared__ float s_red[8][kFold];                    // per-warp sums of the second layer
     __shared__ __align__(16) float s_z[SMAX][12];        // logits | value, then d loss / d logits | d loss / d value
-    __shared__ float s_part[SMAX][3];                    // per-sample policy loss, entropy, value loss
+    __shared__ float s_part[SMAX][kParts];               // per-sample policy loss, entropy, value loss
     __shared__ float s_red8[8];
     __shared__ float4 s_fold[8];
     __shared__ float s_bias[2];
@@ -231,11 +244,21 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
     const int slice = (kLocal + G - 1) / G;              // parameters per CTA in phase B (<= 256)
     const int e_mine = c * slice + j;
     const bool own = j < slice && e_mine < kLocal;
+    // KL: threads slice, slice + 1 of CTA 0 (slice <= 251, so they exist) reduce the two statistic sums, elements
+    // kLocal and kLocal + 1; own_b / e_b are phase B's owner and element, own alone feeds the sum of squares
+    const bool own_b = KL ? own || (c == 0 && j >= slice && j < slice + 2) : own;
+    const int e_b = KL ? (own ? e_mine : kLocal + j - slice) : e_mine;
     const float invB = 1.0f / (float)B;
     const int step0 = *A.step;
     const float lr = A.lr[0];
     float *const gfull = A.ssq + 2 * kMaxCtas + 8 * kMaxCtas;       // [kLocalPad] reduced gradient (workspace tail)
     unsigned int bar_target = 0;
+    // KL with several GPUs: the sequence base comes from the device (A.seq_base is read in place otherwise: a copy
+    // would change k_ppo_epoch<8>'s machine code)
+    unsigned long long seq_kl = 0;
+    if constexpr (KL) seq_kl = A.world > 1 ? *A.seq_dev : A.seq_base;
+    int n_run = A.n_updates;                             // KL: updates that applied a step
+    int n_eval = A.n_updates;                            // KL: updates whose statistics were formed (and exchanged)
 
     // ---- every CTA keeps ALL parameters and Adam moments for the whole launch: thread j the 48 of hidden unit j
     // (parameters in registers, moments in shared memory), threads 0..9 the second-layer biases.  Every CTA applies
@@ -277,7 +300,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
     for (int u = 0; u < A.n_updates; ++u) {
         const bool stamp = A.prof != nullptr && c == 0 && j == 0;
         if (stamp) A.prof[4 * u] = global_ns();
-        const int par = (int)((A.seq_base + (unsigned long long)u) & 1ull);   // continues across launches (odd n_updates)
+        const int par = (int)(((KL ? seq_kl : A.seq_base) + (unsigned long long)u) & 1ull);     // continues across launches (odd n_updates)
 
         // ---- this CTA's observation rows
         if (j < nS * kIn) s_x[j / kIn][j % kIn] = x_pf;
@@ -373,9 +396,15 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                     s_z[j][q] = g_lp * ((a == q ? 1.0f : 0.0f) - p[q]) + A.ent_coef * invB * p[q] * (lp[q] + H);
                 s_z[j][kQ] = A.vf_coef * d * invB;
                 p0 = fmaxf(t1, t2); p1 = H; p2 = 0.5f * d * d;
+                if constexpr (KL) {
+                    const float log_r = new_lp - l_olp;
+                    s_part[j][3] = (ratio - 1.0f) - log_r;
+                    s_part[j][4] = fabsf(ratio - 1.0f) > A.clip_ratio ? 1.0f : 0.0f;
+                }
             } else {
 #pragma unroll
                 for (int q = 0; q < kZ; ++q) s_z[j][q] = 0.0f;
+                if constexpr (KL) { s_part[j][3] = 0.0f; s_part[j][4] = 0.0f; }
             }
             s_part[j][0] = p0; s_part[j][1] = p1; s_part[j][2] = p2;
         }
@@ -420,6 +449,15 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                 for (int s = 0; s < SMAX; ++s) t += s_z[s][j];
                 __stcg(row + kLocalK * kH + j, t);
             }
+            if constexpr (KL) {                                      // the CTA's KL and clip sums, sample order
+                if (j == kZ) {
+                    float tk = 0.0f, tc = 0.0f;
+#pragma unroll
+                    for (int s = 0; s < SMAX; ++s) { tk += s_part[s][3]; tc += s_part[s][4]; }
+                    __stcg(row + kLocal, tk);
+                    __stcg(row + kLocal + 1, tc);
+                }
+            }
         }
         if (u + 1 < A.n_updates) prefetch(u + 1);
         if (grid_barrier(A.bar, bar_target, A.err, &s_flag)) return;
@@ -427,8 +465,8 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
 
         // ---- phase B: slice c of the gradient, summed over the CTAs (and over the GPUs)
         float gsum = 0.0f;
-        if (own) {
-            const float *col = A.partial + e_mine;
+        if (own_b) {
+            const float *col = A.partial + e_b;
             constexpr int kInFlight = 32;
             float t[kInFlight];
             for (int c2 = 0; c2 < G; c2 += kInFlight) {              // 32 loads in flight, summed in CTA order
@@ -438,9 +476,9 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                 for (int i = 0; i < kInFlight; ++i) gsum += t[i];
             }
         }
-        if (A.world > 1 && own) {
+        if (A.world > 1 && own_b) {
             // push this rank's value of the element to every peer, then collect theirs: one-way NVLink latency
-            const unsigned int seq = (unsigned int)(A.seq_base + (unsigned long long)u + 1ull);
+            const unsigned int seq = (unsigned int)((KL ? seq_kl : A.seq_base) + (unsigned long long)u + 1ull);
             const uint2 mine = make_uint2(__float_as_uint(gsum), seq);
             float val[kMaxWorld];
             unsigned int pending = 0;
@@ -448,7 +486,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
             for (int r = 0; r < kMaxWorld; ++r) {
                 val[r] = 0.0f;
                 if (r < A.world && r != A.rank) {
-                    st_slot_sys(&A.peer[r]->ll[par][A.rank][e_mine], mine);
+                    st_slot_sys(&A.peer[r]->ll[par][A.rank][e_b], mine);
                     pending |= 1u << r;
                 }
             }
@@ -459,7 +497,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                 uint2 got[kMaxWorld];
 #pragma unroll
                 for (int r = 0; r < kMaxWorld; ++r)
-                    if (pending & (1u << r)) got[r] = ld_slot_sys(&me->ll[par][r][e_mine]);
+                    if (pending & (1u << r)) got[r] = ld_slot_sys(&me->ll[par][r][e_b]);
 #pragma unroll
                 for (int r = 0; r < kMaxWorld; ++r)
                     if ((pending & (1u << r)) && got[r].y == seq) { val[r] = __uint_as_float(got[r].x); pending &= ~(1u << r); }
@@ -474,7 +512,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                 if (r < A.world) t += (r == A.rank) ? gsum : val[r];
             gsum = t * (1.0f / (float)A.world);
         }
-        if (own) __stcg(gfull + e_mine, gsum);
+        if (own_b) __stcg(gfull + e_b, gsum);
         {   // this CTA's line of the norm / statistics table: slice sum of squares, loss partial sums of its samples
             const float ss = block_sum_256(own ? gsum * gsum : 0.0f, s_red8);
             if (j == 0) {
@@ -514,6 +552,11 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
             tot = s_fold[0];
 #pragma unroll
             for (int w8 = 1; w8 < 8; ++w8) { const float4 o = s_fold[w8]; tot.x += o.x; tot.y += o.y; tot.z += o.z; tot.w += o.w; }
+            if constexpr (KL) {                                       // same bits in every CTA and on every rank
+                const float kl = __ldcg(gfull + kLocal) * invB, clip_frac = __ldcg(gfull + kLocal + 1) * invB;
+                if (c == 0 && j == 0) { A.kl_out[2 * u] = kl; A.kl_out[2 * u + 1] = clip_frac; }
+                if ((double)kl > A.target_kl) { n_run = u; n_eval = u + 1; break; }
+            }
             const float coef = fminf(A.max_grad_norm / (sqrtf(tot.x) + 1.0e-6f), 1.0f);    // clip_grad_norm_
 #ifdef CARENV_EPOCH_PROF2
             if (stamp) A.prof[4 * A.n_updates + 4 * u] = global_ns();
@@ -566,7 +609,16 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
             const int f = local_to_flat(kLocalK * kH + j);
             *param_ptr(A.P, f) = s_b2[j]; A.m[f] = s_b2m[j]; A.v[f] = s_b2v[j];
         }
-        if (j == 0) *A.step = step0 + A.n_updates;
+        if constexpr (KL) {
+            for (int i = 2 * n_eval + j; i < 2 * A.n_updates; i += kEpochThreads) A.kl_out[i] = __int_as_float(0x7fc00000);
+            if (j == 0) {
+                *A.step = step0 + n_run;
+                *A.n_done = n_run;
+                if (A.world > 1) *A.seq_dev = seq_kl + (unsigned long long)n_eval;
+            }
+        } else {
+            if (j == 0) *A.step = step0 + A.n_updates;
+        }
     }
 }
 

@@ -306,6 +306,8 @@ class PopulationPPOUpdate:
             raise ValueError("batch_size must be in 2..1024")
         self.pop, self.batch, self.betas, self.eps = pop, int(batch_size), betas, eps
         self.generators = [torch.Generator(device=pop.device).manual_seed(s * 1000 + 1) for s in pop.seeds]
+        self.kl = None                   # launch(target_kl=...): [P, n_updates, 2] approx KL, clip fraction
+        self.n_done = None               # launch(target_kl=...): [P] int32 updates that applied a step
 
     def draw_indices(self, T: int, n_updates: int) -> torch.Tensor:
         """int64 ``[P, n_updates, batch]`` global rows of the ``[T * N]`` flat arrays."""
@@ -316,15 +318,24 @@ class PopulationPPOUpdate:
         base = (torch.arange(pop.P, device=pop.device, dtype=torch.int64) * n).view(-1, 1, 1)
         return ((k // n) * N + base + k % n).contiguous()
 
-    def run_epoch(self, obs, act, old_logp, adv, ret, T: int, n_updates: int) -> torch.Tensor:
+    def run_epoch(self, obs, act, old_logp, adv, ret, T: int, n_updates: int,
+                  target_kl: float | None = None) -> torch.Tensor:
         """Draw every member's indices and run the epoch; returns the indices."""
         idx = self.draw_indices(T, n_updates)
-        self.launch(obs, idx, act, old_logp, adv, ret)
+        if target_kl is None:
+            self.launch(obs, idx, act, old_logp, adv, ret)
+        else:
+            self.launch(obs, idx, act, old_logp, adv, ret, target_kl=target_kl)
         return idx
 
-    def launch(self, obs, idx, act, old_logp, adv, ret) -> None:
+    def launch(self, obs, idx, act, old_logp, adv, ret, target_kl: float | None = None) -> None:
         """One launch for the updates ``idx[:, u]`` of every member (``idx`` int64 ``[P, n_updates, batch]``).
-        Asynchronous."""
+        Asynchronous.
+
+        ``target_kl`` (positive, ``inf`` for statistics only) launches ``carenv_ppo_epoch_pop_kl``: ``self.kl``
+        [P, n_updates, 2] gets every member's per-update approx KL and clip fraction (NaN after its stopping update),
+        ``self.n_done`` [P] int32 its applied updates; each member stops at its first update whose approx KL exceeds
+        ``target_kl``.  ``None`` launches exactly what it launched before."""
         pop = self.pop
         if idx.dtype != torch.int64 or idx.dim() != 3 or idx.shape[0] != pop.P or idx.shape[2] != self.batch \
                 or not idx.is_contiguous() or idx.device != pop.device:
@@ -334,15 +345,29 @@ class PopulationPPOUpdate:
                 raise ValueError(f"{name} must be a contiguous float32 tensor on {pop.device}")
         if obs.shape[-1] != OBS:
             raise ValueError("obs must have 18 columns")
+        if target_kl is not None:
+            if not float(target_kl) > 0.0:
+                raise ValueError("target_kl must be positive (inf: statistics without stopping)")
+            shape = (pop.P, int(idx.shape[1]), 2)
+            if self.kl is None or tuple(self.kl.shape) != shape:
+                self.kl = torch.empty(shape, device=pop.device)
+            if self.n_done is None or self.n_done.shape[0] != pop.P:
+                self.n_done = torch.zeros(pop.P, dtype=torch.int32, device=pop.device)
         if idx.shape[1] == 0:
+            if target_kl is not None:
+                self.n_done.zero_()
             return
-        with torch.cuda.device(pop.device):
-            rc = pop.L.carenv_ppo_epoch_pop(
-                pop.P, *[_p(t) for t in pop.params], _p(obs), _p(idx), _p(act), _p(old_logp), _p(adv), _p(ret),
+        args = (pop.P, *[_p(t) for t in pop.params], _p(obs), _p(idx), _p(act), _p(old_logp), _p(adv), _p(ret),
                 self.batch, int(idx.shape[1]), _p(pop.lr), _p(pop.clip_ratio), _p(pop.vf_coef), _p(pop.ent_coef),
                 _p(pop.max_grad_norm), self.betas[0], self.betas[1], self.eps, _p(pop.exp_avg), _p(pop.exp_avg_sq),
                 _p(pop.step_count), _p(pop.sums), _stream(pop.device))
-        _lib.check(rc, "carenv_ppo_epoch_pop")
+        with torch.cuda.device(pop.device):
+            if target_kl is None:
+                rc, what = pop.L.carenv_ppo_epoch_pop(*args), "carenv_ppo_epoch_pop"
+            else:
+                rc = pop.L.carenv_ppo_epoch_pop_kl(*args, float(target_kl), _p(self.kl), _p(self.n_done))
+                what = "carenv_ppo_epoch_pop_kl"
+        _lib.check(rc, what)
 
 
 # ---- command line --------------------------------------------------------------------------------------------------
@@ -405,6 +430,9 @@ def check_args(args) -> tuple[list[dict], list[tuple[int, dict]]]:
         raise SystemExit("the population is empty")
     if not 2 <= args.batch_size <= 1024:
         raise SystemExit("--batch-size must be in 2..1024")
+    from .train_ppo import kl_target
+
+    kl_target(args)
     settings, members = expand_grid(seeds, lists)
     if args.pbt_every < 0:
         raise SystemExit("--pbt-every must be >= 0 (0: no population-based training)")
@@ -455,8 +483,10 @@ def train_population(args) -> dict:
     from . import Buffer, VecCarEnv, builtin_track
     from . import pbt
     from .shard import shard_range
+    from .train_ppo import explained_variance, kl_record, kl_target
 
     settings, members = check_args(args)
+    tau = kl_target(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -522,7 +552,14 @@ def train_population(args) -> dict:
                 obs_b, act_b, _, logp_b = buf.get()
                 pop.sums.zero_()
                 upd.run_epoch(obs_b.view(-1, OBS), act_b.view(-1), logp_b.view(-1), adv.view(-1), ret.view(-1), T,
-                              args.train_iters * n_mb)
+                              args.train_iters * n_mb, target_kl=tau)
+                kl_recs = None
+                if tau is not None:                              # per member, over its own [T, n] block
+                    val_b = buf.val_buf
+                    kl_all, done = upd.kl.tolist(), upd.n_done.tolist()
+                    kl_recs = [{**kl_record(kl_all[p], done[p]),
+                                "explained_variance": explained_variance(cols(ret, p), cols(val_b, p))}
+                               for p in range(pop.P)]
                 pop.decay_lr()
                 lr_now = pop.lr.tolist()                         # train_ppo records the decayed rate
                 sums = (pop.sums / args.train_iters).tolist()
@@ -546,6 +583,8 @@ def train_population(args) -> dict:
                     if evals is not None:
                         rec["eval"] = evals[p]
                         eval_ret[p] = rec["eval"]["mean_return"]
+                    if kl_recs is not None:
+                        rec.update(kl_recs[p])
                     if pbt_on:
                         rec["current_hparams"] = current[p]
                     history.append(rec)

@@ -66,6 +66,8 @@ class FusedPPOUpdate:
         self._sync = None
         self._comm = None
         self._comm_world = 1
+        self.kl = None                   # run_epoch(target_kl=...): [n_updates, 2] approx KL, clip fraction
+        self.n_done = None               # run_epoch(target_kl=...): [1] int32 updates that applied a step
 
     # ---- one launch per epoch ---------------------------------------------------------------------------------
     def connect(self, group=None):
@@ -96,10 +98,16 @@ class FusedPPOUpdate:
     def __del__(self):                   # not collective: a communicator that was never closed is left to process exit
         self._comm = None
 
-    def run_epoch(self, obs, idx, act, old_logp, adv, ret, world: int = 1, n_ctas: int = 0, prof=None):
+    def run_epoch(self, obs, idx, act, old_logp, adv, ret, world: int = 1, n_ctas: int = 0, prof=None,
+                  target_kl: float | None = None):
         """All ``idx.shape[0]`` minibatch updates (rows of ``idx`` [n_updates, batch] int64) in ONE launch: forward,
         loss, backward, gradient all-reduce over NVLink peer memory (``world`` > 1, after :meth:`connect`), clip,
-        Adam, statistics into ``self.sums``.  Asynchronous; :meth:`check_epoch` reads the kernel's error word."""
+        Adam, statistics into ``self.sums``.  Asynchronous; :meth:`check_epoch` reads the kernel's error word.
+
+        ``target_kl`` (a positive float, ``inf`` for statistics only) launches ``carenv_ppo_epoch_kl``: ``self.kl``
+        [n_updates, 2] gets each update's approx KL and clip fraction (NaN after the stopping update), ``self.n_done``
+        [1] int32 the updates that applied a step; the epoch stops at the first update whose approx KL exceeds
+        ``target_kl``.  ``None`` launches exactly what it launched before."""
         if idx.dtype != torch.int64 or idx.dim() != 2 or idx.shape[1] != self.batch or not idx.is_contiguous() \
                 or idx.device != self.device:
             raise ValueError(f"idx must be a contiguous int64 [n_updates, {self.batch}] tensor on {self.device}")
@@ -112,20 +120,33 @@ class FusedPPOUpdate:
             raise ValueError("prof must be an int64 device tensor of n_updates x 4 elements")
         if world > 1 and (self._comm is None or self._comm_world != world):
             raise _lib.CarEnvError("run_epoch(world > 1) needs connect() on every rank first")
+        if target_kl is not None and not float(target_kl) > 0.0:
+            raise ValueError("target_kl must be positive (inf: statistics without stopping)")
+        if target_kl is not None:
+            n_upd = int(idx.shape[0])
+            if self.kl is None or self.kl.shape[0] != n_upd:
+                self.kl = torch.empty((n_upd, 2), device=self.device)
+            if self.n_done is None:
+                self.n_done = torch.zeros(1, dtype=torch.int32, device=self.device)
         if idx.shape[0] == 0:            # no updates; an empty idx has no storage (data_ptr 0), which the C ABI refuses
+            if target_kl is not None:
+                self.n_done.zero_()
             return
         if self._epoch_ws is None:
             self._epoch_ws = torch.zeros(self.L.carenv_ppo_epoch_workspace_floats(), device=self.device)
             self._sync = torch.zeros(2, dtype=torch.int32, device=self.device)
+        args = (*[_p(p) for p in self.params], _p(obs), _p(idx), _p(act), _p(old_logp), _p(adv), _p(ret), self.batch,
+                int(idx.shape[0]), self.clip_ratio, self.vf_coef, self.ent_coef, _p(self.exp_avg), _p(self.exp_avg_sq),
+                _p(self.lr), _p(self.step_count), self.betas[0], self.betas[1], self.eps, self.max_grad_norm,
+                _p(self.sums), _p(self._epoch_ws), _p(self._sync), self._comm if world > 1 else None, int(n_ctas),
+                _p(prof) if prof is not None else None, self._stream())
         with torch.cuda.device(self.device):
-            rc = self.L.carenv_ppo_epoch(*[_p(p) for p in self.params], _p(obs), _p(idx), _p(act), _p(old_logp), _p(adv),
-                                         _p(ret), self.batch, int(idx.shape[0]), self.clip_ratio, self.vf_coef,
-                                         self.ent_coef, _p(self.exp_avg), _p(self.exp_avg_sq), _p(self.lr),
-                                         _p(self.step_count), self.betas[0], self.betas[1], self.eps,
-                                         self.max_grad_norm, _p(self.sums), _p(self._epoch_ws), _p(self._sync),
-                                         self._comm if world > 1 else None, int(n_ctas),
-                                         _p(prof) if prof is not None else None, self._stream())
-        _lib.check(rc, "carenv_ppo_epoch")
+            if target_kl is None:
+                rc, what = self.L.carenv_ppo_epoch(*args), "carenv_ppo_epoch"
+            else:
+                rc = self.L.carenv_ppo_epoch_kl(*args, float(target_kl), _p(self.kl), _p(self.n_done))
+                what = "carenv_ppo_epoch_kl"
+        _lib.check(rc, what)
 
     def check_epoch(self):
         """Synchronises and raises if a wait inside run_epoch's kernel timed out (a peer rank that never launched)."""

@@ -122,7 +122,50 @@ def parse_args(argv=None):
                         "the epoch's record under \"eval\".  Default 0: no evaluation")
     p.add_argument("--eval-episodes", type=int, default=1024, help="episodes per evaluation, over all ranks")
     p.add_argument("--eval-greedy", action="store_true", help="evaluate with argmax actions instead of sampled ones")
+    p.add_argument("--target-kl", type=float, default=None,
+                   help="stop an epoch's updates at the first minibatch whose approx KL, mean((ratio - 1) - log ratio) "
+                        "at the parameters before its step, exceeds this (compared against the target itself, not "
+                        "Stable-Baselines3's 1.5 x target).  Epoch records gain approx_kl, clip_fraction, updates and "
+                        "explained_variance")
+    p.add_argument("--kl-stats", action="store_true",
+                   help="the epoch-record statistics of --target-kl without stopping (a target of +inf)")
     return p.parse_args(argv)
+
+
+def kl_target(args) -> float | None:
+    """The target KL of --target-kl / --kl-stats (+inf: statistics only), None without either.  Refuses, before any
+    device work, a target that is NaN or <= 0 and the update paths that cannot report or stop."""
+    if args.target_kl is None and not args.kl_stats:
+        return None
+    tau = float("inf") if args.target_kl is None else float(args.target_kl)
+    if not tau > 0.0:
+        raise SystemExit(f"--target-kl must be positive, got {args.target_kl}")
+    if args.graph_update:
+        raise SystemExit("--target-kl / --kl-stats do not work with --graph-update: a captured update cannot stop")
+    if args.fused_update and (args.per_minibatch_update or args.compact_obs):
+        raise SystemExit("--target-kl / --kl-stats with --fused-update need the one-launch epoch kernel: the "
+                         "per-minibatch kernels (--per-minibatch-update, --compact-obs) have no KL output")
+    return tau
+
+
+def explained_variance(ret, val, world: int = 1) -> float:
+    """1 - Var(ret - val) / Var(ret) over every sample of the rollout (of every rank: float64 sums all-reduced)."""
+    r, d = ret.reshape(-1).double(), (ret - val).reshape(-1).double()
+    z = torch.stack([torch.tensor(float(r.numel()), dtype=torch.float64, device=r.device), r.sum(), (r * r).sum(),
+                     d.sum(), (d * d).sum()])
+    if world > 1:
+        dist.all_reduce(z, op=dist.ReduceOp.SUM)
+    n, sr, srr, sd, sdd = z.tolist()
+    var_r, var_d = srr / n - (sr / n) ** 2, sdd / n - (sd / n) ** 2
+    return 1.0 - var_d / var_r if var_r > 0.0 else float("nan")
+
+
+def kl_record(kl_rows, n_done: int) -> dict:
+    """approx_kl and clip_fraction: means over the evaluated updates (the stopping one included); updates: applied."""
+    n_eval = min(n_done + 1, len(kl_rows))
+    rows = kl_rows[:n_eval]
+    mean = lambda k: sum(r[k] for r in rows) / len(rows) if rows else float("nan")
+    return {"approx_kl": mean(0), "clip_fraction": mean(1), "updates": int(n_done)}
 
 
 def track_list(args) -> tuple[list[str], list[str]]:
@@ -146,6 +189,7 @@ def track_list(args) -> tuple[list[str], list[str]]:
 
 def train(args) -> list[dict]:
     names, paths = track_list(args)
+    tau = kl_target(args)
     multi = len(paths) > 1
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -323,7 +367,8 @@ def train(args) -> list[dict]:
                 idx_static = torch.zeros(args.batch_size, dtype=torch.int64, device=dev)
 
                 def update_step():
-                    """One minibatch: draw indices, clipped-surrogate loss, backward, (all-reduce), clip, Adam."""
+                    """One minibatch: draw indices, clipped-surrogate loss, backward, (all-reduce), clip, Adam.  With
+                    --target-kl / --kl-stats: returns True, without a step, when the approx KL exceeds the target."""
                     torch.randint(0, T * n, (args.batch_size,), device=dev, out=idx_static)
                     idx = idx_static
                     if fused_upd is not None:
@@ -334,6 +379,16 @@ def train(args) -> list[dict]:
                     obs_mb = envs.observe(obs_f, idx) if args.compact_obs else obs_f[idx]
                     _, new_logp, ent, new_val = agent.act(obs_mb, act_f[idx])
                     ratio = torch.exp(new_logp - logp_f[idx])
+                    if tau is not None:
+                        with torch.no_grad():
+                            st = torch.stack([((ratio - 1.0) - (new_logp - logp_f[idx])).mean(),
+                                              ((ratio - 1.0).abs() > args.clip_ratio).float().mean()])
+                            if world > 1:                           # every rank's minibatch: one small all-reduce
+                                dist.all_reduce(st, op=dist.ReduceOp.SUM)
+                                st /= world
+                        kl_rows.append(st)
+                        if tau != float("inf") and float(st[0]) > tau:
+                            return True
                     a = adv_f[idx]
                     a = (a - a.mean()) / torch.clamp(a.std(), min=1e-5)
                     pol = torch.max(-a * ratio, -a * torch.clamp(ratio, 1 - args.clip_ratio, 1 + args.clip_ratio)).mean()
@@ -353,6 +408,7 @@ def train(args) -> list[dict]:
                     nn.utils.clip_grad_norm_(params, args.max_grad_norm)
                     opt.step()
                     sums.add_(torch.stack([pol.detach(), vl.detach(), e.detach(), loss.detach()]))
+                    return False
 
                 update_graph = None
                 if graph_update and not epoch_kernel:           # obs_f, act_f, ... are views of the static buffer tensors
@@ -369,14 +425,18 @@ def train(args) -> list[dict]:
             sums.zero_()
             if fused_upd is not None:
                 fused_upd.sums.zero_()
+            kl_rows, n_done, stopped = [], 0, False
             if epoch_kernel:
                 idx_all = torch.randint(0, T * n, (args.train_iters * n_mb, args.batch_size), device=dev)
-                fused_upd.run_epoch(obs_f, idx_all, act_f, logp_f, adv_f, ret_f, world=world)
+                fused_upd.run_epoch(obs_f, idx_all, act_f, logp_f, adv_f, ret_f, world=world, target_kl=tau)
             for _ in range(0 if epoch_kernel else args.train_iters * n_mb):
                 if update_graph is not None:
                     update_graph.replay()
+                elif stopped:                                    # the stopped epoch still draws its indices
+                    torch.randint(0, T * n, (args.batch_size,), device=dev, out=idx_static)
                 else:
-                    update_step()
+                    stopped = update_step()
+                    n_done += not stopped
             if fused_upd is not None:
                 fused_upd.lr.mul_(args.learning_rate_decay)
                 sums.copy_(fused_upd.sums)
@@ -390,6 +450,13 @@ def train(args) -> list[dict]:
                    "episodes": episodes, "policy_loss": s[0], "value_loss": s[1], "entropy": s[2], "total_loss": s[3],
                    "lr": float(fused_upd.lr if fused_upd is not None else opt.param_groups[0]["lr"]), "sps": global_step / (time.time() - t_start),
                    "wall_s": time.time() - t_start}
+            if tau is not None:
+                if epoch_kernel:
+                    kl_rows, n_done = fused_upd.kl.tolist(), int(fused_upd.n_done.item())
+                else:
+                    kl_rows = torch.stack(kl_rows).tolist() if kl_rows else []
+                rec.update(kl_record(kl_rows, n_done))
+                rec["explained_variance"] = explained_variance(ret_f, val_b.reshape(-1), world)
             if by_track is not None:
                 rec["by_track"] = by_track
             if args.eval_every > 0 and epoch % args.eval_every == 0:
