@@ -10,7 +10,10 @@
 // k_ppo_epoch_pop: all n_updates minibatch updates of an epoch for all P members in ONE ordinary cluster launch.
 // Member p is one thread-block cluster of kPopCluster CTAs x 256 threads (grid P x kPopCluster); clusters never wait
 // for each other, so P may exceed the number of co-resident clusters.  Inside a cluster the plan and the arithmetic are
-// k_ppo_epoch's (ppo_epoch.cuh), with the grid replaced by the cluster:
+// k_ppo_epoch's, with the grid replaced by the cluster.  The two kernels share one copy of the parameter staging and
+// write-back, the advantage statistics, the forward with its warp fold, the backward and the Adam bias corrections
+// (the helpers in ppo_epoch.cuh); the per-sample loss and the Adam step are still written out in both, since moving
+// them into helpers changed the machine code (ppo_epoch.cuh says by how much):
 //
 //   phase A   thread j owns hidden unit j's 48 parameters in registers; CTA r takes samples [r*S, r*S + S) of the
 //             member's minibatch (S = ceil(B / kPopCluster)) in chunks of kEpochSamples and accumulates its partial
@@ -100,8 +103,6 @@ template <bool KL = false>
 __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const PopEpochArgs A) {
     using namespace ppo;
     constexpr int SMAX = kEpochSamples;
-    constexpr int kZ = 10;                               // 9 logits + the value per sample
-    constexpr int kFold = kZ * SMAX;
     constexpr int kParts = KL ? 5 : 3;                   // policy loss, entropy, value loss (, KL term, clipped)
     static_assert(SMAX * kIn <= kEpochThreads, "one thread per staged observation element");
     extern __shared__ __align__(16) float s_dyn[];
@@ -109,7 +110,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     float *const s_g = s_v + kLocalK * kH;               // this CTA's partial gradient, local order
     float *const s_slice = s_g + kLocalPad;              // reduced slice r of the gradient
     __shared__ __align__(16) float s_x[SMAX][20];
-    __shared__ float s_red[8][kFold];
+    __shared__ float s_red[8][kZ * SMAX];
     __shared__ __align__(16) float s_z[SMAX][12];
     __shared__ float s_part[SMAX][kParts];
     __shared__ float s_red8[8];
@@ -141,26 +142,15 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     const uint32_t a_g = tc::smem_u32(s_g), a_slice = tc::smem_u32(s_slice), a_line = tc::smem_u32(&s_line);
 
     float w[kLocalK];
-#pragma unroll
-    for (int k = 0; k < kLocalK; ++k) {
-        const int f = local_to_flat(k * kH + j);
-        w[k] = *param_ptr(P, f);
-        s_m[k * kH + j] = gm[f];
-        s_v[k * kH + j] = gv[f];
-    }
-    if (j < kZ) {
-        const int f = local_to_flat(kLocalK * kH + j);
-        s_b2[j] = *param_ptr(P, f); s_b2m[j] = gm[f]; s_b2v[j] = gv[f];
-    }
+    stage_unit(P, gm, gv, j, w, s_m, s_v, s_b2, s_b2m, s_b2v);
     for (int i = j; i < SMAX * 20; i += kEpochThreads) (&s_x[0][0])[i] = 0.0f;   // the padding columns stay zero
 
     // gathers of the next chunk (or of the next update's first chunk and advantages) are issued a chunk ahead
-    constexpr int kPer = kMaxBatch / kEpochThreads;
-    float x_pf = 0.0f, al_pf[kPer], l_act = 0.0f, l_olp = 0.0f, l_adv = 0.0f, l_ret = 0.0f;
+    float x_pf = 0.0f, al_pf[kAdvPer], l_act = 0.0f, l_olp = 0.0f, l_adv = 0.0f, l_ret = 0.0f;
     auto load_adv = [&](int u2) {
         const long long *idx = idx_p + (size_t)u2 * (size_t)B;
 #pragma unroll
-        for (int i = 0; i < kPer; ++i) {
+        for (int i = 0; i < kAdvPer; ++i) {
             const int t = j + i * kEpochThreads;
             al_pf[i] = t < B ? A.adv[idx[t]] : 0.0f;
         }
@@ -179,22 +169,9 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     __syncthreads();
 
     for (int u = 0; u < A.n_updates; ++u) {
-        // ---- advantage statistics of the member's whole minibatch (train.py:236-237), the same bits in every CTA
+        // ---- advantage statistics of the member's whole minibatch, the same bits in every CTA
         float a_mean, a_inv;
-        {
-            float sum = 0.0f;
-#pragma unroll
-            for (int i = 0; i < kPer; ++i) sum += al_pf[i];
-            a_mean = block_sum_256(sum, s_red8) * invB;
-            float s2 = 0.0f;
-#pragma unroll
-            for (int i = 0; i < kPer; ++i) {
-                const float d = j + i * kEpochThreads < B ? al_pf[i] - a_mean : 0.0f;
-                s2 += d * d;
-            }
-            const float var = block_sum_256(s2, s_red8) / (float)(B > 1 ? B - 1 : 1);
-            a_inv = 1.0f / fmaxf(sqrtf(var), 1.0e-5f);
-        }
+        advantage_stats(al_pf, j, B, invB, s_red8, a_mean, a_inv);
         float lp0 = 0.0f, lp1 = 0.0f, lp2 = 0.0f;       // loss partial sums of the CTA's samples (thread 0)
         float lp3 = 0.0f, lp4 = 0.0f;                   // KL: KL and clip sums of the CTA's samples (thread 0)
 
@@ -208,43 +185,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
             else if (u + 1 < A.n_updates) { load_chunk(u + 1, 0); load_adv(u + 1); }
 
             float pre_a[SMAX], pre_c[SMAX];
-            {
-                float contrib[kFold];
-#pragma unroll
-                for (int s = 0; s < SMAX; ++s) {
-                    const float4 *xv = reinterpret_cast<const float4 *>(s_x[s]);
-                    float x[20];
-#pragma unroll
-                    for (int i = 0; i < 5; ++i) { const float4 t = xv[i]; x[4 * i] = t.x; x[4 * i + 1] = t.y; x[4 * i + 2] = t.z; x[4 * i + 3] = t.w; }
-                    float pa = w[kIn], pb = 0.0f, pc = 0.0f, qa = w[2 * kIn + 1 + kQ], qb = 0.0f, qc = 0.0f;
-#pragma unroll
-                    for (int k = 0; k < kIn; k += 3) {
-                        pa = fmaf(w[k], x[k], pa); pb = fmaf(w[k + 1], x[k + 1], pb); pc = fmaf(w[k + 2], x[k + 2], pc);
-                        qa = fmaf(w[kIn + 1 + kQ + k], x[k], qa); qb = fmaf(w[kIn + 2 + kQ + k], x[k + 1], qb);
-                        qc = fmaf(w[kIn + 3 + kQ + k], x[k + 2], qc);
-                    }
-                    const bool on = s < nc;
-                    pre_a[s] = on ? (pa + pb) + pc : 0.0f;
-                    pre_c[s] = on ? (qa + qb) + qc : 0.0f;
-                    const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
-#pragma unroll
-                    for (int q = 0; q < kQ; ++q) contrib[s * kZ + q] = w[kIn + 1 + q] * ha;
-                    contrib[s * kZ + kQ] = w[kLocalK - 1] * hc;
-                }
-                warp_fold<kFold, 16, kFold>(contrib, lane);
-                constexpr int kRem = fold_rem<kFold, 16>();
-                const int base = fold_base<kFold, 16>(lane);
-#pragma unroll
-                for (int i = 0; i < kRem; ++i) s_red[warp][base + i] = contrib[i];
-            }
-            __syncthreads();
-            if (j < kFold) {
-                float t = s_red[0][j];
-#pragma unroll
-                for (int w8 = 1; w8 < 8; ++w8) t += s_red[w8][j];
-                s_z[j / kZ][j % kZ] = t;
-            }
-            __syncthreads();
+            unit_forward(w, s_x, nc, j, lane, warp, pre_a, pre_c, s_red, s_z);
 
             // ---- loss terms and their derivatives, thread = sample
             if (j < SMAX) {
@@ -306,31 +247,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
                 float g[kLocalK];
 #pragma unroll
                 for (int k = 0; k < kLocalK; ++k) g[k] = ch == 0 ? 0.0f : s_g[k * kH + j];
-#pragma unroll
-                for (int s = 0; s < SMAX; ++s) {
-                    const float4 *xv = reinterpret_cast<const float4 *>(s_x[s]);
-                    float x[20];
-#pragma unroll
-                    for (int i = 0; i < 5; ++i) { const float4 t = xv[i]; x[4 * i] = t.x; x[4 * i + 1] = t.y; x[4 * i + 2] = t.z; x[4 * i + 3] = t.w; }
-                    const float4 *zv = reinterpret_cast<const float4 *>(s_z[s]);
-                    const float4 d0 = zv[0], d1 = zv[1], d2 = zv[2];
-                    const float dz[kQ] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w, d2.x};
-                    const float dv = d2.y;
-                    const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
-                    float dh = 0.0f;
-#pragma unroll
-                    for (int q = 0; q < kQ; ++q) { g[kIn + 1 + q] = fmaf(dz[q], ha, g[kIn + 1 + q]); dh = fmaf(dz[q], w[kIn + 1 + q], dh); }
-                    dh = pre_a[s] > 0.0f ? dh : 0.0f;
-                    const float dc = pre_c[s] > 0.0f ? dv * w[kLocalK - 1] : 0.0f;
-                    g[kLocalK - 1] = fmaf(dv, hc, g[kLocalK - 1]);
-#pragma unroll
-                    for (int k = 0; k < kIn; ++k) {
-                        g[k] = fmaf(dh, x[k], g[k]);
-                        g[kIn + 1 + kQ + k] = fmaf(dc, x[k], g[kIn + 1 + kQ + k]);
-                    }
-                    g[kIn] += dh;
-                    g[2 * kIn + 1 + kQ] += dc;
-                }
+                unit_backward(w, s_x, s_z, pre_a, pre_c, g);
 #pragma unroll
                 for (int k = 0; k < kLocalK; ++k) s_g[k * kH + j] = g[k];
                 if (j < kZ) {                                        // second-layer biases: sum of dz over the samples
@@ -367,11 +284,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
                 if (j == 0) s_line_kl = make_float4(lp3, lp4, 0.0f, 0.0f);
             }
         }
-        if (j == 64) {                                                // bias corrections of this step
-            const int t_step = step0 + u + 1;
-            const float bc1 = 1.0f - powf(A.beta1, (float)t_step), bc2 = 1.0f - powf(A.beta2, (float)t_step);
-            s_bias[0] = lr / bc1; s_bias[1] = rsqrtf(bc2);
-        }
+        if (j == 64) adam_bias_corrections(s_bias, step0 + u + 1, lr, A.beta1, A.beta2);
         cluster_sync_all();                                           // every reduced slice of the cluster is complete
         const float step_size = s_bias[0], inv_sqrt_bc2 = s_bias[1];
 
@@ -451,17 +364,7 @@ __global__ void __launch_bounds__(ppo::kEpochThreads, 1) k_ppo_epoch_pop(const P
     }
     cluster_sync_all();                                               // the peers' last DSMEM reads of this CTA
     if (r == 0) {
-#pragma unroll
-        for (int k = 0; k < kLocalK; ++k) {
-            const int f = local_to_flat(k * kH + j);
-            *param_ptr(P, f) = w[k];
-            gm[f] = s_m[k * kH + j];
-            gv[f] = s_v[k * kH + j];
-        }
-        if (j < kZ) {
-            const int f = local_to_flat(kLocalK * kH + j);
-            *param_ptr(P, f) = s_b2[j]; gm[f] = s_b2m[j]; gv[f] = s_b2v[j];
-        }
+        write_back_unit(P, gm, gv, j, w, s_m, s_v, s_b2, s_b2m, s_b2v);
         if constexpr (KL) {
             float *rows = A.kl_out + 2 * pq * (size_t)A.n_updates;
             for (int i = 2 * n_eval + j; i < 2 * A.n_updates; i += kEpochThreads) rows[i] = __int_as_float(0x7fc00000);

@@ -209,6 +209,161 @@ __device__ __forceinline__ float adam_quotient(float num, float v, float inv_sqr
 
 constexpr int kEpochSamples = 8;                     // samples per CTA: G = max(64, ceil(B / 8)) CTAs cover B <= 1,024
 constexpr int kEpochSmemBytes = 2 * kLocalK * kH * (int)sizeof(float);   // Adam moments of the 48 x 256 unit parameters
+constexpr int kZ = kQ + 1;                           // 9 logits + the value per sample
+constexpr int kAdvPer = kMaxBatch / kEpochThreads;   // 4 advantage values per thread (whole minibatch)
+
+// The per-CTA arithmetic of an epoch update, shared by k_ppo_epoch and k_ppo_epoch_pop (population.cuh): thread j
+// owns hidden unit j of both nets, its 48 parameters w in registers (local order: W1a row, b1a, W2a column, W1c row,
+// b1c, W2c), their Adam moments in s_m / s_v ([48][256]); threads j < kZ also own second-layer bias j (s_b2, moments
+// s_b2m / s_b2v).  Every helper keeps the operation order the kernels had when each held its own copy, and both
+// kernels compile to the same instructions as they did then.  Two pieces are still written out in both kernels,
+// because moving them into a helper changed the machine code: the per-sample loss (softmax, clipped surrogate,
+// d loss / d logits: 1 to 130 instructions of each of the four instantiations; shared with k_ppo_forward as well, 1,223
+// of its instructions and 4 more registers) and the Adam step of phase C (about 1,000 instructions of each, 16 more
+// registers in k_ppo_epoch<8, false>; read from the argument struct inside the helper, 31 and 26 in k_ppo_epoch).
+
+// parameters and moments of unit j (and bias j) from the flat layout of P, m, v
+__device__ __forceinline__ void stage_unit(const MutableParams &P, const float *m, const float *v, const int j,
+                                           float (&w)[kLocalK], float *s_m, float *s_v, float (&s_b2)[kZ],
+                                           float (&s_b2m)[kZ], float (&s_b2v)[kZ]) {
+#pragma unroll
+    for (int k = 0; k < kLocalK; ++k) {
+        const int f = local_to_flat(k * kH + j);
+        w[k] = *param_ptr(P, f);
+        s_m[k * kH + j] = m[f];
+        s_v[k * kH + j] = v[f];
+    }
+    if (j < kZ) {
+        const int f = local_to_flat(kLocalK * kH + j);
+        s_b2[j] = *param_ptr(P, f); s_b2m[j] = m[f]; s_b2v[j] = v[f];
+    }
+}
+
+// the inverse of stage_unit
+__device__ __forceinline__ void write_back_unit(const MutableParams &P, float *m, float *v, const int j,
+                                                const float (&w)[kLocalK], const float *s_m, const float *s_v,
+                                                const float (&s_b2)[kZ], const float (&s_b2m)[kZ],
+                                                const float (&s_b2v)[kZ]) {
+#pragma unroll
+    for (int k = 0; k < kLocalK; ++k) {
+        const int f = local_to_flat(k * kH + j);
+        *param_ptr(P, f) = w[k];
+        m[f] = s_m[k * kH + j];
+        v[f] = s_v[k * kH + j];
+    }
+    if (j < kZ) {
+        const int f = local_to_flat(kLocalK * kH + j);
+        *param_ptr(P, f) = s_b2[j]; m[f] = s_b2m[j]; v[f] = s_b2v[j];
+    }
+}
+
+// advantage mean and 1 / max(std, 1e-5) of the whole minibatch (train.py:236-237, unbiased std) from the values
+// thread j holds (element j + i * 256): the same bits in every CTA
+__device__ __forceinline__ void advantage_stats(const float (&al)[kAdvPer], const int j, const int B, const float invB,
+                                                float *red8, float &a_mean, float &a_inv) {
+    float sum = 0.0f;
+#pragma unroll
+    for (int i = 0; i < kAdvPer; ++i) sum += al[i];
+    a_mean = block_sum_256(sum, red8) * invB;
+    float s2 = 0.0f;
+#pragma unroll
+    for (int i = 0; i < kAdvPer; ++i) {
+        const float d = j + i * kEpochThreads < B ? al[i] - a_mean : 0.0f;
+        s2 += d * d;
+    }
+    const float var = block_sum_256(s2, red8) / (float)(B > 1 ? B - 1 : 1);
+    a_inv = 1.0f / fmaxf(sqrtf(var), 1.0e-5f);
+}
+
+__device__ __forceinline__ void load_row(const float (&row)[20], float (&x)[20]) {
+    const float4 *xv = reinterpret_cast<const float4 *>(row);
+#pragma unroll
+    for (int i = 0; i < 5; ++i) { const float4 t = xv[i]; x[4 * i] = t.x; x[4 * i + 1] = t.y; x[4 * i + 2] = t.z; x[4 * i + 3] = t.w; }
+}
+
+// Forward of unit j for the SMAX observation rows of s_x (rows s >= n count as absent): pre-activations of both nets,
+// then the second-layer products folded over the 256 threads (transposing warp butterfly + 8-way smem fold, fixed
+// order) into s_z[s] = 9 logits | value, second-layer biases not added.  Ends with the block synchronised.
+template <int SMAX>
+__device__ __forceinline__ void unit_forward(const float (&w)[kLocalK], const float (&s_x)[SMAX][20], const int n,
+                                             const int j, const int lane, const int warp, float (&pre_a)[SMAX], float (&pre_c)[SMAX],
+                                             float (&s_red)[8][kZ * SMAX], float (&s_z)[SMAX][12]) {
+    constexpr int kFold = kZ * SMAX;
+    {
+        float contrib[kFold];
+#pragma unroll
+        for (int s = 0; s < SMAX; ++s) {
+            float x[20];
+            load_row(s_x[s], x);
+            float pa = w[kIn], pb = 0.0f, pc = 0.0f, qa = w[2 * kIn + 1 + kQ], qb = 0.0f, qc = 0.0f;   // ppo_update.cuh's order
+#pragma unroll
+            for (int k = 0; k < kIn; k += 3) {
+                pa = fmaf(w[k], x[k], pa); pb = fmaf(w[k + 1], x[k + 1], pb); pc = fmaf(w[k + 2], x[k + 2], pc);
+                qa = fmaf(w[kIn + 1 + kQ + k], x[k], qa); qb = fmaf(w[kIn + 2 + kQ + k], x[k + 1], qb);
+                qc = fmaf(w[kIn + 3 + kQ + k], x[k + 2], qc);
+            }
+            const bool on = s < n;
+            pre_a[s] = on ? (pa + pb) + pc : 0.0f;
+            pre_c[s] = on ? (qa + qb) + qc : 0.0f;
+            const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
+#pragma unroll
+            for (int q = 0; q < kQ; ++q) contrib[s * kZ + q] = w[kIn + 1 + q] * ha;
+            contrib[s * kZ + kQ] = w[kLocalK - 1] * hc;
+        }
+        warp_fold<kFold, 16, kFold>(contrib, lane);
+        constexpr int kRem = fold_rem<kFold, 16>();
+        const int base = fold_base<kFold, 16>(lane);
+#pragma unroll
+        for (int i = 0; i < kRem; ++i) s_red[warp][base + i] = contrib[i];   // lanes holding copies write the same bits
+    }
+    __syncthreads();
+    if (j < kFold) {
+        float t = s_red[0][j];
+#pragma unroll
+        for (int w8 = 1; w8 < 8; ++w8) t += s_red[w8][j];
+        s_z[j / kZ][j % kZ] = t;
+    }
+    __syncthreads();
+}
+
+// Backward of unit j over the SMAX rows: adds to g the gradients of its 48 parameters, given s_z[s] = d loss / d logits
+// | d loss / d value and unit_forward's pre-activations
+template <int SMAX>
+__device__ __forceinline__ void unit_backward(const float (&w)[kLocalK], const float (&s_x)[SMAX][20],
+                                              const float (&s_z)[SMAX][12], const float (&pre_a)[SMAX],
+                                              const float (&pre_c)[SMAX], float (&g)[kLocalK]) {
+#pragma unroll
+    for (int s = 0; s < SMAX; ++s) {
+        float x[20];
+        load_row(s_x[s], x);
+        const float4 *zv = reinterpret_cast<const float4 *>(s_z[s]);
+        const float4 d0 = zv[0], d1 = zv[1], d2 = zv[2];
+        const float dz[kQ] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w, d2.x};
+        const float dv = d2.y;
+        const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
+        float dh = 0.0f;
+#pragma unroll
+        for (int q = 0; q < kQ; ++q) { g[kIn + 1 + q] = fmaf(dz[q], ha, g[kIn + 1 + q]); dh = fmaf(dz[q], w[kIn + 1 + q], dh); }
+        dh = pre_a[s] > 0.0f ? dh : 0.0f;                        // ReLU'(pre), zero at pre == 0 like torch
+        const float dc = pre_c[s] > 0.0f ? dv * w[kLocalK - 1] : 0.0f;
+        g[kLocalK - 1] = fmaf(dv, hc, g[kLocalK - 1]);
+#pragma unroll
+        for (int k = 0; k < kIn; ++k) {
+            g[k] = fmaf(dh, x[k], g[k]);
+            g[kIn + 1 + kQ + k] = fmaf(dc, x[k], g[kIn + 1 + kQ + k]);
+        }
+        g[kIn] += dh;
+        g[2 * kIn + 1 + kQ] += dc;
+    }
+}
+
+// Adam bias corrections of step t: s_bias = {lr / (1 - beta1^t), 1 / sqrt(1 - beta2^t)}.  powf is ~150 instructions,
+// so one thread forms them while a barrier is pending.
+__device__ __forceinline__ void adam_bias_corrections(float (&s_bias)[2], const int t, const float lr,
+                                                      const float beta1, const float beta2) {
+    const float bc1 = 1.0f - powf(beta1, (float)t), bc2 = 1.0f - powf(beta2, (float)t);
+    s_bias[0] = lr / bc1; s_bias[1] = rsqrtf(bc2);
+}
 
 // KL = true adds the PPO diagnostics and the early stop (carenv_ppo_epoch_kl): phase A also sums each sample's
 // (ratio - 1) - log ratio and |ratio - 1| > clip_ratio; the two CTA sums ride in the partial-gradient row at columns
@@ -220,13 +375,11 @@ constexpr int kEpochSmemBytes = 2 * kLocalK * kH * (int)sizeof(float);   // Adam
 template <int SMAX, bool KL = false>
 __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs A) {
     static_assert(SMAX * kIn <= kEpochThreads, "one thread per staged observation element");
-    constexpr int kZ = 10;                               // 9 logits + the value per sample
-    constexpr int kFold = kZ * SMAX;
-    constexpr int kParts = KL ? 5 : 3;                   // policy loss, entropy, value loss (, KL term, clipped)
+    constexpr int kParts = KL ? 5 : 3;                  // policy loss, entropy, value loss (, KL term, clipped)
     extern __shared__ __align__(16) float s_dyn[];       // m [48][256] | v [48][256]: this CTA's copy of the Adam moments
     float *const s_m = s_dyn, *const s_v = s_dyn + kLocalK * kH;
     __shared__ __align__(16) float s_x[SMAX][20];        // observation rows of the CTA's samples
-    __shared__ float s_red[8][kFold];                    // per-warp sums of the second layer
+    __shared__ float s_red[8][kZ * SMAX];                // per-warp sums of the second layer
     __shared__ __align__(16) float s_z[SMAX][12];        // logits | value, then d loss / d logits | d loss / d value
     __shared__ float s_part[SMAX][kParts];               // per-sample policy loss, entropy, value loss
     __shared__ float s_red8[8];
@@ -265,27 +418,16 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
     // the same Adam step to its copy (same operations on the same reduced gradient: same bits), so the next forward
     // needs neither a reload nor a third grid barrier; CTA 0 writes the result back at the end.
     float w[kLocalK];
-#pragma unroll
-    for (int k = 0; k < kLocalK; ++k) {
-        const int f = local_to_flat(k * kH + j);
-        w[k] = *param_ptr(A.P, f);
-        s_m[k * kH + j] = A.m[f];
-        s_v[k * kH + j] = A.v[f];
-    }
-    if (j < kZ) {
-        const int f = local_to_flat(kLocalK * kH + j);
-        s_b2[j] = *param_ptr(A.P, f); s_b2m[j] = A.m[f]; s_b2v[j] = A.v[f];
-    }
+    stage_unit(A.P, A.m, A.v, j, w, s_m, s_v, s_b2, s_b2m, s_b2v);
     for (int i = j; i < SMAX * 20; i += kEpochThreads) (&s_x[0][0])[i] = 0.0f;   // rows >= nS and the padding stay zero
 
     // ---- gathers of the next update are issued before the grid barriers and land while the CTA waits
-    constexpr int kPer = kMaxBatch / kEpochThreads;      // 4 advantage values per thread (whole minibatch)
-    float x_pf = 0.0f, al_pf[kPer], l_act = 0.0f, l_olp = 0.0f, l_adv = 0.0f, l_ret = 0.0f;
+    float x_pf = 0.0f, al_pf[kAdvPer], l_act = 0.0f, l_olp = 0.0f, l_adv = 0.0f, l_ret = 0.0f;
     auto prefetch = [&](int u2) {
         const long long *idx = A.idx + (size_t)u2 * (size_t)B;
         if (j < nS * kIn) x_pf = A.obs[(size_t)idx[s0 + j / kIn] * kIn + j % kIn];
 #pragma unroll
-        for (int i = 0; i < kPer; ++i) {
+        for (int i = 0; i < kAdvPer; ++i) {
             const int t = j + i * kEpochThreads;
             al_pf[i] = t < B ? A.adv[idx[t]] : 0.0f;
         }
@@ -307,61 +449,12 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
 
         // ---- advantage statistics of the whole minibatch (train.py:236-237), the same bits in every CTA
         float a_mean, a_inv;
-        {
-            float sum = 0.0f;
-#pragma unroll
-            for (int i = 0; i < kPer; ++i) sum += al_pf[i];
-            a_mean = block_sum_256(sum, s_red8) * invB;
-            float s2 = 0.0f;
-#pragma unroll
-            for (int i = 0; i < kPer; ++i) {
-                const float d = j + i * kEpochThreads < B ? al_pf[i] - a_mean : 0.0f;
-                s2 += d * d;
-            }
-            const float var = block_sum_256(s2, s_red8) / (float)(B > 1 ? B - 1 : 1);
-            a_inv = 1.0f / fmaxf(sqrtf(var), 1.0e-5f);
-        }
+        advantage_stats(al_pf, j, B, invB, s_red8, a_mean, a_inv);
         __syncthreads();                                              // s_x complete
 
         // ---- forward: pre-activations of unit j for the CTA's samples, second-layer products
         float pre_a[SMAX], pre_c[SMAX];
-        {
-            float contrib[kFold];
-#pragma unroll
-            for (int s = 0; s < SMAX; ++s) {
-                const float4 *xv = reinterpret_cast<const float4 *>(s_x[s]);
-                float x[20];
-#pragma unroll
-                for (int i = 0; i < 5; ++i) { const float4 t = xv[i]; x[4 * i] = t.x; x[4 * i + 1] = t.y; x[4 * i + 2] = t.z; x[4 * i + 3] = t.w; }
-                float pa = w[kIn], pb = 0.0f, pc = 0.0f, qa = w[2 * kIn + 1 + kQ], qb = 0.0f, qc = 0.0f;   // ppo_update.cuh's order
-#pragma unroll
-                for (int k = 0; k < kIn; k += 3) {
-                    pa = fmaf(w[k], x[k], pa); pb = fmaf(w[k + 1], x[k + 1], pb); pc = fmaf(w[k + 2], x[k + 2], pc);
-                    qa = fmaf(w[kIn + 1 + kQ + k], x[k], qa); qb = fmaf(w[kIn + 2 + kQ + k], x[k + 1], qb);
-                    qc = fmaf(w[kIn + 3 + kQ + k], x[k + 2], qc);
-                }
-                const bool on = s < nS;
-                pre_a[s] = on ? (pa + pb) + pc : 0.0f;
-                pre_c[s] = on ? (qa + qb) + qc : 0.0f;
-                const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
-#pragma unroll
-                for (int q = 0; q < kQ; ++q) contrib[s * kZ + q] = w[kIn + 1 + q] * ha;
-                contrib[s * kZ + kQ] = w[kLocalK - 1] * hc;
-            }
-            warp_fold<kFold, 16, kFold>(contrib, lane);
-            constexpr int kRem = fold_rem<kFold, 16>();
-            const int base = fold_base<kFold, 16>(lane);
-#pragma unroll
-            for (int i = 0; i < kRem; ++i) s_red[warp][base + i] = contrib[i];   // lanes holding copies write the same bits
-        }
-        __syncthreads();
-        if (j < kFold) {
-            float t = s_red[0][j];
-#pragma unroll
-            for (int w8 = 1; w8 < 8; ++w8) t += s_red[w8][j];
-            s_z[j / kZ][j % kZ] = t;
-        }
-        __syncthreads();
+        unit_forward(w, s_x, nS, j, lane, warp, pre_a, pre_c, s_red, s_z);
 
         // ---- loss terms and their derivatives, thread = sample (ppo_update.cuh: k_ppo_forward)
         if (j < SMAX) {
@@ -415,31 +508,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
             float g[kLocalK];
 #pragma unroll
             for (int k = 0; k < kLocalK; ++k) g[k] = 0.0f;
-#pragma unroll
-            for (int s = 0; s < SMAX; ++s) {
-                const float4 *xv = reinterpret_cast<const float4 *>(s_x[s]);
-                float x[20];
-#pragma unroll
-                for (int i = 0; i < 5; ++i) { const float4 t = xv[i]; x[4 * i] = t.x; x[4 * i + 1] = t.y; x[4 * i + 2] = t.z; x[4 * i + 3] = t.w; }
-                const float4 *zv = reinterpret_cast<const float4 *>(s_z[s]);
-                const float4 d0 = zv[0], d1 = zv[1], d2 = zv[2];
-                const float dz[kQ] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w, d2.x};
-                const float dv = d2.y;
-                const float ha = fmaxf(pre_a[s], 0.0f), hc = fmaxf(pre_c[s], 0.0f);
-                float dh = 0.0f;
-#pragma unroll
-                for (int q = 0; q < kQ; ++q) { g[kIn + 1 + q] = fmaf(dz[q], ha, g[kIn + 1 + q]); dh = fmaf(dz[q], w[kIn + 1 + q], dh); }
-                dh = pre_a[s] > 0.0f ? dh : 0.0f;                    // ReLU'(pre), zero at pre == 0 like torch
-                const float dc = pre_c[s] > 0.0f ? dv * w[kLocalK - 1] : 0.0f;
-                g[kLocalK - 1] = fmaf(dv, hc, g[kLocalK - 1]);
-#pragma unroll
-                for (int k = 0; k < kIn; ++k) {
-                    g[k] = fmaf(dh, x[k], g[k]);
-                    g[kIn + 1 + kQ + k] = fmaf(dc, x[k], g[kIn + 1 + kQ + k]);
-                }
-                g[kIn] += dh;
-                g[2 * kIn + 1 + kQ] += dc;
-            }
+            unit_backward(w, s_x, s_z, pre_a, pre_c, g);
             float *row = A.partial + (size_t)c * kLocalPad;
 #pragma unroll
             for (int k = 0; k < kLocalK; ++k) __stcg(row + k * kH + j, g[k]);
@@ -522,12 +591,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
                 __stcg(reinterpret_cast<float4 *>(A.stat) + par * kMaxCtas + c, make_float4(ss, p0, p1, p2));
             }
         }
-        // bias corrections of this step, by one thread while the barrier is pending (powf is ~150 instructions)
-        if (j == 64) {
-            const int t_step = step0 + u + 1;
-            const float bc1 = 1.0f - powf(A.beta1, (float)t_step), bc2 = 1.0f - powf(A.beta2, (float)t_step);
-            s_bias[0] = lr / bc1; s_bias[1] = rsqrtf(bc2);
-        }
+        if (j == 64) adam_bias_corrections(s_bias, step0 + u + 1, lr, A.beta1, A.beta2);
         if (grid_barrier(A.bar, bar_target, A.err, &s_flag)) return;
         const float step_size = s_bias[0], inv_sqrt_bc2 = s_bias[1];
         if (stamp) A.prof[4 * u + 2] = global_ns();
@@ -598,17 +662,7 @@ __global__ void __launch_bounds__(kEpochThreads, 1) k_ppo_epoch(const EpochArgs 
     }
     // ---- write the parameters and moments back (every CTA holds the same bits; CTA 0 writes)
     if (c == 0) {
-#pragma unroll
-        for (int k = 0; k < kLocalK; ++k) {
-            const int f = local_to_flat(k * kH + j);
-            *param_ptr(A.P, f) = w[k];
-            A.m[f] = s_m[k * kH + j];
-            A.v[f] = s_v[k * kH + j];
-        }
-        if (j < kZ) {
-            const int f = local_to_flat(kLocalK * kH + j);
-            *param_ptr(A.P, f) = s_b2[j]; A.m[f] = s_b2m[j]; A.v[f] = s_b2v[j];
-        }
+        write_back_unit(A.P, A.m, A.v, j, w, s_m, s_v, s_b2, s_b2m, s_b2v);
         if constexpr (KL) {
             for (int i = 2 * n_eval + j; i < 2 * A.n_updates; i += kEpochThreads) A.kl_out[i] = __int_as_float(0x7fc00000);
             if (j == 0) {
