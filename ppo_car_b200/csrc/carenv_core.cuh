@@ -391,10 +391,36 @@ struct WallAcc2 {
 #if !defined(__CUDACC__)
 struct float4 { float x, y, z, w; };
 #endif
+// Candidate table of the culled pair kernels (build_cull_table, carenv_tables.h): a square grid of kCullCell px cells
+// over the track; entry [cell][k mod 6] has bit jp set unless segment pair jp provably cannot be the nearest hit of any
+// of the 12 rays of a heading k from anywhere in the cell.  Row nx * ny (positions off the grid) has every bit set.
+constexpr int kCullClasses = 6;     // the 12 ray directions of heading k are k + 6i: they depend on k mod 6 only
+struct CullGrid {
+    const uint16_t *mask;   // [nx * ny + 1][kCullClasses]
+    float x0, y0, inv_cell;
+    int nx, ny;
+};
 struct TabView {
     const float4 *base;     // this thread's copy
     int row_f4;             // float4 per row
+    CullGrid cull;          // read by the CULL instantiations only
 };
+
+// Pairs that may hold a nearest hit for the position (px, py) and heading k.  The cell is found in float32 from the
+// float32 position: far less than the table's dilation of the cells (kCullDilate) away from the float64 one.  On the
+// GPU the entry is OR-ed over the lanes that run together, so the mask is warp-uniform and every lane keeps a superset
+// of its own candidates.
+CE_HD unsigned cull_keep(const CullGrid &g, double px, double py, int k) {
+    const float fx = fmul(fsub((float)px, g.x0), g.inv_cell), fy = fmul(fsub((float)py, g.y0), g.inv_cell);
+    const bool on = fx >= 0.0f && fx < (float)g.nx && fy >= 0.0f && fy < (float)g.ny;   // false for NaN too
+    const int cell = on ? (int)fx + g.nx * (int)fy : g.nx * g.ny;
+#if defined(__CUDA_ARCH__)
+    const unsigned m = __ldg(g.mask + cell * kCullClasses + k % kCullClasses);
+    return __reduce_or_sync(__activemask(), m);
+#else
+    return g.mask[cell * kCullClasses + k % kCullClasses];
+#endif
+}
 
 // (q_l, q_{l+3}) = hx*(s_l, c_l) + ((-hy, hy)*(c_l, s_l) - (cp_l, cp_{l+3})): two FFMA2 whose wall-point operands
 // come straight from uniform registers — the same IEEE operations per component as wall_point.
@@ -421,34 +447,43 @@ CE_HD void wall_chain_start2(WallAcc2 &w, const SegF &f) {
 
 // TAB: the denominators come from the table rows tb[l] (entry jp) instead of two DMUL + two DFMA + two F2F per segment
 // and line pair — same values (seg_den).
+// hits = false (culled pairs, see cull_keep): only the end points' offsets, the guards and un; the reciprocals, the
+// denominators and the folds into Rp / Rm are skipped.  The guards gq / gu are then what the full pair gives, so every
+// slow-path decision is unchanged; a line whose guard did not trip has exact hit masks, and on it a culled pair is
+// missed or strictly farther than a kept hit, so Rp and Rm are unchanged too (DESIGN.md §3).
 template <bool TAB>
 CE_HD void wall_pair(WallAcc2 &w, const SegF &f0, const SegD &g0, const SegF &f1, const SegD &g1, double px,
-                     double py, const float4 *const *tb = nullptr, int jp = 0) {
+                     double py, const float4 *const *tb = nullptr, int jp = 0, bool hits = true) {
     P2 QB0[3], QB1[3];
     const SegHead h0 = seg_head(f0), h1 = seg_head(f1);     // bhx, ex, -bhy, bhy: one 128-bit uniform load each
     wall_point2(w, h0.bhx, h0.nbhy, h0.bhy, QB0);
     wall_point2(w, h1.bhx, h1.nbhy, h1.bhy, QB1);
     const float un0 = (float)dfma(g0.ey, px, dfma(-g0.ex, py, g0.K));
     const float un1 = (float)dfma(g1.ey, px, dfma(-g1.ex, py, g1.K));
-    const float inv0 = frcp(un0), inv1 = frcp(un1);
     w.gu = fmin3(w.gu, fabsf(un0), fabsf(un1));
+    if (hits) {
+        const float inv0 = frcp(un0), inv1 = frcp(un1);
+#pragma unroll
+        for (int l = 0; l < 3; ++l) {
+            P2 D0, D1;
+            if (TAB) {
+                const float4 t = tb[l][jp];
+                D0 = p2(t.x, t.y); D1 = p2(t.z, t.w);
+            } else {
+                float a0, a3, b0, b3;
+                seg_den(g0.ex, g0.ey, w.T64[l].y, w.T64[l].x, a0, a3);
+                seg_den(g1.ex, g1.ey, w.T64[l].y, w.T64[l].x, b0, b3);
+                D0 = p2(a0, a3); D1 = p2(b0, b3);
+            }
+            const P2 R0 = pmul(D0, p2(inv0, inv0)), R1 = pmul(D1, p2(inv1, inv1));
+            const P2 H0 = pmul(R0, p2(sat_mul(w.QA[l].x, -QB0[l].x), sat_mul(w.QA[l].y, -QB0[l].y)));
+            const P2 H1 = pmul(R1, p2(sat_mul(QB0[l].x, -QB1[l].x), sat_mul(QB0[l].y, -QB1[l].y)));
+            w.Rp[l] = fmax3(w.Rp[l], H0.x, H1.x); w.Rm[l] = fmin3(w.Rm[l], H0.x, H1.x);
+            w.Rp[l + 3] = fmax3(w.Rp[l + 3], H0.y, H1.y); w.Rm[l + 3] = fmin3(w.Rm[l + 3], H0.y, H1.y);
+        }
+    }
 #pragma unroll
     for (int l = 0; l < 3; ++l) {
-        P2 D0, D1;
-        if (TAB) {
-            const float4 t = tb[l][jp];
-            D0 = p2(t.x, t.y); D1 = p2(t.z, t.w);
-        } else {
-            float a0, a3, b0, b3;
-            seg_den(g0.ex, g0.ey, w.T64[l].y, w.T64[l].x, a0, a3);
-            seg_den(g1.ex, g1.ey, w.T64[l].y, w.T64[l].x, b0, b3);
-            D0 = p2(a0, a3); D1 = p2(b0, b3);
-        }
-        const P2 R0 = pmul(D0, p2(inv0, inv0)), R1 = pmul(D1, p2(inv1, inv1));
-        const P2 H0 = pmul(R0, p2(sat_mul(w.QA[l].x, -QB0[l].x), sat_mul(w.QA[l].y, -QB0[l].y)));
-        const P2 H1 = pmul(R1, p2(sat_mul(QB0[l].x, -QB1[l].x), sat_mul(QB0[l].y, -QB1[l].y)));
-        w.Rp[l] = fmax3(w.Rp[l], H0.x, H1.x); w.Rm[l] = fmin3(w.Rm[l], H0.x, H1.x);
-        w.Rp[l + 3] = fmax3(w.Rp[l + 3], H0.y, H1.y); w.Rm[l + 3] = fmin3(w.Rm[l + 3], H0.y, H1.y);
         w.gq[l] = fmin3(w.gq[l], fabsf(QB0[l].x), fabsf(QB1[l].x));
         w.gq[l + 3] = fmin3(w.gq[l + 3], fabsf(QB0[l].y), fabsf(QB1[l].y));
         w.QA[l] = QB1[l];
@@ -518,7 +553,8 @@ __device__ __forceinline__ void cast_walls_warp(const EnvState &s, const Tables 
 // Round 1 measured a full unroll of 24 segments as instruction-cache bound (1.5 "no instruction" stalls per issue);
 // with the pair arithmetic the 24-segment wall block is about 900 instructions and 4.4 % faster (DESIGN.md §3).
 // TAB (U > 1 only): denominators from the per-track table `tv` (k_rollout_tab) instead of being recomputed.
-template <int U, bool TAB = false, int NS = 0>
+// CULL (TAB and NS > 0 only): the hit part of a pair runs only where the candidate table tv->cull keeps it (cull_keep).
+template <int U, bool TAB = false, int NS = 0, bool CULL = false>
 CE_HD bool cast_walls(const EnvState &s, const TrackParams &P, const Tables &T, float dist[kNumRays],
                       unsigned long long *stats, const WarpSeg *ws = nullptr, const TabView *tv = nullptr) {
     const float R0 = kNoHitR;
@@ -547,12 +583,14 @@ CE_HD bool cast_walls(const EnvState &s, const TrackParams &P, const Tables &T, 
 #pragma unroll
         for (int l = 0; l < 6; ++l) { w.Rp[l] = R0; w.Rm[l] = -R0; w.gq[l] = 1.0e30f; }
         w.gu = 1.0e30f;
+        static_assert(!CULL || (TAB && NS > 0), "the culled pair path is the table kernel's full unroll");
+        const unsigned keep = CULL ? cull_keep(tv->cull, s.px, s.py, s.k) : ~0u;
         auto segments = [&](int j0) {                       // segments j0 .. j0 + U - 1
             if (P.segf[j0].chain_start) wall_chain_start2(w, P.segf[j0]);
 #pragma unroll
             for (int u = 0; u < U; u += 2)
                 wall_pair<TAB>(w, P.segf[j0 + u], P.segd[j0 + u], P.segf[j0 + u + 1], P.segd[j0 + u + 1], s.px, s.py,
-                               tb, (j0 + u) >> 1);
+                               tb, (j0 + u) >> 1, !CULL || ((keep >> ((j0 + u) >> 1)) & 1u));
         };
         if (NS > 0) {
             // every segment index is a constant: the records are constant-bank operands, no indexed loads, no loop
@@ -660,7 +698,7 @@ CE_HD void pose_observation(const EnvState &s, float vx10, float vy10, const flo
 // ---- one CarEnv.step with same-step autoreset --------------------------------------------------
 // `final_obs` (optional, 18 floats): receives the observation of the state the step ended in BEFORE the autoreset —
 // gymnasium's info["final_observation"]; it equals o.obs wherever the episode did not end.
-template <int U, bool TAB = false, int NS = 0>
+template <int U, bool TAB = false, int NS = 0, bool CULL = false>
 CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackParams &P, const Tables &T,
                     StepResult &o, unsigned long long *stats, const WarpSeg *ws = nullptr, const TabView *tv = nullptr,
                     float *final_obs = nullptr) {
@@ -682,7 +720,7 @@ CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackPar
     integrate(s, thrust, k_pre, T);
 
     float dist[kNumRays];
-    bool destroyed = cast_walls<U, TAB, NS>(s, P, T, dist, stats, ws, tv);
+    bool destroyed = cast_walls<U, TAB, NS, CULL>(s, P, T, dist, stats, ws, tv);
     destroyed = destroyed || (P.start_destroyed != 0);
     s.t += 1;
     o.terminated = 0; o.truncated = 0;

@@ -71,6 +71,7 @@ struct Handle {
     HostTrack host;
     unsigned char *d_blob;    // trig64 | acc64 | gates | trig32 | trig32s | walls64 | segf | segd | den4
     const float4 *d_den4;     // [72][n_pairs] denominators of the pair kernels (null: track without pairs)
+    CullGrid cull;            // candidate table of the culled table kernels (mask in d_blob after den4; null: none)
     int host_ranges;          // tuning hook: sub-ranges of the host-buffer step (0 = by size)
     float *cur_fobs;          // pre-reset ("final") observations for the launch being dispatched (else null)
     int4 *cur_rec;            // step records instead of reward / flag arrays for the launch being dispatched (else null)
@@ -322,9 +323,10 @@ k_rollout(const __grid_constant__ TrackParams P, const Tables G, int n_envs, int
 #define CARENV_TAB_THREADS 512
 #endif
 constexpr int kTabThreads = CARENV_TAB_THREADS;
-template <typename ActT, typename FlagT, int U, int NS = 0>
+template <typename ActT, typename FlagT, int U, int NS = 0, bool CULL = false>
 __global__ void __launch_bounds__(kTabThreads, 1)
-k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4, int n_pairs,
+k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4, const CullGrid cull,
+              int n_pairs,
               int row_f4, int copies, int table_bytes, int n_envs, int n_steps, int epb_main, int n_main, int epb_last,
               int n_blocks,
               double2 *__restrict__ pos, double2 *__restrict__ vel, int4 *__restrict__ ints,
@@ -343,7 +345,7 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
         for (int c = 0; c < copies; ++c) tab[c * copy_f4 + k * row_f4 + jp] = v;
     }
     const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
-    const TabView tv{tab + (threadIdx.x & (copies - 1)) * copy_f4, row_f4};
+    const TabView tv{tab + (threadIdx.x & (copies - 1)) * copy_f4, row_f4, cull};
 
     // blocks [0, n_main) hold epb_main environments each (full rounds: four warps per scheduler), the blocks of the
     // last round epb_last (a multiple of 128: every scheduler of the SM gets the same number of warps)
@@ -367,7 +369,7 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
             const int a = a_next;
             if (t + 1 < n_steps) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
-            env_step<U, true, NS>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
+            env_step<U, true, NS, CULL>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
                 float2 *dst = reinterpret_cast<float2 *>(obs_out + idx * kObsDim);
 #pragma unroll
@@ -395,9 +397,10 @@ k_rollout_tab(const __grid_constant__ TrackParams P, const Tables G, const float
 // is at least n_steps long, so the first part has finished by then; the flag makes it safe).  Every warp is busy for
 // the same number of steps and every scheduler keeps four warps until the very end.  Per-environment arithmetic is
 // untouched: results are bit-identical to k_rollout_tab / k_rollout.
-template <typename ActT, typename FlagT, int U, int NS = 0>
+template <typename ActT, typename FlagT, int U, int NS = 0, bool CULL = false>
 __global__ void __launch_bounds__(kTabThreads, 1)
-k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4, int n_pairs,
+k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, const float4 *__restrict__ den4,
+                     const CullGrid cull, int n_pairs,
                      int row_f4, int copies, int table_bytes, int n_envs, int n_steps, int *__restrict__ flags,
                      double2 *__restrict__ pos, double2 *__restrict__ vel, int4 *__restrict__ ints,
                      const ActT *__restrict__ actions, double reward_scale, float *__restrict__ obs_out,
@@ -414,7 +417,7 @@ k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, cons
         for (int c = 0; c < copies; ++c) tab[c * copy_f4 + k * row_f4 + jp] = v;
     }
     const Tables T = stage_tables(G, P.n_gates, P.n_seg, smem);      // ends with __syncthreads()
-    const TabView tv{tab + (threadIdx.x & (copies - 1)) * copy_f4, row_f4};
+    const TabView tv{tab + (threadIdx.x & (copies - 1)) * copy_f4, row_f4, cull};
 
     // (the warp index through a shuffle: the compiler then knows that it — and with it every item bound below, the
     // trip count of the step loop included — is warp-uniform; derived from threadIdx alone the loop counted as
@@ -459,7 +462,7 @@ k_rollout_tab_sliced(const __grid_constant__ TrackParams P, const Tables G, cons
             const int a = a_next;
             if (t + 1 < t1) a_next = action_index(actions[idx + (size_t)n_envs]);
             StepResult o;
-            env_step<U, true, NS>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
+            env_step<U, true, NS, CULL>(s, a, reward_scale, P, T, o, stats, nullptr, &tv);
             if (obs_mode == kObsFull) {
                 float2 *dst = reinterpret_cast<float2 *>(obs_out + idx * kObsDim);
 #pragma unroll
@@ -787,6 +790,8 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
                        void *trunc_out, int32_t *info_out, cudaStream_t stream, int obs_mode) {
     // The segment loop fully unrolled (NS = n_seg) for the segment counts of the shipped tracks, big_track (24) and
     // track.json (16): no indexed constant loads and no loop overhead (DESIGN.md §3).  Other tracks run the U loop.
+    // big_track's unroll skips the segment pairs the candidate table culls (CULL, cast_walls): 3.7 of 12 pairs per
+    // warp-step, 5 % faster.  track.json's does not: it culls 1 of 8 and the lookup costs more (3 % slower, §3).
     const int n_seg = h->host.P.n_seg;
     const int n_pairs = h->host.n_pairs;
     const int row_f4 = (n_pairs + 7) / 8 * 8;                // rows are multiples of 128 bytes
@@ -828,14 +833,14 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
                 auto launch_s = [&](auto kern) -> int {
                     CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_s));
                     kern<<<sms, block, smem_s, stream>>>(
-                        h->host.P, h->dev, h->d_den4, n_pairs, row_f4, copies, table_bytes, n_envs, n_steps, h->d_flags,
+                        h->host.P, h->dev, h->d_den4, h->cull, n_pairs, row_f4, copies, table_bytes, n_envs, n_steps, h->d_flags,
                         reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints),
                         static_cast<const ActT *>(actions), reward_scale, obs_out, reward_out, static_cast<FlagT *>(term_out),
                         static_cast<FlagT *>(trunc_out), reinterpret_cast<int4 *>(info_out), h->cur_rec, h->d_stats, obs_mode);
                     CU(cudaGetLastError());
                     return 0;
                 };
-                if (U == 6 && n_seg == 24) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 6, 24>);
+                if (U == 6 && n_seg == 24) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 6, 24, true>);
                 if (U == 4 && n_seg == 16) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 4, 16>);
                 if (U == 6) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 6>);
                 if (U == 4) return launch_s(k_rollout_tab_sliced<ActT, FlagT, 4>);
@@ -858,7 +863,8 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
     auto launch = [&](auto kern) -> int {
         CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<grid, block, smem, stream>>>(
-            h->host.P, h->dev, h->d_den4, n_pairs, row_f4, copies, table_bytes, n_envs, n_steps, epb_main, n_main, epb_last,
+            h->host.P, h->dev, h->d_den4, h->cull, n_pairs, row_f4, copies, table_bytes, n_envs, n_steps, epb_main, n_main,
+            epb_last,
             n_blocks,
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints),
             static_cast<const ActT *>(actions), reward_scale, obs_out, reward_out, static_cast<FlagT *>(term_out),
@@ -866,7 +872,7 @@ int launch_rollout_tab(Handle *h, int U, int n_envs, int n_steps, double *pos, d
         CU(cudaGetLastError());
         return 0;
     };
-    if (U == 6 && n_seg == 24) return launch(k_rollout_tab<ActT, FlagT, 6, 24>);
+    if (U == 6 && n_seg == 24) return launch(k_rollout_tab<ActT, FlagT, 6, 24, true>);
     if (U == 4 && n_seg == 16) return launch(k_rollout_tab<ActT, FlagT, 4, 16>);
     if (U == 6) return launch(k_rollout_tab<ActT, FlagT, 6>);
     if (U == 4) return launch(k_rollout_tab<ActT, FlagT, 4>);
@@ -981,7 +987,8 @@ int carenv_create(const double *walls, int n_walls, const double *gates, int n_g
     h->smem_bytes = big ? o_segd + b_segd : o_walls + b_walls;
     if (h->smem_bytes > 200 * 1024) { delete h; return fail(CARENV_E_TRACK, "track tables do not fit in shared memory"); }
     const size_t o_den4 = (o_segd + b_segd + 15) / 16 * 16, b_den4 = sizeof(float) * h->host.den4.size();
-    cudaError_t e = cudaMalloc(&h->d_blob, o_den4 + b_den4 + 16);
+    const size_t o_cull = o_den4 + b_den4, b_cull = sizeof(uint16_t) * h->host.cull.size();
+    cudaError_t e = cudaMalloc(&h->d_blob, o_cull + b_cull + 16);
     if (e == cudaSuccess) e = cudaMalloc(&h->d_stats, sizeof(unsigned long long) * kNumStats);
     if (e == cudaSuccess) e = cudaMemset(h->d_stats, 0, sizeof(unsigned long long) * kNumStats);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob, h->host.trig64.data(), b_trig64, cudaMemcpyHostToDevice);
@@ -990,6 +997,7 @@ int carenv_create(const double *walls, int n_walls, const double *gates, int n_g
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob + o_trig32, h->host.trig32.data(), b_trig32 / 2, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob + o_trig32 + b_trig32 / 2, h->host.trig32s.data(), b_trig32 / 2, cudaMemcpyHostToDevice);
     if (e == cudaSuccess && b_den4) e = cudaMemcpy(h->d_blob + o_den4, h->host.den4.data(), b_den4, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && b_cull) e = cudaMemcpy(h->d_blob + o_cull, h->host.cull.data(), b_cull, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob + o_walls, h->host.walls64.data(), b_walls, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob + o_segf, h->host.segf.data(), b_segf, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_blob + o_segd, h->host.segd.data(), b_segd, cudaMemcpyHostToDevice);
@@ -1004,6 +1012,8 @@ int carenv_create(const double *walls, int n_walls, const double *gates, int n_g
     h->dev.trig32 = reinterpret_cast<const F2 *>(h->d_blob + o_trig32);
     h->dev.trig32s = h->dev.trig32 + kHeadings;
     h->d_den4 = b_den4 ? reinterpret_cast<const float4 *>(h->d_blob + o_den4) : nullptr;
+    h->cull = h->host.cull_grid;
+    h->cull.mask = b_cull ? reinterpret_cast<const uint16_t *>(h->d_blob + o_cull) : nullptr;
     h->dev.walls64 = reinterpret_cast<const double *>(h->d_blob + o_walls);
     h->dev.segf = reinterpret_cast<const SegF *>(h->d_blob + o_segf);
     h->dev.segd = reinterpret_cast<const SegD *>(h->d_blob + o_segd);
