@@ -37,6 +37,7 @@ extern "C" {
 #define CARENV_ABI_VERSION 1
 #define CARENV_OBS_DIM 18      /* 6 + num_rays, lib/car_env.py:513-519 */
 #define CARENV_NUM_ACTIONS 9   /* spaces.Discrete(9), lib/car_env.py:525 */
+#define CARENV_TIME_LIMIT 1000 /* an episode is truncated at its 1000th step, lib/car_env.py:491 */
 #define CARENV_MAX_SEGMENTS 2048   /* up to 128: geometry as kernel constants (fast kernels); above: staged in shared memory */
 
 #define CARENV_E_INVAL (-1)    /* bad argument (null pointer, size, dtype) */
@@ -199,6 +200,15 @@ int carenv_stats(void *handle, unsigned long long out4_host[4], int reset_counte
 int gae_reverse_scan(const float *rew, const float *val, const float *term, const float *trunc,
                      const float *last_val, const float *last_term, const float *last_trunc, float *adv, float *ret,
                      int T, int N, double gamma, double gae_lambda, void *stream);
+
+/* gae_reverse_scan with time-limit bootstrapping (Pardo et al. 2018, "Time Limits in Reinforcement Learning"): a row t
+ * whose successor has trunc == 1 and term == 0 (for row T - 1: last_trunc / last_term) uses nv = boot[t][e] — the
+ * critic's value of the observation its episode ended in, before the autoreset (carenv_final_values) — instead of
+ * val[t + 1][e] / last_val[e].  boot [T][N] float32 is read nowhere else (other entries may hold anything, NaN
+ * included); every other operation is gae_reverse_scan's, so without truncation flags the results are the same bits. */
+int gae_reverse_scan_boot(const float *rew, const float *val, const float *term, const float *trunc,
+                          const float *last_val, const float *last_term, const float *last_trunc, const float *boot,
+                          float *adv, float *ret, int T, int N, double gamma, double gae_lambda, void *stream);
 
 /* Fused rollout (the loop of train.py:173-195 in one launch): for n_steps steps, per environment:
  * actor/critic forward (lib/model.py:10-40, float32), categorical sample by inverse CDF on a Philox4x32-10
@@ -417,6 +427,7 @@ int carenv_policy_rollout_tc_pop(void *handle, int n_members, const float *packe
                                  float *term_buf, float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg,
                                  void *stream);
 int carenv_ppo_epoch_pop_cluster_size(void);
+
 int carenv_ppo_epoch_pop_resident_clusters(int *n_clusters);
 int carenv_ppo_epoch_pop(int n_members, float *w1_actor, float *b1_actor, float *w2_actor, float *b2_actor,
                          float *w1_critic, float *b1_critic, float *w2_critic, float *b2_critic, const float *obs,
@@ -445,6 +456,70 @@ int carenv_tc_gemm_test(const float *A, const float *B, float *D, void *stream);
 /* Measurement helper (no reference counterpart): an FFMA-only kernel, blocks x 256 threads x
  * iters x 64 FFMA, used by bench.py to measure the FP32-pipe peak the step kernel is compared with. */
 int carenv_bench_ffma(int blocks, int iters, float *scratch, void *stream);
+
+
+/* Final observations of truncated episodes from the fused rollouts, for time-limit bootstrapping (gae_reverse_scan_boot).
+ * Every rollout entry point has a _final twin with the same arguments plus
+ *   final_obs [n_slots][N][18] float32, final_row [n_slots][N] int32 (device; N = the launch's columns: n_envs, or
+ *   n_members * n_envs_per_member for the _pop twins), n_slots >= ceil(n_steps / CARENV_TIME_LIMIT)
+ * An environment truncates at most ceil(n_steps / CARENV_TIME_LIMIT) times in n_steps steps whatever its starting
+ * time step.  Its k-th truncation in the call writes the observation the episode ended in (before the autoreset) to
+ * final_obs[k][e] and the row t of that step to final_row[k][e], rows in increasing order; the slots it does not use
+ * get final_row = -1 (their final_obs is not written).  All other outputs are bit-identical to the plain entry point.
+ * The twins return CARENV_E_INVAL for null slot pointers and for n_slots < ceil(n_steps / CARENV_TIME_LIMIT).
+ *   carenv_final_values   boot[final_row[k][c]][c] = critic(final_obs[k][c]) for every used slot with a row below
+ *       n_rows (float32 CUDA cores; other entries of boot [n_rows][N] are not written).  Critic tensors in nn.Linear
+ *       layout, stacked [n_members][...] as above; column c belongs to member c / n_envs_per_member, whose values do not
+ *       depend on the other members and equal the call with n_members = 1 on that member alone. */
+int carenv_policy_rollout_final(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                                unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                                int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                                float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                float *final_obs, int32_t *final_row, int n_slots);
+int carenv_policy_rollout_tc_final(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                                   unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                                   int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc,
+                                   double reward_scale, float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                   float *term_buf, float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg,
+                                   void *stream, float *final_obs, int32_t *final_row, int n_slots);
+int carenv_policy_rollout_warp_final(void *handle, const float *w1_actor, const float *b1_actor,
+                                     const float *w2_actor, const float *b2_actor, const float *w1_critic,
+                                     const float *b1_critic, const float *w2_critic, const float *b2_critic, int n_envs,
+                                     int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                                     double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                     float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                     float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                     float *logp_buf, float *last_val, float *u_dbg, void *stream, float *final_obs,
+                                     int32_t *final_row, int n_slots);
+int carenv_policy_rollout_tc_multi_final(void *multi, const int32_t *track_ids, const float *packed_weights,
+                                         int n_envs, int n_steps, int env_offset, unsigned long long seed,
+                                         unsigned long long step0, double *pos, double *vel, int32_t *ints,
+                                         float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                         float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                         float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
+                                         float *u_dbg, void *stream, float *final_obs, int32_t *final_row,
+                                         int n_slots);
+int carenv_policy_rollout_warp_pop_final(void *handle, int n_members, const float *w1_actor, const float *b1_actor,
+                                         const float *w2_actor, const float *b2_actor, const float *w1_critic,
+                                         const float *b1_critic, const float *w2_critic, const float *b2_critic,
+                                         int n_envs_per_member, int n_steps, const unsigned long long *seeds,
+                                         unsigned long long step0, double *pos, double *vel, int32_t *ints,
+                                         float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                         float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                         float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
+                                         float *u_dbg, void *stream, float *final_obs, int32_t *final_row,
+                                         int n_slots);
+int carenv_policy_rollout_tc_pop_final(void *handle, int n_members, const float *packed_weights,
+                                       int n_envs_per_member, int n_steps, const unsigned long long *seeds,
+                                       unsigned long long step0, double *pos, double *vel, int32_t *ints,
+                                       float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                       float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                       float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
+                                       float *u_dbg, void *stream, float *final_obs, int32_t *final_row, int n_slots);
+int carenv_final_values(int n_members, const float *w1_critic, const float *b1_critic, const float *w2_critic,
+                        const float *b2_critic, const float *final_obs, const int32_t *final_row, int n_slots,
+                        int n_envs_per_member, int n_rows, float *boot, void *stream);
 
 #ifdef __cplusplus
 }

@@ -130,6 +130,16 @@ def lib():
     L.carenv_ppo_epoch_pop_resident_clusters.argtypes = [vp]
     L.carenv_policy_eval_pop.argtypes = [vp, i32] + [vp] * 4 + [C.c_longlong, C.c_ulonglong, i32, vp, vp, i32, vp, vp,
                                                                vp]
+    # final-observation twins: the plain arguments plus final_obs, final_row, n_slots
+    L.gae_reverse_scan_boot.argtypes = [vp] * 10 + [i32, i32, f64, f64, vp]
+    for name in ("carenv_policy_rollout", "carenv_policy_rollout_tc", "carenv_policy_rollout_warp",
+                 "carenv_policy_rollout_tc_multi", "carenv_policy_rollout_warp_pop", "carenv_policy_rollout_tc_pop"):
+        getattr(L, name + "_final").argtypes = getattr(L, name).argtypes + [vp, vp, i32]
+    L.carenv_final_values.argtypes = [i32] + [vp] * 6 + [i32, i32, i32, vp, vp]
+    for name in ("carenv_policy_rollout_final", "carenv_policy_rollout_tc_final", "carenv_policy_rollout_warp_final",
+                 "carenv_policy_rollout_tc_multi_final", "carenv_policy_rollout_warp_pop_final",
+                 "carenv_policy_rollout_tc_pop_final", "carenv_final_values", "gae_reverse_scan_boot"):
+        getattr(L, name).restype = i32
     for name in ("carenv_pack_policy_pop", "carenv_policy_rollout_warp_pop", "carenv_policy_rollout_tc_pop",
                  "carenv_ppo_epoch_pop", "carenv_ppo_epoch_pop_kl", "carenv_ppo_epoch_pop_cluster_size", "carenv_ppo_epoch_pop_resident_clusters",
                  "carenv_policy_eval_pop"):

@@ -698,10 +698,12 @@ CE_HD void pose_observation(const EnvState &s, float vx10, float vy10, const flo
 // ---- one CarEnv.step with same-step autoreset --------------------------------------------------
 // `final_obs` (optional, 18 floats): receives the observation of the state the step ended in BEFORE the autoreset —
 // gymnasium's info["final_observation"]; it equals o.obs wherever the episode did not end.
+// `trunc_obs` (optional, 18 floats): receives that observation only in a step that truncates the episode — written
+// inside the autoreset branch, so the fused rollouts carry one pointer instead of 18 more live floats.
 template <int U, bool TAB = false, int NS = 0, bool CULL = false>
 CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackParams &P, const Tables &T,
                     StepResult &o, unsigned long long *stats, const WarpSeg *ws = nullptr, const TabView *tv = nullptr,
-                    float *final_obs = nullptr) {
+                    float *final_obs = nullptr, float *trunc_obs = nullptr) {
     int thrust, turn;
     decode_action(action, thrust, turn);
     double reward = thrust > 0 ? 0.01 : 0.0;
@@ -744,6 +746,10 @@ CE_HD void env_step(EnvState &s, int action, double reward_scale, const TrackPar
 #endif
     {
         if (done) {
+            if (trunc_obs && o.truncated) {
+#pragma unroll
+                for (int i = 0; i < kObsDim; ++i) trunc_obs[i] = o.obs[i];
+            }
             s.px = P.start_x; s.py = P.start_y; s.vx = 0.0; s.vy = 0.0;
             s.k = 0; s.t = 0; s.next_gate = 0; s.passed = 0;
 #pragma unroll

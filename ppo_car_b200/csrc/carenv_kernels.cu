@@ -575,17 +575,21 @@ __device__ __forceinline__ void gae_load(GaeBatch<kGaeUnroll> &b, const float *_
 
 // kGaeUnroll = 8 (80 registers) is best up to ~65 k columns, 16 (164 registers, more loads in flight per
 // thread) beyond: 5.92 vs 4.69 TB/s at [1024, 65536], 5.30 vs 5.45 at [1024, 131072], 5.81 vs 5.94 at [128, 1 M].
-template <int kGaeUnroll>
+// BOOT (gae_reverse_scan_boot): time-limit bootstrapping.  A row whose successor has trunc == 1 and term == 0 (for row
+// T - 1: last_trunc / last_term) takes nv = boot[t] — the critic's value of the observation its episode ended in —
+// instead of val[t + 1] / last_val; boot is read nowhere else.  Every other operation is k_gae's.
+template <int kGaeUnroll, bool BOOT = false>
 __global__ void __launch_bounds__(128)
 k_gae(const float *__restrict__ rew, const float *__restrict__ val, const float *__restrict__ term,
       const float *__restrict__ trunc, const float *__restrict__ last_val, const float *__restrict__ last_term,
       const float *__restrict__ last_trunc, float *__restrict__ adv, float *__restrict__ ret, int T, int N, float g,
-      float gl) {
+      float gl, const float *__restrict__ boot) {
   // grid-stride over the columns: the launch sizes the grid to ONE balanced wave of resident threads
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < N; e += gridDim.x * blockDim.x) {
     float nv = last_val[e];
     float tm = __fadd_rn(1.0f, -last_term[e]);
     float um = __fadd_rn(1.0f, -last_trunc[e]);
+    bool cut = BOOT && last_trunc[e] == 1.0f && last_term[e] == 0.0f;   // the successor ended by truncation
     float a = 0.0f;
     int t = T - 1;
     GaeBatch<kGaeUnroll> cur, nxt;
@@ -596,6 +600,7 @@ k_gae(const float *__restrict__ rew, const float *__restrict__ val, const float 
 #pragma unroll
         for (int i = 0; i < kGaeUnroll; ++i) {
             const size_t k = (size_t)(t - i) * (size_t)N + (size_t)e;
+            if (BOOT && cut) nv = __ldcs(boot + k);
             const float delta = __fadd_rn(__fadd_rn(cur.r[i], __fmul_rn(__fmul_rn(g, nv), tm)), -cur.v[i]);
             a = __fadd_rn(delta, __fmul_rn(__fmul_rn(__fmul_rn(gl, tm), um), a));
             __stcs(adv + k, a);
@@ -603,19 +608,28 @@ k_gae(const float *__restrict__ rew, const float *__restrict__ val, const float 
             nv = cur.v[i];
             tm = __fadd_rn(1.0f, -cur.te[i]);
             um = __fadd_rn(1.0f, -cur.tr[i]);
+            if (BOOT) cut = cur.tr[i] == 1.0f && cur.te[i] == 0.0f;
         }
         if (more) cur = nxt;
     }
     for (; t >= 0; --t) {
         const size_t k = (size_t)t * (size_t)N + (size_t)e;
         const float r = __ldcs(rew + k), v = __ldcs(val + k);
+        if (BOOT && cut) nv = __ldcs(boot + k);
         const float delta = __fadd_rn(__fadd_rn(r, __fmul_rn(__fmul_rn(g, nv), tm)), -v);
         a = __fadd_rn(delta, __fmul_rn(__fmul_rn(__fmul_rn(gl, tm), um), a));
         __stcs(adv + k, a);
         __stcs(ret + k, __fadd_rn(a, v));
         nv = v;
-        tm = __fadd_rn(1.0f, -__ldcs(term + k));
-        um = __fadd_rn(1.0f, -__ldcs(trunc + k));
+        if (BOOT) {
+            const float te = __ldcs(term + k), tr = __ldcs(trunc + k);
+            tm = __fadd_rn(1.0f, -te);
+            um = __fadd_rn(1.0f, -tr);
+            cut = tr == 1.0f && te == 0.0f;
+        } else {
+            tm = __fadd_rn(1.0f, -__ldcs(term + k));
+            um = __fadd_rn(1.0f, -__ldcs(trunc + k));
+        }
     }
   }
 }
@@ -1419,9 +1433,10 @@ int carenv_stats(void *handle, unsigned long long out[4], int reset_counters) {
     return 0;
 }
 
-int gae_reverse_scan(const float *rew, const float *val, const float *term, const float *trunc,
-                     const float *last_val, const float *last_term, const float *last_trunc, float *adv, float *ret,
-                     int T, int N, double gamma, double gae_lambda, void *stream) {
+// gae_reverse_scan (boot == nullptr: k_gae<U>) and gae_reverse_scan_boot (k_gae<U, true>): the same launch choice
+static int gae_launch(const float *rew, const float *val, const float *term, const float *trunc, const float *last_val,
+                      const float *last_term, const float *last_trunc, const float *boot, float *adv, float *ret, int T,
+                      int N, double gamma, double gae_lambda, void *stream) {
     if (T < 0 || N < 0) return fail(CARENV_E_INVAL, "negative T / N");
     if (T == 0 || N == 0) return 0;
     if (!rew || !val || !term || !trunc || !last_val || !last_term || !last_trunc || !adv || !ret)
@@ -1447,14 +1462,26 @@ int gae_reverse_scan(const float *rew, const float *val, const float *term, cons
         threads = (N + k - 1) / k;
     }
     const int grid = (threads + block - 1) / block;
-    if (wide)
-        k_gae<16><<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(rew, val, term, trunc, last_val, last_term,
-                                                                       last_trunc, adv, ret, T, N, g, gl);
-    else
-        k_gae<8><<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(rew, val, term, trunc, last_val, last_term,
-                                                                      last_trunc, adv, ret, T, N, g, gl);
+    auto kern = wide ? (boot ? k_gae<16, true> : k_gae<16>) : (boot ? k_gae<8, true> : k_gae<8>);
+    kern<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(rew, val, term, trunc, last_val, last_term, last_trunc,
+                                                               adv, ret, T, N, g, gl, boot);
     CU(cudaGetLastError());
     return 0;
+}
+
+int gae_reverse_scan(const float *rew, const float *val, const float *term, const float *trunc,
+                     const float *last_val, const float *last_term, const float *last_trunc, float *adv, float *ret,
+                     int T, int N, double gamma, double gae_lambda, void *stream) {
+    return gae_launch(rew, val, term, trunc, last_val, last_term, last_trunc, nullptr, adv, ret, T, N, gamma,
+                      gae_lambda, stream);
+}
+
+int gae_reverse_scan_boot(const float *rew, const float *val, const float *term, const float *trunc,
+                          const float *last_val, const float *last_term, const float *last_trunc, const float *boot,
+                          float *adv, float *ret, int T, int N, double gamma, double gae_lambda, void *stream) {
+    if (!boot && T > 0 && N > 0) return fail(CARENV_E_INVAL, "null pointer");
+    return gae_launch(rew, val, term, trunc, last_val, last_term, last_trunc, boot, adv, ret, T, N, gamma, gae_lambda,
+                      stream);
 }
 
 /* Measurement helper: launches blocks x 256 threads, each doing iters * 64 FFMA (2 flop each). */

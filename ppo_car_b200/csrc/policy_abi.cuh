@@ -232,11 +232,27 @@ int carenv_ppo_epoch_kl(float *w1a, float *b1a, float *w2a, float *b2a, float *w
 
 int carenv_policy_weights_floats(void) { return kPolicyFloats; }
 
-int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
-                          unsigned long long seed, unsigned long long step0, double *pos, double *vel, int32_t *ints,
-                          float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
-                          float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
-                          float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+// Final-observation slots of the carenv_policy_rollout*_final twins (FINAL instantiations); obs == nullptr: the plain
+// entry points, which launch the kernels they always launched.
+static_assert(kTimeLimit == CARENV_TIME_LIMIT, "time limit");
+struct SlotArgs {
+    float *obs = nullptr;
+    int32_t *row = nullptr;
+    int n = 0;
+};
+static int slot_args_ok(const SlotArgs &f, int n_steps) {
+    if (!f.obs || !f.row) return fail(CARENV_E_INVAL, "null pointer");
+    const long long need = n_steps > 0 ? ((long long)n_steps + CARENV_TIME_LIMIT - 1) / CARENV_TIME_LIMIT : 0;
+    if (f.n < need) return fail(CARENV_E_INVAL, "n_slots must be at least ceil(n_steps / CARENV_TIME_LIMIT)");
+    return 0;
+}
+
+static int policy_rollout_impl(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                               unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                               int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                               float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                               float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                               const SlotArgs &fs) {
     Handle *h = static_cast<Handle *>(handle);
     if (!h) return fail(CARENV_E_INVAL, "null handle");
     if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
@@ -260,13 +276,41 @@ int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs,
             h->host.P, h->dev, packed_weights, n_envs, n_steps, env_offset, seed, step0,
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
             cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull);
+            last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, fs.obs, fs.row, fs.n);
         CU(cudaGetLastError());
         return 0;
     };
+    if (fs.obs) {
+        if (U == 4) return launch(k_policy_rollout<4, true>);
+        if (U == 2) return launch(k_policy_rollout<2, true>);
+        return launch(k_policy_rollout<1, true>);
+    }
     if (U == 4) return launch(k_policy_rollout<4>);
     if (U == 2) return launch(k_policy_rollout<2>);
     return launch(k_policy_rollout<1>);
+}
+
+int carenv_policy_rollout(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                          unsigned long long seed, unsigned long long step0, double *pos, double *vel, int32_t *ints,
+                          float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                          float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                          float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    return policy_rollout_impl(handle, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos, vel, ints, cur_obs,
+                               cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf,
+                               trunc_buf, logp_buf, last_val, u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_final(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                                unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                                int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                                float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                float *final_obs, int32_t *final_row, int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_impl(handle, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos, vel, ints, cur_obs,
+                               cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf,
+                               trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
 }
 
 /* Small batches: one warp per environment, network parameters in nn.Linear layout (k_policy_rollout_warp). */
@@ -277,7 +321,8 @@ static int policy_rollout_warp_launch(Handle *h, const ppo::Params &W, int n_mem
                                       unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
                                       float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
                                       float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
-                                      float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+                                      float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                      const SlotArgs &fs) {
     if (h->host.P.n_seg > 32)
         return fail(CARENV_E_TRACK, "the warp-per-environment rollout kernel supports tracks with at most 32 wall segments");
     DeviceGuard guard(h->device);
@@ -285,25 +330,26 @@ static int policy_rollout_warp_launch(Handle *h, const ppo::Params &W, int n_mem
     const int table_bytes = (int)((h->smem_bytes + 15) / 16 * 16);
     const size_t smem = (size_t)table_bytes + sizeof(float) * kWpFloats;
     if (smem > 227 * 1024) return fail(CARENV_E_TRACK, "track tables too large for the warp-per-environment rollout kernel");
-    auto kern = n_members > 0 ? k_policy_rollout_warp<true> : k_policy_rollout_warp<false>;
+    auto kern = fs.obs ? (n_members > 0 ? k_policy_rollout_warp<true, true> : k_policy_rollout_warp<false, true>)
+                       : (n_members > 0 ? k_policy_rollout_warp<true> : k_policy_rollout_warp<false>);
     CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const dim3 grid((n_envs + 3) / 4, n_members > 0 ? n_members : 1);
     kern<<<grid, 128, smem, static_cast<cudaStream_t>(stream)>>>(
         h->host.P, h->dev, W, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
         reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale, obs_buf,
         act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, h->d_stats, table_bytes,
-        h->pose_rows ? kObsPose : kObsFull, seeds, n_members * n_envs);
+        h->pose_rows ? kObsPose : kObsFull, seeds, n_members * n_envs, fs.obs, fs.row, fs.n);
     CU(cudaGetLastError());
     return 0;
 }
 
-int carenv_policy_rollout_warp(void *handle, const float *w1a, const float *b1a, const float *w2a, const float *b2a,
-                               const float *w1c, const float *b1c, const float *w2c, const float *b2c, int n_envs,
-                               int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
-                               double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
-                               float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf, float *rew_buf,
-                               float *val_buf, float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
-                               float *u_dbg, void *stream) {
+static int policy_rollout_warp_impl(void *handle, const float *w1a, const float *b1a, const float *w2a,
+                                    const float *b2a, const float *w1c, const float *b1c, const float *w2c,
+                                    const float *b2c, int n_envs, int n_steps, int env_offset, unsigned long long seed,
+                                    unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                    float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                    float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                    float *logp_buf, float *last_val, float *u_dbg, void *stream, const SlotArgs &fs) {
     Handle *h = static_cast<Handle *>(handle);
     if (!h) return fail(CARENV_E_INVAL, "null handle");
     if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
@@ -314,7 +360,34 @@ int carenv_policy_rollout_warp(void *handle, const float *w1a, const float *b1a,
     return policy_rollout_warp_launch(h, ppo::Params{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c}, 0, n_envs, n_steps,
                                       env_offset, seed, nullptr, step0, pos, vel, ints, cur_obs, cur_term, cur_trunc,
                                       reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-                                      last_val, u_dbg, stream);
+                                      last_val, u_dbg, stream, fs);
+}
+
+int carenv_policy_rollout_warp(void *handle, const float *w1a, const float *b1a, const float *w2a, const float *b2a,
+                               const float *w1c, const float *b1c, const float *w2c, const float *b2c, int n_envs,
+                               int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                               double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                               float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf, float *rew_buf,
+                               float *val_buf, float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
+                               float *u_dbg, void *stream) {
+    return policy_rollout_warp_impl(handle, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, n_envs, n_steps, env_offset, seed,
+                                    step0, pos, vel, ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf,
+                                    rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_warp_final(void *handle, const float *w1a, const float *b1a, const float *w2a,
+                                     const float *b2a, const float *w1c, const float *b1c, const float *w2c,
+                                     const float *b2c, int n_envs, int n_steps, int env_offset, unsigned long long seed,
+                                     unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                     float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                     float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                     float *logp_buf, float *last_val, float *u_dbg, void *stream, float *final_obs,
+                                     int32_t *final_row, int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_warp_impl(handle, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, n_envs, n_steps, env_offset, seed,
+                                    step0, pos, vel, ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf,
+                                    rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
 }
 
 /* Test hook: D[128,256] = A[128,24] * B[256,24]^T on the tensor cores (tcgen05, kind::tf32). */
@@ -336,7 +409,7 @@ static int policy_rollout_tc_launch(Handle *h, const float *packed_weights, int 
                                     unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
                                     float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
                                     float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
-                                    float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+                                    float *logp_buf, float *last_val, float *u_dbg, void *stream, const SlotArgs &fs) {
     if (h->host.P.n_seg > kMaxSeg)
         return fail(CARENV_E_TRACK, "the fused rollout kernels support tracks with at most 128 wall segments");
     if (h->tc_tiles >= 2 && h->tc_tiles <= 4)
@@ -365,10 +438,20 @@ static int policy_rollout_tc_launch(Handle *h, const float *packed_weights, int 
             reinterpret_cast<double2 *>(pos), reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs,
             cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
             last_val, u_dbg, h->d_stats, table_bytes, h->pose_rows ? kObsPose : kObsFull, h->d_den4, n_pairs, row_f4,
-            nullptr, nullptr, 0, nullptr, seeds, n_members * n_envs);
+            nullptr, nullptr, 0, nullptr, seeds, n_members * n_envs, fs.obs, fs.row, fs.n);
         CU(cudaGetLastError());
         return 0;
     };
+    if (fs.obs && n_members > 0) {
+        if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true, true, true>) : launch(k_policy_rollout_tc3<4, false, true, true>);
+        if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true, true, true>) : launch(k_policy_rollout_tc3<2, false, true, true>);
+        return launch(k_policy_rollout_tc3<1, false, true, true>);
+    }
+    if (fs.obs) {
+        if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true, false, true>) : launch(k_policy_rollout_tc3<4, false, false, true>);
+        if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true, false, true>) : launch(k_policy_rollout_tc3<2, false, false, true>);
+        return launch(k_policy_rollout_tc3<1, false, false, true>);
+    }
     if (n_members > 0) {
         if (U == 4) return tab ? launch(k_policy_rollout_tc3<4, true, true>) : launch(k_policy_rollout_tc3<4, false, true>);
         if (U == 2) return tab ? launch(k_policy_rollout_tc3<2, true, true>) : launch(k_policy_rollout_tc3<2, false, true>);
@@ -381,11 +464,12 @@ static int policy_rollout_tc_launch(Handle *h, const float *packed_weights, int 
 
 /* Tensor-core variant of carenv_policy_rollout (same arguments; packed_weights in the layout of
  * ppo_car_b200/policy.py: pack_policy_weights_tc): k_policy_rollout_tc3. */
-int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
-                             unsigned long long seed, unsigned long long step0, double *pos, double *vel,
-                             int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
-                             float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
-                             float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+static int policy_rollout_tc_impl(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                                  unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                                  int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc,
+                                  double reward_scale, float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                  float *term_buf, float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg,
+                                  void *stream, const SlotArgs &fs) {
     Handle *h = static_cast<Handle *>(handle);
     if (!h) return fail(CARENV_E_INVAL, "null handle");
     if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
@@ -395,7 +479,30 @@ int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_en
         return fail(CARENV_E_INVAL, "null pointer");
     return policy_rollout_tc_launch(h, packed_weights, 0, n_envs, n_steps, env_offset, seed, nullptr, step0, pos, vel,
                                     ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
-                                    term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream);
+                                    term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
+}
+
+int carenv_policy_rollout_tc(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                             unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                             int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                             float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                             float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    return policy_rollout_tc_impl(handle, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos, vel, ints,
+                                  cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
+                                  term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_tc_final(void *handle, const float *packed_weights, int n_envs, int n_steps, int env_offset,
+                                   unsigned long long seed, unsigned long long step0, double *pos, double *vel,
+                                   int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc,
+                                   double reward_scale, float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                   float *term_buf, float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg,
+                                   void *stream, float *final_obs, int32_t *final_row, int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_tc_impl(handle, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos, vel, ints,
+                                  cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
+                                  term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
 }
 
 /* Largest wall-segment count over the tracks of a multi-track handle: the handle keeps its TrackParams on the device
@@ -412,12 +519,13 @@ static int multi_max_seg(const MultiTrack *m, cudaStream_t stream, int *max_seg)
 
 /* carenv_policy_rollout_tc on several tracks (k_policy_rollout_tc3<0, false>): environment e runs on track
  * track_ids[e] of the multi-track handle (clamped to 0..n_tracks - 1 as carenv_multi_rollout does). */
-int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const float *packed_weights, int n_envs,
-                                   int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
-                                   double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
-                                   float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
-                                   float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
-                                   float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+static int policy_rollout_tc_multi_impl(void *multi, const int32_t *track_ids, const float *packed_weights, int n_envs,
+                                        int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                                        double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                        float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                        float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                        float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                        const SlotArgs &fs) {
     MultiTrack *m = static_cast<MultiTrack *>(multi);
     if (!m) return fail(CARENV_E_INVAL, "null handle");
     if (n_envs < 0 || n_steps < 0) return fail(CARENV_E_INVAL, "negative n_envs / n_steps");
@@ -436,13 +544,55 @@ int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const 
     const size_t smem = 128 + (size_t)((kTcWeightFloats * 4 + 127) / 128 * 128) + (size_t)2 * 2 * tc::kABytes +
                         (size_t)2 * 128 * 12 * sizeof(float);
     static const TrackParams kNoTrack{};                     // P and G of the single-track instantiations: unused
-    auto kern = k_policy_rollout_tc3<0, false>;
+    auto kern = fs.obs ? k_policy_rollout_tc3<0, false, false, true> : k_policy_rollout_tc3<0, false>;
     CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<(n_envs + 255) / 256, 256 + 128 + 32, smem, st>>>(
         kNoTrack, Tables{}, packed_weights, n_envs, n_steps, env_offset, seed, step0, reinterpret_cast<double2 *>(pos),
         reinterpret_cast<double2 *>(vel), reinterpret_cast<int4 *>(ints), cur_obs, cur_term, cur_trunc, reward_scale,
         obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, m->d_stats, 0, kObsFull,
-        nullptr, 0, 0, m->d_params, m->d_tables, m->n_tracks, track_ids, nullptr, 0);
+        nullptr, 0, 0, m->d_params, m->d_tables, m->n_tracks, track_ids, nullptr, 0, fs.obs, fs.row, fs.n);
+    CU(cudaGetLastError());
+    return 0;
+}
+
+int carenv_policy_rollout_tc_multi(void *multi, const int32_t *track_ids, const float *packed_weights, int n_envs,
+                                   int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
+                                   double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                   float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                   float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                   float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    return policy_rollout_tc_multi_impl(multi, track_ids, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos,
+                                        vel, ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf,
+                                        val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_tc_multi_final(void *multi, const int32_t *track_ids, const float *packed_weights,
+                                         int n_envs, int n_steps, int env_offset, unsigned long long seed,
+                                         unsigned long long step0, double *pos, double *vel, int32_t *ints,
+                                         float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                         float *obs_buf, float *act_buf, float *rew_buf, float *val_buf,
+                                         float *term_buf, float *trunc_buf, float *logp_buf, float *last_val,
+                                         float *u_dbg, void *stream, float *final_obs, int32_t *final_row,
+                                         int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_tc_multi_impl(multi, track_ids, packed_weights, n_envs, n_steps, env_offset, seed, step0, pos,
+                                        vel, ints, cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf,
+                                        val_buf, term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
+}
+
+/* Critic values of the final-observation slots (k_final_values): one thread per slot and column. */
+int carenv_final_values(int n_members, const float *w1c, const float *b1c, const float *w2c, const float *b2c,
+                        const float *final_obs, const int32_t *final_row, int n_slots, int n_envs, int n_rows,
+                        float *boot, void *stream) {
+    if (n_members < 1 || n_envs < 1 || n_slots < 0 || n_rows < 0 || (long long)n_members * n_envs > 0x7fffffffll)
+        return fail(CARENV_E_INVAL, "n_members and n_envs must be positive, n_slots and n_rows non-negative");
+    if (!w1c || !b1c || !w2c || !b2c || !final_obs || !final_row || !boot) return fail(CARENV_E_INVAL, "null pointer");
+    const long long total = (long long)n_slots * n_members * n_envs;
+    if (total == 0) return 0;
+    const ppo::Params W{nullptr, nullptr, nullptr, nullptr, w1c, b1c, w2c, b2c};
+    k_final_values<<<(unsigned)((total + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+        W, final_obs, final_row, n_slots, n_members * n_envs, n_envs, n_rows, boot);
     CU(cudaGetLastError());
     return 0;
 }

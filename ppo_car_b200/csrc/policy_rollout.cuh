@@ -56,7 +56,40 @@ __global__ void __launch_bounds__(128) k_tc_gemm_test(const float *__restrict__ 
 #define CARENV_POLICY_MIN_BLOCKS 3
 #endif
 constexpr int kPolicyBlock = CARENV_POLICY_BLOCK;
-template <int U>
+
+// ---- final-observation slots (FINAL instantiations, C ABI carenv_policy_rollout*_final) ---------------------------
+// An environment truncates at most S = ceil(n_steps / kTimeLimit) times in a launch, whatever its starting time step.
+// Its k-th truncation writes the observation the episode ended in (before the autoreset) to final_obs[k][e] and the
+// row t of that step to final_row[k][e] ([S][stride](,18) arrays); when the rollout ends, the slots it did not use get
+// row -1.  The writes sit in the autoreset branch of env_step (about once per 1000 env-steps); the step loop carries
+// the two slot pointers and a count.  obs == nullptr: this thread writes nothing (idle or non-leader threads).
+struct FinalSlots {
+    float *obs;
+    int *row;
+    int used;
+};
+__device__ __forceinline__ FinalSlots final_slots_begin(bool writer, float *final_obs, int *final_row, int n_slots,
+                                                        int e) {
+    return FinalSlots{writer && n_slots > 0 ? final_obs + (size_t)e * kObsDim : nullptr,
+                      writer ? final_row + e : nullptr, 0};
+}
+// after the step of row t: a truncation takes the slot just written and moves to the next one
+__device__ __forceinline__ void final_slots_step(FinalSlots &f, int truncated, int t, int n_slots, int stride) {
+    if (truncated) {
+        if (f.obs) {
+            *f.row = t;
+            f.row += stride;
+            f.obs += (size_t)stride * kObsDim;
+        }
+        if (++f.used >= n_slots) f.obs = nullptr;            // n_slots >= S (checked by the launchers): never taken
+    }
+}
+__device__ __forceinline__ void final_slots_end(FinalSlots &f, int n_slots, int stride) {
+    if (f.row)
+        for (int k = f.used; k < n_slots; ++k, f.row += stride) *f.row = -1;
+}
+
+template <int U, bool FINAL = false>
 __global__ void __launch_bounds__(kPolicyBlock, CARENV_POLICY_MIN_BLOCKS)
 k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const float *__restrict__ weights,
                  int n_envs, int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
@@ -65,7 +98,8 @@ k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const fl
                  double reward_scale, float *__restrict__ obs_buf, float *__restrict__ act_buf,
                  float *__restrict__ rew_buf, float *__restrict__ val_buf, float *__restrict__ term_buf,
                  float *__restrict__ trunc_buf, float *__restrict__ logp_buf, float *__restrict__ last_val,
-                 float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode) {
+                 float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode,
+                 float *__restrict__ final_obs, int *__restrict__ final_row, int n_slots) {
     extern __shared__ __align__(16) unsigned char smem[];
     float *sw = reinterpret_cast<float *>(smem + table_bytes);
     for (int i = threadIdx.x; i < kPolicyFloats / 4; i += blockDim.x)
@@ -89,6 +123,8 @@ k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const fl
     }
     float tc = cur_term[e], uc = cur_trunc[e];
     const uint32_t gid = (uint32_t)(env_offset + e);
+    FinalSlots fs{};
+    if constexpr (FINAL) fs = final_slots_begin(true, final_obs, final_row, n_slots, e);
     PolicyOut po;
     for (int t = 0; t < n_steps; ++t) {
         const size_t idx = (size_t)t * (size_t)n_envs + (size_t)e;
@@ -113,7 +149,12 @@ k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const fl
         trunc_buf[idx] = uc;
         if (u_dbg) u_dbg[idx] = u;
         StepResult o;
-        env_step<U>(s, a, reward_scale, P, T, o, stats);
+        if constexpr (FINAL) {
+            env_step<U>(s, a, reward_scale, P, T, o, stats, nullptr, nullptr, nullptr, fs.obs);
+            final_slots_step(fs, o.truncated, t, n_slots, n_envs);
+        } else {
+            env_step<U>(s, a, reward_scale, P, T, o, stats);
+        }
         rew_buf[idx] = o.reward;
 #pragma unroll
         for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];
@@ -130,6 +171,7 @@ k_policy_rollout(const __grid_constant__ TrackParams P, const Tables G, const fl
     }
     cur_term[e] = tc;
     cur_trunc[e] = uc;
+    if constexpr (FINAL) final_slots_end(fs, n_slots, n_envs);
     if (last_val) {                                          // bootstrap value of the state after the rollout
         policy_forward(obs, sw, po);
         last_val[e] = po.value;
@@ -155,8 +197,42 @@ __device__ __forceinline__ ppo::Params member_params(const ppo::Params &W, int p
                        W.w2c + q * kHidden,           W.b2c + q};
 }
 
+// Critic pass over the final-observation slots (carenv_final_values): thread i = slot k * N + column c; a used slot
+// (0 <= final_row[k][c] < n_rows) gets boot[final_row[k][c]][c] = critic(final_obs[k][c]), float32 CUDA cores.  Column c
+// belongs to member c / n_per_member of stacked nn.Linear critic tensors (one policy: n_per_member = N), and each
+// thread reads only its member's parameters, so a member's values do not depend on the others.
+__global__ void __launch_bounds__(128)
+k_final_values(const ppo::Params W, const float *__restrict__ final_obs, const int *__restrict__ final_row, int n_slots,
+               int N, int n_per_member, int n_rows, float *__restrict__ boot) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)n_slots * N) return;
+    const int row = final_row[i];
+    if (row < 0 || row >= n_rows) return;
+    const int c = (int)(i % N);
+    const ppo::Params m = member_params(W, c / n_per_member);
+    float x[kObsDim];
+    {
+        const float2 *src = reinterpret_cast<const float2 *>(final_obs + (size_t)i * kObsDim);
+#pragma unroll
+        for (int k = 0; k < kObsDim / 2; ++k) { const float2 v = src[k]; x[2 * k] = v.x; x[2 * k + 1] = v.y; }
+    }
+    float v0 = 0.0f, v1 = 0.0f;
+#pragma unroll 2
+    for (int j = 0; j < kHidden; ++j) {
+        const float *w = m.w1c + j * kObsDim;
+        float h = __ldg(m.b1c + j);
+#pragma unroll
+        for (int k = 0; k < kObsDim; ++k) h = fmaf(__ldg(w + k), x[k], h);
+        if (j & 1) v1 = fmaf(__ldg(m.w2c + j), fmaxf(h, 0.0f), v1);
+        else v0 = fmaf(__ldg(m.w2c + j), fmaxf(h, 0.0f), v0);
+    }
+    boot[(size_t)row * N + c] = (v0 + v1) + __ldg(m.b2c);
+}
+
 // Moves every per-environment pointer to column col0 (the member's first environment): afterwards the kernel indexes
-// them with the member-local env e and, for the [T, N] rows, with the population's row stride N.
+// them with the member-local env e and, for the [T, N] rows, with the population's row stride N.  FINAL: the
+// final-observation slots [S][N](,18) as well.
+template <bool FINAL>
 __device__ __forceinline__ void pop_shift_columns(int col0, double2 *__restrict__ &pos, double2 *__restrict__ &vel,
                                                   int4 *__restrict__ &ints, float *__restrict__ &cur_obs,
                                                   float *__restrict__ &cur_term, float *__restrict__ &cur_trunc,
@@ -164,7 +240,8 @@ __device__ __forceinline__ void pop_shift_columns(int col0, double2 *__restrict_
                                                   float *__restrict__ &act_buf, float *__restrict__ &rew_buf,
                                                   float *__restrict__ &val_buf, float *__restrict__ &term_buf,
                                                   float *__restrict__ &trunc_buf, float *__restrict__ &logp_buf,
-                                                  float *__restrict__ &u_dbg) {
+                                                  float *__restrict__ &u_dbg, float *__restrict__ &final_obs,
+                                                  int *__restrict__ &final_row) {
     const size_t c = (size_t)col0;
     pos += c; vel += c; ints += c;
     cur_obs += c * kObsDim; cur_term += c; cur_trunc += c;
@@ -172,6 +249,10 @@ __device__ __forceinline__ void pop_shift_columns(int col0, double2 *__restrict_
     obs_buf += c * kObsDim;                                  // full observation rows only (the launchers refuse poses)
     act_buf += c; rew_buf += c; val_buf += c; term_buf += c; trunc_buf += c; logp_buf += c;
     if (u_dbg) u_dbg += c;
+    if constexpr (FINAL) {
+        final_obs += c * kObsDim;
+        final_row += c;
+    }
 }
 
 // Packing of the reference network's parameters (nn.Linear layout: weight [out][in], lib/model.py:10-26) into the
@@ -296,7 +377,8 @@ __device__ __forceinline__ void second_layer_chunk16_x2(uint32_t a, const float 
 // POP (carenv_policy_rollout_tc_pop, single-track U only): blockIdx.y = member p, as in k_policy_rollout_warp<true>:
 // packed weights [P][kTcWeightFloats], seeds[p], n_envs environments per member at columns p * n_envs + e of arrays
 // with row_stride columns.
-template <int U, bool TAB, bool POP = false>
+// FINAL: final-observation slots (final_slots_begin above); only active threads write.
+template <int U, bool TAB, bool POP = false, bool FINAL = false>
 __global__ void __launch_bounds__(256 + 128 + 32, 1)
 k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, const float *__restrict__ weights,
                      int n_envs, int n_steps, int env_offset, unsigned long long seed, unsigned long long step0,
@@ -308,7 +390,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
                      float *__restrict__ u_dbg, unsigned long long *stats, int table_bytes, int obs_mode,
                      const float4 *__restrict__ den4, int n_pairs, int row_f4, const TrackParams *__restrict__ mt_params,
                      const Tables *__restrict__ mt_tables, int n_tracks, const int *__restrict__ track_ids,
-                     const unsigned long long *__restrict__ seeds, int row_stride) {
+                     const unsigned long long *__restrict__ seeds, int row_stride, float *__restrict__ final_obs,
+                     int *__restrict__ final_row, int n_slots) {
     static_assert(!POP || U != 0, "populations run on one track");
     constexpr int kGroups = 2, kCols = 256, kHalf = 128, kEnvThreads = kGroups * 128, kCriticThreads = 128;
     extern __shared__ __align__(16) unsigned char smem[];
@@ -318,8 +401,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
         weights += (size_t)p * kTcWeightFloats;
         seed = seeds[p];
         stride = row_stride;
-        pop_shift_columns(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
-                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg);
+        pop_shift_columns<FINAL>(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
+                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg, final_obs, final_row);
     }
     // [tables | pad to a 128-byte boundary | weights | A tiles (hi, lo per group) | exchanged partial logits [group][128][12]
     //  | TAB: the denominator table of k_rollout_tab, ONE copy whose rows are skewed by 16 bytes (row_f4 is odd in
@@ -469,6 +552,8 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
         }
         float tc_ = cur_term[e], uc = cur_trunc[e];
         const uint32_t gid = (uint32_t)(env_offset + e);
+        FinalSlots fs{};
+        if constexpr (FINAL) fs = final_slots_begin(active, final_obs, final_row, n_slots, e);
 
         auto write_row = [&](int f) {
             if (f > 0) tc::mbar_wait(b_full_c, (uint32_t)((f - 1) & 1));   // the previous pass's MMAs have read the tile
@@ -555,7 +640,13 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
                 logp_buf[idx] = logp;
             }
             StepResult o;
-            env_step<U, TAB>(s, a, reward_scale, PE, TE, o, active ? stats : nullptr, nullptr, TAB ? &tv : nullptr);
+            if constexpr (FINAL) {
+                env_step<U, TAB>(s, a, reward_scale, PE, TE, o, active ? stats : nullptr, nullptr, TAB ? &tv : nullptr,
+                                 nullptr, fs.obs);
+                final_slots_step(fs, o.truncated, t, n_slots, stride);
+            } else {
+                env_step<U, TAB>(s, a, reward_scale, PE, TE, o, active ? stats : nullptr, nullptr, TAB ? &tv : nullptr);
+            }
             if (active) rew_buf[idx] = o.reward;
 #pragma unroll
             for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];
@@ -578,6 +669,7 @@ k_policy_rollout_tc3(const __grid_constant__ TrackParams P, const Tables G, cons
             cur_term[e] = tc_;
             cur_trunc[e] = uc;
         }
+        if constexpr (FINAL) final_slots_end(fs, n_slots, stride);
     }
     tc::tc_fence_before();
     __syncthreads();
@@ -603,7 +695,8 @@ constexpr int kWpFloats = 2 * kHidden * kWpRow + kHidden * kWpW2 + kHidden + 12;
 // environment count and env e of member p is global column p * n_envs + e of every [N] and [T, N] array
 // (row_stride = N).  The CTA stages member p's parameters and otherwise runs the single-policy code unchanged, so
 // member p's rows are those of k_policy_rollout_warp<false> on that member alone with env_offset = 0.
-template <bool POP>
+// FINAL: final-observation slots (final_slots_begin above), written by lane 0.
+template <bool POP, bool FINAL = false>
 __global__ void __launch_bounds__(128)
 k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, const ppo::Params W, int n_envs, int n_steps,
                       int env_offset, unsigned long long seed, unsigned long long step0, double2 *__restrict__ pos,
@@ -613,7 +706,7 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
                       float *__restrict__ val_buf, float *__restrict__ term_buf, float *__restrict__ trunc_buf,
                       float *__restrict__ logp_buf, float *__restrict__ last_val, float *__restrict__ u_dbg,
                       unsigned long long *stats, int table_bytes, int obs_mode, const unsigned long long *__restrict__ seeds,
-                      int row_stride) {
+                      int row_stride, float *__restrict__ final_obs, int *__restrict__ final_row, int n_slots) {
     extern __shared__ __align__(16) unsigned char smem[];
     ppo::Params Wm = W;
     int stride = n_envs;
@@ -622,8 +715,8 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
         Wm = member_params(W, p);
         seed = seeds[p];
         stride = row_stride;
-        pop_shift_columns(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
-                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg);
+        pop_shift_columns<FINAL>(p * n_envs, pos, vel, ints, cur_obs, cur_term, cur_trunc, last_val, obs_buf, act_buf, rew_buf,
+                          val_buf, term_buf, trunc_buf, logp_buf, u_dbg, final_obs, final_row);
     }
     float *sw1 = reinterpret_cast<float *>(smem + table_bytes);   // [512][20]: rows 0..255 actor, 256..511 critic
     float *sw2 = sw1 + 2 * kHidden * kWpRow;                      // [256][12]
@@ -665,6 +758,8 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
     float tc_ = cur_term[e], uc = cur_trunc[e];
     const uint32_t gid = (uint32_t)(env_offset + e);
     unsigned long long *my_stats = lane == 0 ? stats : nullptr;
+    FinalSlots fs{};
+    if constexpr (FINAL) fs = final_slots_begin(lane == 0, final_obs, final_row, n_slots, e);
 
     // pre-activation of one hidden unit (row of sw1) for the observation in `obs`
     auto unit = [&](const float *row) {
@@ -734,7 +829,12 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
             if (u_dbg) u_dbg[idx] = u;
         }
         StepResult o;
-        env_step<kWarpPerEnv>(s, a, reward_scale, P, T, o, my_stats, &ws);
+        if constexpr (FINAL) {
+            env_step<kWarpPerEnv>(s, a, reward_scale, P, T, o, my_stats, &ws, nullptr, nullptr, fs.obs);
+            final_slots_step(fs, o.truncated, t, n_slots, stride);
+        } else {
+            env_step<kWarpPerEnv>(s, a, reward_scale, P, T, o, my_stats, &ws);
+        }
         if (lane == 0) rew_buf[idx] = o.reward;
 #pragma unroll
         for (int i = 0; i < kObsDim; ++i) obs[i] = o.obs[i];
@@ -753,4 +853,5 @@ k_policy_rollout_warp(const __grid_constant__ TrackParams P, const Tables G, con
         cur_trunc[e] = uc;
         if (last_val) last_val[e] = po.value;
     }
+    if constexpr (FINAL) final_slots_end(fs, n_slots, stride);
 }

@@ -416,13 +416,14 @@ static int rollout_pop_args_ok(Handle *h, int n_members, int n_envs, int n_steps
     return 0;
 }
 
-int carenv_policy_rollout_warp_pop(void *handle, int n_members, const float *w1a, const float *b1a, const float *w2a,
-                                   const float *b2a, const float *w1c, const float *b1c, const float *w2c,
-                                   const float *b2c, int n_envs, int n_steps, const unsigned long long *seeds,
-                                   unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
-                                   float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
-                                   float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
-                                   float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+static int policy_rollout_warp_pop_impl(void *handle, int n_members, const float *w1a, const float *b1a,
+                                        const float *w2a, const float *b2a, const float *w1c, const float *b1c,
+                                        const float *w2c, const float *b2c, int n_envs, int n_steps,
+                                        const unsigned long long *seeds, unsigned long long step0, double *pos,
+                                        double *vel, int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc,
+                                        double reward_scale, float *obs_buf, float *act_buf, float *rew_buf,
+                                        float *val_buf, float *term_buf, float *trunc_buf, float *logp_buf,
+                                        float *last_val, float *u_dbg, void *stream, const SlotArgs &fs) {
     Handle *h = static_cast<Handle *>(handle);
     const void *ptrs[] = {w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, pos, vel, ints, cur_obs, cur_term, cur_trunc,
                           obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf};
@@ -431,14 +432,46 @@ int carenv_policy_rollout_warp_pop(void *handle, int n_members, const float *w1a
     return policy_rollout_warp_launch(h, ppo::Params{w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c}, n_members, n_envs,
                                       n_steps, 0, 0, seeds, step0, pos, vel, ints, cur_obs, cur_term, cur_trunc,
                                       reward_scale, obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf,
-                                      last_val, u_dbg, stream);
+                                      last_val, u_dbg, stream, fs);
 }
 
-int carenv_policy_rollout_tc_pop(void *handle, int n_members, const float *packed_weights, int n_envs, int n_steps,
-                                 const unsigned long long *seeds, unsigned long long step0, double *pos, double *vel,
-                                 int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
-                                 float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
-                                 float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+int carenv_policy_rollout_warp_pop(void *handle, int n_members, const float *w1a, const float *b1a, const float *w2a,
+                                   const float *b2a, const float *w1c, const float *b1c, const float *w2c,
+                                   const float *b2c, int n_envs, int n_steps, const unsigned long long *seeds,
+                                   unsigned long long step0, double *pos, double *vel, int32_t *ints, float *cur_obs,
+                                   float *cur_term, float *cur_trunc, double reward_scale, float *obs_buf,
+                                   float *act_buf, float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                   float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    return policy_rollout_warp_pop_impl(handle, n_members, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, n_envs, n_steps,
+                                        seeds, step0, pos, vel, ints, cur_obs, cur_term, cur_trunc, reward_scale,
+                                        obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val,
+                                        u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_warp_pop_final(void *handle, int n_members, const float *w1a, const float *b1a,
+                                         const float *w2a, const float *b2a, const float *w1c, const float *b1c,
+                                         const float *w2c, const float *b2c, int n_envs, int n_steps,
+                                         const unsigned long long *seeds, unsigned long long step0, double *pos,
+                                         double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                         float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                         float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                         float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                         float *final_obs, int32_t *final_row, int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_warp_pop_impl(handle, n_members, w1a, b1a, w2a, b2a, w1c, b1c, w2c, b2c, n_envs, n_steps,
+                                        seeds, step0, pos, vel, ints, cur_obs, cur_term, cur_trunc, reward_scale,
+                                        obs_buf, act_buf, rew_buf, val_buf, term_buf, trunc_buf, logp_buf, last_val,
+                                        u_dbg, stream, fs);
+}
+
+static int policy_rollout_tc_pop_impl(void *handle, int n_members, const float *packed_weights, int n_envs,
+                                      int n_steps, const unsigned long long *seeds, unsigned long long step0,
+                                      double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                      float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                      float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                      float *logp_buf, float *last_val, float *u_dbg, void *stream,
+                                      const SlotArgs &fs) {
     Handle *h = static_cast<Handle *>(handle);
     const void *ptrs[] = {packed_weights, pos, vel, ints, cur_obs, cur_term, cur_trunc, obs_buf, act_buf, rew_buf,
                           val_buf, term_buf, trunc_buf, logp_buf};
@@ -446,7 +479,31 @@ int carenv_policy_rollout_tc_pop(void *handle, int n_members, const float *packe
         return rc;
     return policy_rollout_tc_launch(h, packed_weights, n_members, n_envs, n_steps, 0, 0, seeds, step0, pos, vel, ints,
                                     cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
-                                    term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream);
+                                    term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
+}
+
+int carenv_policy_rollout_tc_pop(void *handle, int n_members, const float *packed_weights, int n_envs, int n_steps,
+                                 const unsigned long long *seeds, unsigned long long step0, double *pos, double *vel,
+                                 int32_t *ints, float *cur_obs, float *cur_term, float *cur_trunc, double reward_scale,
+                                 float *obs_buf, float *act_buf, float *rew_buf, float *val_buf, float *term_buf,
+                                 float *trunc_buf, float *logp_buf, float *last_val, float *u_dbg, void *stream) {
+    return policy_rollout_tc_pop_impl(handle, n_members, packed_weights, n_envs, n_steps, seeds, step0, pos, vel, ints,
+                                      cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
+                                      term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, SlotArgs{});
+}
+
+int carenv_policy_rollout_tc_pop_final(void *handle, int n_members, const float *packed_weights, int n_envs,
+                                       int n_steps, const unsigned long long *seeds, unsigned long long step0,
+                                       double *pos, double *vel, int32_t *ints, float *cur_obs, float *cur_term,
+                                       float *cur_trunc, double reward_scale, float *obs_buf, float *act_buf,
+                                       float *rew_buf, float *val_buf, float *term_buf, float *trunc_buf,
+                                       float *logp_buf, float *last_val, float *u_dbg, void *stream, float *final_obs,
+                                       int32_t *final_row, int n_slots) {
+    const SlotArgs fs{final_obs, final_row, n_slots};
+    if (const int rc = slot_args_ok(fs, n_steps)) return rc;
+    return policy_rollout_tc_pop_impl(handle, n_members, packed_weights, n_envs, n_steps, seeds, step0, pos, vel, ints,
+                                      cur_obs, cur_term, cur_trunc, reward_scale, obs_buf, act_buf, rew_buf, val_buf,
+                                      term_buf, trunc_buf, logp_buf, last_val, u_dbg, stream, fs);
 }
 
 int carenv_ppo_epoch_pop_cluster_size(void) { return kPopCluster; }

@@ -112,6 +112,14 @@ def _p(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def final_slot_args(buf) -> tuple:
+    """The trailing (final_obs, final_row, n_slots) arguments of the ``*_final`` entry points for a
+    ``Buffer(bootstrap_truncated=True)``, or () for a buffer without slots (the plain entry points)."""
+    if getattr(buf, "final_obs_buf", None) is None:
+        return ()
+    return _p(buf.final_obs_buf), _p(buf.final_row_buf), buf.final_row_buf.shape[0]
+
+
 def fused_rollout(env, packed: torch.Tensor, buf, cur_obs: torch.Tensor, cur_term: torch.Tensor,
                   cur_trunc: torch.Tensor, seed: int, step0: int, env_offset: int = 0,
                   last_val: torch.Tensor | None = None, u_dbg: torch.Tensor | None = None,
@@ -122,7 +130,10 @@ def fused_rollout(env, packed: torch.Tensor, buf, cur_obs: torch.Tensor, cur_ter
 
     ``env`` may be a :class:`MultiTrackVecEnv` (C ABI carenv_policy_rollout_tc_multi): every environment runs on its
     track (``env.track_ids``) and its rows are bit-identical to a single-track run on that track.  That needs the
-    tensor-core packing and full observation rows (no ``Buffer(compact_obs=True)``)."""
+    tensor-core packing and full observation rows (no ``Buffer(compact_obs=True)``).
+
+    A ``Buffer(bootstrap_truncated=True)`` runs the ``*_final`` twin, which also fills ``final_obs_buf`` /
+    ``final_row_buf``; every other output is the same bits."""
     from .vec_env import MultiTrackVecEnv
 
     multi = isinstance(env, MultiTrackVecEnv)
@@ -146,22 +157,28 @@ def fused_rollout(env, packed: torch.Tensor, buf, cur_obs: torch.Tensor, cur_ter
         if not tensor_cores:
             raise ValueError("several tracks run on the tensor-core kernel only: pack the weights with "
                              "pack_policy_weights_tc")
+        slots = final_slot_args(buf)
+        fn = L.carenv_policy_rollout_tc_multi_final if slots else L.carenv_policy_rollout_tc_multi
         with torch.cuda.device(env.device):
-            rc = L.carenv_policy_rollout_tc_multi(
-                env._multi, _p(env.track_ids), _p(packed), n, T, int(env_offset), int(seed) & (2 ** 64 - 1),
-                int(step0), _p(env.pos), _p(env.vel), _p(env.ints), _p(cur_obs), _p(cur_term), _p(cur_trunc),
-                float(env.reward_scaling), _p(rows), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf),
-                _p(buf.term_buf), _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream())
+            rc = fn(env._multi, _p(env.track_ids), _p(packed), n, T, int(env_offset), int(seed) & (2 ** 64 - 1),
+                    int(step0), _p(env.pos), _p(env.vel), _p(env.ints), _p(cur_obs), _p(cur_term), _p(cur_trunc),
+                    float(env.reward_scaling), _p(rows), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf),
+                    _p(buf.term_buf), _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream(),
+                    *slots)
         _lib.check(rc, "carenv_policy_rollout_tc_multi")
         buf.ptr = T
         return
     env.set_option("pose_rows", int(compact))               # obs_buf argument = 32-byte pose records
-    fn = L.carenv_policy_rollout_tc if tensor_cores else L.carenv_policy_rollout
+    slots = final_slot_args(buf)
+    if slots:
+        fn = L.carenv_policy_rollout_tc_final if tensor_cores else L.carenv_policy_rollout_final
+    else:
+        fn = L.carenv_policy_rollout_tc if tensor_cores else L.carenv_policy_rollout
     with torch.cuda.device(env.device):
         rc = fn(env._handle, _p(packed), n, T, int(env_offset), int(seed) & (2 ** 64 - 1), int(step0), _p(env.pos),
                 _p(env.vel), _p(env.ints), _p(cur_obs), _p(cur_term), _p(cur_trunc), float(env.reward_scaling),
                 _p(rows), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf), _p(buf.term_buf),
-                _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream())
+                _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream(), *slots)
     _lib.check(rc, "carenv_policy_rollout_tc" if tensor_cores else "carenv_policy_rollout")
     buf.ptr = T
 
@@ -193,11 +210,13 @@ def fused_rollout_warp(env, actor, critic, buf, cur_obs: torch.Tensor, cur_term:
         raise ValueError("buffer shape does not match the environment")
     env.set_option("pose_rows", int(compact))
     L = _lib.lib()
+    slots = final_slot_args(buf)
+    fn = L.carenv_policy_rollout_warp_final if slots else L.carenv_policy_rollout_warp
     with torch.cuda.device(env.device):
-        rc = L.carenv_policy_rollout_warp(env._handle, *[_p(p) for p in params], n, T, int(env_offset),
-                                          int(seed) & (2 ** 64 - 1), int(step0), _p(env.pos), _p(env.vel), _p(env.ints),
-                                          _p(cur_obs), _p(cur_term), _p(cur_trunc), float(env.reward_scaling), _p(rows),
-                                          _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf), _p(buf.term_buf),
-                                          _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream())
+        rc = fn(env._handle, *[_p(p) for p in params], n, T, int(env_offset), int(seed) & (2 ** 64 - 1), int(step0),
+                _p(env.pos), _p(env.vel), _p(env.ints), _p(cur_obs), _p(cur_term), _p(cur_trunc),
+                float(env.reward_scaling), _p(rows), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf),
+                _p(buf.term_buf), _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream(),
+                *slots)
     _lib.check(rc, "carenv_policy_rollout_warp")
     buf.ptr = T

@@ -257,7 +257,9 @@ def population_rollout(env, pop: Population, buf, cur_obs: torch.Tensor, cur_ter
     """Fill every row of ``buf`` (``Buffer(.., T, P * n, ..)``) for all members with one launch.  Member p's columns
     are bit-identical to ``fused_rollout_warp`` / ``fused_rollout`` of member p alone with ``seed = seeds[p]``,
     ``env_offset = 0`` and n environments.  ``packed`` is an optional ``[P, floats]`` buffer the tensor-core path packs
-    into (allocated per call otherwise)."""
+    into (allocated per call otherwise).  A ``Buffer(bootstrap_truncated=True)`` runs the ``*_final`` twin, which also
+    fills its final-observation slots."""
+    from .policy import final_slot_args
     from .vec_env import MultiTrackVecEnv
 
     if isinstance(env, MultiTrackVecEnv):
@@ -279,16 +281,18 @@ def population_rollout(env, pop: Population, buf, cur_obs: torch.Tensor, cur_ter
               float(env.reward_scaling), _p(buf.obs_buf), _p(buf.act_buf), _p(buf.rew_buf), _p(buf.val_buf),
               _p(buf.term_buf), _p(buf.trunc_buf), _p(buf.logprob_buf), _p(last_val), _p(u_dbg), env._stream())
     L = pop.L
+    slots = final_slot_args(buf)
+    sfx = "_final" if slots else ""
     with torch.cuda.device(env.device):
         if use_warp_kernel(env, n):
-            rc = L.carenv_policy_rollout_warp_pop(env._handle, pop.P, *[_p(t) for t in pop.params], n, T,
-                                                  _p(pop.seeds_dev), int(step0), *common)
-            what = "carenv_policy_rollout_warp_pop"
+            what = "carenv_policy_rollout_warp_pop" + sfx
+            rc = getattr(L, what)(env._handle, pop.P, *[_p(t) for t in pop.params], n, T, _p(pop.seeds_dev),
+                                  int(step0), *common, *slots)
         else:
             packed = pop.pack(True, out=packed)
-            rc = L.carenv_policy_rollout_tc_pop(env._handle, pop.P, _p(packed), n, T, _p(pop.seeds_dev), int(step0),
-                                                *common)
-            what = "carenv_policy_rollout_tc_pop"
+            what = "carenv_policy_rollout_tc_pop" + sfx
+            rc = getattr(L, what)(env._handle, pop.P, _p(packed), n, T, _p(pop.seeds_dev), int(step0), *common,
+                                  *slots)
     _lib.check(rc, what)
     buf.ptr = T
 
@@ -508,7 +512,7 @@ def train_population(args) -> dict:
         pop = Population([s for s, _ in mine], n, [h for _, h in mine], dev)
         N = pop.num_envs
         env = VecCarEnv(N, track, device=dev, reward_scaling=args.reward_scaling, float_flags=True, with_info=False)
-        buf = Buffer((OBS,), T, N, dev, args.gamma, args.gae_lambda)
+        buf = Buffer((OBS,), T, N, dev, args.gamma, args.gae_lambda, bootstrap_truncated=args.bootstrap_truncated)
         upd = PopulationPPOUpdate(pop, args.batch_size)
         next_obs = env.reset()[0].clone()
         next_term, next_trunc = torch.zeros(N, device=dev), torch.zeros(N, device=dev)
@@ -542,6 +546,8 @@ def train_population(args) -> dict:
                 with torch.no_grad():
                     population_rollout(env, pop, buf, next_obs, next_term, next_trunc, step0=(epoch - 1) * T,
                                        last_val=last_val, packed=packed)
+                    if args.bootstrap_truncated:
+                        buf.final_values(pop)
                     adv, ret = buf.calculate_advantages(last_val.reshape(1, -1), next_term.reshape(1, -1),
                                                         next_trunc.reshape(1, -1))
                 # per member as train_ppo sums its own contiguous [T, n] block: the same reduction, the same bits

@@ -129,6 +129,11 @@ def parse_args(argv=None):
                         "explained_variance")
     p.add_argument("--kl-stats", action="store_true",
                    help="the epoch-record statistics of --target-kl without stopping (a target of +inf)")
+    p.add_argument("--bootstrap-truncated", action="store_true",
+                   help="time-limit bootstrapping: the last step of an episode cut by the 1000-step limit is "
+                        "bootstrapped from the critic's value of the observation the episode ended in instead of the "
+                        "next episode's reset observation (the reference's GAE).  Changes the targets only; the rollout "
+                        "rows are the same bits")
     return p.parse_args(argv)
 
 
@@ -178,7 +183,10 @@ def track_list(args) -> tuple[list[str], list[str]]:
                               ("--fused-cuda-cores", args.fused_cuda_cores,
                                "the multi-track fused rollout runs on the tensor cores"),
                               ("--cuda-graph", args.cuda_graph,
-                               "the eager rollout is not captured; --fused-rollout is one launch per epoch")):
+                               "the eager rollout is not captured; --fused-rollout is one launch per epoch"),
+                              ("--bootstrap-truncated without --fused-rollout",
+                               args.bootstrap_truncated and not args.fused_rollout,
+                               "the eager multi-track step has no final observation; use --fused-rollout")):
             if on:
                 raise SystemExit(f"{flag} does not work with several tracks: {why}")
         if args.n_envs < len(paths):
@@ -204,12 +212,14 @@ def train(args) -> list[dict]:
     n = hi - lo
     T = args.n_steps
 
+    boot_trunc = bool(args.bootstrap_truncated)
+    eager_boot = boot_trunc and not args.fused_rollout          # the eager loop stores critic(final observation)
     if multi:
         envs = MultiTrackVecEnv(track_paths=paths, track_ids=track_blocks(args.n_envs, len(paths), lo, hi), device=dev,
                                 reward_scaling=args.reward_scaling, float_flags=True)
     else:
         envs = VecCarEnv(n, paths[0], device=dev, reward_scaling=args.reward_scaling, float_flags=True,
-                         with_info=False)
+                         with_info=False, final_observation=eager_boot)
     obs_dim = envs.single_observation_space.shape
     agent = ActorCritic(obs_dim[0], envs.single_action_space.n).to(dev)
     graph_update = bool(args.graph_update)                 # with world > 1 the NCCL all-reduce is captured too
@@ -234,7 +244,8 @@ def train(args) -> list[dict]:
     params = [p for p in agent.parameters()]
     if args.compact_obs and not args.fused_rollout:
         raise SystemExit("--compact-obs needs --fused-rollout")
-    buf = Buffer(obs_dim, T, n, dev, args.gamma, args.gae_lambda, compact_obs=args.compact_obs)
+    buf = Buffer(obs_dim, T, n, dev, args.gamma, args.gae_lambda, compact_obs=args.compact_obs,
+                 bootstrap_truncated=boot_trunc)
     torch.manual_seed(args.seed * 1000 + rank + 1)     # different sampling noise per shard
 
     # the rollout state lives in three static tensors so that the loop below can be captured in a graph
@@ -260,8 +271,10 @@ def train(args) -> list[dict]:
         for _ in range(T):
             act, logp, _, val = agent.act(next_obs)
             buf.store(next_obs, act, 0.0, val.view(-1), next_term, next_trunc, logp)
-            o, rew, te, tr, _ = envs.step(act)
+            o, rew, te, tr, info = envs.step(act)
             buf.rew_buf[buf.ptr - 1].copy_(rew)
+            if eager_boot:                                  # read by the GAE only where the step truncated
+                buf.boot_buf[buf.ptr - 1].copy_(agent.value(info["final_observation"]).view(-1))
             next_obs.copy_(o)
             next_term.copy_(te)
             next_trunc.copy_(tr)
@@ -338,11 +351,15 @@ def train(args) -> list[dict]:
                 if warp_rollout:
                     fused_rollout_warp(envs, agent.actor, agent.critic, buf, next_obs, next_term, next_trunc,
                                        seed=args.seed, step0=(epoch - 1) * T, env_offset=lo, last_val=last_val)
+                    if boot_trunc:
+                        buf.final_values(agent.critic)
                     boot = last_val.reshape(1, -1)
                 elif packed is not None:
                     pack_policy(agent.actor, agent.critic, out=packed)
                     fused_rollout(envs, packed, buf, next_obs, next_term, next_trunc, seed=args.seed,
                                   step0=(epoch - 1) * T, env_offset=lo, last_val=last_val)
+                    if boot_trunc:
+                        buf.final_values(agent.critic)
                     boot = last_val.reshape(1, -1)
                 else:
                     if graph is not None:
